@@ -8,6 +8,7 @@ controls, full trajectory materialised as predictor.predict_core returns it.  On
 
   python bench.py --gpus N --steps K --warmup W            # ours (CUDA through the C ABI)
   python bench.py --impl reference --gpus N ...            # the reference algorithm's CPU port on the host cores
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed pass computed (DIR/*.npy)
 
 Prints ONE JSON line on rank 0.  Also measured inside the same run and attached to the line:
   e2e           same pass through cps_rollout_host with pinned HOST buffers (H2D of s0+Q, D2H of the trajectory)
@@ -99,6 +100,33 @@ def make_inputs(B, T, seed):
     return s0, Q
 
 
+DUMP_TRAJ_BYTES = 48 << 20   # --dump-outputs: trajectories of at most this many bytes (64 MB for everything written)
+
+
+def dump_index(B, T, seed=0):
+    """The cartpoles --dump-outputs writes: a fixed, seeded sample of n of the B (every one when their trajectories fit
+    in DUMP_TRAJ_BYTES), sorted."""
+    n = int(min(B, max(1, DUMP_TRAJ_BYTES // ((T + 1) * 6 * 4))))
+    return np.arange(B) if n == B else np.sort(np.random.default_rng(seed).choice(B, n, replace=False))
+
+
+def write_dump(out_dir, traj_sample, idx):
+    """trajectory.npy = the sampled cartpoles' trajectories ([T+1, 6, n] float32, time-major like the full result);
+    cartpole_index.npy = their indices in the batch (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "trajectory.npy"), np.ascontiguousarray(traj_sample, dtype=np.float32))
+    np.save(os.path.join(out_dir, "cartpole_index.npy"), idx.astype(np.float64))
+
+
+def dump_outputs(out_dir, traj):
+    """--dump-outputs: what the timed rollouts returned in their last pass (traj [T+1, 6, B] on the device), so that two
+    builds can be compared output for output."""
+    import torch
+    T1, _, B = traj.shape
+    idx = dump_index(B, T1 - 1)
+    write_dump(out_dir, traj.index_select(2, torch.from_numpy(idx).to(traj.device)).cpu().numpy(), idx)
+
+
 def cpu_port_rate(B_sample, T, threads=None, repeats=1, seed=0):
     """state-steps/s of the oracle port (cps_oracle_rollout_v0, OpenMP) on this host."""
     from oracle import oracle as O
@@ -137,6 +165,13 @@ def run_reference(args):
         t1 = time.perf_counter()
         O.rollout("ODE_v0", s0, Qr, n=N_SUB, dt=DT)
         times.append(time.perf_counter() - t1)
+    if args.dump_outputs:
+        # the timed sample's size depends on the host, so the port rolls out the cartpoles --impl ours dumps, from the
+        # inputs --impl ours uses (rank 0): the two arms can be compared output for output
+        s0_all, Q_all = make_inputs(args.batch, T, seed=1234)
+        idx = dump_index(args.batch, T)
+        traj = O.rollout("ODE_v0", s0_all[idx], np.ascontiguousarray(Q_all[:, idx].T), n=N_SUB, dt=DT)   # [n, T+1, 6]
+        write_dump(args.dump_outputs, traj.transpose(1, 2, 0), idx)
     total = float(np.sum(times))
     value = B_sample * T * N_SUB * args.steps / total
     sample = f"{B_sample} of {args.batch} cartpoles x {T * N_SUB} substeps per step"
@@ -735,6 +770,8 @@ def run_ours(args):
     launches = (args.steps if graph is not None else eng.launch_count() - launches0)
     kernel_label = eng.rollout_last_kernel() or "rollout_kernel"   # what the timed passes dispatched to
     total_ms = t_all0.elapsed_time(t_all1)
+    if args.dump_outputs and rank == 0:   # traj still holds the last timed pass
+        dump_outputs(args.dump_outputs, traj)
     per_rank = None
     if world > 1:
         # every rank's own device time and per-launch kernel time: with no communication in the timed region, the spread
@@ -897,7 +934,7 @@ def run_ours(args):
                        "timed_region": ("one CUDA graph replay of the %d passes" % args.steps) if graph is not None
                        else ("%d separate launches" % args.steps)},
             "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                    "ms_per_step": 1e3 * e2e_s / e2e_steps, "api": "cps_rollout_host (pinned host buffers), full trajectory returned",
+                    "steps": e2e_steps, "ms_per_step": 1e3 * e2e_s / e2e_steps, "api": "cps_rollout_host (pinned host buffers), full trajectory returned",
                     "numa_bound_cpus": len(numa_cpus) if numa_cpus else None, "pcie": e2e_bus,
                     "final_states_only": {"value": e2e_final_value, "unit": UNIT, "h2d_bytes_per_step": h2d,
                                           "d2h_bytes_per_step": int(final_pin.numel() * 4),
@@ -914,7 +951,8 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed passes of the headline figure (the e2e legs time max(2, min(steps, 5)), e2e.steps)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=B_DEFAULT, help="cartpoles per GPU")
@@ -924,7 +962,12 @@ def main():
     ap.add_argument("--no-mppi", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="time K separate launches instead of one CUDA graph of K passes")
     ap.add_argument("--mppi-calls", type=int, default=1000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's batch) as DIR/<name>.npy; "
+                         "--impl reference: the CPU port's rollouts of the same sampled cartpoles")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,4 +1,4 @@
-"""Runs in a subprocess of tests/test_reference_dropin.py (build container only: needs /root/reference).
+"""Runs in a subprocess of tests/test_reference_dropin.py (needs the reference checkout at CPS_REFERENCE_ROOT).
 
 Drives the UNMODIFIED reference controller_mpc in a scratch workspace (SURVEY Appendix B.10) whose
 config selects `optimizer: mppi-b200`; the plugin stub is found by the reference's own glob.  There is no GPU
@@ -17,6 +17,7 @@ import numpy as np  # noqa: E402
 import yaml  # noqa: E402
 
 from oracle import ref_loader as R  # noqa: E402
+from tests.dropin_recorder import recording_engine  # noqa: E402
 
 
 def main():
@@ -54,38 +55,8 @@ def main():
         pode.predictor_ODE.__init__ = lambda self, *a, **k: _init(self, *a, **dict(k, computation_library=PyTorchLibrary()))
 
         calls = []
-
-        class FakeEngine:
-            def __init__(self, **kw):
-                import torch
-                calls.append(("create", {k: v for k, v in kw.items()}))
-                self.device = torch.device("cpu")
-                self.K, self.T, self.p = kw["num_rollouts"], kw["horizon"], kw["interp_period"]
-                self.n_ind = int(np.ceil((self.T - 1) / self.p)) + 1
-                self.u_nom = np.zeros(self.T, np.float32)
-
-            def set_cost_params(self, v):
-                calls.append(("cost_params", [float(x) for x in v]))
-
-            def set_mppi_params(self, *a):
-                calls.append(("mppi_params", [float(x) for x in a]))
-
-            def set_variable_parameters(self, *a):
-                calls.append(("variable", [float(x) for x in a]))
-
-            def mppi_reset(self, v):
-                calls.append(("reset", float(v)))
-
-            def mppi_step_host(self, s, noise, layout, u_prev):
-                calls.append(("step", dict(s=[float(x) for x in s], noise_shape=list(noise.shape), layout=int(layout),
-                                           u_prev=float(u_prev))))
-                return 0.25
-
-            def get_u_nom(self):
-                return self.u_nom
-
         import cartpolesimulation_b200.optimizer_mppi_b200 as mod
-        mod.Engine = FakeEngine
+        mod.Engine = recording_engine(calls)
 
         from Control_Toolkit.Controllers.controller_mpc import controller_mpc
         ctrl = controller_mpc(environment_name="CartPole",
