@@ -20,13 +20,15 @@
 // rpgd_update_kernel is the rest of grad_step (:176-180): tf.clip_by_norm per plan, the Adam step (Keras legacy Adam =
 // ResourceApplyAdam) and the clip to the control limits.
 // Cost plugins: quadratic_boundary_grad_minimal (the plugin the shipped RPGD configuration uses) and quadratic_boundary_grad;
-// predictor "ODE".
+// predictor "ODE" here, the neural predictor in cps_net_grad.cu (cps_plan_cost_grad hands it over; the RPGD update and
+// bookkeeping below serve both).
 #include <cuda_runtime.h>
 
 #include <cmath>
 #include <cstring>
 #include <new>
 
+#include "cps_grad_partials.cuh"
 #include "cps_internal.cuh"
 
 #define CPS_GRAD_MAX_SUBSTEPS 32
@@ -63,15 +65,6 @@ struct GradArgs {
 
 namespace {
 
-// sincosf / cosf for the angles a rollout produces: fold_angle leaves every angle after the first substep in [-pi, pi], where
-// sincos_folded is bit-identical to the math library (cps_selftest_sincos); anything else (a caller-supplied unwrapped
-// initial angle) takes the library call, out of line.
-static __device__ __noinline__ void sincos_library(float a, float *s, float *c) { sincosf(a, s, c); }
-__device__ __forceinline__ void sincos_th(float th, float &s, float &c) {
-    if (__builtin_expect(fabsf(th) <= CPS_PI_F, 1)) sincos_folded(th, s, c);
-    else sincos_library(th, &s, &c);
-}
-
 struct Sub { float th, w, v, sn, c; };
 
 // One Euler-Cromer substep of predictor_ODE with cos / sin taken from the angle (cartpole_equations.py:71-99, 245-262).
@@ -91,38 +84,6 @@ __device__ __forceinline__ Sub grad_substep(const OdeParams &P, float &th, float
     th = fold_angle(fmaf(w, P.h, th));
     x = fmaf(v, P.h, x);
     return in;
-}
-
-// Partial derivatives of the stage cost with respect to (angle, angleD, position).
-// quadratic_boundary_grad_minimal (Control_Toolkit_ASF/Cost_Functions/CartPole/quadratic_boundary_grad_minimal.py:62-130);
-// w: [dd_q, db, ep, ekp, cc*R, bf = f thl, 1/((1-f) thl)] as in stage_cost<COST_GRADMIN>.
-__device__ __forceinline__ void gradmin_partials(const CostParams &C, float th, float w, float x, float &d_th, float &d_w,
-                                                 float &d_x) {
-    float sn, c;
-    sincos_th(th, sn, c);
-    const float dist = (x - C.target_position) * C.inv_2thl;
-    const float apos = fabsf(x);
-    const float over = (apos > C.w[5]) ? (apos - C.w[5]) * C.w[6] : 0.0f;
-    d_x = fmaf(C.w[0] * 2.0f * dist, C.inv_2thl, C.w[1] * 2.0f * over * C.w[6] * copysignf(1.0f, x));
-    d_th = C.w[2] * 2.0f * (1.0f - C.target_equilibrium * c) * (C.target_equilibrium * sn);
-    d_w = 2.0f * C.w[3] * w;
-}
-// quadratic_boundary_grad (quadratic_boundary_grad.py:62-142, 202-240); w as in stage_cost<COST_GRAD>:
-// [dd_q, dd_lin, db, ep, ekp, cc*R, ccrc, bf, 1/((1-f) thl), tmax, cos(admissible angle)].  The kinetic term is
-// |angleD^2 - tmax scaling(angle)| with the target under stop_gradient (:133-139): no derivative with respect to the angle.
-__device__ __forceinline__ float sgnf(float x) { return (float)(x > 0.0f) - (float)(x < 0.0f); }   // d|x|/dx with 0 at 0, as autograd
-__device__ __forceinline__ void grad_partials(const CostParams &C, float th, float w, float x, float &d_th, float &d_w,
-                                              float &d_x) {
-    float sn, c;
-    sincos_th(th, sn, c);
-    const float e = C.target_equilibrium;
-    const float dist = (x - C.target_position) * C.inv_2thl;
-    const float apos = fabsf(x);
-    const float over = (apos > C.w[7]) ? (apos - C.w[7]) * C.w[8] : 0.0f;
-    d_x = fmaf(C.w[0] * 2.0f * dist, C.inv_2thl, C.w[2] * 2.0f * over * C.w[8] * copysignf(1.0f, x)) + C.w[1] * sgnf(dist) * C.inv_2thl;
-    d_th = C.w[3] * 2.0f * (2.0f - e * c) * (e * sn);
-    const float scaling = (e * (c - C.w[10]) > 0.0f) ? 0.0f : 0.5f * (1.0f - e * c);
-    d_w = C.w[4] * sgnf(fmaf(w, w, -C.w[9] * scaling)) * 2.0f * w;
 }
 
 // ---- forward: one thread per plan; cost and a checkpoint per control step ---------------------------------------------------
@@ -416,18 +377,23 @@ void cps_grad_free(cps_handle *h) {
 
 static int grad_state(cps_handle *h, GradState **out) {
     if (h->grad) { *out = h->grad; return CPS_OK; }
-    if (h->cfg.integrator != CPS_EULER_CROMER)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_plan_cost_grad: the adjoint is built for predictor \"ODE\" (Euler-Cromer)");
+    const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
+    if (h->cfg.integrator != CPS_EULER_CROMER && !neural)
+        return fail(h, CPS_ERR_UNSUPPORTED, "cps_plan_cost_grad: the adjoint is built for predictor \"ODE\" (Euler-Cromer) and the "
+                    "neural predictor");
     if (h->cfg.cost_id != CPS_COST_QB_GRAD_MINIMAL && h->cfg.cost_id != CPS_COST_QB_GRAD)
         return fail(h, CPS_ERR_UNSUPPORTED, "cps_plan_cost_grad: the adjoint is built for the quadratic_boundary_grad_minimal and quadratic_boundary_grad plugins");
-    if (h->cfg.substeps > CPS_GRAD_MAX_SUBSTEPS)
+    if (!neural && h->cfg.substeps > CPS_GRAD_MAX_SUBSTEPS)
         return fail(h, CPS_ERR_UNSUPPORTED, "cps_plan_cost_grad: at most 32 substeps per control step");
     GradState *G = new (std::nothrow) GradState();
     if (!G) return fail(h, CPS_ERR_INVALID, "cps_plan_cost_grad: out of host memory");
     memset(G, 0, sizeof(*G));
     const size_t K = h->cfg.num_rollouts, T = h->cfg.horizon;
-    cudaError_t e = cudaMalloc(&G->d_ck, sizeof(float) * 4 * K * T);
-    if (e == cudaSuccess) e = cudaMalloc(&G->d_jac, sizeof(float) * CPS_GRAD_REC * K * T);
+    cudaError_t e = cudaSuccess;
+    if (!neural) {   // the neural adjoint keeps its records in the network's workspace (cps_net_grad.cu)
+        e = cudaMalloc(&G->d_ck, sizeof(float) * 4 * K * T);
+        if (e == cudaSuccess) e = cudaMalloc(&G->d_jac, sizeof(float) * CPS_GRAD_REC * K * T);
+    }
     if (e == cudaSuccess) e = cudaMalloc(&G->d_J, sizeof(float) * K);
     if (e == cudaSuccess) e = cudaMalloc(&G->d_G, sizeof(float) * K * T);
     if (e == cudaSuccess) e = cudaMalloc(&G->d_m, sizeof(float) * K * T);
@@ -453,6 +419,8 @@ extern "C" int cps_plan_cost_grad(cps_handle *h, const float *s_dev, const float
     int rc = grad_state(h, &G);
     if (rc != CPS_OK) return rc;
     const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
+        return cps_net_plan_cost_grad(h, s_dev, Q_dev, q_layout, u_prev, J_out_dev ? J_out_dev : G->d_J, G_out_dev);
     GradArgs a;
     memset(&a, 0, sizeof(a));
     a.ode = h->ode; a.cost = h->cost;

@@ -144,6 +144,11 @@ void cps_grad_free(cps_handle *h);
 int cps_fold_cost_for(cps_handle *h, float target_equilibrium, CostParams *out);
 // cps_net.cu
 void cps_net_free(cps_handle *h);
+// cps_net_grad.cu: cps_plan_cost / cps_plan_cost_grad with CPS_PREDICTOR_NEURAL
+int cps_net_plan_cost(cps_handle *h, const float *s_dev, const float *Q_dev, int q_layout, int K, int T, float u_prev,
+                      float *J_out_dev, float *traj_out_dev, int traj_layout);
+int cps_net_plan_cost_grad(cps_handle *h, const float *s_dev, const float *Q_dev, int q_layout, float u_prev, float *J_out_dev,
+                           float *G_out_dev);
 int cps_net_mppi_step(cps_handle *h, const float *s_dev, const float *noise_dev, int noise_layout, float u_prev,
                       float *u_nom_dev, float *u_out_dev, float *J_out_dev, float *traj_out_dev, int traj_layout,
                       float *u_run_out_dev);

@@ -28,6 +28,8 @@ struct NetState {
     float *d_href;      // stored hidden state [htot] (memory_states_ref; rows are identical across the batch)
     int ht;             // common hidden size if the kernels have a specialisation for it (64, 32), else 0
     unsigned char *d_tc;  // tensor-core kernel image (fp16 hi/lo weights in UMMA core-matrix order + epilogue constants), or null
+    float *d_gws;         // net_grad_kernel's records of the forward pass (cps_net_grad.cu), grown on demand
+    size_t gws_bytes;
 };
 
 struct NetArgs {

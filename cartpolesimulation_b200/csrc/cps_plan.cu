@@ -759,7 +759,7 @@ static int plan_state(cps_handle *h, PlanState **out) {
 
 static int plan_check(cps_handle *h, const char *who) {
     if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
-        return fail(h, CPS_ERR_UNSUPPORTED, "%s: ODE predictors only (neural predictor: cps_net_rollout + cps_trajectory_cost)", who);
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: ODE predictors only (neural predictor: cps_plan_cost, or cps_net_rollout + cps_trajectory_cost)", who);
     if (h->cfg.cost_id == CPS_COST_NONE || h->cfg.cost_id == CPS_COST_LEGACY_MPPI)
         return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: the handle has no cost-function plugin", who);
     if (h->cfg.flags & (CPS_FLAG_SUBSTEP_SINCOS | CPS_FLAG_FAST_DIV))
@@ -794,6 +794,8 @@ extern "C" int cps_plan_cost(cps_handle *h, const float *s_dev, const float *Q_d
     if (!h) return CPS_ERR_INVALID;
     if (!s_dev || !Q_dev || !J_out_dev) return fail(h, CPS_ERR_INVALID, "cps_plan_cost: null pointer");
     if (K < 1 || T < 1) return fail(h, CPS_ERR_INVALID, "cps_plan_cost: K and T must be positive");
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
+        return cps_net_plan_cost(h, s_dev, Q_dev, q_layout, K, T, u_prev, J_out_dev, traj_out_dev, traj_layout);
     int rc = plan_check(h, "cps_plan_cost");
     if (rc != CPS_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));

@@ -7,8 +7,8 @@ reads (`u`, `logging_values`, `num_rollouts`, `mpc_horizon`, `optimizer_name`; C
 `predict_and_cost` (predictor.predict_core + cost_function.get_trajectory_cost) and the selection on the sorted costs
 run as one CUDA kernel launch per evaluation (cps_plan_random_action / cps_cem_step); a CEM solve is `cem_outer_it`
 launches with no host round trip in between.  The predictor and cost-function objects handed in are only inspected
-for their configuration, so this package's wrappers and the reference's own work alike.  ODE / ODE_v0 predictors;
-no CPU fallback.
+for their configuration, so this package's wrappers and the reference's own work alike.  ODE / ODE_v0 predictors (RPGD
+also the neural predictor); no CPU fallback.
 
 Semantics kept from the reference: `self.u` (the `u_prev` of the cost's control-change term) is the last RETURNED
 control, 0.0 initially (Optimizers/__init__.py:35); CEM samples Q = clip(mean + normal * stdev) (:66-68), takes the
@@ -24,7 +24,7 @@ import torch
 from . import _lib as L
 from . import config as cfgmod
 from .core import Engine
-from .optimizer_mppi_b200 import CudaNormalGenerator, _extract_cost, _extract_predictor
+from .optimizer_mppi_b200 import CudaNormalGenerator, _extract_cost, _extract_net_spec, _extract_predictor
 from .predictors import read_variable
 
 
@@ -38,6 +38,7 @@ class CudaGenerator(CudaNormalGenerator):
 
 class _forward_optimizer:
     supported_computation_libraries = ("Numpy", "TF", "Pytorch")
+    PREDICTORS = ("ODE", "ODE_v0")   # predictor types configure accepts
     NOISE_RING = 256   # solves per device RNG call when the optimizer draws its own numbers
 
     def _ring_draw(self, shape, draw):
@@ -81,9 +82,10 @@ class _forward_optimizer:
             raise ValueError(f"{type(self).__name__} implements the CartPole path: 6 states, 1 control input")
         self.num_states, self.num_control_inputs = int(num_states), int(num_control_inputs)
         ptype, n = _extract_predictor(self.predictor, predictor_specification)
-        if ptype not in ("ODE", "ODE_v0"):
-            raise NotImplementedError(f"{type(self).__name__} supports the ODE / ODE_v0 predictors, not {ptype!r} "
-                                      "(no CPU fallback)")
+        if ptype not in self.PREDICTORS:
+            raise NotImplementedError(f"{type(self).__name__} supports the {' / '.join(self.PREDICTORS)} predictors, not "
+                                      f"{ptype!r} (no CPU fallback)")
+        net_spec = _extract_net_spec(self.predictor) if ptype == "neural" else None
         if dt is None:
             dt = getattr(self.predictor, "dt", None) or 0.02
         cost_name, cost_cfg = _extract_cost(self.cost_function)
@@ -92,6 +94,8 @@ class _forward_optimizer:
                              integrator=ptype, cost=cost_name, device=self._device_arg)
         self.device = self.engine.device
         self.cost_name, self.predictor_type = cost_name, ptype
+        if net_spec is not None:
+            self.engine.net_load(net_spec)
         self.engine.set_cost_params(cfgmod.cost_vector(cost_name, cost_cfg))
         # only the control limits of this block are used by the planners
         self.engine.set_mppi_params(lo=float(self.action_low[0]), hi=float(self.action_high[0]))
@@ -334,8 +338,16 @@ class optimizer_rpgd_b200(_forward_optimizer):
     The gradient -- a GradientTape around predict_and_cost in the reference -- is one adjoint kernel launch
     (cps_rpgd_grad_step: gradient, clip_by_norm, Adam, clip to the limits); the plans and the Adam moments stay on the
     device, the per-solve bookkeeping of step() (:297-356: argsort of K costs, gather, shift) is a handful of torch index
-    operations on those device tensors.  Predictor "ODE"; cost quadratic_boundary_grad_minimal (the shipped configuration) or
-    quadratic_boundary_grad; no CPU fallback."""
+    operations on those device tensors.  Predictors "ODE" and "neural" (plain GRU / Dense networks; differential D_* networks
+    are not supported); cost quadratic_boundary_grad_minimal (the shipped configuration) or quadratic_boundary_grad; no CPU
+    fallback.
+
+    Hidden state of a recurrent network: step() does not advance it.  optimizer_rpgd_tf's predict_and_cost is
+    predict_core + get_trajectory_cost (:167-168), whereas optimizer_mppi advances the memory inside its _predict_and_cost
+    (optimizer_mppi.py:191); every rollout and gradient here starts from the stored hidden state of this optimizer's engine
+    and leaves it as it was.  A caller that wants the memory to follow the plant calls `engine.net_update(s, u)` after each step."""
+
+    PREDICTORS = ("ODE", "ODE_v0", "neural")
 
     def __init__(self, predictor, cost_function, control_limits, computation_library=None, seed=None,
                  mpc_horizon: int = 35, num_rollouts: int = 16, outer_its: int = 4, sample_stdev: float = 0.5,
@@ -446,7 +458,11 @@ class optimizer_rpgd_b200(_forward_optimizer):
             self.Q_tf.copy_(Qn)
         self.count += 1
         if self.calculate_optimal_trajectory:
-            traj, _ = self.engine.rollout(s_dev, self.u_nom.reshape(1, T).to(self.device))
+            u_nom = self.u_nom.reshape(1, T).to(self.device)
+            if self.predictor_type == "neural":
+                traj, _ = self.engine.net_rollout(s_dev, u_nom)
+            else:
+                traj, _ = self.engine.rollout(s_dev, u_nom)
             self.optimal_trajectory = traj.cpu().numpy()
         self.u = np.array(self.optimal_control_sequence[0, 0, 0], dtype=np.float32)   # already on the host: no second sync
         return self.u

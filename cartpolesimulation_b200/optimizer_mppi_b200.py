@@ -81,6 +81,20 @@ def _extract_predictor(predictor, predictor_specification):
     return ptype, n
 
 
+def _extract_net_spec(predictor):
+    """The network of a configured neural predictor: this package's predictor_autoregressive_neural (net_spec) or the
+    reference's own object (torch net + net_info + normalization_info)."""
+    from . import neural
+    inner = getattr(predictor, "predictor", predictor)
+    net_spec = getattr(inner, "net_spec", None)
+    if net_spec is None:
+        if not hasattr(inner, "net_info"):
+            raise ValueError("neural predictor: configure the PredictorWrapper before the optimizer "
+                             "(controller_mpc.py:69-76 does)")
+        net_spec = neural.spec_from_reference_predictor(inner)
+    return net_spec
+
+
 class optimizer_mppi_b200:
     supported_computation_libraries = ("Numpy", "TF", "Pytorch")
     NOISE_RING = 256   # solves per device RNG call when the optimizer draws its own noise
@@ -128,18 +142,7 @@ class optimizer_mppi_b200:
         ptype, n = _extract_predictor(self.predictor, predictor_specification)
         if ptype not in ("ODE", "ODE_v0", "neural"):
             raise ValueError(f"optimizer_mppi_b200 does not support predictor type {ptype!r} (no CPU fallback)")
-        net_spec = None
-        if ptype == "neural":
-            # the network comes from the configured predictor: this package's predictor_autoregressive_neural
-            # (net_spec) or the reference's own object (torch net + net_info + normalization_info)
-            from . import neural
-            inner = getattr(self.predictor, "predictor", self.predictor)
-            net_spec = getattr(inner, "net_spec", None)
-            if net_spec is None:
-                if not hasattr(inner, "net_info"):
-                    raise ValueError("neural predictor: configure the PredictorWrapper before the optimizer "
-                                     "(controller_mpc.py:69-76 does)")
-                net_spec = neural.spec_from_reference_predictor(inner)
+        net_spec = _extract_net_spec(self.predictor) if ptype == "neural" else None
         cost_name, cost_cfg = _extract_cost(self.cost_function)
         self.dt = float(dt)
         self.engine = Engine(num_rollouts=self.num_rollouts, horizon=self.mpc_horizon, dt=self.dt, substeps=n,

@@ -405,7 +405,13 @@ int cps_fleet_noise(cps_handle *h, long long period, float *out_dev);
  * the caller (random action) or in the kernel (CEM) to the control limits of cps_set_mppi_params (lo, hi).
  *
  * cps_plan_cost: J_out_dev[k] = get_trajectory_cost(predict_core(s, Q), Q, u_prev)[k] for K plans of length T
- * (any K, T; Q_dev [K][T] CPS_ROLLOUT_MAJOR or [T][K] CPS_TIME_MAJOR); traj_out_dev as in cps_mppi_step or NULL. */
+ * (any K, T; Q_dev [K][T] CPS_ROLLOUT_MAJOR or [T][K] CPS_TIME_MAJOR); traj_out_dev as in cps_mppi_step or NULL.
+ * cps_plan_cost also takes CPS_PREDICTOR_NEURAL: the plain (not D_*) network loaded with cps_net_load, started from the
+ * handle's stored hidden state (read, never written), with quadratic_boundary_grad_minimal or quadratic_boundary_grad, the
+ * forward pass of cps_plan_cost_grad (the same J bit for bit; trajectories those of cps_net_rollout on the FP32 kernel).
+ * No network loaded: CPS_ERR_NOT_CONFIGURED; differential networks, other cost plugins, CPS_FLAG_NET_TENSOR_CORES or a
+ * network whose shared-memory image exceeds 227 KB: CPS_ERR_UNSUPPORTED.  The fused planners below
+ * (cps_plan_random_action*, cps_cem_*, cps_cem_gmm_*) stay ODE-only. */
 int cps_plan_cost(cps_handle *h, const float *s_dev, const float *Q_dev, int q_layout, int K, int T, float u_prev,
                   float *J_out_dev, float *traj_out_dev, int traj_layout);
 /* optimizer_random_action_tf.step (:52-79) for the handle's (K, T): u_out_dev[0] = Q[argmin J, 0], ties to the lowest
@@ -477,7 +483,15 @@ int cps_selftest_sincos(cps_handle *h, long long *mismatches_out);
  * the reference differentiates), cost quadratic_boundary_grad_minimal (the shipped RPGD configuration) or
  * quadratic_boundary_grad (u_prev enters its control-change term; its kinetic term's target is under stop_gradient, as in
  * the plugin); anything else: CPS_ERR_UNSUPPORTED.
- * cps_rpgd_grad_step is grad_step (:166-180) on the device: the gradient, tf.clip_by_norm over each plan (gradmax_clip), one
+ * CPS_PREDICTOR_NEURAL (predictor_autoregressive_neural): one launch per gradient, a tile of 16 or 32 plans per CTA runs the
+ * FP32 network forward over the horizon and then the reverse sweep through the GRU / Dense layers, the normalised-output
+ * feedback, de-normalisation, angle augmentation and the cost plugin (records in a handle-owned workspace that grows on
+ * demand, (T+1) x Htot x K floats and a little more).  All plans start from the handle's stored hidden state, which the call
+ * reads and never writes (no gradient flows into it or into s); the same two cost plugins.  No network loaded:
+ * CPS_ERR_NOT_CONFIGURED; differential (D_*) networks, CPS_FLAG_NET_TENSOR_CORES (that flag forces a kernel without a
+ * gradient) or a network whose shared-memory image with the adjoint's buffers exceeds 227 KB: CPS_ERR_UNSUPPORTED.
+ * cps_rpgd_grad_step is grad_step (:166-180) on the device (either predictor, as cps_plan_cost_grad; with the neural one the
+ * stored hidden state is left as it is): the gradient, tf.clip_by_norm over each plan (gradmax_clip), one
  * Adam step (Keras legacy Adam: lr_t = lr sqrt(1 - b2^t) / (1 - b1^t), m, v per element, handle-owned, t = iterations since
  * cps_rpgd_reset) and the clip to the control limits, in place on Q_dev [K][T].  cps_rpgd_adam_state exposes the device
  * buffers of m and v ([K][T]) and the iteration count for the warm-start bookkeeping of step() (:297-356). */
