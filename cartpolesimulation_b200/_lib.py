@@ -61,6 +61,16 @@ class cps_fleet_plant_models(C.Structure):
                 ("latency", C.c_double)]
 
 
+class cps_rpgd_fleet_config(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("n_experiments", C.c_int), ("sim_substeps", C.c_int),
+                ("draw_source", C.c_int), ("dt_simulation", C.c_double), ("seed", C.c_ulonglong),
+                ("experiment_offset", C.c_longlong), ("outer_its", C.c_int), ("first_iter_count", C.c_int),
+                ("resamp_per", C.c_int), ("opt_keep_k", C.c_int), ("shift_previous", C.c_int),
+                ("learning_rate", C.c_float), ("adam_beta_1", C.c_float), ("adam_beta_2", C.c_float),
+                ("adam_epsilon", C.c_float), ("gradmax_clip", C.c_float), ("sample_stdev", C.c_float),
+                ("sample_mean", C.c_float)]
+
+
 # name -> (restype, argtypes); every symbol include/cps.h declares
 _FP = C.POINTER(C.c_float)
 _VP = C.c_void_p
@@ -119,6 +129,14 @@ SYMBOLS = {
     "cps_fleet_relabel_masked": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "cps_fleet_reset": (C.c_int, [_VP, C.c_longlong]),
     "cps_fleet_noise": (C.c_int, [_VP, C.c_longlong, _VP]),
+    "cps_rpgd_fleet_create": (C.c_int, [_VP, C.POINTER(cps_rpgd_fleet_config)]),
+    "cps_rpgd_fleet_set_states": (C.c_int, [_VP, _FP, _VP, C.c_longlong]),
+    "cps_rpgd_fleet_step": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "cps_rpgd_fleet_get_states": (C.c_int, [_VP, _FP, _FP]),
+    "cps_rpgd_fleet_get_plans": (C.c_int, [_VP, _FP, _FP, _FP, C.POINTER(C.c_int), C.POINTER(C.c_longlong),
+                                           C.POINTER(C.c_longlong)]),
+    "cps_rpgd_fleet_period": (C.c_longlong, [_VP]),
+    "cps_rpgd_fleet_draws": (C.c_int, [_VP, C.c_longlong, _VP]),
     "cps_plan_cost": (C.c_int, [_VP, _VP, _VP, C.c_int, C.c_int, C.c_int, C.c_float, _VP, _VP, C.c_int]),
     "cps_plan_random_action": (C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, _VP, _VP, _VP]),
     "cps_plan_random_action_host": (C.c_int, [_VP, _FP, _VP, C.c_int, C.c_float, _FP]),

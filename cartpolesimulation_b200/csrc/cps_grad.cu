@@ -32,7 +32,6 @@
 #include "cps_internal.cuh"
 
 #define CPS_GRAD_MAX_SUBSTEPS 32
-#define CPS_GRAD_REC 20   /* floats per (control step, plan) record: M[3][4], r[4], cost partials (3), control term */
 
 struct GradState {
     float *d_ck;        // [T][4][K] checkpoints
@@ -63,6 +62,17 @@ struct GradArgs {
     int *nonfinite;
 };
 
+// The fleet variants' per-experiment inputs (cps_rpgd_fleet.cu): plan k belongs to experiment k / kpe.
+struct FleetGradExt {
+    const CostParams *costs;   // [E] folded for each experiment's targets of the period
+    const float *u_prev;       // [E]
+    int kpe;                   // plans per experiment
+};
+struct FleetGradArgs {
+    GradArgs g;                // K = E * kpe plans [E * kpe][T]; s = the fleet's states [E][8]
+    FleetGradExt x;
+};
+
 namespace {
 
 struct Sub { float th, w, v, sn, c; };
@@ -89,25 +99,31 @@ __device__ __forceinline__ Sub grad_substep(const OdeParams &P, float &th, float
 // ---- forward: one thread per plan; cost and a checkpoint per control step ---------------------------------------------------
 // The integration and the cost are plan_kernel's (control_step with the rotation substeps, stage_cost): J is bit-identical
 // to cps_plan_cost's, and the sequential part of the gradient runs at the solve kernels' speed.
-template <int NSUB>
-__global__ void __launch_bounds__(128) plan_grad_fwd_kernel(const __grid_constant__ GradArgs a) {
+// FLEET (cps_rpgd_fleet.cu): the plans of E experiments in one launch, plan k of experiment k / fx.kpe with that experiment's
+// state, u_prev and cost parameters (fx); a null a.ck skips the checkpoints (costs only).  Per plan the arithmetic is the same.
+template <int NSUB, bool FLEET>
+__device__ __forceinline__ void grad_fwd(const GradArgs &a, const FleetGradExt &fx) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= a.K) return;
-    const CostParams &C = a.cost;
+    const int e = FLEET ? k / fx.kpe : 0;
+    const CostParams &C = FLEET ? fx.costs[e] : a.cost;
     const int T = a.T, K = a.K;
-    State z = load_state(a.use_inline ? a.s_inline : a.s);
+    const bool want_ck = !FLEET || a.ck != nullptr;
+    State z = load_state(FLEET ? a.s + (long long)e * 8 : (a.use_inline ? a.s_inline : a.s));
     const OdeParams ode = pin_params(a.ode, z.th);
     float c_cost = cosf(z.th);
     const float *q = a.Q + (long long)k * a.qs_k;
-    float *ck = a.ck + k;
-    float Jacc = 0.0f, up = a.u_prev;
+    float *ck = want_ck ? a.ck + k : nullptr;   // costs only (fleet): no checkpoint buffer
+    float Jacc = 0.0f, up = FLEET ? fx.u_prev[e] : a.u_prev;
     float qn = q[0];
 #pragma unroll 1
     for (int t = 0; t < T; ++t) {
         const float u = qn;
         if (t + 1 < T) qn = q[(long long)(t + 1) * a.qs_t];   // prefetch under the integration
-        ck[((long long)t * 4 + 0) * K] = z.th; ck[((long long)t * 4 + 1) * K] = z.w;
-        ck[((long long)t * 4 + 2) * K] = z.x;  ck[((long long)t * 4 + 3) * K] = z.v;
+        if (want_ck) {
+            ck[((long long)t * 4 + 0) * K] = z.th; ck[((long long)t * 4 + 1) * K] = z.w;
+            ck[((long long)t * 4 + 2) * K] = z.x;  ck[((long long)t * 4 + 3) * K] = z.v;
+        }
         Jacc += a.full ? stage_cost<COST_GRAD>(C, c_cost, z.w, z.x, u, up) : stage_cost<COST_GRADMIN>(C, c_cost, z.w, z.x, u, 0.0f);
         control_step<1, SC_ROTATE, false, false, false, NSUB>(ode, z, u);
         c_cost = z.c;
@@ -116,6 +132,14 @@ __global__ void __launch_bounds__(128) plan_grad_fwd_kernel(const __grid_constan
     const float J = __fdiv_rn(Jacc, (float)(T + 1));   // the plugin's terminal cost is zero
     if (a.J) a.J[k] = J;
     if (!isfinite(J)) atomicAdd(a.nonfinite, 1);
+}
+template <int NSUB>
+__global__ void __launch_bounds__(128) plan_grad_fwd_kernel(const __grid_constant__ GradArgs a) {
+    grad_fwd<NSUB, false>(a, FleetGradExt());
+}
+template <int NSUB>
+__global__ void __launch_bounds__(128) fleet_grad_fwd_kernel(const __grid_constant__ FleetGradArgs f) {
+    grad_fwd<NSUB, true>(f.g, f.x);
 }
 
 // ---- transposed Jacobian of every control step, in parallel over (control step, plan) ------------------------------------
@@ -126,9 +150,12 @@ __global__ void __launch_bounds__(128) plan_grad_fwd_kernel(const __grid_constan
 // (a_x passes through unchanged: the position enters no right-hand side) --, r[4], the row that gives d/d(uk), and the
 // terms the cost adds at the step's boundary.
 // Sequential work per plan shrinks from T x n reverse substeps to T small matrix-vector products (plan_grad_rev_kernel).
-template <int NSUB>
-__device__ __forceinline__ void step_record(const GradArgs &a, int t, int k, float *o, long long stride) {
+template <int NSUB, bool FLEET = false>
+__device__ __forceinline__ void step_record(const GradArgs &a, int t, int k, float *o, long long stride,
+                                            const FleetGradExt &fx = FleetGradExt()) {
     const int K = a.K;
+    const int e = FLEET ? k / fx.kpe : 0;
+    const CostParams &C = FLEET ? fx.costs[e] : a.cost;
     const OdeParams &P = a.ode;
     const int n = NSUB ? NSUB : P.n;
     const float *ck = a.ck + k;
@@ -188,15 +215,15 @@ __device__ __forceinline__ void step_record(const GradArgs &a, int t, int k, flo
     // state and its control term, with the 1 / (T + 1) of the mean
     float d_th, d_w, d_x, d_u;
     if (a.full) {
-        grad_partials(a.cost, th0, w0, x0, d_th, d_w, d_x);
+        grad_partials(C, th0, w0, x0, d_th, d_w, d_x);
         // cc u_t^2 + ccrc (u_t - u_{t-1})^2 of this stage and ccrc (u_{t+1} - u_t)^2 of the next (_control_change_rate_cost, :174-180)
         const float *q = a.Q + (long long)k * a.qs_k;
-        const float up = (t > 0) ? q[(long long)(t - 1) * a.qs_t] : a.u_prev;
-        d_u = 2.0f * a.cost.w[5] * u + 2.0f * a.cost.w[6] * (u - up);
-        if (t + 1 < a.T) d_u -= 2.0f * a.cost.w[6] * (q[(long long)(t + 1) * a.qs_t] - u);
+        const float up = (t > 0) ? q[(long long)(t - 1) * a.qs_t] : (FLEET ? fx.u_prev[e] : a.u_prev);
+        d_u = 2.0f * C.w[5] * u + 2.0f * C.w[6] * (u - up);
+        if (t + 1 < a.T) d_u -= 2.0f * C.w[6] * (q[(long long)(t + 1) * a.qs_t] - u);
     } else {
-        gradmin_partials(a.cost, th0, w0, x0, d_th, d_w, d_x);
-        d_u = 2.0f * a.cost.w[4] * u;
+        gradmin_partials(C, th0, w0, x0, d_th, d_w, d_x);
+        d_u = 2.0f * C.w[4] * u;
     }
     o[16 * stride] = a.inv_T1 * d_th;
     o[17 * stride] = a.inv_T1 * d_w;
@@ -212,6 +239,16 @@ __global__ void __launch_bounds__(128) plan_grad_jac_kernel(const __grid_constan
     if (gid >= (long long)K * a.T) return;
     const int k = (int)(gid % K), t = (int)(gid / K);
     step_record<NSUB>(a, t, k, a.jac + (long long)t * CPS_GRAD_REC * K + k, K);
+}
+// (six blocks per SM as plan_grad_jac_kernel<10>: the per-experiment cost parameters would otherwise lift it to 96 registers)
+template <int NSUB>
+__global__ void __launch_bounds__(128, 6) fleet_grad_jac_kernel(const __grid_constant__ FleetGradArgs f) {
+    const GradArgs &a = f.g;
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int K = a.K;
+    if (gid >= (long long)K * a.T) return;
+    const int k = (int)(gid % K), t = (int)(gid / K);
+    step_record<NSUB, true>(a, t, k, a.jac + (long long)t * CPS_GRAD_REC * K + k, K, f.x);
 }
 
 // One control step of the reverse sweep from its record r.
@@ -555,5 +592,55 @@ extern "C" int cps_rpgd_set_iterations(cps_handle *h, long long iterations) {
     int rc = grad_state(h, &G);
     if (rc != CPS_OK) return rc;
     G->adam_iterations = iterations;
+    return CPS_OK;
+}
+
+// ---- cps_rpgd_fleet.cu: the plans of E experiments in one launch per kernel ------------------------------------------------
+// G != nullptr: the gradient -- forward with checkpoints, Jacobians to global records, reverse (the global-record path of
+// cps_plan_cost_grad for every E: the launches per period do not depend on E; the records and the arithmetic per plan are the
+// same as the fused kernel's, so J and G match cps_plan_cost_grad bit for bit).  G == nullptr: the costs only, J [n_plans].
+int cps_grad_fleet(cps_handle *h, int n_plans, int kpe, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
+                   const float *u_prev_dev, float *ck, float *jac, float *J, float *G) {
+    const int T = h->cfg.horizon;
+    FleetGradArgs f;
+    memset(&f, 0, sizeof(f));
+    GradArgs &a = f.g;
+    a.ode = h->ode;
+    a.s = s_dev;
+    a.Q = Q_dev;
+    a.qs_k = T; a.qs_t = 1; a.gs_k = T; a.gs_t = 1;
+    a.K = n_plans; a.T = T;
+    a.full = h->cfg.cost_id == CPS_COST_QB_GRAD ? 1 : 0;
+    a.inv_T1 = 1.0f / (float)(T + 1);
+    a.ck = G ? ck : nullptr; a.jac = jac; a.J = J; a.G = G;
+    a.nonfinite = h->d_nonfinite;
+    f.x.costs = costs_dev; f.x.u_prev = u_prev_dev; f.x.kpe = kpe;
+    const int block = 128, grid = (n_plans + block - 1) / block;
+    if (a.ode.n == 10) fleet_grad_fwd_kernel<10><<<grid, block, 0, h->stream>>>(f);
+    else fleet_grad_fwd_kernel<0><<<grid, block, 0, h->stream>>>(f);
+    h->launches += 1;
+    if (G) {
+        const long long pairs = (long long)n_plans * T;
+        if (a.ode.n == 10) fleet_grad_jac_kernel<10><<<(unsigned)((pairs + 127) / 128), 128, 0, h->stream>>>(f);
+        else fleet_grad_jac_kernel<0><<<(unsigned)((pairs + 127) / 128), 128, 0, h->stream>>>(f);
+        plan_grad_rev_kernel<<<grid, block, 0, h->stream>>>(a);
+        h->launches += 2;
+    }
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
+}
+
+// rpgd_update_kernel over n_plans plans [n_plans][T] (one warp each); lr_t computed by the caller
+int cps_grad_fleet_update(cps_handle *h, int n_plans, float *Q_dev, const float *G_dev, float *m_dev, float *v_dev, float lr_t,
+                          float beta_1, float beta_2, float epsilon, float gradmax_clip) {
+    RpgdArgs a;
+    a.Q = Q_dev; a.G = G_dev; a.m = m_dev; a.v = v_dev;
+    a.K = n_plans; a.T = h->cfg.horizon;
+    a.clip_norm = gradmax_clip; a.lr_t = lr_t;
+    a.beta1 = beta_1; a.beta2 = beta_2; a.eps = epsilon;
+    a.lo = h->mppi_in[5]; a.hi = h->mppi_in[6];
+    rpgd_update_kernel<<<(a.K + 3) / 4, 128, 0, h->stream>>>(a);
+    h->launches += 1;
+    CUDA_TRY(h, cudaGetLastError());
     return CPS_OK;
 }

@@ -65,6 +65,7 @@ struct FinalizeArgs {
 
 struct NetState;    // cps_net.cu
 struct FleetState;  // cps_fleet.cu
+struct RpgdFleetState;  // cps_rpgd_fleet.cu
 struct PlanState;   // cps_plan.cu
 struct GmmState;    // cps_gmm.cu
 struct GradState;   // cps_grad.cu
@@ -115,6 +116,7 @@ struct cps_handle {
     PlanState *plan;    // forward-only planners (cps_plan_*, cps_cem_*), owned
     GmmState *gmm;      // CEM with a Gaussian-mixture sampling distribution (cps_cem_gmm_*), owned
     GradState *grad;    // adjoint workspace and Adam moments (cps_plan_cost_grad, cps_rpgd_*), owned
+    RpgdFleetState *rfleet;  // closed-loop experiments under RPGD (cps_rpgd_fleet_create), owned
 };
 
 extern thread_local std::string g_create_err;
@@ -134,12 +136,21 @@ static inline size_t mppi_smem_floats(MppiParams &mp, int cost_id, int block, in
 
 // cps_fleet.cu
 void cps_fleet_free(cps_handle *h);
+// cps_rpgd_fleet.cu
+void cps_rpgd_fleet_free(cps_handle *h);
 // cps_plan.cu
 void cps_plan_free(cps_handle *h);
 // cps_gmm.cu
 void cps_gmm_free(cps_handle *h);
 // cps_grad.cu
+#define CPS_GRAD_REC 20   /* floats per (control step, plan) record: M[3][4], r[4], cost partials (3), control term */
 void cps_grad_free(cps_handle *h);
+// the RPGD fleet's gradient (G != nullptr; ck [T][4][n_plans], jac [T][CPS_GRAD_REC][n_plans]) or costs (G == nullptr) of
+// n_plans = E * kpe plans [n_plans][T] from the fleet's states [E][8], per-experiment cost parameters and u_prev [E]
+int cps_grad_fleet(cps_handle *h, int n_plans, int kpe, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
+                   const float *u_prev_dev, float *ck, float *jac, float *J, float *G);
+int cps_grad_fleet_update(cps_handle *h, int n_plans, float *Q_dev, const float *G_dev, float *m_dev, float *v_dev, float lr_t,
+                          float beta_1, float beta_2, float epsilon, float gradmax_clip);
 // cps_lib.cu: cost parameters folded for a given target equilibrium
 int cps_fold_cost_for(cps_handle *h, float target_equilibrium, CostParams *out);
 // cps_net.cu

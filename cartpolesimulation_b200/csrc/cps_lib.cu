@@ -397,6 +397,7 @@ extern "C" void cps_destroy(cps_handle *h) {
     cudaSetDevice(h->cfg.device);
     cps_net_free(h);
     cps_fleet_free(h);
+    cps_rpgd_fleet_free(h);
     cps_plan_free(h);
     cps_gmm_free(h);
     cps_grad_free(h);

@@ -267,3 +267,134 @@ class Fleet:
         eng._chk(eng.lib.cps_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
                                         _ptr(noise), _ptr(record), _ptr(J_out)))
         return record
+
+
+class RpgdFleet:
+    """E closed-loop experiments under RPGD, the reference's shipped default optimizer (Control_Toolkit_ASF/
+    config_controllers.yml:2), on one device: one cps_handle with an RPGD fleet attached (include/cps.h "RPGD fleet").
+
+    Every controller period does, for every experiment, what optimizer_rpgd_b200.step does (Adam steps on the gradient
+    of predict_and_cost, the costs of the improved plans, u = the cheapest plan's first input, the shifted warm start and
+    every `resamp_per` solves the resampling of the worst plans), then what Fleet's plant does, with no host round trip.
+    The keywords are optimizer_rpgd_b200's (same defaults; opt_keep_k and first_iter_count are derived as it derives
+    them) and Fleet's.  Predictor "ODE", cost quadratic_boundary_grad_minimal or quadratic_boundary_grad; uniform
+    resampling and the plant-side models (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+
+    def __init__(self, n_experiments: int, num_rollouts: int = 16, mpc_horizon: int = 35, outer_its: int = 4,
+                 resamp_per: int = 10, opt_keep_k_ratio: float = 0.75, period_interpolation_inducing_points: int = 4,
+                 learning_rate: float = 0.05, adam_beta_1: float = 0.9, adam_beta_2: float = 0.999,
+                 adam_epsilon: float = 1e-8, gradmax_clip: float = 5.0, sample_stdev: float = 0.5,
+                 sample_mean: float = 0.0, shift_previous: int = 1, warmup: bool = False, warmup_iterations: int = 250,
+                 control_limits=(-1.0, 1.0), SAMPLING_DISTRIBUTION: str = "normal", dt: float = 0.02,
+                 substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
+                 cost_config: dict | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
+                 experiment_offset: int = 0, dt_simulation: float = 0.002):
+        if SAMPLING_DISTRIBUTION == "uniform":
+            raise NotImplementedError("RpgdFleet resamples from the normal distribution only (SAMPLING_DISTRIBUTION='normal')")
+        if SAMPLING_DISTRIBUTION != "normal":
+            raise ValueError(f"RPGD cannot interpret sampling type {SAMPLING_DISTRIBUTION}")
+        if noise not in ("philox", "supplied"):
+            raise ValueError("noise must be 'philox' or 'supplied'")
+        n_sim = int(round(dt / dt_simulation))
+        if n_sim < 1 or abs(n_sim * dt_simulation - dt) > 1e-9:
+            raise ValueError("dt (control) must be a multiple of dt_simulation")
+        self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
+        self.outer_its, self.resamp_per, self.shift_previous = int(outer_its), int(resamp_per), int(shift_previous)
+        self.first_iter_count = int(warmup_iterations) if warmup else self.outer_its   # as optimizer_rpgd_b200
+        self.opt_keep_k = int(max(int(self.K * opt_keep_k_ratio), 1))
+        self.noise_source = noise
+        lo, hi = (float(np.asarray(x, dtype=np.float32).reshape(-1)[0]) for x in control_limits)
+        self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost,
+                             interp_period=period_interpolation_inducing_points, device=device)
+        self.n_ind, self.device = self.engine.n_ind, self.engine.device
+        if cost_config is not None:
+            self.engine.set_cost_config(cost_config)
+        self.engine.set_mppi_params(lo=lo, hi=hi)
+        c = L.cps_rpgd_fleet_config(C.sizeof(L.cps_rpgd_fleet_config), self.E, n_sim,
+                                    L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
+                                    float(dt_simulation), int(seed), int(experiment_offset), self.outer_its,
+                                    self.first_iter_count, self.resamp_per, self.opt_keep_k, self.shift_previous,
+                                    float(learning_rate), float(adam_beta_1), float(adam_beta_2), float(adam_epsilon),
+                                    float(gradmax_clip), float(sample_stdev), float(sample_mean))
+        self.engine._chk(self.engine.lib.cps_rpgd_fleet_create(self.engine._h, C.byref(c)))
+
+    def close(self):
+        self.engine.close()
+
+    def set_plant_models(self, *args, **kwargs):
+        raise NotImplementedError("RpgdFleet has no plant-side models (control disturbance, measurement noise, latency)")
+
+    def reset(self, states, period: int = 0, init_draws=None):
+        """optimizer_reset of every experiment and the initial states [E, 6].  init_draws: cuda tensor [E, K, n_ind] of
+        standard normals for the initial plans ('supplied' fleets; a 'philox' fleet draws them, see draws(-1))."""
+        s = np.ascontiguousarray(states, dtype=np.float32)
+        if s.shape != (self.E, 6):
+            raise ValueError(f"states must have shape ({self.E}, 6)")
+        if init_draws is not None:
+            _check_dev(init_draws, "init_draws", self.device)
+            if init_draws.numel() != self.E * self.K * self.n_ind:
+                raise ValueError(f"init_draws has {init_draws.numel()} elements, expected {self.E * self.K * self.n_ind}")
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_rpgd_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP),
+                                                                   _ptr(init_draws), int(period)))
+
+    def states(self, with_u_prev: bool = False):
+        s = np.zeros((self.E, 6), dtype=np.float32)
+        u_prev = np.zeros(self.E, dtype=np.float32) if with_u_prev else None
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_rpgd_fleet_get_states(
+            self.engine._h, s.ctypes.data_as(L._FP), None if u_prev is None else u_prev.ctypes.data_as(L._FP)))
+        return (s, u_prev) if with_u_prev else s
+
+    def plans(self) -> dict:
+        """The optimizer state of every experiment: Q, m, v [E, K, T], ages [E, K] (int32), and the shared Adam iteration
+        and solve counters."""
+        Q, m, v = (np.zeros((self.E, self.K, self.T), dtype=np.float32) for _ in range(3))
+        ages = np.zeros((self.E, self.K), dtype=np.int32)
+        it, solves = C.c_longlong(), C.c_longlong()
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_rpgd_fleet_get_plans(
+            self.engine._h, Q.ctypes.data_as(L._FP), m.ctypes.data_as(L._FP), v.ctypes.data_as(L._FP),
+            ages.ctypes.data_as(C.POINTER(C.c_int)), C.byref(it), C.byref(solves)))
+        return dict(Q=Q, m=m, v=v, ages=ages, adam_iterations=int(it.value), solves=int(solves.value))
+
+    @property
+    def period(self) -> int:
+        return int(self.engine.lib.cps_rpgd_fleet_period(self.engine._h))
+
+    def nonfinite_costs(self) -> int:
+        """Non-finite plan costs met so far (a NaN state or target makes them so; such costs sort after every number, as
+        torch.sort does, and the run goes on).  Synchronises."""
+        self.engine.use_current_stream()
+        return self.engine.nonfinite_costs()
+
+    def draws(self, period: int) -> torch.Tensor:
+        """The draws a 'philox' fleet uses: period >= 0 its resampling draws [E, K - opt_keep_k, n_ind]; period = -1 the
+        draws of reset() [E, K, n_ind]."""
+        rows = self.K if period < 0 else self.K - self.opt_keep_k
+        out = torch.empty((self.E, rows, self.n_ind), device=self.device, dtype=torch.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_rpgd_fleet_draws(self.engine._h, int(period), _ptr(out)))
+        return out
+
+    def run(self, n_periods: int, target_position=None, target_equilibrium=None, draws=None, record=None, J_out=None,
+            Q_opt=None):
+        """cps_rpgd_fleet_step: n_periods controller periods, no synchronisation.  target_position / target_equilibrium:
+        cuda tensors [n_periods, E] or None; draws: [n_periods, E, K - opt_keep_k, n_ind] for a 'supplied' fleet (read in
+        resampling periods only); record [n_periods, E, 16], J_out [n_periods, E, K] (costs of the improved plans) and
+        Q_opt [n_periods, E, K, T] (plans after the Adam steps) or None."""
+        eng = self.engine
+        eng.use_current_stream()
+        for t, name, numel in ((target_position, "target_position", n_periods * self.E),
+                               (target_equilibrium, "target_equilibrium", n_periods * self.E),
+                               (draws, "draws", n_periods * self.E * (self.K - self.opt_keep_k) * self.n_ind),
+                               (record, "record", n_periods * self.E * L.FLEET_RECORD),
+                               (J_out, "J_out", n_periods * self.E * self.K),
+                               (Q_opt, "Q_opt", n_periods * self.E * self.K * self.T)):
+            if t is not None:
+                _check_dev(t, name, self.device)
+                if t.numel() != numel:
+                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+        eng._chk(eng.lib.cps_rpgd_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
+                                             _ptr(draws), _ptr(record), _ptr(J_out), _ptr(Q_opt)))
+        return record

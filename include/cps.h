@@ -396,6 +396,60 @@ int cps_fleet_reset(cps_handle *h, long long period);
 /* The draws CPS_FLEET_NOISE_PHILOX uses in controller period `period`: out_dev [E][n_ind][K]. */
 int cps_fleet_noise(cps_handle *h, long long period, float *out_dev);
 
+/* ---- RPGD fleet: E closed-loop experiments under the reference's default optimizer ------------------------------ */
+/* The data generator with controller_mpc and optimizer rpgd (Control_Toolkit_ASF/config_controllers.yml:2): per controller
+ * period every experiment runs exactly what optimizer_rpgd_tf.step (Control_Toolkit/Optimizers/optimizer_rpgd_tf.py:231-377)
+ * does -- first_iter_count Adam steps on the first solve after a reset, outer_its after that (gradient, clip_by_norm per
+ * plan, Adam, clip to the control limits), the costs of the improved plans, their stable order, u = Q[best, 0], the plans
+ * shifted by shift_previous (last input repeated) and, on resampling solves (solves % resamp_per == 0, the first one
+ * included), the K - opt_keep_k worst plans replaced by clip(normal * sample_stdev + sample_mean) at the inducing points,
+ * interpolated with Interpolator's tent weights (the kept plans move to rows K - keep.. in cost order with their shifted
+ * moments and ages, the fresh ones start with zero moments and age) -- then the plant advances one controller period with
+ * Q = u and writes the record row of cps_fleet_step.  u becomes the experiment's u_prev for the next solve's cost.
+ * Each experiment owns its plans [K][T], Adam moments, ages, u_prev, state and targets (target_position /
+ * target_equilibrium select the folded cost parameters per experiment and period, as in cps_fleet_step); all advance in
+ * lockstep, so the solve counter and Adam's iteration count (lr_t) are shared.
+ * The handle: predictor CPS_EULER_CROMER, cost CPS_COST_QB_GRAD_MINIMAL or CPS_COST_QB_GRAD, K <= 4096, T, dt, substeps;
+ * interp_period = period_interpolation_inducing_points; control limits from cps_set_mppi_params (lo, hi).  Anything else:
+ * CPS_ERR_UNSUPPORTED.  opt_keep_k outside [1, K], shift_previous < 0 or dt not a multiple of dt_simulation:
+ * CPS_ERR_INVALID.  Per period 3 + 4 x (Adam steps) launches, whatever E (cps_launch_count).
+ * Non-finite costs (e.g. from a NaN state or target) are not an error: they sort after every number, as in torch.sort,
+ * and every one the fleet's forward passes meet is added to the handle's counter (cps_nonfinite_costs). */
+typedef struct cps_rpgd_fleet_config {
+    int struct_size;                 /* = sizeof(cps_rpgd_fleet_config) */
+    int n_experiments;               /* E on this device */
+    int sim_substeps;                /* plant ticks per controller period */
+    int draw_source;                 /* CPS_FLEET_NOISE_SUPPLIED | CPS_FLEET_NOISE_PHILOX: the sampling draws */
+    double dt_simulation;            /* plant tick, 0.002 s */
+    unsigned long long seed;
+    long long experiment_offset;     /* global index of local experiment 0 (Philox counters) */
+    int outer_its, first_iter_count, resamp_per, opt_keep_k, shift_previous;
+    float learning_rate, adam_beta_1, adam_beta_2, adam_epsilon, gradmax_clip, sample_stdev, sample_mean;
+} cps_rpgd_fleet_config;
+int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config *cfg);
+/* optimizer_reset for every experiment: plans from the draws init_draws_dev [E][K][n_ind] (NULL on a Philox fleet, which
+ * draws them itself), zero moments and ages, solve counter and Adam iterations 0, u_prev = 0; states s_host [E][6]
+ * (angle_cos / angle_sin taken as given); the period counter. */
+int cps_rpgd_fleet_set_states(cps_handle *h, const float *s_host, const float *init_draws_dev, long long period);
+/* n_periods controller periods, stream-ordered, no synchronisation.  tp_dev / te_dev [n_periods][E] or NULL (0 / +1);
+ * draws_dev [n_periods][E][K - opt_keep_k][n_ind] standard normals (read only in resampling periods; NULL on a Philox
+ * fleet); record_dev [n_periods][E][CPS_FLEET_RECORD], J_out_dev [n_periods][E][K] (costs of the improved plans) and
+ * Q_opt_out_dev [n_periods][E][K][T] (plans after the Adam steps, before the bookkeeping: optimizer_rpgd_tf's Q_logged)
+ * may each be NULL. */
+int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *draws_dev,
+                        float *record_dev, float *J_out_dev, float *Q_opt_out_dev);
+/* s_host [E][6], u_prev_host [E]; either may be NULL.  Synchronises. */
+int cps_rpgd_fleet_get_states(cps_handle *h, float *s_host, float *u_prev_host);
+/* Optimizer state: Q_host, m_host, v_host [E][K][T], ages_host [E][K], the shared Adam iteration and solve counters; any
+ * may be NULL.  Synchronises. */
+int cps_rpgd_fleet_get_plans(cps_handle *h, float *Q_host, float *m_host, float *v_host, int *ages_host,
+                             long long *adam_iterations, long long *solves);
+long long cps_rpgd_fleet_period(const cps_handle *h);
+/* The draws a Philox fleet uses: period >= 0 the resampling draws of that period [E][K - opt_keep_k][n_ind]; period = -1
+ * the draws of a reset [E][K][n_ind].  Counters (plan row, tag + draw group, period, experiment_offset + e): disjoint
+ * from the MPPI fleet's rollout and plant-side draws. */
+int cps_rpgd_fleet_draws(cps_handle *h, long long period, float *out_dev);
+
 /* ---- forward-only planners: predict_and_cost and the selection step (SURVEY 8f row f3) ----------------------- */
 /* optimizer_random_action_tf / optimizer_cem_tf / optimizer_cem_gmm_tf evaluate K candidate input plans from one state
  * with predictor.predict_core(s, Q) followed by cost_function.get_trajectory_cost(trajectory, Q, u_prev)
@@ -521,8 +575,9 @@ int cps_net_last_kernel(const cps_handle *h);
 /* Which kernel the last cps_rollout / cps_rollout_host chunk of this handle launched: 0 none yet, 1 rollout_kernel (one
  * cartpole per thread), 2 rollout_pair_kernel (two per thread, packed FP32; large time-major batches). */
 int cps_rollout_last_kernel(const cps_handle *h);
-/* Cumulative count of non-finite trajectory costs seen by cps_mppi_step since cps_create (the reference propagates
- * NaN silently into exp(); this library does the same arithmetic but counts it).  Synchronises. */
+/* Cumulative count of non-finite trajectory costs seen by cps_mppi_step, cps_plan_cost_grad / cps_rpgd_grad_step and
+ * cps_rpgd_fleet_step since cps_create (the reference propagates NaN silently; this library does the same arithmetic but
+ * counts it).  Synchronises. */
 int cps_nonfinite_costs(cps_handle *h, int *count_out);
 
 #ifdef __cplusplus
