@@ -160,6 +160,13 @@ int cps_net_plan_cost(cps_handle *h, const float *s_dev, const float *Q_dev, int
                       float *J_out_dev, float *traj_out_dev, int traj_layout);
 int cps_net_plan_cost_grad(cps_handle *h, const float *s_dev, const float *Q_dev, int q_layout, float u_prev, float *J_out_dev,
                            float *G_out_dev);
+// the RPGD fleet with CPS_PREDICTOR_NEURAL: cps_net_grad_fleet_prepare runs the network checks of cps_plan_cost_grad and
+// sizes the workspace for E experiments; cps_net_grad_fleet is net_grad_kernel over E experiments x K plans [E][K][T] from
+// the fleet's states [E][8], per-experiment cost parameters and u_prev [E]: the gradient (G != nullptr, J and G [E][K][T])
+// or the costs only (G == nullptr), per plan bit-identical to cps_plan_cost_grad / cps_plan_cost
+int cps_net_grad_fleet_prepare(cps_handle *h, int E, const char *who);
+int cps_net_grad_fleet(cps_handle *h, int E, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
+                       const float *u_prev_dev, float *J_dev, float *G_dev);
 int cps_net_mppi_step(cps_handle *h, const float *s_dev, const float *noise_dev, int noise_layout, float u_prev,
                       float *u_nom_dev, float *u_out_dev, float *J_out_dev, float *traj_out_dev, int traj_layout,
                       float *u_run_out_dev);

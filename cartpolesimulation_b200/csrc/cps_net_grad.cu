@@ -27,6 +27,13 @@
 // transposed copy of the weights (the 2 x 64 GRU image is 156 KB of the 227 KB).  The gate adjoints are kept [unit][R + 4]:
 // the padding makes the 16-byte loads of eight consecutive units fall on distinct banks.
 // FP32 on CUDA cores (FFMA2), no tensor cores: the shipped RPGD size is 16 plans, and the gradient wants fp32 accuracy.
+//
+// net_grad_kernel<R, HT, GRAD, FLEET = true> (cps_rpgd_fleet.cu): the plans of E experiments in one launch.  The tiles are
+// laid per experiment (grid = E x ceil(K / R), R chosen from the per-experiment K as the single-experiment call chooses it),
+// so every CTA holds plans of one experiment only and runs, per plan, exactly the arithmetic of cps_plan_cost_grad /
+// cps_plan_cost for that experiment alone.  CTA b takes experiment e = b / ceil(K / R): its state s + 8 e, u_prev[e] and
+// folded cost parameters costs[e]; Q, G [E][K][T] and J [E][K] are indexed by the global plan e K + k.  The weights and the
+// stored hidden state h0 are shared and read-only.  FLEET = false compiles to the code it compiled to before FLEET existed.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -54,6 +61,14 @@ struct NetGradArgs {
     float *ws;                  // GRAD: per CTA [T+1][htot][R] hidden states, [T][8][R] inputs, [T][8][R] outputs
     long long ws_cta;           // floats per CTA
     int *nonfinite;
+};
+
+// FLEET's per-experiment inputs (unused otherwise): CTA b holds plans of experiment b / tiles.  With FLEET, NetGradArgs' K
+// is the number of plans per experiment, s the fleet's states [E][8], Q and G [E][K][T], J [E][K].
+struct NetFleetExt {
+    const CostParams *costs;    // [E] folded for each experiment's targets of the period
+    const float *u_prev;        // [E]
+    int tiles;                  // CTAs per experiment, ceil(K / R)
 };
 
 namespace {
@@ -97,8 +112,9 @@ __device__ __forceinline__ void copy4(float *dst, const float *src, int n, int t
     for (int i = 4 * tid; i < n; i += 4 * nt) *reinterpret_cast<float4 *>(dst + i) = *reinterpret_cast<const float4 *>(src + i);
 }
 
-template <int R, int HT, bool GRAD>
-__global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_constant__ NetGradArgs a) {
+template <int R, int HT, bool GRAD, bool FLEET>
+__global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_constant__ NetGradArgs a,
+                                                                 const __grid_constant__ NetFleetExt fx) {
     constexpr int NC = R * 8, NT = NC + 32, RP = R + 4, G8 = R / NET_RT;
     extern __shared__ __align__(16) float smem[];
     __shared__ __align__(8) unsigned long long s_bar;
@@ -107,6 +123,9 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_co
     const bool row_warp = tid >= NC;
     const int T = a.T;
     const bool gru = N.type == CPS_NET_GRU;
+    // FLEET: the CTA's experiment and its per-experiment inputs (read where the single-experiment call reads its own)
+    const int e = FLEET ? (int)blockIdx.x / fx.tiles : 0;
+    const CostParams &C = FLEET ? fx.costs[e] : a.cost;
 
     // ---- shared-memory carve-up (net_kernel's, then the adjoints) --------------------------------------------------
     float *wsm = smem;                              // [n_weights]
@@ -131,14 +150,16 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_co
     }
     __syncthreads();  // also publishes the mbarrier init
 
+    const unsigned tile = FLEET ? blockIdx.x - (unsigned)(e * fx.tiles) : blockIdx.x;
+    const long long pbase = FLEET ? (long long)e * a.K : 0;   // the experiment's first plan
     const int r_row = lane % R;
     const bool row_lead = row_warp && lane < R;
-    const int k = blockIdx.x * R + r_row;
+    const int k = tile * R + r_row;
     const bool active = row_lead && k < a.K;
     const int kc = min(k, a.K - 1);
-    const float *qrow = a.Q + (long long)kc * a.qs_k;
+    const float *qrow = a.Q + (pbase + kc) * a.qs_k;
     float *traj = (a.traj && active) ? a.traj + (long long)k * a.ts_k : nullptr;
-    float Jacc = 0.0f, up = a.u_prev, u_cur = 0.0f, u_nxt = row_warp ? qrow[0] : 0.0f;
+    float Jacc = 0.0f, up = FLEET ? fx.u_prev[e] : a.u_prev, u_cur = 0.0f, u_nxt = row_warp ? qrow[0] : 0.0f;
     weights_copy_wait(&s_bar);
     __syncthreads();
 
@@ -151,9 +172,9 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_co
         if (row_warp) {
             if (t == 0) {
 #pragma unroll
-                for (int c = 0; c < 6; ++c) st[c] = a.s[c];
+                for (int c = 0; c < 6; ++c) st[c] = (FLEET ? a.s + (long long)e * 8 : a.s)[c];
                 if (row_lead)
-                    for (int i = 0; i < N.n_state_in; ++i) xin[(1 + i) * R + r_row] = fmaf(N.norm_a[1 + i], a.s[N.in_idx[i]], N.norm_b[1 + i]);
+                    for (int i = 0; i < N.n_state_in; ++i) xin[(1 + i) * R + r_row] = fmaf(N.norm_a[1 + i], (FLEET ? a.s + (long long)e * 8 : a.s)[N.in_idx[i]], N.norm_b[1 + i]);
             } else {
                 out_layer_row<R>(N, wsm, hlast_base + (gru ? p * hstride : 0), lane, y);
                 if (row_lead) {
@@ -176,7 +197,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_co
 #pragma unroll
                 for (int c = 0; c < 6; ++c) traj[(long long)t * a.ts_t + c * a.ts_c] = st[c];
             }
-            Jacc += stage_cost_rt(a.cost_id, a.cost, cosf(st[IDX_ANGLE]), st[IDX_ANGLED], st[IDX_POS], u_cur, up);
+            Jacc += stage_cost_rt(a.cost_id, C, cosf(st[IDX_ANGLE]), st[IDX_ANGLED], st[IDX_POS], u_cur, up);
             up = u_cur;
             if (t + 1 < T) u_nxt = qrow[(long long)(t + 1) * a.qs_t];
             for (int l = 0; l < N.n_layers; ++l) cta_sync();
@@ -195,7 +216,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_co
         }
         const float J = __fdiv_rn(Jacc, (float)(T + 1));   // mean over the T + 1 entries (true division, as torch.mean)
         if (active) {
-            a.J[k] = J;
+            a.J[pbase + k] = J;
             if (!isfinite(J)) atomicAdd(a.nonfinite, 1);
         }
     }
@@ -225,8 +246,8 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_co
                 for (int o = 0; o < 6; ++o) yv[o] = (o < N.n_out) ? wsY[((long long)t * 8 + o) * R + r_row] : 0.0f;
                 compose_state(N, yv, st);
                 float d_th, d_w, d_x;
-                if (full) grad_partials(a.cost, st[IDX_ANGLE], st[IDX_ANGLED], st[IDX_POS], d_th, d_w, d_x);
-                else gradmin_partials(a.cost, st[IDX_ANGLE], st[IDX_ANGLED], st[IDX_POS], d_th, d_w, d_x);
+                if (full) grad_partials(C, st[IDX_ANGLE], st[IDX_ANGLED], st[IDX_POS], d_th, d_w, d_x);
+                else gradmin_partials(C, st[IDX_ANGLE], st[IDX_ANGLED], st[IDX_POS], d_th, d_w, d_x);
                 d_th *= a.inv_T1; d_w *= a.inv_T1; d_x *= a.inv_T1;
                 float d_sin = 0.0f, d_cos = 0.0f;
                 if (atan2_angle) {   // angle = atan2(sin, cos)
@@ -350,30 +371,31 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_grad_kernel(const __grid_co
             const float u = qrow[(long long)t * a.qs_t];
             float du;
             if (full) {   // cc u_t^2 + ccrc (u_t - u_{t-1})^2 of this stage and ccrc (u_{t+1} - u_t)^2 of the next
-                const float upv = (t > 0) ? qrow[(long long)(t - 1) * a.qs_t] : a.u_prev;
-                du = 2.0f * a.cost.w[5] * u + 2.0f * a.cost.w[6] * (u - upv);
-                if (t + 1 < T) du -= 2.0f * a.cost.w[6] * (qrow[(long long)(t + 1) * a.qs_t] - u);
+                const float upv = (t > 0) ? qrow[(long long)(t - 1) * a.qs_t] : (FLEET ? fx.u_prev[e] : a.u_prev);
+                du = 2.0f * C.w[5] * u + 2.0f * C.w[6] * (u - upv);
+                if (t + 1 < T) du -= 2.0f * C.w[6] * (qrow[(long long)(t + 1) * a.qs_t] - u);
             } else {
-                du = 2.0f * a.cost.w[4] * u;
+                du = 2.0f * C.w[4] * u;
             }
-            if (active) a.G[(long long)k * a.gs_k + (long long)t * a.gs_t] = fmaf(N.norm_a[0], dX[r_row], a.inv_T1 * du);
+            if (active) a.G[(pbase + k) * a.gs_k + (long long)t * a.gs_t] = fmaf(N.norm_a[0], dX[r_row], a.inv_T1 * du);
         }
     }
 }
 
-typedef void (*net_grad_fn)(const NetGradArgs);
+typedef void (*net_grad_fn)(const NetGradArgs, const NetFleetExt);
 
-template <int R, bool GRAD>
+template <int R, bool GRAD, bool FLEET>
 net_grad_fn pick2(int ht) {
     switch (ht) {
-    case 64: return net_grad_kernel<R, 64, GRAD>;
-    case 32: return net_grad_kernel<R, 32, GRAD>;
-    default: return net_grad_kernel<R, 0, GRAD>;
+    case 64: return net_grad_kernel<R, 64, GRAD, FLEET>;
+    case 32: return net_grad_kernel<R, 32, GRAD, FLEET>;
+    default: return net_grad_kernel<R, 0, GRAD, FLEET>;
     }
 }
+template <bool FLEET>
 net_grad_fn pick(int R, int ht, bool grad) {
-    if (R == 32) return grad ? pick2<32, true>(ht) : pick2<32, false>(ht);
-    return grad ? pick2<16, true>(ht) : pick2<16, false>(ht);
+    if (R == 32) return grad ? pick2<32, true, FLEET>(ht) : pick2<32, false, FLEET>(ht);
+    return grad ? pick2<16, true, FLEET>(ht) : pick2<16, false, FLEET>(ht);
 }
 
 int hidden_max(const NetDev &N) {
@@ -415,26 +437,36 @@ int tile_rows(const NetDev &N, int K) {
     return (K > 148 * 16 && smem_bytes(N, 32, true) <= 227 * 1024) ? 32 : 16;
 }
 
+// The forward records of the gradient: floats per CTA of R plans over T steps
+long long ws_floats_per_cta(const NetDev &N, int R, int T) { return (long long)(T + 1) * N.htot * R + 16LL * T * R; }
+
+// Makes the handle's workspace hold at least `need` bytes (grown on demand; K = 2000, T = 50, 2 x 64 GRU: 53 MB)
+int grow_ws(cps_handle *h, size_t need) {
+    NetState *S = h->net;
+    if (need > S->gws_bytes) {
+        cudaFree(S->d_gws);
+        S->d_gws = nullptr;
+        S->gws_bytes = 0;
+        CUDA_TRY(h, cudaMalloc(&S->d_gws, need));
+        S->gws_bytes = need;
+    }
+    return CPS_OK;
+}
+
 int launch(cps_handle *h, NetGradArgs &a, bool grad) {
     NetState *S = h->net;
     const int R = tile_rows(S->dev, a.K);
     const size_t smem = smem_bytes(S->dev, R, grad);
     const int grid = (a.K + R - 1) / R;
     if (grad) {
-        a.ws_cta = (long long)(a.T + 1) * S->dev.htot * R + 16LL * a.T * R;
-        const size_t need = sizeof(float) * (size_t)a.ws_cta * grid;
-        if (need > S->gws_bytes) {   // grows on demand; K = 2000, T = 50, 2 x 64 GRU: 53 MB
-            cudaFree(S->d_gws);
-            S->d_gws = nullptr;
-            S->gws_bytes = 0;
-            CUDA_TRY(h, cudaMalloc(&S->d_gws, need));
-            S->gws_bytes = need;
-        }
+        a.ws_cta = ws_floats_per_cta(S->dev, R, a.T);
+        const int rc = grow_ws(h, sizeof(float) * (size_t)a.ws_cta * grid);
+        if (rc != CPS_OK) return rc;
         a.ws = S->d_gws;
     }
-    net_grad_fn fn = pick(R, S->ht, grad);
+    net_grad_fn fn = pick<false>(R, S->ht, grad);
     CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fn<<<grid, R * 8 + 32, smem, h->stream>>>(a);
+    fn<<<grid, R * 8 + 32, smem, h->stream>>>(a, NetFleetExt());
     h->launches += 1;
     CUDA_TRY(h, cudaGetLastError());
     return CPS_OK;
@@ -482,4 +514,43 @@ int cps_net_plan_cost_grad(cps_handle *h, const float *s_dev, const float *Q_dev
     a.G = G_out_dev;
     if (q_layout == CPS_TIME_MAJOR) { a.gs_k = 1; a.gs_t = K; } else { a.gs_k = T; a.gs_t = 1; }
     return launch(h, a, true);
+}
+
+// ---- cps_rpgd_fleet.cu: the plans of E experiments in one launch -----------------------------------------------------------
+int cps_net_grad_fleet_prepare(cps_handle *h, int E, const char *who) {
+    int rc = check(h, who, true);
+    if (rc != CPS_OK) return rc;
+    const NetDev &N = h->net->dev;
+    const int K = h->cfg.num_rollouts, T = h->cfg.horizon, R = tile_rows(N, K);
+    return grow_ws(h, sizeof(float) * (size_t)ws_floats_per_cta(N, R, T) * (size_t)E * (size_t)((K + R - 1) / R));
+}
+
+int cps_net_grad_fleet(cps_handle *h, int E, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
+                       const float *u_prev_dev, float *J_dev, float *G_dev) {
+    const bool grad = G_dev != nullptr;
+    int rc = check(h, "cps_rpgd_fleet_step", grad);
+    if (rc != CPS_OK) return rc;
+    NetState *S = h->net;
+    const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
+    const int R = tile_rows(S->dev, K), tiles = (K + R - 1) / R;   // the tile of the single-experiment call
+    NetGradArgs a;
+    NetFleetExt x;
+    common(h, a, s_dev, Q_dev, CPS_ROLLOUT_MAJOR, K, T, 0.0f);
+    a.J = J_dev;
+    a.G = G_dev;
+    a.gs_k = T; a.gs_t = 1;
+    x.costs = costs_dev; x.u_prev = u_prev_dev; x.tiles = tiles;
+    const long long grid = (long long)E * tiles;
+    if (grad) {
+        a.ws_cta = ws_floats_per_cta(S->dev, R, T);
+        if ((rc = grow_ws(h, sizeof(float) * (size_t)a.ws_cta * (size_t)grid)) != CPS_OK) return rc;
+        a.ws = S->d_gws;
+    }
+    const size_t smem = smem_bytes(S->dev, R, grad);
+    net_grad_fn fn = pick<true>(R, S->ht, grad);
+    CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fn<<<(unsigned)grid, R * 8 + 32, smem, h->stream>>>(a, x);
+    h->launches += 1;
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
 }

@@ -3,16 +3,21 @@
 //
 // One controller period of EVERY experiment, no host round trip (launches independent of E):
 //   rpgd_fleet_cost_kernel     the cost parameters of each experiment's targets, folded once into an [E] array;
-//   per Adam step              the three ODE adjoint kernels of cps_grad.cu over all E x K plans (plan k belongs to
-//                              experiment k / K and takes its state, u_prev and cost parameters; per plan the arithmetic
-//                              of cps_plan_cost_grad) and rpgd_update_kernel over all E x K plans;
-//   costs                      the adjoint's forward over all plans without checkpoints (J of cps_plan_cost bit for bit);
+//   per Adam step              predictor "ODE": the three ODE adjoint kernels of cps_grad.cu over all E x K plans (plan k
+//                              belongs to experiment k / K and takes its state, u_prev and cost parameters; per plan the
+//                              arithmetic of cps_plan_cost_grad); neural predictor: net_grad_kernel<.., FLEET> of
+//                              cps_net_grad.cu, one launch over E experiments x K plans with the single-experiment tiling
+//                              (the same per-plan arithmetic, the stored hidden state read and never written); then
+//                              rpgd_update_kernel over all E x K plans;
+//   costs                      the adjoint's forward over all plans without checkpoints / records (J of cps_plan_cost bit
+//                              for bit);
 //   rpgd_fleet_finish_kernel   one block per experiment: stable ranks of its K costs, u = the cheapest plan's first
 //                              input, the shifted / permuted plans, moments and ages into the other half of a ping-pong
 //                              pair (fresh plans built in the kernel from the draws), then the plant period in the
 //                              reference's mixed float32 / float64 arithmetic (cps_plant.cuh, as cps_fleet.cu) and the
 //                              record row.
 // The solve counter and Adam's iteration count are shared (lockstep), so lr_t is one host-computed scalar per Adam step.
+// Launches per period: 3 + 4 x (Adam steps) with predictor "ODE", 3 + 2 x (Adam steps) with the neural predictor.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -200,7 +205,8 @@ struct RpgdFleetState {
     float *d_Q[2], *d_m[2], *d_v[2];  // ping-pong plans and Adam moments [E][K][T]
     int *d_ages[2];                   // [E][K]
     int cur;                          // which half holds the current plans
-    float *d_ck, *d_jac, *d_J, *d_G;  // adjoint workspace: [T][4][EK], [T][CPS_GRAD_REC][EK], [EK], [EK][T]
+    float *d_ck, *d_jac, *d_J, *d_G;  // adjoint workspace: [T][4][EK], [T][CPS_GRAD_REC][EK] (ODE only; the neural adjoint
+                                      // keeps its records in the network's workspace), [EK], [EK][T]
     CostParams *d_costs;              // [E] this period's folded cost parameters
     float *d_draws;                   // Philox reset draws [E][K][n_ind]
     size_t finish_smem;
@@ -230,13 +236,15 @@ extern "C" int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config 
     if (!h) return CPS_ERR_INVALID;
     if (!cfg || cfg->struct_size != (int)sizeof(cps_rpgd_fleet_config))
         return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: cps_rpgd_fleet_config size mismatch");
-    if (h->cfg.integrator != CPS_EULER_CROMER)
+    const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
+    if (h->cfg.integrator != CPS_EULER_CROMER && !neural)
         return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: the adjoint of an RPGD fleet is built for predictor \"ODE\" "
-                    "(Euler-Cromer)");
+                    "(Euler-Cromer) and the neural predictor");
     if (h->cfg.cost_id != CPS_COST_QB_GRAD_MINIMAL && h->cfg.cost_id != CPS_COST_QB_GRAD)
         return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: the adjoint is built for the quadratic_boundary_grad_minimal and "
                     "quadratic_boundary_grad plugins");
-    if (h->cfg.substeps > 32) return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: at most 32 substeps per control step");
+    if (!neural && h->cfg.substeps > 32)
+        return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: at most 32 substeps per control step");
     const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
     if (K > 4096) return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: at most 4096 plans (ranks by counting)");
     if (cfg->n_experiments < 1 || cfg->sim_substeps < 1 || !(cfg->dt_simulation > 0.0))
@@ -259,6 +267,8 @@ extern "C" int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config 
         return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: (K - opt_keep_k) x n_ind too large for the finish kernel's "
                     "shared memory");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    int rc;   // neural: the network checks of cps_plan_cost_grad, and the workspace sized now rather than mid-run
+    if (neural && (rc = cps_net_grad_fleet_prepare(h, cfg->n_experiments, "cps_rpgd_fleet_create")) != CPS_OK) return rc;
     cps_rpgd_fleet_free(h);
     RpgdFleetState *F = new (std::nothrow) RpgdFleetState();
     if (!F) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: out of host memory");
@@ -276,8 +286,10 @@ extern "C" int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config 
         CUDA_TRY(h, cudaMalloc(&F->d_v[i], sizeof(float) * n));
         CUDA_TRY(h, cudaMalloc(&F->d_ages[i], sizeof(int) * EK));
     }
-    CUDA_TRY(h, cudaMalloc(&F->d_ck, sizeof(float) * 4 * n));
-    CUDA_TRY(h, cudaMalloc(&F->d_jac, sizeof(float) * CPS_GRAD_REC * n));
+    if (!neural) {
+        CUDA_TRY(h, cudaMalloc(&F->d_ck, sizeof(float) * 4 * n));
+        CUDA_TRY(h, cudaMalloc(&F->d_jac, sizeof(float) * CPS_GRAD_REC * n));
+    }
     CUDA_TRY(h, cudaMalloc(&F->d_J, sizeof(float) * EK));
     CUDA_TRY(h, cudaMalloc(&F->d_G, sizeof(float) * n));
     CUDA_TRY(h, cudaMalloc(&F->d_costs, sizeof(CostParams) * E));
@@ -350,8 +362,10 @@ extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp
     if (!philox && !draws_dev && F->nf > 0) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_step: this fleet expects supplied draws");
     if (philox && draws_dev) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_step: this fleet generates its draws (Philox); pass NULL");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
+    int rc;   // neural: the network may have been reloaded since create (another size): check it, grow the workspace
+    if (neural && (rc = cps_net_grad_fleet_prepare(h, F->E, "cps_rpgd_fleet_step")) != CPS_OK) return rc;
     CostParams up, dn;
-    int rc;
     if ((rc = cps_fold_cost_for(h, 1.0f, &up)) != CPS_OK) return rc;
     if ((rc = cps_fold_cost_for(h, -1.0f, &dn)) != CPS_OK) return rc;
     const cps_rpgd_fleet_config &c = F->cfg;
@@ -377,8 +391,9 @@ extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp
         float *Q = F->d_Q[F->cur], *m = F->d_m[F->cur], *v = F->d_v[F->cur];
         const int its = F->solves == 0 ? c.first_iter_count : c.outer_its;
         for (int it = 0; it < its; ++it) {   // grad_step (:166-180)
-            if ((rc = cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, F->d_ck, F->d_jac, F->d_J, F->d_G)) != CPS_OK)
-                return rc;
+            rc = neural ? cps_net_grad_fleet(h, (int)E, F->d_s, Q, F->d_costs, F->d_uprev, F->d_J, F->d_G)
+                        : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, F->d_ck, F->d_jac, F->d_J, F->d_G);
+            if (rc != CPS_OK) return rc;
             F->adam_iterations += 1;
             const double t = (double)F->adam_iterations;   // ResourceApplyAdam, as cps_rpgd_grad_step
             const float lr_t = (float)((double)c.learning_rate * sqrt(1.0 - pow((double)c.adam_beta_2, t)) /
@@ -388,8 +403,9 @@ extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp
                 return rc;
         }
         // get_action (:182-224): the costs of the improved plans
-        if ((rc = cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, nullptr, nullptr, F->d_J, nullptr)) != CPS_OK)
-            return rc;
+        rc = neural ? cps_net_grad_fleet(h, (int)E, F->d_s, Q, F->d_costs, F->d_uprev, F->d_J, nullptr)
+                    : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, nullptr, nullptr, F->d_J, nullptr);
+        if (rc != CPS_OK) return rc;
         const int nxt = F->cur ^ 1;
         a.J = F->d_J; a.Q = Q; a.m = m; a.v = v; a.ages = F->d_ages[F->cur];
         a.Q2 = F->d_Q[nxt]; a.m2 = F->d_m[nxt]; a.v2 = F->d_v[nxt]; a.ages2 = F->d_ages[nxt];

@@ -277,8 +277,13 @@ class RpgdFleet:
     of predict_and_cost, the costs of the improved plans, u = the cheapest plan's first input, the shifted warm start and
     every `resamp_per` solves the resampling of the worst plans), then what Fleet's plant does, with no host round trip.
     The keywords are optimizer_rpgd_b200's (same defaults; opt_keep_k and first_iter_count are derived as it derives
-    them) and Fleet's.  Predictor "ODE", cost quadratic_boundary_grad_minimal or quadratic_boundary_grad; uniform
-    resampling and the plant-side models (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+    them) and Fleet's.  Predictor "ODE", or "neural" with `network`: the spec dict Engine.net_load takes
+    (neural.load_model(...)[0], neural.build_net_spec, neural.synthetic_net_spec), loaded before the fleet is created.  The
+    network lives in the controller only; the plant stays the CartPole ODE.  Every gradient and cost reads the network's
+    stored hidden state (zero after loading; engine.net_set_state before reset() sets another) and never advances it, as
+    optimizer_rpgd_b200 and the reference's RPGD.  Cost quadratic_boundary_grad_minimal or quadratic_boundary_grad;
+    uniform resampling and the plant-side models (Fleet.set_plant_models) are not implemented and raise
+    NotImplementedError."""
 
     def __init__(self, n_experiments: int, num_rollouts: int = 16, mpc_horizon: int = 35, outer_its: int = 4,
                  resamp_per: int = 10, opt_keep_k_ratio: float = 0.75, period_interpolation_inducing_points: int = 4,
@@ -288,7 +293,12 @@ class RpgdFleet:
                  control_limits=(-1.0, 1.0), SAMPLING_DISTRIBUTION: str = "normal", dt: float = 0.02,
                  substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
                  cost_config: dict | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
-                 experiment_offset: int = 0, dt_simulation: float = 0.002):
+                 experiment_offset: int = 0, dt_simulation: float = 0.002, network: dict | None = None):
+        if integrator == "neural" and network is None:
+            raise NotImplementedError("RpgdFleet with integrator='neural' needs the network: pass network=<spec dict as "
+                                      "Engine.net_load takes, e.g. neural.load_model(...)[0]>")
+        if network is not None and integrator != "neural":
+            raise ValueError(f"network= is the neural predictor's model; integrator={integrator!r} takes none")
         if SAMPLING_DISTRIBUTION == "uniform":
             raise NotImplementedError("RpgdFleet resamples from the normal distribution only (SAMPLING_DISTRIBUTION='normal')")
         if SAMPLING_DISTRIBUTION != "normal":
@@ -310,6 +320,8 @@ class RpgdFleet:
         if cost_config is not None:
             self.engine.set_cost_config(cost_config)
         self.engine.set_mppi_params(lo=lo, hi=hi)
+        if network is not None:
+            self.engine.net_load(network)
         c = L.cps_rpgd_fleet_config(C.sizeof(L.cps_rpgd_fleet_config), self.E, n_sim,
                                     L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
                                     float(dt_simulation), int(seed), int(experiment_offset), self.outer_its,

@@ -409,10 +409,18 @@ int cps_fleet_noise(cps_handle *h, long long period, float *out_dev);
  * Each experiment owns its plans [K][T], Adam moments, ages, u_prev, state and targets (target_position /
  * target_equilibrium select the folded cost parameters per experiment and period, as in cps_fleet_step); all advance in
  * lockstep, so the solve counter and Adam's iteration count (lr_t) are shared.
- * The handle: predictor CPS_EULER_CROMER, cost CPS_COST_QB_GRAD_MINIMAL or CPS_COST_QB_GRAD, K <= 4096, T, dt, substeps;
- * interp_period = period_interpolation_inducing_points; control limits from cps_set_mppi_params (lo, hi).  Anything else:
- * CPS_ERR_UNSUPPORTED.  opt_keep_k outside [1, K], shift_previous < 0 or dt not a multiple of dt_simulation:
- * CPS_ERR_INVALID.  Per period 3 + 4 x (Adam steps) launches, whatever E (cps_launch_count).
+ * The handle: predictor CPS_EULER_CROMER (substeps <= 32) or CPS_PREDICTOR_NEURAL, cost CPS_COST_QB_GRAD_MINIMAL or
+ * CPS_COST_QB_GRAD, K <= 4096, T, dt; interp_period = period_interpolation_inducing_points; control limits from
+ * cps_set_mppi_params (lo, hi).  Anything else: CPS_ERR_UNSUPPORTED.  opt_keep_k outside [1, K], shift_previous < 0 or dt
+ * not a multiple of dt_simulation: CPS_ERR_INVALID.
+ * CPS_PREDICTOR_NEURAL: the network is loaded before create (cps_net_load; none: CPS_ERR_NOT_CONFIGURED) and must be one
+ * cps_plan_cost_grad accepts (not differential, no CPS_FLAG_NET_TENSOR_CORES, fits shared memory with the adjoint's
+ * buffers; else CPS_ERR_UNSUPPORTED).  Create sizes the adjoint's workspace for E experiments; step re-checks the network
+ * (it may have been reloaded) and grows the workspace if needed.  Every gradient and cost reads the stored hidden state
+ * (cps_net_set_state; zero after load) and never writes it, as optimizer_rpgd_tf's predictor does.  The plant stays the
+ * CartPole ODE; the network lives only in the controller.
+ * Per period 3 + 4 x (Adam steps) launches with CPS_EULER_CROMER, 3 + 2 x (Adam steps) with CPS_PREDICTOR_NEURAL, whatever E
+ * (cps_launch_count).
  * Non-finite costs (e.g. from a NaN state or target) are not an error: they sort after every number, as in torch.sort,
  * and every one the fleet's forward passes meet is added to the handle's counter (cps_nonfinite_costs). */
 typedef struct cps_rpgd_fleet_config {
