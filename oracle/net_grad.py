@@ -27,7 +27,8 @@ def _t(a, dtype, device=None):
 
 def predict(spec, s0, Q, h0=None, dtype=torch.float64):
     """Trajectories [K, T+1, 6] of the network on plans Q [K, T] (tensor; may require grad) from s0 ([6] or [K, 6]) and
-    the shared initial hidden state h0 ([Htot], concatenated over the layers; None = zeros).  Runs on Q's device."""
+    the initial hidden state h0 ([Htot] shared or [K, Htot], concatenated over the layers; None = zeros).  Runs on Q's
+    device."""
     K, T = Q.shape
     dev = Q.device
     s0 = _t(s0, dtype, dev)
@@ -41,10 +42,12 @@ def predict(spec, s0, Q, h0=None, dtype=torch.float64):
     ns = len(in_idx)
     h = []
     if gru:
-        hv = torch.zeros(int(sum(spec["hsz"])), dtype=dtype, device=dev) if h0 is None else _t(h0, dtype, dev).reshape(-1)
+        Ht = int(sum(spec["hsz"]))
+        hv = torch.zeros(Ht, dtype=dtype, device=dev) if h0 is None else _t(h0, dtype, dev)
+        hv = hv.reshape(-1, Ht).expand(K, Ht)
         off = 0
         for H in spec["hsz"]:
-            h.append(hv[off:off + H].reshape(1, H).expand(K, H))
+            h.append(hv[:, off:off + H])
             off += H
     has = set(out_idx)
 

@@ -84,3 +84,103 @@ def write_model_dir(root, z):
     sd = {str(k): torch.from_numpy(np.array(z["w__" + str(k)])) for k in z["state_dict_keys"]}
     torch.save(sd, os.path.join(d, "ckpt.pt"))
     return os.path.join(root, full)
+
+
+# ---- networks of any architecture the loader accepts -------------------------------------------------------------
+SHIPPED_IN = ["Q", "angleD", "angle_cos", "angle_sin", "position", "positionD"]
+SHIPPED_OUT = SHIPPED_IN[1:]
+ANGLE_IN, ANGLE_OUT = ["Q", "angle", "angleD", "position", "positionD"], ["angle", "angleD", "position", "positionD"]
+PERM_IN = ["Q", "position", "angle_sin", "angleD", "angle_cos", "positionD"]
+PERM_OUT = PERM_IN[1:] + ["angle"]
+EXTRA_IN, EXTRA_OUT = ["Q", "angle_cos", "angle_sin"], ["angle_cos", "angle_sin", "angleD", "position", "positionD"]
+NOIN_IN, NOIN_OUT = ["Q"], ["angle", "angleD", "position", "positionD"]
+
+# id: (type, hidden sizes, inputs, outputs) -- one line per kernel branch the entry exists for
+ARCHS = {
+    "g_mixed": ("GRU", (48, 40), SHIPPED_IN, SHIPPED_OUT),        # HT = 0, 2 layers; tensor-core eligible
+    "g_3x32": ("GRU", (32, 32, 32), SHIPPED_IN, SHIPPED_OUT),     # HT = 32 with 3 layers
+    "g_1x64": ("GRU", (64,), SHIPPED_IN, SHIPPED_OUT),            # HT = 64 with 1 layer
+    "g_4deep": ("GRU", (16, 24, 8, 40), SHIPPED_IN, SHIPPED_OUT),  # HT = 0, 4 layers (hoff of layers 2, 3)
+    "g_wide": ("GRU", (96,), SHIPPED_IN, SHIPPED_OUT),            # H0 > 64: layer 0 without the split; gradient at R = 32
+    "d_128": ("Dense", (128, 128), SHIPPED_IN, SHIPPED_OUT),      # widest Dense; gradient falls back to R = 16 at large K
+    "d_odd": ("Dense", (7,), SHIPPED_IN, SHIPPED_OUT),            # 1 layer of odd width (out_layer_row's two lane halves)
+    "d_angle": ("Dense", (24, 24, 24), ANGLE_IN, ANGLE_OUT),      # `angle` output: sin / cos rebuilt by sinf / cosf
+    "g_perm": ("GRU", (33, 31), PERM_IN, PERM_OUT),               # permuted in_idx / out_idx; angle, sin and cos all output
+    "g_extra": ("GRU", (1, 5), EXTRA_IN, EXTRA_OUT),              # H = 1; n_state_in < n_out (outputs not fed back)
+    "g_noin": ("GRU", (20, 12), NOIN_IN, NOIN_OUT),               # n_state_in = 0 (n_in = 1)
+    "tc_angle": ("GRU", (64, 64), ANGLE_IN, ANGLE_OUT),           # tensor cores: n_in = 5, `angle` output
+    "tc_perm": ("GRU", (40, 56), PERM_IN, PERM_OUT),              # tensor cores: permuted indices, n_out = 6
+    "tc_extra": ("GRU", (32, 32), EXTRA_IN, EXTRA_OUT),           # tensor cores (narrow image): n_state_in < n_out
+    "tc_noin": ("GRU", (24, 16), NOIN_IN, NOIN_OUT),              # tensor cores (narrow image): n_in = 1
+}
+
+
+def arch_norm(outputs=()):
+    """(columns, table) normalisation of the reference's shipped ranges (neural.DEFAULT_RANGES), plus symmetric ranges
+    of the D_* columns a differential network's outputs name (those of the reference's differential recordings)."""
+    from cartpolesimulation_b200.neural import DEFAULT_RANGES
+    rng = dict(DEFAULT_RANGES)
+    d_ranges = {"D_angle": 18.38, "D_angleD": 90.0, "D_angle_cos": 15.0, "D_angle_sin": 15.0, "D_position": 1.125,
+                "D_positionD": 9.0}
+    for o in outputs:
+        if o.startswith("D_"):
+            rng[o] = (d_ranges[o], -d_ranges[o])
+    cols = list(rng)
+    table = np.array([[0.0] * len(cols), [1.0] * len(cols), [rng[c][0] for c in cols], [rng[c][1] for c in cols]])
+    return cols, table
+
+
+def arch_net(net_type, hsz, inputs, outputs, seed, dt=None):
+    """(engine spec, oracle spec) of one randomly initialised network.
+
+    Weights as torch initialises GRUCell / Linear, U(-1/sqrt(H), 1/sqrt(H)) with H the layer's width (the input width for
+    the output layer).  A layout that rebuilds the angle as atan2(sin, cos) gets output rows for angle_cos / angle_sin
+    with the bias (cos phi, sin phi) and weights scaled by 0.1, so that |(sin, cos)| stays near 1: an untrained network
+    would put it near 0, where atan2 amplifies any rounding without bound and hides the kernels' own error.
+    The engine spec comes from the product's neural.build_net_spec; the oracle spec holds the same weights unpacked into
+    layers / out_layer tuples (oracle/net_grad.py, oracle.net_rollout)."""
+    from cartpolesimulation_b200.neural import build_net_spec
+    rng = np.random.default_rng(seed)
+    gru = net_type == "GRU"
+    G = 3 if gru else 1
+    layers, n_in = [], len(inputs)
+    u = lambda k, shape: rng.uniform(-k, k, shape).astype(np.float32)
+    for H in hsz:
+        k = 1.0 / np.sqrt(H)
+        layers.append((u(k, (G * H, n_in)), u(k, (G * H, H)), u(k, G * H), u(k, G * H)) if gru else
+                      (u(k, (H, n_in)), u(k, H)))
+        n_in = H
+    k = 1.0 / np.sqrt(n_in)
+    w_out, b_out = u(k, (len(outputs), n_in)), u(k, len(outputs))
+    norm = arch_norm(outputs)
+    spec = build_net_spec(net_type, inputs, outputs, list(hsz), np.zeros(1), norm, dt)
+    names = [(o[2:] if o[:2] == "D_" else o) for o in outputs]
+    if "angle" not in names and "angle_cos" in names and "angle_sin" in names and not spec["differential"]:
+        phi = rng.uniform(-np.pi, np.pi)
+        A, B = spec["denorm_A"], spec["denorm_B"]
+        for name, v in (("angle_cos", np.cos(phi)), ("angle_sin", np.sin(phi))):
+            o = names.index(name)
+            w_out[o] *= np.float32(0.1)
+            b_out[o] = np.float32((v - B[o]) / A[o])
+    from oracle import oracle as O
+    spec["weights"] = O.pack_net_weights(net_type, layers, (w_out, b_out))
+    diff = None
+    if spec["differential"]:
+        diff = dict(p1=spec["diff_p1"], p2=spec["diff_p2"], on_a=spec["out_norm_a"], on_b=spec["out_norm_b"],
+                    out_to_in=spec["out_to_in"])
+    osp = dict(net_type=net_type, hsz=list(hsz), layers=layers, out_layer=(w_out, b_out), in_idx=spec["in_idx"],
+               out_idx=spec["out_idx"], norm_a=spec["norm_a"], norm_b=spec["norm_b"], denorm_A=spec["denorm_A"],
+               denorm_B=spec["denorm_B"], diff=diff)
+    return spec, osp
+
+
+def arch(name, seed=None):
+    """arch_net of a catalogue entry (seed: the entry's position, unless given)."""
+    t, hsz, i, o = ARCHS[name]
+    return arch_net(t, hsz, i, o, list(ARCHS).index(name) if seed is None else seed)
+
+
+def atan2_layout(osp):
+    """Whether the network's layout rebuilds the angle as atan2(sin, cos) (no `angle` output, both sin and cos)."""
+    out = set(osp["out_idx"])
+    return 0 not in out and 2 in out and 3 in out

@@ -510,8 +510,8 @@ def test_tc_padded_gru32_mppi_vs_reference_golden(run):
 @pytest.mark.parametrize("K", [500, 6000, 12000])   # 32 / 64 / 128 live rollouts per CTA
 def test_tc_padded_widths_match_fp32_kernel(hsz, K):
     """two-layer GRUs narrower than the tensor-core kernel's 64 units (zero-padded image; k-steps and half-layer jobs that hold
-    only padding are skipped): same costs, control, nominal inputs and stored hidden state as the FP32 kernel, which is
-    pinned against the reference for arbitrary widths."""
+    only padding are skipped): same costs, control, nominal inputs and stored hidden state as the FP32 kernel, which
+    tests/test_gpu_net_arch.py pins against the oracle for arbitrary widths."""
     import torch
     from cartpolesimulation_b200 import _lib as L
     from cartpolesimulation_b200.core import Engine

@@ -43,16 +43,12 @@ def test_restatement_costs_match_oracle_trajectory_cost(name, cost):
     assert e < 2e-6   # float32 oracle against a float64 sum: measured <= 4.9e-7
 
 
-@pytest.mark.parametrize("name", NETS)
-@pytest.mark.parametrize("cost", COSTS)
-def test_autograd_gradient_matches_finite_differences(name, cost):
+def fd_gradient_error(sp, cost, s0, h0):
+    """max |autograd - central finite differences| / max |finite differences| of dJ/dQ on three random plans."""
     from oracle import net_grad as NG
-    z, _ = load_golden(name)
-    sp = net_spec_from_golden(z)
     rng = np.random.default_rng(3)
     K, T = 3, 6
     Q = np.clip(rng.normal(0, 0.5, (K, T)), -1, 1)
-    h0 = z["h_after_updates"].reshape(-1) if "h_after_updates" in z.files else None
     kw = dict(u_prev=-0.3, target_position=0.03, target_equilibrium=1.0, h0=h0)
     if cost == "quadratic_boundary_grad":
         from oracle import oracle as O
@@ -60,15 +56,23 @@ def test_autograd_gradient_matches_finite_differences(name, cost):
         # the kinetic term's target is under stop_gradient, which a finite difference does not see: weight 0 here
         cfg.update({"dd_linear_weight_up": 25.0, "ccrc_weight_up": 1.5, "ekp_weight_up": 0.0})
         kw["cost_cfg"] = cfg
-    _, G = NG.plan_cost_grad(sp, cost, z["s0"], Q, **kw)
+    _, G = NG.plan_cost_grad(sp, cost, s0, Q, **kw)
     eps = 1e-6
     Gfd = np.zeros_like(Q)
     for t in range(T):
         d = np.zeros_like(Q)
         d[:, t] = eps
-        Jp = NG.plan_cost(sp, cost, z["s0"], torch.from_numpy(Q + d), **kw).numpy()
-        Jm = NG.plan_cost(sp, cost, z["s0"], torch.from_numpy(Q - d), **kw).numpy()
+        Jp = NG.plan_cost(sp, cost, s0, torch.from_numpy(Q + d), **kw).numpy()
+        Jm = NG.plan_cost(sp, cost, s0, torch.from_numpy(Q - d), **kw).numpy()
         Gfd[:, t] = (Jp - Jm) / (2 * eps)
-    e = float(np.abs(G - Gfd).max() / np.abs(Gfd).max())
+    return float(np.abs(G - Gfd).max() / np.abs(Gfd).max())
+
+
+@pytest.mark.parametrize("name", NETS)
+@pytest.mark.parametrize("cost", COSTS)
+def test_autograd_gradient_matches_finite_differences(name, cost):
+    z, _ = load_golden(name)
+    h0 = z["h_after_updates"].reshape(-1) if "h_after_updates" in z.files else None
+    e = fd_gradient_error(net_spec_from_golden(z), cost, z["s0"], h0)
     record("net_grad_oracle_vs_finite_differences", f"{name}/{cost}", G=e)
     assert e < 1e-6
