@@ -175,11 +175,21 @@ static void fold_ode(cps_handle *h) {
     o.d3 = (float)(J / (mp * Lh * kp1 * Lh));
     o.u_scale = (float)(kp1 * umax);
     o.h = (float)((double)h->cfg.dt / (double)h->cfg.substeps);
-    {   // rotation substeps: the step folded into the angular-acceleration constants (ode_rhs_w)
+    {   // rotation substeps: the step folded into the angular-acceleration constants (ode_rhs_w) and the rotation (rotate_cs)
         const double hh = (double)h->cfg.dt / (double)h->cfg.substeps;
+        const double hd2 = hh * (1.0 / (kp1 * Lh));
+        o.yc1 = (float)(hd2 * (mp * g));
+        o.yc2 = (float)(hd2 * (kp1 * mp * Lh));
+        o.yc3 = (float)(hd2 * (J / Lh));
+        o.yc5 = (float)(hd2 * (kp1 * M));
+        o.yu_scale = (float)(hd2 * (kp1 * umax));
+        o.v_y = (float)(kp1 * Lh);
         o.hd1 = (float)(hh * (g / (kp1 * Lh)));
-        o.hd2 = (float)(hh * (1.0 / (kp1 * Lh)));
         o.hd3 = (float)(hh * (J / (mp * Lh * kp1 * Lh)));
+        o.rot_c2 = (float)(-hh * hh / 2.0);
+        o.rot_s3 = (float)(-hh * hh * hh / 6.0);
+        o.rot_c4 = (float)(hh * hh * hh * hh / 24.0);
+        o.w_rot_max = (float)((double)CPS_ROT_MAX / hh);
     }
     o.thl = h->phys[CPS_PH_TRACK_HALF_LENGTH];
     o.bounce = (float)(2.0 / (0.5 * L));
