@@ -129,6 +129,8 @@ SYMBOLS = {
     "cps_fleet_relabel_masked": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "cps_fleet_reset": (C.c_int, [_VP, C.c_longlong]),
     "cps_fleet_noise": (C.c_int, [_VP, C.c_longlong, _VP]),
+    "cps_fleet_get_net_states": (C.c_int, [_VP, _FP]),
+    "cps_fleet_set_net_states": (C.c_int, [_VP, _FP]),
     "cps_rpgd_fleet_create": (C.c_int, [_VP, C.POINTER(cps_rpgd_fleet_config)]),
     "cps_rpgd_fleet_set_states": (C.c_int, [_VP, _FP, _VP, C.c_longlong]),
     "cps_rpgd_fleet_step": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),

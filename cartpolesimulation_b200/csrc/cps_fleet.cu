@@ -19,6 +19,7 @@
 #include <cstdint>
 #include <cstring>
 #include <new>
+#include <vector>
 
 #include "cps_internal.cuh"
 #include "cps_plant.cuh"
@@ -283,6 +284,45 @@ __global__ void __launch_bounds__(256, 4) fleet_kernel(const __grid_constant__ F
     }
 }
 
+// Neural fleets (CPS_PREDICTOR_NEURAL): the solve is net_kernel / net_tc_kernel<.., FLEET> (cps_net.cu, cps_net_tc.cu),
+// which leaves each experiment's u in u_prev[e]; this kernel is the plant period that follows, one thread per experiment:
+// fleet_kernel's record row and plant with Q_applied = Q (plant-side models are not offered on neural fleets).
+struct NetPlantArgs {
+    PlantParams plant;
+    float *s;                   // [E][8]
+    const float *u;             // [E] the controls the solve just chose
+    const float *tp, *te;       // [E] targets of this period (null: 0 / +1)
+    float *record;              // [E][CPS_FLEET_RECORD] of this period, or null
+    double time;                // period * dt_control
+    int E;
+};
+__global__ void __launch_bounds__(128) fleet_net_plant_kernel(const __grid_constant__ NetPlantArgs a) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= a.E) return;
+    const PlantParams &P = a.plant;
+    float s[6];
+#pragma unroll
+    for (int c = 0; c < 6; ++c) s[c] = a.s[(size_t)e * 8 + c];
+    const float Q = a.u[e];
+    const float u = __fmul_rn(P.u_max, Q);
+    double aDD, pDD;
+    plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
+    if (a.record) {
+        float *r = a.record + (size_t)e * CPS_FLEET_RECORD;
+        r[0] = (float)a.time;
+        r[1] = s[IDX_ANGLE]; r[2] = s[IDX_ANGLED]; r[3] = (float)aDD; r[4] = s[IDX_COS]; r[5] = s[IDX_SIN];
+        r[6] = s[IDX_POS]; r[7] = s[IDX_POSD]; r[8] = (float)pDD;
+        r[9] = Q; r[10] = Q; r[11] = u; r[12] = a.tp ? a.tp[e] : 0.0f; r[13] = a.te ? a.te[e] : 1.0f; r[14] = 0.0f; r[15] = 0.0f;
+    }
+    for (int i = 0; i < P.n_sim; ++i) {
+        plant_tick(P, s, aDD, pDD);
+        plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
+    }
+    float *so = a.s + (size_t)e * 8;
+#pragma unroll
+    for (int c = 0; c < 6; ++c) so[c] = s[c];
+}
+
 // (Re)start of the observation chain: ring = the reference's initial buffer (zeros, cos = 1, latency_adder.py:26-28), nothing
 // pushed yet; the first solve sees the TRUE state, as the controller call of set_cartpole_state_at_t0 does
 // (CartPole/__init__.py:869-880: self.s, no noise, no latency).
@@ -306,6 +346,12 @@ struct FleetState {
     long long period;
     CostParams cost_up, cost_dn;
     PlantModels pm;            // plant-side models (cps_fleet_set_plant_models); pm.pushed counts the ring pushes
+    // neural fleets (CPS_PREDICTOR_NEURAL): the controller runs net_kernel / net_tc_kernel<.., FLEET>
+    int neural;
+    int htot;                  // hidden-state floats per experiment of the network the fleet was created for
+    float *d_h;                // [E][htot] each experiment's hidden state
+    float *d_noise;            // Philox: [E][n_ind][K] the period's draws (fleet_noise_kernel), read like supplied ones
+    size_t part_cap;           // floats allocated at d_partials
 };
 
 void cps_fleet_free(cps_handle *h) {
@@ -313,6 +359,7 @@ void cps_fleet_free(cps_handle *h) {
     if (!F) return;
     cudaFree(F->d_s); cudaFree(F->d_unom); cudaFree(F->d_uprev); cudaFree(F->d_partials); cudaFree(F->d_tickets);
     cudaFree(F->pm.obs); cudaFree(F->pm.ring);
+    cudaFree(F->d_h); cudaFree(F->d_noise);
     delete F;
     h->fleet = nullptr;
 }
@@ -338,6 +385,41 @@ static fleet_fn pick_fleet(int integ, int cost, bool philox, bool pair, bool n10
     return integ == CPS_EULER_V0 ? pick_fleet1<0>(cost, philox, pair, n10) : pick_fleet1<1>(cost, philox, pair, n10);
 }
 
+// A fleet whose controller predicts with the loaded network: per experiment a hidden state next to the ODE fleet's state,
+// warm start and last control; partials and tickets for the network kernel's tiling; a draw workspace for Philox.
+static int fleet_create_neural(cps_handle *h, const cps_fleet_config *cfg) {
+    NetFleetPlan p;
+    int rc = cps_net_mppi_fleet_plan(h, cfg->n_experiments, "cps_fleet_create", &p);
+    if (rc != CPS_OK) return rc;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    cps_fleet_free(h);
+    FleetState *F = new (std::nothrow) FleetState();
+    if (!F) return fail(h, CPS_ERR_INVALID, "cps_fleet_create: out of host memory");
+    memset(F, 0, sizeof(*F));
+    F->cfg = *cfg;
+    F->E = cfg->n_experiments;
+    F->neural = 1;
+    F->htot = cps_net_state_size(h);
+    F->bpe = p.tiles;
+    h->fleet = F;
+    const size_t E = F->E, K = h->cfg.num_rollouts, T = h->cfg.horizon, hn = F->htot > 0 ? F->htot : 1;
+    F->part_cap = E * p.tiles * (h->n_red + 2);
+    CUDA_TRY(h, cudaMalloc(&F->d_s, sizeof(float) * E * 8));
+    CUDA_TRY(h, cudaMalloc(&F->d_unom, sizeof(float) * E * T));
+    CUDA_TRY(h, cudaMalloc(&F->d_uprev, sizeof(float) * E));
+    CUDA_TRY(h, cudaMalloc(&F->d_partials, sizeof(float) * F->part_cap));
+    CUDA_TRY(h, cudaMalloc(&F->d_tickets, sizeof(unsigned) * E));
+    CUDA_TRY(h, cudaMalloc(&F->d_h, sizeof(float) * E * hn));
+    if (cfg->noise_source == CPS_FLEET_NOISE_PHILOX) CUDA_TRY(h, cudaMalloc(&F->d_noise, sizeof(float) * E * h->n_ind * K));
+    CUDA_TRY(h, cudaMemset(F->d_s, 0, sizeof(float) * E * 8));
+    CUDA_TRY(h, cudaMemset(F->d_unom, 0, sizeof(float) * E * T));
+    CUDA_TRY(h, cudaMemset(F->d_uprev, 0, sizeof(float) * E));
+    CUDA_TRY(h, cudaMemset(F->d_tickets, 0, sizeof(unsigned) * E));
+    CUDA_TRY(h, cudaMemset(F->d_h, 0, sizeof(float) * E * hn));
+    CUDA_TRY(h, cudaDeviceSynchronize());
+    return CPS_OK;
+}
+
 extern "C" int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg) {
     if (!h) return CPS_ERR_INVALID;
     if (!cfg || cfg->struct_size != (int)sizeof(cps_fleet_config))
@@ -346,12 +428,11 @@ extern "C" int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg) {
         return fail(h, CPS_ERR_INVALID, "cps_fleet_create: need n_experiments >= 1, sim_substeps >= 1, dt_simulation > 0");
     if (cfg->noise_source != CPS_FLEET_NOISE_SUPPLIED && cfg->noise_source != CPS_FLEET_NOISE_PHILOX)
         return fail(h, CPS_ERR_INVALID, "cps_fleet_create: unknown noise source %d", cfg->noise_source);
-    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_create: fleets run with the ODE predictors only");
     if (h->cfg.cost_id == CPS_COST_NONE) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_create: the handle has no cost function");
     if (h->cfg.noise_mode != CPS_NOISE_INDUCING)
         return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_create: fleets use inducing-point noise (CPS_NOISE_INDUCING)");
     if (cfg->n_experiments > 65535) return fail(h, CPS_ERR_INVALID, "cps_fleet_create: at most 65535 experiments per handle");
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) return fleet_create_neural(h, cfg);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     cps_fleet_free(h);
     FleetState *F = new (std::nothrow) FleetState();
@@ -406,6 +487,17 @@ extern "C" int cps_fleet_set_states(cps_handle *h, const float *s_host, long lon
     delete[] tmp;
     CUDA_TRY(h, er);
     F->period = period;
+    if (F->neural && F->htot > 0) {   // every experiment starts from the handle's stored state (what a fresh predictor holds)
+        std::vector<float> h0((size_t)F->htot), all((size_t)F->E * F->htot);
+        if (F->htot != cps_net_state_size(h))
+            return fail(h, CPS_ERR_INVALID, "cps_fleet_set_states: the loaded network's hidden state differs from the fleet's; "
+                        "recreate the fleet (cps_fleet_create)");
+        int rc = cps_net_get_state(h, h0.data());
+        if (rc != CPS_OK) return rc;
+        for (int e = 0; e < F->E; ++e) memcpy(&all[(size_t)e * F->htot], h0.data(), sizeof(float) * F->htot);
+        CUDA_TRY(h, cudaMemcpyAsync(F->d_h, all.data(), sizeof(float) * all.size(), cudaMemcpyHostToDevice, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    }
     if (F->pm.on) {   // ring = the reference's initial buffer; the first solve sees the true state
         F->pm.pushed = 0;
         fleet_observe_reset_kernel<<<(F->E + 127) / 128, 128, 0, h->stream>>>(F->pm, F->d_s, F->E);
@@ -419,6 +511,8 @@ extern "C" int cps_fleet_set_plant_models(cps_handle *h, const cps_fleet_plant_m
     if (!h) return CPS_ERR_INVALID;
     FleetState *F = h->fleet;
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_set_plant_models: no fleet (cps_fleet_create)");
+    if (F->neural) return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_set_plant_models: plant-side models are not offered on fleets "
+                               "with the neural predictor");
     if (!m || m->struct_size != (int)sizeof(cps_fleet_plant_models))
         return fail(h, CPS_ERR_INVALID, "cps_fleet_set_plant_models: cps_fleet_plant_models size mismatch");
     if (m->control_noise_mode < 0 || m->control_noise_mode > 2) return fail(h, CPS_ERR_INVALID, "cps_fleet_set_plant_models: control_noise_mode must be 0 (OFF), 1 (additive) or 2 (truncnorm)");
@@ -500,6 +594,28 @@ extern "C" int cps_fleet_get_states(cps_handle *h, float *s_host, float *u_nom_h
     return CPS_OK;
 }
 
+// [E][htot] hidden states of a neural fleet, host <-> device; synchronises
+static int fleet_net_states_io(cps_handle *h, float *host, bool get, const char *who) {
+    if (!h) return CPS_ERR_INVALID;
+    FleetState *F = h->fleet;
+    if (!F || !F->neural) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no fleet with the neural predictor (cps_fleet_create)", who);
+    if (!host) return fail(h, CPS_ERR_INVALID, "%s: null pointer", who);
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    const size_t bytes = sizeof(float) * (size_t)F->E * F->htot;
+    if (bytes) {
+        CUDA_TRY(h, get ? cudaMemcpyAsync(host, F->d_h, bytes, cudaMemcpyDeviceToHost, h->stream)
+                        : cudaMemcpyAsync(F->d_h, host, bytes, cudaMemcpyHostToDevice, h->stream));
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    }
+    return CPS_OK;
+}
+extern "C" int cps_fleet_get_net_states(cps_handle *h, float *out_host) {
+    return fleet_net_states_io(h, out_host, true, "cps_fleet_get_net_states");
+}
+extern "C" int cps_fleet_set_net_states(cps_handle *h, const float *in_host) {
+    return fleet_net_states_io(h, const_cast<float *>(in_host), false, "cps_fleet_set_net_states");
+}
+
 extern "C" long long cps_fleet_period(const cps_handle *h) { return (h && h->fleet) ? h->fleet->period : -1; }
 
 // CostParams for a given target equilibrium: fold_cost() depends on it for quadratic_boundary_grad (weight set, w[9]).
@@ -575,15 +691,80 @@ static int fleet_launch(cps_handle *h, const char *who, int n_periods, const flo
     return CPS_OK;
 }
 
+// cps_fleet_step on a neural fleet: per period [Philox draws ->] the network solve of all experiments -> the plant
+static int fleet_step_neural(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *noise_dev,
+                             float *record_dev, float *J_out_dev) {
+    const char *who = "cps_fleet_step";
+    FleetState *F = h->fleet;
+    if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "%s: negative number of periods", who);
+    const bool philox = F->cfg.noise_source == CPS_FLEET_NOISE_PHILOX;
+    if (!philox && !noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied noise", who);
+    if (philox && noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its noise (Philox); pass NULL", who);
+    NetFleetPlan p;
+    int rc = cps_net_mppi_fleet_plan(h, F->E, who, &p);
+    if (rc != CPS_OK) return rc;
+    if (cps_net_state_size(h) != F->htot)
+        return fail(h, CPS_ERR_INVALID, "%s: the loaded network has %d hidden-state floats, the fleet was created for %d; "
+                    "recreate the fleet (cps_fleet_create)", who, cps_net_state_size(h), F->htot);
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    const size_t E = F->E, K = h->cfg.num_rollouts, need = E * p.tiles * (h->n_red + 2);
+    if (need > F->part_cap) {   // a different tiling than at create (CPS_TC_ROWS)
+        cudaFree(F->d_partials);
+        F->d_partials = nullptr;
+        F->part_cap = 0;
+        CUDA_TRY(h, cudaMalloc(&F->d_partials, sizeof(float) * need));
+        F->part_cap = need;
+    }
+    F->bpe = p.tiles;
+    CostParams cost_up, cost_dn;
+    if ((rc = cps_fold_cost_for(h, 1.0f, &cost_up)) != CPS_OK) return rc;
+    if ((rc = cps_fold_cost_for(h, -1.0f, &cost_dn)) != CPS_OK) return rc;
+    NetPlantArgs pa;
+    PlantParams &P = pa.plant;
+    P.k = h->phys[CPS_PH_K]; P.m_cart = h->phys[CPS_PH_M_CART]; P.g = h->phys[CPS_PH_G]; P.J_fric = h->phys[CPS_PH_J_FRIC];
+    P.M_fric = h->phys[CPS_PH_M_FRIC]; P.u_max = h->phys[CPS_PH_U_MAX]; P.thl = h->phys[CPS_PH_TRACK_HALF_LENGTH];
+    P.L = (double)h->phys[CPS_PH_L]; P.m_pole = (double)h->phys[CPS_PH_M_POLE];
+    P.dt = F->cfg.dt_simulation; P.n_sim = F->cfg.sim_substeps;
+    pa.s = F->d_s; pa.u = F->d_uprev; pa.E = F->E;
+    const double dt_control = F->cfg.dt_simulation * F->cfg.sim_substeps;
+    for (int j = 0; j < n_periods; ++j) {
+        const float *tp = tp_dev ? tp_dev + (size_t)j * E : nullptr, *te = te_dev ? te_dev + (size_t)j * E : nullptr;
+        const float *noise = noise_dev ? noise_dev + (size_t)j * E * h->n_ind * K : F->d_noise;
+        if (philox) {   // the draws cps_fleet_noise returns for this period
+            fleet_noise_kernel<<<dim3((unsigned)(K + 255) / 256, F->E), 256, 0, h->stream>>>(
+                F->cfg.seed, (unsigned)F->period, (unsigned)F->cfg.experiment_offset, F->E, (int)K, h->n_ind, F->d_noise);
+            h->launches += 1;
+        }
+        if ((rc = cps_net_mppi_fleet(h, F->E, p, F->d_s, F->d_unom, F->d_uprev, F->d_h, tp, te, cost_up, cost_dn, noise,
+                                     F->d_partials, F->d_tickets, J_out_dev ? J_out_dev + (size_t)j * E * K : nullptr)) != CPS_OK)
+            return rc;
+        pa.tp = tp; pa.te = te;
+        pa.record = record_dev ? record_dev + (size_t)j * E * CPS_FLEET_RECORD : nullptr;
+        pa.time = (double)F->period * dt_control;
+        fleet_net_plant_kernel<<<(F->E + 127) / 128, 128, 0, h->stream>>>(pa);
+        h->launches += 1;
+        F->period += 1;
+    }
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
+}
+
 extern "C" int cps_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *noise_dev,
                               float *record_dev, float *J_out_dev) {
     if (!h) return CPS_ERR_INVALID;
+    if (h->fleet && h->fleet->neural) return fleet_step_neural(h, n_periods, tp_dev, te_dev, noise_dev, record_dev, J_out_dev);
     return fleet_launch(h, "cps_fleet_step", n_periods, tp_dev, te_dev, noise_dev, record_dev, J_out_dev, nullptr, nullptr, nullptr, nullptr);
+}
+
+static int fleet_reject_neural(cps_handle *h, const char *who) {
+    return fail(h, CPS_ERR_UNSUPPORTED, "%s: not offered on fleets with the neural predictor (no plant-side models, no "
+                "relabelling with a network)", who);
 }
 
 extern "C" int cps_fleet_step_noisy(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *noise_dev,
                                     float *record_dev, float *J_out_dev, const float *ctrl_draws_dev, const float *meas_draws_dev) {
     if (!h) return CPS_ERR_INVALID;
+    if (h->fleet && h->fleet->neural) return fleet_reject_neural(h, "cps_fleet_step_noisy");
     if (!h->fleet || !h->fleet->pm.on)
         return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_step_noisy: no plant-side models (cps_fleet_set_plant_models)");
     return fleet_launch(h, "cps_fleet_step_noisy", n_periods, tp_dev, te_dev, noise_dev, record_dev, J_out_dev, nullptr, nullptr, nullptr,
@@ -594,6 +775,7 @@ extern "C" int cps_fleet_relabel(cps_handle *h, int n_rows, const float *states_
                                  const float *L_dev, const float *m_pole_dev, const float *noise_dev, float *Q_out_dev,
                                  float *J_out_dev) {
     if (!h) return CPS_ERR_INVALID;
+    if (h->fleet && h->fleet->neural) return fleet_reject_neural(h, "cps_fleet_relabel");
     if (!states_dev || !Q_out_dev) return fail(h, CPS_ERR_INVALID, "cps_fleet_relabel: null pointer");
     return fleet_launch(h, "cps_fleet_relabel", n_rows, tp_dev, te_dev, noise_dev, nullptr, J_out_dev, states_dev, L_dev, m_pole_dev, Q_out_dev);
 }
@@ -602,6 +784,7 @@ extern "C" int cps_fleet_relabel_masked(cps_handle *h, int n_rows, const float *
                                         const float *L_dev, const float *m_pole_dev, const float *noise_dev, float *Q_out_dev,
                                         float *J_out_dev, const int *active_dev) {
     if (!h) return CPS_ERR_INVALID;
+    if (h->fleet && h->fleet->neural) return fleet_reject_neural(h, "cps_fleet_relabel_masked");
     if (!states_dev || !Q_out_dev) return fail(h, CPS_ERR_INVALID, "cps_fleet_relabel_masked: null pointer");
     return fleet_launch(h, "cps_fleet_relabel_masked", n_rows, tp_dev, te_dev, noise_dev, nullptr, J_out_dev, states_dev, L_dev,
                         m_pole_dev, Q_out_dev, active_dev);

@@ -170,6 +170,16 @@ int cps_net_grad_fleet(cps_handle *h, int E, const float *s_dev, const float *Q_
 int cps_net_mppi_step(cps_handle *h, const float *s_dev, const float *noise_dev, int noise_layout, float u_prev,
                       float *u_nom_dev, float *u_out_dev, float *J_out_dev, float *traj_out_dev, int traj_layout,
                       float *u_run_out_dev);
+// the MPPI fleet with CPS_PREDICTOR_NEURAL: cps_net_mppi_fleet_plan runs the network checks of cps_mppi_step and picks the
+// kernel (kernel 1 net_kernel, 2 net_tc_kernel), its rollouts per CTA, CTAs per experiment and shared memory;
+// cps_net_mppi_fleet is one launch of that kernel over E experiments x K rollouts, per experiment the arithmetic of
+// cps_mppi_step: states [E][8], warm starts [E][T], u_prev [E] (<- u), hidden states [E][htot] (advanced on (u, s)),
+// draws [E][n_ind][K], partials [E][tiles][2 + n_red], tickets [E], J_out [E][K] or null
+struct NetFleetPlan { int kernel, rows, tiles; size_t smem; };
+int cps_net_mppi_fleet_plan(cps_handle *h, int E, const char *who, NetFleetPlan *p);
+int cps_net_mppi_fleet(cps_handle *h, int E, const NetFleetPlan &p, const float *s_dev, float *u_nom_dev, float *u_prev_dev,
+                       float *hid_dev, const float *tp_dev, const float *te_dev, const CostParams &cost_up, const CostParams &cost_dn,
+                       const float *noise_dev, float *partials_dev, unsigned *tickets_dev, float *J_out_dev);
 
 static inline int fail(cps_handle *h, int code, const char *fmt, ...) {
     char buf[512];

@@ -29,8 +29,9 @@
 
 #include "cps_net_fp32.cuh"
 
-template <int R, int HT, bool MPPI>
-__global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constant__ NetArgs a) {
+template <int R, int HT, bool MPPI, bool FLEET>
+__global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constant__ NetArgs a,
+                                                            const __grid_constant__ NetFleetMppiExt fx) {
     constexpr int NC = R * 8, NT = NC + 32;
     extern __shared__ __align__(16) float smem[];
     __shared__ __align__(8) unsigned long long s_bar;
@@ -43,6 +44,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
     // differential networks: autoregression_loop.run takes the integrating helper only in its general loop; with
     // horizon == 1 the "0th iteration" branch hands out the raw network output (autoregression.py:49-70)
     const bool diff = N.differential && T > 1;
+    const int e = FLEET ? (int)blockIdx.y : 0;   // FLEET: the CTA's experiment
 
     // ---- shared-memory carve-up ------------------------------------------------------------------------------
     float *wsm = smem;                              // [n_weights]
@@ -55,6 +57,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
     float *s_w1 = s_w0 + (MPPI ? a.mp.p : 0);
     float *s_red = s_w1 + (MPPI ? a.mp.p : 0);      // [n_red + 2 + 16]
     float *s_rs = s_red + (MPPI ? a.mp.n_red + 2 + 16 : 0);   // MAX_COST plugins: row-sum slots [32][R] (RowSumPlan)
+    CostParams *s_cost = reinterpret_cast<CostParams *>(s_rs + 32 * R);   // FLEET: the experiment's cost parameters
 
     // ---- weights: one bulk asynchronous copy global -> shared ---------------------------------------------------
     if (tid == 0) weights_copy_start(&s_bar, wsm, a.weights, N.n_weights);
@@ -64,16 +67,17 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
         for (int idx = tid; idx < N.htot * R; idx += NT) {
             const int j = idx / R, r = idx % R;
             const int b = min(row0 + r, a.B - 1);
-            hb[idx] = a.h0[(long long)b * a.hs_b + j];
+            hb[idx] = FLEET ? fx.h[(long long)e * N.htot + j] : a.h0[(long long)b * a.hs_b + j];
         }
     }
     if (MPPI) {
         // warm-start shift at the START of the solve (optimizer_mppi.py:183)
-        for (int t = tid; t < T; t += NT) s_unom[t] = a.u_nom[min(t + 1, T - 1)];
+        for (int t = tid; t < T; t += NT) s_unom[t] = (FLEET ? fx.u_nom + (long long)e * T : a.u_nom)[min(t + 1, T - 1)];
         for (int j = tid; j < a.mp.p; j += NT) {
             s_w0[j] = (float)(a.mp.p - j) / (float)a.mp.p;
             s_w1[j] = (float)j / (float)a.mp.p;
         }
+        if (FLEET && tid == 0) fleet_cost_stage(fx, e, s_cost);
     }
     __syncthreads();  // also publishes the mbarrier init
 
@@ -83,7 +87,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
     const int k = row0 + r_row;
     const bool active = row_lead && k < a.B;
     const int kc = min(k, a.B - 1);
-    float Jacc = 0.0f, corr = 0.0f, up = a.u_prev, u_cur = 0.0f, du_cur = 0.0f, u_nxt = 0.0f, du_nxt = 0.0f;
+    float Jacc = 0.0f, corr = 0.0f, up = FLEET ? fx.u_prev[e] : a.u_prev, u_cur = 0.0f, du_cur = 0.0f, u_nxt = 0.0f, du_nxt = 0.0f;
     // default / quadratic_boundary: the T+1 cost entries are summed in the reference backend's order (cps_device.cuh)
     const bool rowsum = MPPI && (a.cost_id == CPS_COST_DEFAULT || a.cost_id == CPS_COST_QUADRATIC_BOUNDARY);
     const RowSumPlan rsp = row_sum_plan(T + 1);
@@ -98,7 +102,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
     if (row_warp) {
         traj = (a.traj_out && active) ? a.traj_out + (long long)k * a.ts_k : nullptr;
         if (MPPI) {
-            nz = a.noise + (long long)kc * a.ns_k;
+            nz = (FLEET ? a.noise + (long long)e * a.mp.n_ind * a.B : a.noise) + (long long)kc * a.ns_k;
             na = nz[0] * a.mp.sigma;
             nb = (a.mp.n_ind > 1) ? nz[a.ns_i] * a.mp.sigma : 0.0f;
         } else {
@@ -135,13 +139,13 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
             // (1) this step's network input: control + state features (the initial state, or the previous output)
             if (t == 0) {
 #pragma unroll
-                for (int c = 0; c < 6; ++c) st[c] = a.s0[(long long)kc * a.ss_b + c];
+                for (int c = 0; c < 6; ++c) st[c] = (FLEET ? fx.s + (long long)e * 8 : a.s0)[(long long)kc * a.ss_b + c];
                 if (row_lead) {
                     for (int i = 0; i < N.n_state_in; ++i)
-                        xin[(1 + i) * R + r_row] = fmaf(N.norm_a[1 + i], a.s0[(long long)kc * a.ss_b + N.in_idx[i]], N.norm_b[1 + i]);
+                        xin[(1 + i) * R + r_row] = fmaf(N.norm_a[1 + i], (FLEET ? fx.s + (long long)e * 8 : a.s0)[(long long)kc * a.ss_b + N.in_idx[i]], N.norm_b[1 + i]);
                     if (diff)  // dmah.set_starting_point (autoregression.py:145-146)
                         for (int o = 0; o < N.n_out; ++o)
-                            snorm[o * R + r_row] = fmaf(N.on_a[o], a.s0[(long long)kc * a.ss_b + N.out_idx[o]], N.on_b[o]);
+                            snorm[o * R + r_row] = fmaf(N.on_a[o], (FLEET ? fx.s + (long long)e * 8 : a.s0)[(long long)kc * a.ss_b + N.out_idx[o]], N.on_b[o]);
                 }
             } else {
                 out_layer_row<R>(N, wsm, hlast_base + (N.type == CPS_NET_GRU ? p * hstride : 0), lane, y);
@@ -172,7 +176,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
                 for (int c = 0; c < 6; ++c) traj[(long long)t * a.ts_t + c * a.ts_c] = st[c];
             }
             if (MPPI) {
-                const float stc = stage_cost_rt(a.cost_id, a.cost, cosf(st[IDX_ANGLE]), st[IDX_ANGLED], st[IDX_POS], u_cur, up);
+                const float stc = stage_cost_rt(a.cost_id, FLEET ? *s_cost : a.cost, cosf(st[IDX_ANGLE]), st[IDX_ANGLED], st[IDX_POS], u_cur, up);
                 if (rowsum) { if (row_lead) row_sum_push(rsp, sl, R, rs_tail, t, stc); }
                 else Jacc += stc;
                 corr = fmaf(a.mp.cc_half_nu * du_cur, du_cur,
@@ -205,13 +209,13 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
         if (MPPI) {
             if (rowsum) {
                 if (row_lead) {
-                    row_sum_push(rsp, sl, R, rs_tail, T, terminal_cost<COST_DEFAULT>(a.cost, st[IDX_ANGLE], st[IDX_POS]));
+                    row_sum_push(rsp, sl, R, rs_tail, T, terminal_cost<COST_DEFAULT>(FLEET ? *s_cost : a.cost, st[IDX_ANGLE], st[IDX_POS]));
                     Jacc = row_sum_finish(rsp, sl, R, rs_tail);
                 }
             }
             J = __fdiv_rn(Jacc, a.mp.T1) + corr;   // mean over T+1 entries (true division, as torch.mean) + correction
             if (active) {
-                if (a.J_out) a.J_out[k] = J;
+                if (a.J_out) (FLEET ? a.J_out + (long long)e * a.B : a.J_out)[k] = J;
                 if (!isfinite(J)) atomicAdd(a.nonfinite, 1);
             }
         }
@@ -230,7 +234,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
     if (row_warp) {
         const float m = warp_min(active ? J : INFINITY);
         const float wgt = active ? expf(-(J - m) * mp.inv_lambda) : 0.0f;
-        float *part = a.partials + (size_t)blockIdx.x * rec;
+        float *part = (FLEET ? a.partials + (size_t)e * gridDim.x * rec : a.partials) + (size_t)blockIdx.x * rec;
         const float S = warp_sum(wgt);
         if (lane == 0) { part[0] = m; part[1] = S; }
         for (int i = 0; i < mp.n_red; ++i) {
@@ -241,21 +245,24 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
     }
     __threadfence();
     __syncthreads();
-    if (tid == 0) s_ticket = atomicAdd(a.ticket, 1u);
+    if (tid == 0) s_ticket = atomicAdd(FLEET ? fx.tickets + e : a.ticket, 1u);
     __syncthreads();
     if (s_ticket != gridDim.x - 1) return;
     __threadfence();
-    merge_and_finish(mp, a.partials, gridDim.x, s_red, s_unom, a.u_nom, a.u_out, a.shard_out, false, &a.px);
-    if (tid == 0) *a.ticket = 0u;
-    if (a.shard_out || !a.h_ref || N.type != CPS_NET_GRU) return;
+    // FLEET: the experiment's tiles, warm start and last control
+    merge_and_finish(mp, FLEET ? a.partials + (size_t)e * gridDim.x * rec : a.partials, gridDim.x, s_red, s_unom,
+                     FLEET ? fx.u_nom + (long long)e * T : a.u_nom, FLEET ? fx.u_prev + e : a.u_out, a.shard_out, false, &a.px);
+    if (tid == 0) *(FLEET ? fx.tickets + e : a.ticket) = 0u;
+    if (a.shard_out || !(FLEET ? fx.h : a.h_ref) || N.type != CPS_NET_GRU) return;
 
     // ---- advance the stored hidden state by one step on (u, s) (optimizer_mppi.py:191,194-196) --------------------
     __syncthreads();
-    const float u_sel = __ldcg(a.u_out);
-    for (int idx = tid; idx < N.htot * R; idx += NT) hb[idx] = a.h_ref[idx / R];
+    float *const h_ref = FLEET ? fx.h + (long long)e * N.htot : a.h_ref;
+    const float u_sel = __ldcg(FLEET ? fx.u_prev + e : a.u_out);
+    for (int idx = tid; idx < N.htot * R; idx += NT) hb[idx] = h_ref[idx / R];
     for (int idx = tid; idx < N.n_in * R; idx += NT) {
         const int i = idx / R;
-        const float v = (i == 0) ? u_sel : a.s0[N.in_idx[i - 1]];
+        const float v = (i == 0) ? u_sel : (FLEET ? fx.s + (long long)e * 8 : a.s0)[N.in_idx[i - 1]];
         xin[idx] = fmaf(N.norm_a[i], v, N.norm_b[i]);
     }
     __syncthreads();
@@ -264,7 +271,7 @@ __global__ void __launch_bounds__(R * 8 + 32, 1) net_kernel(const __grid_constan
     } else {
         compute_step<R, HT>(N, wsm, hb, hstride, 0, xin, tid);
     }
-    for (int j = tid; j < N.htot; j += NT) a.h_ref[j] = hb[hstride + j * R];
+    for (int j = tid; j < N.htot; j += NT) h_ref[j] = hb[hstride + j * R];
 }
 
 // =====================================================================================================
@@ -277,14 +284,14 @@ static size_t net_smem_bytes(const NetDev &N, int R, bool mppi, const MppiParams
     return f * sizeof(float);
 }
 
-typedef void (*net_fn)(const NetArgs);
+typedef void (*net_fn)(const NetArgs, const NetFleetMppiExt);
 
-template <int R, bool MPPI>
+template <int R, bool MPPI, bool FLEET = false>
 static net_fn pick_net2(int ht) {
     switch (ht) {
-    case 64: return net_kernel<R, 64, MPPI>;
-    case 32: return net_kernel<R, 32, MPPI>;
-    default: return net_kernel<R, 0, MPPI>;
+    case 64: return net_kernel<R, 64, MPPI, FLEET>;
+    case 32: return net_kernel<R, 32, MPPI, FLEET>;
+    default: return net_kernel<R, 0, MPPI, FLEET>;
     }
 }
 static net_fn pick_net(int R, int ht, bool mppi) {
@@ -297,6 +304,8 @@ bool cps_net_tc_eligible(const NetDev &N);
 void cps_net_tc_build_image(const NetDev &N, const float *w, std::vector<unsigned char> &img);
 int cps_net_tc_launch(cps_handle *h, NetArgs &a, bool mppi, int n_rows);
 size_t cps_net_tc_smem(const MppiParams *mp, bool mppi);
+int cps_net_tc_rows(cps_handle *h, long long n_rows);
+int cps_net_tc_fleet_launch(cps_handle *h, NetArgs &a, const NetFleetMppiExt &x, int E);
 
 void cps_net_free(cps_handle *h) {
     if (!h || !h->net) return;
@@ -440,7 +449,7 @@ static int net_launch(cps_handle *h, NetArgs &a, bool mppi, int n_rows) {
     net_fn fn = pick_net(R, S->ht, mppi);
     CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int grid = (n_rows + R - 1) / R;
-    fn<<<grid, R * 8 + 32, smem, h->stream>>>(a);
+    fn<<<grid, R * 8 + 32, smem, h->stream>>>(a, NetFleetMppiExt());
     h->launches += 1;
     h->net_last_kernel = 1;
     CUDA_TRY(h, cudaGetLastError());
@@ -543,4 +552,65 @@ int cps_net_mppi_step(cps_handle *h, const float *s_dev, const float *noise_dev,
     if (h->px.world > 1) a.px.epoch = ++h->px.epoch;
     a.h_ref = h->net->d_href;
     return net_launch(h, a, true, (int)K);
+}
+
+// ---- cps_fleet.cu: MPPI fleets on the neural predictor ----------------------------------------------------------------
+// The kernel an MPPI fleet of E experiments runs, chosen as net_launch chooses it for a single solve: the tensor-core kernel
+// for the GRUs it takes (live rollouts per CTA from the fleet's E x K rollouts by cps_net_tc_launch's rule), else the FP32
+// kernel with R from the per-experiment K, so that every experiment runs the arithmetic of one cps_mppi_step.  Both stage
+// the experiment's cost parameters in shared memory behind the single solve's carve-up.
+int cps_net_mppi_fleet_plan(cps_handle *h, int E, const char *who, NetFleetPlan *p) {
+    if (!h->net) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: neural predictor without a network (cps_net_load)", who);
+    if (h->cfg.noise_mode != CPS_NOISE_INDUCING)
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: the neural predictor supports CPS_NOISE_INDUCING only", who);
+    if ((h->cfg.cost_id == CPS_COST_DEFAULT || h->cfg.cost_id == CPS_COST_QUADRATIC_BOUNDARY) && row_sum_slots(h->cfg.horizon + 1) > 32)
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: default / quadratic_boundary with the neural predictor support horizons below 511", who);
+    NetState *S = h->net;
+    const unsigned fl = h->cfg.flags;
+    const int K = h->cfg.num_rollouts;
+    if ((fl & CPS_FLAG_NET_TENSOR_CORES) && !S->d_tc)
+        return fail(h, CPS_ERR_UNSUPPORTED, "CPS_FLAG_NET_TENSOR_CORES: the tensor-core kernel supports plain (not differential, D_*) 2 x 64 GRU networks only");
+    const size_t tc_smem = cps_net_tc_smem(&h->mp, true) + sizeof(CostParams);
+    if (S->d_tc && !(fl & CPS_FLAG_NET_FP32) && ((fl & CPS_FLAG_NET_TENSOR_CORES) || tc_smem <= 227 * 1024)) {
+        if (tc_smem > 227 * 1024) return fail(h, CPS_ERR_UNSUPPORTED, "%s: horizon too large for the tensor-core kernel's shared memory", who);
+        p->kernel = 2;
+        p->rows = cps_net_tc_rows(h, (long long)E * K);
+        p->smem = tc_smem;
+    } else {
+        int R = (K > 148 * 16) ? 32 : 16;
+        if (net_smem_bytes(S->dev, R, true, &h->mp) > 227 * 1024) R = 16;
+        p->kernel = 1;
+        p->rows = R;
+        p->smem = net_smem_bytes(S->dev, R, true, &h->mp) + sizeof(CostParams);
+        if (p->smem > 227 * 1024)
+            return fail(h, CPS_ERR_UNSUPPORTED, "%s: the network needs %zu bytes of shared memory per CTA here (limit 227 KB)", who, p->smem);
+    }
+    p->tiles = (K + p->rows - 1) / p->rows;
+    return CPS_OK;
+}
+
+int cps_net_mppi_fleet(cps_handle *h, int E, const NetFleetPlan &p, const float *s_dev, float *u_nom_dev, float *u_prev_dev,
+                       float *hid_dev, const float *tp_dev, const float *te_dev, const CostParams &cost_up, const CostParams &cost_dn,
+                       const float *noise_dev, float *partials_dev, unsigned *tickets_dev, float *J_out_dev) {
+    NetState *S = h->net;
+    const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
+    NetArgs a;
+    memset(&a, 0, sizeof(a));
+    a.net = S->dev; a.weights = S->d_weights; a.tc = S->d_tc;
+    a.B = K; a.T = T;
+    a.cost_id = h->cfg.cost_id; a.cost = h->cost; a.mp = h->mp;
+    a.noise = noise_dev; a.ns_i = K; a.ns_k = 1;
+    a.J_out = J_out_dev; a.partials = partials_dev; a.nonfinite = h->d_nonfinite;
+    a.tc_rows = p.rows;
+    NetFleetMppiExt x;
+    x.s = s_dev; x.u_nom = u_nom_dev; x.u_prev = u_prev_dev; x.h = hid_dev; x.tp = tp_dev; x.te = te_dev;
+    x.cost_up = cost_up; x.cost_dn = cost_dn; x.tickets = tickets_dev;
+    if (p.kernel == 2) return cps_net_tc_fleet_launch(h, a, x, E);
+    net_fn fn = (p.rows == 32) ? pick_net2<32, true, true>(S->ht) : pick_net2<16, true, true>(S->ht);
+    CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
+    fn<<<dim3(p.tiles, E), p.rows * 8 + 32, p.smem, h->stream>>>(a, x);
+    h->launches += 1;
+    h->net_last_kernel = 1;
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
 }

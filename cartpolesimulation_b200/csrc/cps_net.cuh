@@ -62,6 +62,30 @@ struct NetArgs {
     int tc_rows;              // net_tc_kernel: live rollouts per CTA (32 | 64: the first 8 | 16 lanes of each tensor-memory lane quarter | 128)
 };
 
+// The MPPI fleet's per-experiment inputs (net_kernel / net_tc_kernel with FLEET = true; unused otherwise).  Grid
+// (tiles, E): CTA (x, e = blockIdx.y) holds rollouts of experiment e only, and the experiment's gridDim.x tiles merge as the
+// tiles of one cps_mppi_step do.  With FLEET, NetArgs' B is the rollouts per experiment K, noise the draws [E][n_ind][K]
+// (ns_i = K, ns_k = 1), partials [E][gridDim.x][2 + n_red] and J_out [E][K] or null; s0, h0, u_nom, u_prev, u_out, cost,
+// ticket and h_ref are taken from here instead.
+struct NetFleetMppiExt {
+    const float *s;               // [E][8] states
+    float *u_nom;                 // [E][T] warm starts
+    float *u_prev;                // [E] last controls; the solve's u replaces them (optimizer_mppi.py:210)
+    float *h;                     // [E][htot] hidden states: the rollouts' h0, advanced on (u, s) by the experiment's last CTA
+    const float *tp, *te;         // [E] targets of this period (null: 0 / +1)
+    CostParams cost_up, cost_dn;  // folded for target_equilibrium = +1 / -1
+    unsigned *tickets;            // [E]
+};
+
+// The experiment's cost parameters, as fleet_kernel selects them; staged once per CTA in shared memory.
+__device__ __forceinline__ void fleet_cost_stage(const NetFleetMppiExt &fx, int e, CostParams *dst) {
+    const float tp = fx.tp ? fx.tp[e] : 0.0f, te = fx.te ? fx.te[e] : 1.0f;
+    CostParams c = (te == 1.0f) ? fx.cost_up : fx.cost_dn;
+    c.target_position = tp;
+    c.target_equilibrium = te;
+    *dst = c;
+}
+
 // ---- small device helpers ---------------------------------------------------------------------------------------
 __device__ __forceinline__ float sigmoid_f(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
 // 1 - 2/(1 + e^{2x}): absolute error ~1e-7, saturates correctly for large |x|

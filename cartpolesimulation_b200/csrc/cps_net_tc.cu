@@ -45,8 +45,11 @@ namespace {
 // NARROW: both layers have at most 32 units (the reference's shipped GRU-6IN-32H1-32H2-5OUT): the second half-layer jobs
 // (units 32..63) hold only padding -- their MMAs and epilogues are skipped, the hand-offs stay, so the pipeline's barrier
 // protocol is the same -- and the products over a hidden state take 2 k-steps instead of 4.
-template <bool MPPI, bool NARROW = false>
-__global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant__ NetArgs a) {
+//
+// FLEET (MPPI only): grid (tiles, E); CTA (x, e = blockIdx.y) solves for experiment e with the per-experiment inputs of fx
+// (cps_net.cuh NetFleetMppiExt), its cost parameters staged in shared memory behind the single solve's carve-up.
+template <bool MPPI, bool NARROW = false, bool FLEET = false>
+__global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant__ NetArgs a, const __grid_constant__ NetFleetMppiExt fx) {
     constexpr int NKH = NARROW ? 2 : 4;
     constexpr bool JB = !NARROW;
     extern __shared__ __align__(128) unsigned char smem[];
@@ -66,6 +69,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
     const int sub = (warp >> 2) & 3;           // epilogue warps: which 8 of a job's 32 units
     const int row = 32 * (warp & 3) + lane;    // rollout inside the tile (epilogue and row warps)
     const int T = a.T;
+    const int e = FLEET ? (int)blockIdx.y : 0;   // FLEET: the CTA's experiment
     // Small batches are latency-bound by the step's dependence chain, not by throughput: with only the first 16 (or 8) tensor-
     // memory lanes of every lane quarter live (64 / 32 rollouts per CTA) the epilogues take half the time (12 % less again), because the
     // 16-lane access shapes spread those rollouts over all 32 threads of the epilogue warps -- and all four schedulers stay
@@ -86,6 +90,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
     float *s_w1 = s_w0 + (MPPI ? a.mp.p : 0);
     float *s_red = s_w1 + (MPPI ? a.mp.p : 0);             // [4][n_red + 2] then [n_red + 2 + warps]
     float *s_rs = s_red + (MPPI ? 5 * (a.mp.n_red + 2) + 8 : 0);   // MAX_COST plugins: row-sum slots [32][128] (RowSumPlan)
+    CostParams *s_cost = reinterpret_cast<CostParams *>(s_rs + 32 * TC_ROWS);   // FLEET: the experiment's cost parameters
     const float *cst1 = reinterpret_cast<const float *>(smem + O_CST1);
     const float *cst2 = reinterpret_cast<const float *>(smem + O_CST2);
     const float *csto = reinterpret_cast<const float *>(smem + O_CSTO);   // [16][2] output layer, then {c, cn} of the two layers
@@ -117,11 +122,12 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
     }
     if (MPPI) {
-        for (int t = tid; t < T; t += TC_NT) s_unom[t] = a.u_nom[min(t + 1, T - 1)];   // warm-start shift (:183)
+        for (int t = tid; t < T; t += TC_NT) s_unom[t] = (FLEET ? fx.u_nom + (long long)e * T : a.u_nom)[min(t + 1, T - 1)];   // warm-start shift (:183)
         for (int j = tid; j < a.mp.p; j += TC_NT) {
             s_w0[j] = (float)(a.mp.p - j) / (float)a.mp.p;
             s_w1[j] = (float)j / (float)a.mp.p;
         }
+        if (FLEET && tid == 0) fleet_cost_stage(fx, e, s_cost);
     }
     for (int i = tid; i < 2048; i += TC_NT) reinterpret_cast<uint32_t *>(smem + O_X_HI)[i] = 0u;   // x tiles: k = 7..15 stay 0
     tc_fence_before();
@@ -131,7 +137,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
     const uint32_t tl = tmem + ((uint32_t)(32 * (warp & 3)) << 16);   // this warp's lane quarter
 
     // ---- row bookkeeping (row warps) ------------------------------------------------------------------------------------
-    float Jacc = 0.0f, corr = 0.0f, up = a.u_prev, u_cur = 0.0f, du_cur = 0.0f, u_nxt = 0.0f, du_nxt = 0.0f;
+    float Jacc = 0.0f, corr = 0.0f, up = FLEET ? fx.u_prev[e] : a.u_prev, u_cur = 0.0f, du_cur = 0.0f, u_nxt = 0.0f, du_nxt = 0.0f;
     int seg = 0, jj = 0;
     float na = 0.0f, nb = 0.0f;
     const float *nz = nullptr, *qrow = nullptr;
@@ -143,7 +149,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
     float rs_tail = 0.0f;
     if (is_row) {
         if (MPPI) {
-            nz = a.noise + (long long)kc * a.ns_k;
+            nz = (FLEET ? a.noise + (long long)e * a.mp.n_ind * a.B : a.noise) + (long long)kc * a.ns_k;
             na = nz[0] * a.mp.sigma;
             nb = (a.mp.n_ind > 1) ? nz[a.ns_i] * a.mp.sigma : 0.0f;
             if (rowsum) row_sum_init(rsp, sl, TC_ROWS);
@@ -207,7 +213,8 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
                 const int u0 = chunk_u0(ch);
 #pragma unroll
                 for (int i = 0; i < TC_EU; ++i)   // layers narrower than 64 units: the padding units carry (and keep) zero
-                    v[i] = (u0 + i < N.hsz[l]) ? a.h0[(long long)kc * a.hs_b + N.hoff[l] + u0 + i] : 0.0f;
+                    v[i] = (u0 + i < N.hsz[l]) ? (FLEET ? fx.h[(long long)e * N.htot + N.hoff[l] + u0 + i]
+                                                        : a.h0[(long long)kc * a.hs_b + N.hoff[l] + u0 + i]) : 0.0f;
                 if (stk) write_operand8_stacked(tl, (l ? C_AH2_HI : C_AH1_HI) + (u0 >> 1), v, lane);
                 else write_operand8(tl, (l ? C_AH2_HI : C_AH1_HI) + (u0 >> 1), (l ? C_AH2_LO : C_AH1_LO) + (u0 >> 1), v);
             }
@@ -215,11 +222,11 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
     }
     if (is_row) {
 #pragma unroll
-        for (int c = 0; c < 6; ++c) st[c] = a.s0[(long long)kc * a.ss_b + c];
+        for (int c = 0; c < 6; ++c) st[c] = (FLEET ? fx.s + (long long)e * 8 : a.s0)[(long long)kc * a.ss_b + c];
         next_control(0);
 #pragma unroll
         for (int i = 0; i < 6; ++i)
-            feat[i] = (i < N.n_state_in) ? fmaf(N.norm_a[1 + i], a.s0[(long long)kc * a.ss_b + N.in_idx[i]], N.norm_b[1 + i]) : 0.0f;
+            feat[i] = (i < N.n_state_in) ? fmaf(N.norm_a[1 + i], (FLEET ? fx.s + (long long)e * 8 : a.s0)[(long long)kc * a.ss_b + N.in_idx[i]], N.norm_b[1 + i]) : 0.0f;
         write_x(u_nxt, feat, stk);
     }
     bar_wait(wbar, 0);   // weights have landed
@@ -336,7 +343,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
                     for (int c = 0; c < 6; ++c) traj[(long long)t * a.ts_t + c * a.ts_c] = st[c];
                 }
                 if (MPPI) {
-                    const float stc = stage_cost_rt(a.cost_id, a.cost, cosf(st[IDX_ANGLE]), st[IDX_ANGLED], st[IDX_POS], u_cur, up);
+                    const float stc = stage_cost_rt(a.cost_id, FLEET ? *s_cost : a.cost, cosf(st[IDX_ANGLE]), st[IDX_ANGLED], st[IDX_POS], u_cur, up);
                     if (rowsum) row_sum_push(rsp, sl, TC_ROWS, rs_tail, t, stc);
                     else Jacc += stc;
                     corr = fmaf(a.mp.cc_half_nu * du_cur, du_cur,
@@ -396,7 +403,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
         }
         if (MPPI) {
             if (a.cost_id == CPS_COST_DEFAULT || a.cost_id == CPS_COST_QUADRATIC_BOUNDARY) {
-                const float term = terminal_cost<COST_DEFAULT>(a.cost, st[IDX_ANGLE], st[IDX_POS]);
+                const float term = terminal_cost<COST_DEFAULT>(FLEET ? *s_cost : a.cost, st[IDX_ANGLE], st[IDX_POS]);
                 if (rowsum) {
                     row_sum_push(rsp, sl, TC_ROWS, rs_tail, T, term);
                     Jacc = row_sum_finish(rsp, sl, TC_ROWS, rs_tail);
@@ -406,7 +413,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
             }
             J = __fdiv_rn(Jacc, a.mp.T1) + corr;   // mean over T+1 entries (true division, as torch.mean) + correction
             if (active) {
-                if (a.J_out) a.J_out[k] = J;
+                if (a.J_out) (FLEET ? a.J_out + (long long)e * a.B : a.J_out)[k] = J;
                 if (!isfinite(J)) atomicAdd(a.nonfinite, 1);
             }
         }
@@ -453,25 +460,28 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
             }
         }
         __syncthreads();
-        float *part = a.partials + (size_t)blockIdx.x * rec;
+        float *part = (FLEET ? a.partials + (size_t)e * gridDim.x * rec : a.partials) + (size_t)blockIdx.x * rec;
         for (int c = tid; c < mp.n_red + 1; c += TC_NT)
             part[1 + c] = (s_red[1 + c] + s_red[rec + 1 + c]) + (s_red[2 * rec + 1 + c] + s_red[3 * rec + 1 + c]);
         if (tid == 0) part[0] = m;
         __threadfence();
         __syncthreads();
-        if (tid == 0) s_ticket = atomicAdd(a.ticket, 1u);
+        if (tid == 0) s_ticket = atomicAdd(FLEET ? fx.tickets + e : a.ticket, 1u);
         __syncthreads();
         last = s_ticket == gridDim.x - 1;
         if (last) {
             __threadfence();
-            merge_and_finish(mp, a.partials, gridDim.x, s_red, s_unom, a.u_nom, a.u_out, a.shard_out, false, &a.px);
-            if (tid == 0) *a.ticket = 0u;
+            // FLEET: the experiment's tiles, warm start and last control
+            merge_and_finish(mp, FLEET ? a.partials + (size_t)e * gridDim.x * rec : a.partials, gridDim.x, s_red, s_unom,
+                             FLEET ? fx.u_nom + (long long)e * T : a.u_nom, FLEET ? fx.u_prev + e : a.u_out, a.shard_out, false, &a.px);
+            if (tid == 0) *(FLEET ? fx.tickets + e : a.ticket) = 0u;
         }
-        if (last && !a.shard_out && a.h_ref) {
+        if (last && !a.shard_out && (FLEET ? fx.h : a.h_ref)) {
             // ---- advance the stored hidden state by one step on (u, s) (optimizer_mppi.py:191,194-196): one more,
             //      unpipelined, network step with every rollout carrying the stored state --------------------------------
             __syncthreads();
-            const float u_sel = __ldcg(a.u_out);
+            float *const h_ref = FLEET ? fx.h + (long long)e * N.htot : a.h_ref;
+            const float u_sel = __ldcg(FLEET ? fx.u_prev + e : a.u_out);
             const bool upd = row < 32;   // the stored state is one row: the first lane quarter carries it
             if (is_epi && upd) {
                 float v[TC_EU];
@@ -481,7 +491,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
                     for (int ch = 0; ch < 2; ++ch) {
                         const int u0 = chunk_u0(ch);
 #pragma unroll
-                        for (int i = 0; i < TC_EU; ++i) v[i] = (u0 + i < N.hsz[l]) ? a.h_ref[N.hoff[l] + u0 + i] : 0.0f;
+                        for (int i = 0; i < TC_EU; ++i) v[i] = (u0 + i < N.hsz[l]) ? h_ref[N.hoff[l] + u0 + i] : 0.0f;
                         write_operand8(tl, (l ? C_AH2_HI : C_AH1_HI) + (u0 >> 1), (l ? C_AH2_LO : C_AH1_LO) + (u0 >> 1), v);
                     }
                 }
@@ -489,7 +499,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
             if (is_row && upd) {
 #pragma unroll
                 for (int i = 0; i < 6; ++i)
-                    feat[i] = (i < N.n_state_in) ? fmaf(N.norm_a[1 + i], a.s0[N.in_idx[i]], N.norm_b[1 + i]) : 0.0f;
+                    feat[i] = (i < N.n_state_in) ? fmaf(N.norm_a[1 + i], (FLEET ? fx.s + (long long)e * 8 : a.s0)[N.in_idx[i]], N.norm_b[1 + i]) : 0.0f;
                 write_x(u_sel, feat, false);
             }
             tc_sync();
@@ -521,7 +531,7 @@ __global__ void __launch_bounds__(TC_NT, 1) net_tc_kernel(const __grid_constant_
                 gru_epilogue<1, true>(tl, 256, (uint32_t)(TC_EU * sub), cst2, ec2, ecn2, C_AH2_HI, C_AH2_LO, chunk_u0(0), lane);
                 gru_epilogue<1, true>(tl, 0, (uint32_t)(TC_EU * sub), cst2, ec2, ecn2, C_AH2_HI, C_AH2_LO, chunk_u0(1), lane);
                 asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-                store_hidden(row == 0 ? a.h_ref : nullptr, false);
+                store_hidden(row == 0 ? h_ref : nullptr, false);
             }
         }
     }
@@ -637,22 +647,42 @@ void cps_net_tc_build_image(const NetDev &N, const float *w, std::vector<unsigne
 
 int cps_net_tc_image_bytes() { return (int)TC_IMAGE_BYTES; }
 
+// live rollouts per CTA for a launch of n_rows rollouts: 32 or 64 while that still gives every CTA its own SM (see the
+// kernel's comment on rpq)
+int cps_net_tc_rows(cps_handle *h, long long n_rows) {
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->cfg.device);
+    int rows = (n_rows <= 32LL * sms) ? 32 : (n_rows <= 64LL * sms) ? 64 : TC_ROWS;
+    if (const char *e = getenv("CPS_TC_ROWS")) {   // A/B switch (tools/bench_net.py)
+        const int r = atoi(e);
+        if (r == 32 || r == 64 || r == 128) rows = r;
+    }
+    return rows;
+}
+
 int cps_net_tc_launch(cps_handle *h, NetArgs &a, bool mppi, int n_rows) {
     const size_t smem = cps_net_tc_smem(&h->mp, mppi);
     const bool narrow = h->net->dev.hsz[0] <= 32 && h->net->dev.hsz[1] <= 32;
-    void (*fn)(const NetArgs) = narrow ? (mppi ? net_tc_kernel<true, true> : net_tc_kernel<false, true>)
-                                       : (mppi ? net_tc_kernel<true, false> : net_tc_kernel<false, false>);
+    void (*fn)(const NetArgs, const NetFleetMppiExt) = narrow ? (mppi ? net_tc_kernel<true, true> : net_tc_kernel<false, true>)
+                                                              : (mppi ? net_tc_kernel<true, false> : net_tc_kernel<false, false>);
     CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // live rollouts per CTA: 32 or 64 while that still gives every CTA its own SM (see the kernel's comment on rpq)
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->cfg.device);
-    a.tc_rows = (n_rows <= 32 * sms) ? 32 : (n_rows <= 64 * sms) ? 64 : TC_ROWS;
-    if (const char *e = getenv("CPS_TC_ROWS")) {   // A/B switch (tools/bench_net.py)
-        const int r = atoi(e);
-        if (r == 32 || r == 64 || r == 128) a.tc_rows = r;
-    }
+    a.tc_rows = cps_net_tc_rows(h, n_rows);
     const int grid = (n_rows + a.tc_rows - 1) / a.tc_rows;
-    fn<<<grid, TC_NT, smem, h->stream>>>(a);
+    fn<<<grid, TC_NT, smem, h->stream>>>(a, NetFleetMppiExt());
+    h->launches += 1;
+    h->net_last_kernel = 2;
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
+}
+
+// The MPPI fleet (cps_net_mppi_fleet): a.tc_rows and the experiments' draws / partials are set by the caller
+int cps_net_tc_fleet_launch(cps_handle *h, NetArgs &a, const NetFleetMppiExt &x, int E) {
+    const size_t smem = cps_net_tc_smem(&h->mp, true) + sizeof(CostParams);
+    const bool narrow = h->net->dev.hsz[0] <= 32 && h->net->dev.hsz[1] <= 32;
+    void (*fn)(const NetArgs, const NetFleetMppiExt) = narrow ? net_tc_kernel<true, true, true> : net_tc_kernel<true, false, true>;
+    CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const dim3 grid((a.B + a.tc_rows - 1) / a.tc_rows, E);
+    fn<<<grid, TC_NT, smem, h->stream>>>(a, x);
     h->launches += 1;
     h->net_last_kernel = 2;
     CUDA_TRY(h, cudaGetLastError());

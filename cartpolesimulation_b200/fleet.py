@@ -162,16 +162,32 @@ def make_experiments(n_experiments: int, n_periods: int, cfg: DataGenConfig | No
 
 
 class Fleet:
-    """E closed-loop experiments on one device = one cps_handle with a fleet attached."""
+    """E closed-loop experiments on one device = one cps_handle with a fleet attached.
+
+    Predictor "ODE" / "ODE_v0", or "neural" with `network`: the spec dict Engine.net_load takes
+    (neural.load_model(...)[0], neural.build_net_spec, neural.synthetic_net_spec), loaded before the fleet is created;
+    `net_kernel` (None, 'tensor', 'fp32') is Engine's.  The network lives in the controller only; the plant stays the
+    CartPole ODE.  Each experiment then owns a hidden state (net_states / set_net_states), set to the network's stored
+    state by reset() and advanced on (u, s) after every solve, as optimizer_mppi does.  Plant-side models are not offered
+    on neural fleets (set_plant_models raises NotImplementedError)."""
 
     def __init__(self, n_experiments: int, num_rollouts: int = 2000, horizon: int = 50, dt: float = 0.02,
                  substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
                  interp_period: int = 10, device: int | None = None, noise: str = "philox", seed: int = 0,
-                 experiment_offset: int = 0, dt_simulation: float = 0.002, no_pairs: bool = False):
+                 experiment_offset: int = 0, dt_simulation: float = 0.002, no_pairs: bool = False,
+                 network: dict | None = None, net_kernel: str | None = None):
+        if integrator == "neural" and network is None:
+            raise NotImplementedError("Fleet with integrator='neural' needs the network: pass network=<spec dict as "
+                                      "Engine.net_load takes, e.g. neural.load_model(...)[0]>")
+        if network is not None and integrator != "neural":
+            raise ValueError(f"network= is the neural predictor's model; integrator={integrator!r} takes none")
         if noise not in ("philox", "supplied"):
             raise ValueError("noise must be 'philox' or 'supplied'")
         self.engine = Engine(num_rollouts, horizon, dt=dt, substeps=substeps, integrator=integrator, cost=cost,
-                             interp_period=interp_period, device=device, no_pairs=no_pairs)
+                             interp_period=interp_period, device=device, no_pairs=no_pairs, net_kernel=net_kernel)
+        self.neural = network is not None
+        if self.neural:
+            self.engine.net_load(network)
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(horizon)
         self.n_ind, self.device = self.engine.n_ind, self.engine.device
         n_sim = int(round(dt / dt_simulation))
@@ -214,6 +230,23 @@ class Fleet:
         self.engine._chk(self.engine.lib.cps_fleet_noise(self.engine._h, int(period), _ptr(out)))
         return out
 
+    def net_states(self) -> np.ndarray:
+        """[E, Htot]: every experiment's hidden state (neural fleets).  Synchronises."""
+        htot = getattr(self.engine, "net_htot", 0)
+        out = np.zeros((self.E, max(htot, 1)), dtype=np.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_fleet_get_net_states(self.engine._h, out.ctypes.data_as(L._FP)))
+        return out[:, :htot]
+
+    def set_net_states(self, states):
+        """Sets every experiment's hidden state from [E, Htot] (neural fleets; after reset(), which sets them to the
+        network's stored state)."""
+        v = np.ascontiguousarray(states, dtype=np.float32)
+        if v.shape != (self.E, self.engine.net_htot):
+            raise ValueError(f"hidden states must have shape ({self.E}, {self.engine.net_htot})")
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_fleet_set_net_states(self.engine._h, v.ctypes.data_as(L._FP)))
+
     _CONTROL_NOISE = {"OFF": 0, "additive": 1, "truncnorm": 2}
 
     def set_plant_models(self, control_noise_mode: str = "OFF", control_noise: float = 0.0, control_bias: float = 0.0,
@@ -222,6 +255,9 @@ class Fleet:
         """cps_fleet_set_plant_models with the reference's configuration keys (cartpole_physical_parameters.yml:13-24:
         controlDisturbance_mode / controlDisturbance / controlBias, latency, noise.noise_mode / sigma_*).  Call before
         reset(); the first solve after reset() sees the true state (the reference's controller call at t = 0)."""
+        if self.neural:
+            raise NotImplementedError("plant-side models (control disturbance, measurement noise, latency) are not offered "
+                                      "on fleets with the neural predictor")
         if control_noise_mode not in self._CONTROL_NOISE:
             raise ValueError(f"controlDisturbance_mode with value {control_noise_mode} not valid")
         m = L.cps_fleet_plant_models(C.sizeof(L.cps_fleet_plant_models), self._CONTROL_NOISE[control_noise_mode],

@@ -395,6 +395,25 @@ int cps_fleet_relabel_masked(cps_handle *h, int n_rows, const float *states_dev,
 int cps_fleet_reset(cps_handle *h, long long period);
 /* The draws CPS_FLEET_NOISE_PHILOX uses in controller period `period`: out_dev [E][n_ind][K]. */
 int cps_fleet_noise(cps_handle *h, long long period, float *out_dev);
+/* Fleets with the neural predictor (CPS_PREDICTOR_NEURAL; cps_net_load before cps_fleet_create, else
+ * CPS_ERR_NOT_CONFIGURED).  The network lives in the controller only; the plant stays the CartPole ODE.  Each experiment
+ * owns a hidden state [Htot] besides its state, warm start and last control.  A period does, per experiment, what
+ * cps_mppi_step does with the network -- shifted warm start, its own draws, targets, u_prev and hidden state shared by its K
+ * rollouts, merge, then the hidden state advanced one step on (u, s) (optimizer_mppi.py:191,194-196; Dense networks keep
+ * it) -- and then the plant period with the record row of fleets on the ODE predictors (Q_applied = Q).  The solve of all
+ * experiments is one launch of the network kernel cps_mppi_step would pick (the tensor-core kernel for plain GRUs of up to
+ * 2 x 64 units, its rollouts per CTA chosen from E x K; else the FP32 kernel with the single solve's tile for K), so every
+ * experiment runs the arithmetic of one cps_mppi_step.  Launches per period: 2 with supplied draws (solve, plant), 3 with
+ * CPS_FLEET_NOISE_PHILOX (the draws of cps_fleet_noise into a fleet-owned [E][n_ind][K] workspace first), whatever E.
+ * CPS_NOISE_INDUCING only; default / quadratic_boundary need T + 1 < 512.  cps_fleet_set_states also sets every
+ * experiment's hidden state to the handle's stored state (zero after cps_net_load, or what cps_net_set_state set); the
+ * handle's own stored state is never written by the fleet.  cps_fleet_step re-checks the loaded network: one whose Htot
+ * differs from the fleet's gives CPS_ERR_INVALID (recreate the fleet).  cps_fleet_set_plant_models, cps_fleet_step_noisy,
+ * cps_fleet_relabel and cps_fleet_relabel_masked give CPS_ERR_UNSUPPORTED on a neural fleet.
+ * cps_fleet_get_net_states / cps_fleet_set_net_states: the hidden states [E][Htot] (Htot = cps_net_state_size);
+ * synchronise; CPS_ERR_NOT_CONFIGURED on a fleet without the neural predictor. */
+int cps_fleet_get_net_states(cps_handle *h, float *out_host);
+int cps_fleet_set_net_states(cps_handle *h, const float *in_host);
 
 /* ---- RPGD fleet: E closed-loop experiments under the reference's default optimizer ------------------------------ */
 /* The data generator with controller_mpc and optimizer rpgd (Control_Toolkit_ASF/config_controllers.yml:2): per controller
