@@ -134,6 +134,7 @@ SYMBOLS = {
     "cps_rpgd_fleet_create": (C.c_int, [_VP, C.POINTER(cps_rpgd_fleet_config)]),
     "cps_rpgd_fleet_set_states": (C.c_int, [_VP, _FP, _VP, C.c_longlong]),
     "cps_rpgd_fleet_step": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "cps_rpgd_fleet_relabel": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "cps_rpgd_fleet_get_states": (C.c_int, [_VP, _FP, _FP]),
     "cps_rpgd_fleet_get_plans": (C.c_int, [_VP, _FP, _FP, _FP, C.POINTER(C.c_int), C.POINTER(C.c_longlong),
                                            C.POINTER(C.c_longlong)]),

@@ -78,36 +78,6 @@ struct FleetArgs {
     double h_step;                // substep dt / n in double, for the device-side fold
 };
 
-// fold_ode (cps_lib.cu) on the device, same double-precision expressions: the controller's model constants for a
-// per-experiment pole length / mass (add_control_along_trajectories feeds L per recorded row).
-template <int INTEG>
-__device__ __forceinline__ void fold_ode_device(const FleetArgs &a, double L, double mp_in, OdeParams &o) {
-    const double k = a.k, mc = a.m_cart, g = a.g, J = a.J_fric, M = a.M_fric, umax = a.u_max;
-    const double mp = (INTEG == 0) ? (double)a.m_pole_fixed : mp_in;
-    const double kp1 = k + 1.0, Lh = L / 2.0;
-    o.KM = (float)(kp1 * (mc + mp));
-    o.m_p = (float)mp;
-    o.c1 = (float)(mp * g);
-    o.c2 = (float)(kp1 * mp * Lh);
-    o.c3 = (float)(J / Lh);
-    o.c5 = (float)(kp1 * M);
-    o.d1 = (float)(g / (kp1 * Lh));
-    o.d2 = (float)(1.0 / (kp1 * Lh));
-    o.d3 = (float)(J / (mp * Lh * kp1 * Lh));
-    o.bounce = (float)(2.0 / (0.5 * L));
-    const double hh = a.h_step;
-    const double hd2 = hh * (1.0 / (kp1 * Lh));
-    o.yc1 = (float)(hd2 * (mp * g));
-    o.yc2 = (float)(hd2 * (kp1 * mp * Lh));
-    o.yc3 = (float)(hd2 * (J / Lh));
-    o.yc5 = (float)(hd2 * (kp1 * M));
-    o.yu_scale = (float)(hd2 * (kp1 * umax));
-    o.v_y = (float)(kp1 * Lh);
-    o.hd1 = (float)(hh * (g / (kp1 * Lh)));
-    o.hd3 = (float)(hh * (J / (mp * Lh * kp1 * Lh)));
-    // the rotation constants and w_rot_max depend on the step only: the handle's fold stands
-}
-
 // cps_fleet_noise: materialise the draws the kernel generates, [E][n_ind][K]
 __global__ void __launch_bounds__(256) fleet_noise_kernel(unsigned long long seed, unsigned period, unsigned e_offset, int E,
                                                           int K, int n_ind, float *out) {

@@ -72,6 +72,13 @@ struct FleetGradArgs {
     GradArgs g;                // K = E * kpe plans [E * kpe][T]; s = the fleet's states [E][8]
     FleetGradExt x;
 };
+// The same with the controller's model per experiment (cps_rpgd_fleet_relabel with per-row L / m_pole): experiment e
+// integrates with odes[e] instead of g.ode.
+struct FleetGradOdeArgs {
+    GradArgs g;
+    FleetGradExt x;
+    const OdeParams *odes;     // [E]
+};
 
 namespace {
 
@@ -101,8 +108,9 @@ __device__ __forceinline__ Sub grad_substep(const OdeParams &P, float &th, float
 // to cps_plan_cost's, and the sequential part of the gradient runs at the solve kernels' speed.
 // FLEET (cps_rpgd_fleet.cu): the plans of E experiments in one launch, plan k of experiment k / fx.kpe with that experiment's
 // state, u_prev and cost parameters (fx); a null a.ck skips the checkpoints (costs only).  Per plan the arithmetic is the same.
-template <int NSUB, bool FLEET>
-__device__ __forceinline__ void grad_fwd(const GradArgs &a, const FleetGradExt &fx) {
+// ODE_E (FLEET only): the model constants of experiment e from odes[e] rather than a.ode.
+template <int NSUB, bool FLEET, bool ODE_E = false>
+__device__ __forceinline__ void grad_fwd(const GradArgs &a, const FleetGradExt &fx, const OdeParams *odes = nullptr) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= a.K) return;
     const int e = FLEET ? k / fx.kpe : 0;
@@ -110,7 +118,7 @@ __device__ __forceinline__ void grad_fwd(const GradArgs &a, const FleetGradExt &
     const int T = a.T, K = a.K;
     const bool want_ck = !FLEET || a.ck != nullptr;
     State z = load_state(FLEET ? a.s + (long long)e * 8 : (a.use_inline ? a.s_inline : a.s));
-    const OdeParams ode = pin_params(a.ode, z.th);
+    const OdeParams ode = pin_params(ODE_E ? odes[e] : a.ode, z.th);
     float c_cost = cosf(z.th);
     const float *q = a.Q + (long long)k * a.qs_k;
     float *ck = want_ck ? a.ck + k : nullptr;   // costs only (fleet): no checkpoint buffer
@@ -141,6 +149,10 @@ template <int NSUB>
 __global__ void __launch_bounds__(128) fleet_grad_fwd_kernel(const __grid_constant__ FleetGradArgs f) {
     grad_fwd<NSUB, true>(f.g, f.x);
 }
+template <int NSUB>
+__global__ void __launch_bounds__(128) fleet_grad_fwd_ode_kernel(const __grid_constant__ FleetGradOdeArgs f) {
+    grad_fwd<NSUB, true, true>(f.g, f.x, f.odes);
+}
 
 // ---- transposed Jacobian of every control step, in parallel over (control step, plan) ------------------------------------
 // The reverse sweep is linear in the adjoint (a_th, a_w, a_x, a_v), so a control step acts on it as a 4 x 4 matrix that
@@ -150,13 +162,13 @@ __global__ void __launch_bounds__(128) fleet_grad_fwd_kernel(const __grid_consta
 // (a_x passes through unchanged: the position enters no right-hand side) --, r[4], the row that gives d/d(uk), and the
 // terms the cost adds at the step's boundary.
 // Sequential work per plan shrinks from T x n reverse substeps to T small matrix-vector products (plan_grad_rev_kernel).
-template <int NSUB, bool FLEET = false>
+template <int NSUB, bool FLEET = false, bool ODE_E = false>
 __device__ __forceinline__ void step_record(const GradArgs &a, int t, int k, float *o, long long stride,
-                                            const FleetGradExt &fx = FleetGradExt()) {
+                                            const FleetGradExt &fx = FleetGradExt(), const OdeParams *odes = nullptr) {
     const int K = a.K;
     const int e = FLEET ? k / fx.kpe : 0;
     const CostParams &C = FLEET ? fx.costs[e] : a.cost;
-    const OdeParams &P = a.ode;
+    const OdeParams &P = ODE_E ? odes[e] : a.ode;
     const int n = NSUB ? NSUB : P.n;
     const float *ck = a.ck + k;
     float th = ck[((long long)t * 4 + 0) * K], w = ck[((long long)t * 4 + 1) * K];
@@ -249,6 +261,17 @@ __global__ void __launch_bounds__(128, 6) fleet_grad_jac_kernel(const __grid_con
     if (gid >= (long long)K * a.T) return;
     const int k = (int)(gid % K), t = (int)(gid / K);
     step_record<NSUB, true>(a, t, k, a.jac + (long long)t * CPS_GRAD_REC * K + k, K, f.x);
+}
+// the same with experiment e's model constants read from f.odes[e]: they occupy registers, where the kernel above reads
+// them from the parameter bank.  Five blocks per SM (96 registers): at six (80) the NSUB = 10 variant spills 76 bytes.
+template <int NSUB>
+__global__ void __launch_bounds__(128, 5) fleet_grad_jac_ode_kernel(const __grid_constant__ FleetGradOdeArgs f) {
+    const GradArgs &a = f.g;
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int K = a.K;
+    if (gid >= (long long)K * a.T) return;
+    const int k = (int)(gid % K), t = (int)(gid / K);
+    step_record<NSUB, true, true>(a, t, k, a.jac + (long long)t * CPS_GRAD_REC * K + k, K, f.x, f.odes);
 }
 
 // One control step of the reverse sweep from its record r.
@@ -599,8 +622,9 @@ extern "C" int cps_rpgd_set_iterations(cps_handle *h, long long iterations) {
 // G != nullptr: the gradient -- forward with checkpoints, Jacobians to global records, reverse (the global-record path of
 // cps_plan_cost_grad for every E: the launches per period do not depend on E; the records and the arithmetic per plan are the
 // same as the fused kernel's, so J and G match cps_plan_cost_grad bit for bit).  G == nullptr: the costs only, J [n_plans].
+// odes_dev [n_plans / kpe] or nullptr: each experiment's model constants (the _ode kernels), else the handle's.
 int cps_grad_fleet(cps_handle *h, int n_plans, int kpe, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
-                   const float *u_prev_dev, float *ck, float *jac, float *J, float *G) {
+                   const float *u_prev_dev, float *ck, float *jac, float *J, float *G, const OdeParams *odes_dev) {
     const int T = h->cfg.horizon;
     FleetGradArgs f;
     memset(&f, 0, sizeof(f));
@@ -615,14 +639,27 @@ int cps_grad_fleet(cps_handle *h, int n_plans, int kpe, const float *s_dev, cons
     a.ck = G ? ck : nullptr; a.jac = jac; a.J = J; a.G = G;
     a.nonfinite = h->d_nonfinite;
     f.x.costs = costs_dev; f.x.u_prev = u_prev_dev; f.x.kpe = kpe;
+    FleetGradOdeArgs fo;
+    fo.g = f.g; fo.x = f.x; fo.odes = odes_dev;
     const int block = 128, grid = (n_plans + block - 1) / block;
-    if (a.ode.n == 10) fleet_grad_fwd_kernel<10><<<grid, block, 0, h->stream>>>(f);
-    else fleet_grad_fwd_kernel<0><<<grid, block, 0, h->stream>>>(f);
+    if (odes_dev) {
+        if (a.ode.n == 10) fleet_grad_fwd_ode_kernel<10><<<grid, block, 0, h->stream>>>(fo);
+        else fleet_grad_fwd_ode_kernel<0><<<grid, block, 0, h->stream>>>(fo);
+    } else {
+        if (a.ode.n == 10) fleet_grad_fwd_kernel<10><<<grid, block, 0, h->stream>>>(f);
+        else fleet_grad_fwd_kernel<0><<<grid, block, 0, h->stream>>>(f);
+    }
     h->launches += 1;
     if (G) {
         const long long pairs = (long long)n_plans * T;
-        if (a.ode.n == 10) fleet_grad_jac_kernel<10><<<(unsigned)((pairs + 127) / 128), 128, 0, h->stream>>>(f);
-        else fleet_grad_jac_kernel<0><<<(unsigned)((pairs + 127) / 128), 128, 0, h->stream>>>(f);
+        const unsigned jgrid = (unsigned)((pairs + 127) / 128);
+        if (odes_dev) {
+            if (a.ode.n == 10) fleet_grad_jac_ode_kernel<10><<<jgrid, 128, 0, h->stream>>>(fo);
+            else fleet_grad_jac_ode_kernel<0><<<jgrid, 128, 0, h->stream>>>(fo);
+        } else {
+            if (a.ode.n == 10) fleet_grad_jac_kernel<10><<<jgrid, 128, 0, h->stream>>>(f);
+            else fleet_grad_jac_kernel<0><<<jgrid, 128, 0, h->stream>>>(f);
+        }
         plan_grad_rev_kernel<<<grid, block, 0, h->stream>>>(a);
         h->launches += 2;
     }

@@ -146,9 +146,10 @@ void cps_gmm_free(cps_handle *h);
 #define CPS_GRAD_REC 20   /* floats per (control step, plan) record: M[3][4], r[4], cost partials (3), control term */
 void cps_grad_free(cps_handle *h);
 // the RPGD fleet's gradient (G != nullptr; ck [T][4][n_plans], jac [T][CPS_GRAD_REC][n_plans]) or costs (G == nullptr) of
-// n_plans = E * kpe plans [n_plans][T] from the fleet's states [E][8], per-experiment cost parameters and u_prev [E]
+// n_plans = E * kpe plans [n_plans][T] from the fleet's states [E][8], per-experiment cost parameters and u_prev [E];
+// odes_dev [E] per-experiment model constants (relabelling with per-row L / m_pole) or nullptr (the handle's)
 int cps_grad_fleet(cps_handle *h, int n_plans, int kpe, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
-                   const float *u_prev_dev, float *ck, float *jac, float *J, float *G);
+                   const float *u_prev_dev, float *ck, float *jac, float *J, float *G, const OdeParams *odes_dev = nullptr);
 int cps_grad_fleet_update(cps_handle *h, int n_plans, float *Q_dev, const float *G_dev, float *m_dev, float *v_dev, float lr_t,
                           float beta_1, float beta_2, float epsilon, float gradmax_clip);
 // cps_lib.cu: cost parameters folded for a given target equilibrium

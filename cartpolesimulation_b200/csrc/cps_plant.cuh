@@ -16,6 +16,38 @@ struct PlantParams {
     int n_sim;
 };
 
+// fold_ode (cps_lib.cu) on the device, same double-precision expressions: the controller's model constants for a
+// per-experiment pole length / mass (add_control_along_trajectories feeds L per recorded row).  `a` is any argument block
+// with the physical constants k, m_cart, g, J_fric, M_fric, u_max, m_pole_fixed and the substep h_step (FleetArgs of
+// cps_fleet.cu, RpgdRowArgs of cps_rpgd_fleet.cu).
+template <int INTEG, class A>
+__device__ __forceinline__ void fold_ode_device(const A &a, double L, double mp_in, OdeParams &o) {
+    const double k = a.k, mc = a.m_cart, g = a.g, J = a.J_fric, M = a.M_fric, umax = a.u_max;
+    const double mp = (INTEG == 0) ? (double)a.m_pole_fixed : mp_in;
+    const double kp1 = k + 1.0, Lh = L / 2.0;
+    o.KM = (float)(kp1 * (mc + mp));
+    o.m_p = (float)mp;
+    o.c1 = (float)(mp * g);
+    o.c2 = (float)(kp1 * mp * Lh);
+    o.c3 = (float)(J / Lh);
+    o.c5 = (float)(kp1 * M);
+    o.d1 = (float)(g / (kp1 * Lh));
+    o.d2 = (float)(1.0 / (kp1 * Lh));
+    o.d3 = (float)(J / (mp * Lh * kp1 * Lh));
+    o.bounce = (float)(2.0 / (0.5 * L));
+    const double hh = a.h_step;
+    const double hd2 = hh * (1.0 / (kp1 * Lh));
+    o.yc1 = (float)(hd2 * (mp * g));
+    o.yc2 = (float)(hd2 * (kp1 * mp * Lh));
+    o.yc3 = (float)(hd2 * (J / Lh));
+    o.yc5 = (float)(hd2 * (kp1 * M));
+    o.yu_scale = (float)(hd2 * (kp1 * umax));
+    o.v_y = (float)(kp1 * Lh);
+    o.hd1 = (float)(hh * (g / (kp1 * Lh)));
+    o.hd3 = (float)(hh * (J / (mp * Lh * kp1 * Lh)));
+    // the rotation constants and w_rot_max depend on the step only: the handle's fold stands
+}
+
 // ---- Philox4x32-10 (Salmon et al., SC'11), the counter-based generator torch / TF / cuRAND also use ---------------------
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 #pragma unroll

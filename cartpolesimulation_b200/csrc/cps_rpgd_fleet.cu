@@ -18,6 +18,12 @@
 //                              record row.
 // The solve counter and Adam's iteration count are shared (lockstep), so lr_t is one host-computed scalar per Adam step.
 // Launches per period: 3 + 4 x (Adam steps) with predictor "ODE", 3 + 2 x (Adam steps) with the neural predictor.
+//
+// Offline relabelling (cps_rpgd_fleet_relabel) is the same period with the plant replaced by a recording: per row,
+// rpgd_relabel_row_kernel takes the place of rpgd_fleet_cost_kernel -- it also copies the row's recorded states into the
+// fleet's states and, with per-row L / m_pole on predictor "ODE", folds each experiment's model constants (the _ode
+// adjoint kernels of cps_grad.cu read them) -- and rpgd_relabel_finish_kernel does the bookkeeping of
+// rpgd_fleet_finish_kernel, then writes u to u_prev and Q_out instead of integrating.  Same launches per row as per period.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -30,15 +36,52 @@
 
 namespace {
 
-__global__ void __launch_bounds__(128) rpgd_fleet_cost_kernel(const CostParams up, const CostParams dn, const float *tp,
-                                                               const float *te, CostParams *out, int E) {
-    const int e = blockIdx.x * blockDim.x + threadIdx.x;
-    if (e >= E) return;
+// experiment e's cost parameters for its targets (null: 0 / +1)
+__device__ __forceinline__ CostParams fold_cost_e(const CostParams &up, const CostParams &dn, const float *tp, const float *te,
+                                                  int e) {
     const float tpe = tp ? tp[e] : 0.0f, tee = te ? te[e] : 1.0f;
     CostParams c = (tee == 1.0f) ? up : dn;   // quadratic_boundary_grad selects its weight set on the target equilibrium
     c.target_position = tpe;
     c.target_equilibrium = tee;
-    out[e] = c;
+    return c;
+}
+
+__global__ void __launch_bounds__(128) rpgd_fleet_cost_kernel(const CostParams up, const CostParams dn, const float *tp,
+                                                               const float *te, CostParams *out, int E) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= E) return;
+    out[e] = fold_cost_e(up, dn, tp, te, e);
+}
+
+struct RpgdRowArgs {
+    CostParams up, dn;
+    const float *tp, *te;            // [E] targets of this row (null: 0 / +1)
+    const float *states;             // [E][6] recorded states of this row
+    const float *L_row, *mp_row;     // [E] the controller model's pole length / mass of this row, or null
+    CostParams *costs;               // [E] <- folded cost parameters
+    float *s;                        // [E][8] <- the recorded states
+    OdeParams *odes;                 // [E] <- per-experiment model constants, or null (neural, or no per-row L / m_pole)
+    OdeParams ode;                   // the handle's fold (the constants that do not depend on L / m_pole)
+    float k, m_cart, g, J_fric, M_fric, u_max, m_pole_fixed;   // fold_ode_device's inputs
+    float L_default, mp_default;     // the handle's L / m_pole "for controller" when only one of the arrays is given
+    double h_step;
+    int E;
+};
+
+// Relabelling, per row: what rpgd_fleet_cost_kernel does, the row's recorded states into the fleet's, and the model
+// constants of each experiment's L / m_pole.  One thread per experiment.
+__global__ void __launch_bounds__(128) rpgd_relabel_row_kernel(const __grid_constant__ RpgdRowArgs a) {
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= a.E) return;
+    a.costs[e] = fold_cost_e(a.up, a.dn, a.tp, a.te, e);
+#pragma unroll
+    for (int c = 0; c < 6; ++c) a.s[(size_t)e * 8 + c] = a.states[(size_t)e * 6 + c];
+    if (a.odes) {
+        OdeParams o = a.ode;
+        fold_ode_device<CPS_EULER_CROMER>(a, a.L_row ? (double)a.L_row[e] : (double)a.L_default,
+                                          a.mp_row ? (double)a.mp_row[e] : (double)a.mp_default, o);
+        a.odes[e] = o;
+    }
 }
 
 // Input t of a fresh plan from its raw draws d[i * ds], i < n_ind (optimizer_rpgd_b200.sample_actions): the draws scaled,
@@ -119,12 +162,14 @@ struct RpgdFinishArgs {
     float *J_out;                    // [E][K] or null
     float *Q_opt;                    // [E][K][T] or null
     double time;
+    float *Q_out;                    // relabelling: [E] <- u (no plant, no record)
 };
 
 // get_action + the bookkeeping of step() (:182-224, :297-356), then the plant: one block per experiment.  The plant stage
-// reads nothing the bookkeeping writes; a mode that takes the next state from a recording instead (offline relabelling)
-// would replace only that stage.
-__global__ void __launch_bounds__(128) rpgd_fleet_finish_kernel(const __grid_constant__ RpgdFinishArgs a) {
+// reads nothing the bookkeeping writes; REPLAY (offline relabelling: the next state comes from a recording) replaces only
+// that stage, by writing u to Q_out.
+template <bool REPLAY>
+__device__ __forceinline__ void rpgd_finish(const RpgdFinishArgs &a) {
     extern __shared__ float smem[];
     const int e = blockIdx.x, tid = threadIdx.x, nt = blockDim.x, K = a.K, T = a.T;
     float *s_J = smem;
@@ -172,6 +217,10 @@ __global__ void __launch_bounds__(128) rpgd_fleet_finish_kernel(const __grid_con
     // ---- the plant: one controller period with Q held (CartPole/__init__.py:283-324), as fleet_kernel without plant-side models
     const float Qc = Q[(size_t)s_src[0] * T];   // u_nom[0] of the cheapest improved plan
     a.u_prev[e] = Qc;                           // the returned control enters the next solve's cost
+    if (REPLAY) {
+        a.Q_out[e] = Qc;
+        return;
+    }
     const PlantParams &P = a.plant;
     float s[6];
 #pragma unroll
@@ -194,6 +243,12 @@ __global__ void __launch_bounds__(128) rpgd_fleet_finish_kernel(const __grid_con
 #pragma unroll
     for (int c = 0; c < 6; ++c) so[c] = s[c];
 }
+__global__ void __launch_bounds__(128) rpgd_fleet_finish_kernel(const __grid_constant__ RpgdFinishArgs a) {
+    rpgd_finish<false>(a);
+}
+__global__ void __launch_bounds__(128) rpgd_relabel_finish_kernel(const __grid_constant__ RpgdFinishArgs a) {
+    rpgd_finish<true>(a);
+}
 
 }  // namespace
 
@@ -208,6 +263,7 @@ struct RpgdFleetState {
     float *d_ck, *d_jac, *d_J, *d_G;  // adjoint workspace: [T][4][EK], [T][CPS_GRAD_REC][EK] (ODE only; the neural adjoint
                                       // keeps its records in the network's workspace), [EK], [EK][T]
     CostParams *d_costs;              // [E] this period's folded cost parameters
+    OdeParams *d_odes;                // [E] relabelling: each experiment's model constants for its row's L / m_pole (ODE only)
     float *d_draws;                   // Philox reset draws [E][K][n_ind]
     size_t finish_smem;
     int ready;                        // cps_rpgd_fleet_set_states has run
@@ -220,6 +276,7 @@ void cps_rpgd_fleet_free(cps_handle *h) {
     cudaFree(F->d_s); cudaFree(F->d_uprev);
     for (int i = 0; i < 2; ++i) { cudaFree(F->d_Q[i]); cudaFree(F->d_m[i]); cudaFree(F->d_v[i]); cudaFree(F->d_ages[i]); }
     cudaFree(F->d_ck); cudaFree(F->d_jac); cudaFree(F->d_J); cudaFree(F->d_G); cudaFree(F->d_costs); cudaFree(F->d_draws);
+    cudaFree(F->d_odes);
     delete F;
     h->rfleet = nullptr;
 }
@@ -289,13 +346,16 @@ extern "C" int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config 
     if (!neural) {
         CUDA_TRY(h, cudaMalloc(&F->d_ck, sizeof(float) * 4 * n));
         CUDA_TRY(h, cudaMalloc(&F->d_jac, sizeof(float) * CPS_GRAD_REC * n));
+        CUDA_TRY(h, cudaMalloc(&F->d_odes, sizeof(OdeParams) * E));
     }
     CUDA_TRY(h, cudaMalloc(&F->d_J, sizeof(float) * EK));
     CUDA_TRY(h, cudaMalloc(&F->d_G, sizeof(float) * n));
     CUDA_TRY(h, cudaMalloc(&F->d_costs, sizeof(CostParams) * E));
     if (cfg->draw_source == CPS_FLEET_NOISE_PHILOX) CUDA_TRY(h, cudaMalloc(&F->d_draws, sizeof(float) * EK * h->n_ind));
-    if (smem > 48 * 1024)
+    if (smem > 48 * 1024) {
         CUDA_TRY(h, cudaFuncSetAttribute((const void *)rpgd_fleet_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CUDA_TRY(h, cudaFuncSetAttribute((const void *)rpgd_relabel_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    }
     return CPS_OK;
 }
 
@@ -351,20 +411,21 @@ extern "C" int cps_rpgd_fleet_set_states(cps_handle *h, const float *s_host, con
 
 int cps_fold_cost_for(cps_handle *h, float target_equilibrium, CostParams *out);
 
-extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *draws_dev,
-                                   float *record_dev, float *J_out_dev, float *Q_opt_out_dev) {
-    if (!h) return CPS_ERR_INVALID;
+// Shared by cps_rpgd_fleet_step (closed loop: replay_dev == nullptr) and cps_rpgd_fleet_relabel (states from a recording).
+static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, const float *tp_dev, const float *te_dev,
+                             const float *draws_dev, float *record_dev, float *J_out_dev, float *Q_opt_out_dev,
+                             const float *replay_dev, const float *L_dev, const float *mp_dev, float *Q_out_dev) {
     RpgdFleetState *F = h->rfleet;
-    if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_step: no RPGD fleet (cps_rpgd_fleet_create)");
-    if (!F->ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_step: no states yet (cps_rpgd_fleet_set_states)");
-    if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_step: negative number of periods");
+    if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no RPGD fleet (cps_rpgd_fleet_create)", who);
+    if (!F->ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no states yet (cps_rpgd_fleet_set_states)", who);
+    if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "%s: negative number of periods / rows", who);
     const bool philox = F->cfg.draw_source == CPS_FLEET_NOISE_PHILOX;
-    if (!philox && !draws_dev && F->nf > 0) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_step: this fleet expects supplied draws");
-    if (philox && draws_dev) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_step: this fleet generates its draws (Philox); pass NULL");
+    if (!philox && !draws_dev && F->nf > 0) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied draws", who);
+    if (philox && draws_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its draws (Philox); pass NULL", who);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
     int rc;   // neural: the network may have been reloaded since create (another size): check it, grow the workspace
-    if (neural && (rc = cps_net_grad_fleet_prepare(h, F->E, "cps_rpgd_fleet_step")) != CPS_OK) return rc;
+    if (neural && (rc = cps_net_grad_fleet_prepare(h, F->E, who)) != CPS_OK) return rc;
     CostParams up, dn;
     if ((rc = cps_fold_cost_for(h, 1.0f, &up)) != CPS_OK) return rc;
     if ((rc = cps_fold_cost_for(h, -1.0f, &dn)) != CPS_OK) return rc;
@@ -384,15 +445,36 @@ extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp
     P.L = (double)h->phys[CPS_PH_L]; P.m_pole = (double)h->phys[CPS_PH_M_POLE];
     P.dt = c.dt_simulation; P.n_sim = c.sim_substeps;
     const double dt_control = c.dt_simulation * c.sim_substeps;
+    // relabelling: the network reads neither L nor m_pole, so only predictor "ODE" folds per-row model constants
+    const OdeParams *odes = (replay_dev && !neural && (L_dev || mp_dev)) ? F->d_odes : nullptr;
+    RpgdRowArgs ra;
+    memset(&ra, 0, sizeof(ra));
+    ra.up = up; ra.dn = dn;
+    ra.costs = F->d_costs; ra.s = F->d_s; ra.odes = const_cast<OdeParams *>(odes);
+    ra.ode = h->ode;
+    ra.k = P.k; ra.m_cart = P.m_cart; ra.g = P.g; ra.J_fric = P.J_fric; ra.M_fric = P.M_fric; ra.u_max = P.u_max;
+    ra.m_pole_fixed = h->phys[CPS_PH_M_POLE];
+    ra.L_default = h->L_var; ra.mp_default = h->m_pole_var;
+    ra.h_step = (double)h->cfg.dt / (double)h->cfg.substeps;
+    ra.E = (int)E;
     for (int j = 0; j < n_periods; ++j) {
         const float *tp = tp_dev ? tp_dev + (size_t)j * E : nullptr, *te = te_dev ? te_dev + (size_t)j * E : nullptr;
-        rpgd_fleet_cost_kernel<<<(unsigned)((E + 127) / 128), 128, 0, h->stream>>>(up, dn, tp, te, F->d_costs, (int)E);
+        if (replay_dev) {
+            ra.tp = tp; ra.te = te;
+            ra.states = replay_dev + (size_t)j * E * 6;
+            ra.L_row = L_dev ? L_dev + (size_t)j * E : nullptr;
+            ra.mp_row = mp_dev ? mp_dev + (size_t)j * E : nullptr;
+            rpgd_relabel_row_kernel<<<(unsigned)((E + 127) / 128), 128, 0, h->stream>>>(ra);
+        } else {
+            rpgd_fleet_cost_kernel<<<(unsigned)((E + 127) / 128), 128, 0, h->stream>>>(up, dn, tp, te, F->d_costs, (int)E);
+        }
         h->launches += 1;
         float *Q = F->d_Q[F->cur], *m = F->d_m[F->cur], *v = F->d_v[F->cur];
         const int its = F->solves == 0 ? c.first_iter_count : c.outer_its;
         for (int it = 0; it < its; ++it) {   // grad_step (:166-180)
             rc = neural ? cps_net_grad_fleet(h, (int)E, F->d_s, Q, F->d_costs, F->d_uprev, F->d_J, F->d_G)
-                        : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, F->d_ck, F->d_jac, F->d_J, F->d_G);
+                        : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, F->d_ck, F->d_jac, F->d_J, F->d_G,
+                                         odes);
             if (rc != CPS_OK) return rc;
             F->adam_iterations += 1;
             const double t = (double)F->adam_iterations;   // ResourceApplyAdam, as cps_rpgd_grad_step
@@ -404,7 +486,7 @@ extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp
         }
         // get_action (:182-224): the costs of the improved plans
         rc = neural ? cps_net_grad_fleet(h, (int)E, F->d_s, Q, F->d_costs, F->d_uprev, F->d_J, nullptr)
-                    : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, nullptr, nullptr, F->d_J, nullptr);
+                    : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, nullptr, nullptr, F->d_J, nullptr, odes);
         if (rc != CPS_OK) return rc;
         const int nxt = F->cur ^ 1;
         a.J = F->d_J; a.Q = Q; a.m = m; a.v = v; a.ages = F->d_ages[F->cur];
@@ -417,7 +499,9 @@ extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp
         a.J_out = J_out_dev ? J_out_dev + (size_t)j * E * K : nullptr;
         a.Q_opt = Q_opt_out_dev ? Q_opt_out_dev + (size_t)j * E * K * T : nullptr;
         a.time = (double)F->period * dt_control;
-        rpgd_fleet_finish_kernel<<<(unsigned)E, 128, F->finish_smem, h->stream>>>(a);
+        a.Q_out = Q_out_dev ? Q_out_dev + (size_t)j * E : nullptr;
+        if (replay_dev) rpgd_relabel_finish_kernel<<<(unsigned)E, 128, F->finish_smem, h->stream>>>(a);
+        else rpgd_fleet_finish_kernel<<<(unsigned)E, 128, F->finish_smem, h->stream>>>(a);
         h->launches += 1;
         CUDA_TRY(h, cudaGetLastError());
         F->cur = nxt;
@@ -425,6 +509,22 @@ extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp
         F->period += 1;
     }
     return CPS_OK;
+}
+
+extern "C" int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *draws_dev,
+                                   float *record_dev, float *J_out_dev, float *Q_opt_out_dev) {
+    if (!h) return CPS_ERR_INVALID;
+    return rpgd_fleet_launch(h, "cps_rpgd_fleet_step", n_periods, tp_dev, te_dev, draws_dev, record_dev, J_out_dev, Q_opt_out_dev,
+                             nullptr, nullptr, nullptr, nullptr);
+}
+
+extern "C" int cps_rpgd_fleet_relabel(cps_handle *h, int n_rows, const float *states_dev, const float *tp_dev, const float *te_dev,
+                                      const float *L_dev, const float *m_pole_dev, const float *draws_dev, float *Q_out_dev,
+                                      float *J_out_dev) {
+    if (!h) return CPS_ERR_INVALID;
+    if (!states_dev || !Q_out_dev) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_relabel: null pointer");
+    return rpgd_fleet_launch(h, "cps_rpgd_fleet_relabel", n_rows, tp_dev, te_dev, draws_dev, nullptr, J_out_dev, nullptr,
+                             states_dev, L_dev, m_pole_dev, Q_out_dev);
 }
 
 extern "C" int cps_rpgd_fleet_get_states(cps_handle *h, float *s_host, float *u_prev_host) {

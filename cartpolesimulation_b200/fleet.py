@@ -446,3 +446,31 @@ class RpgdFleet:
         eng._chk(eng.lib.cps_rpgd_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
                                              _ptr(draws), _ptr(record), _ptr(J_out), _ptr(Q_opt)))
         return record
+
+    def relabel(self, states, target_position=None, target_equilibrium=None, L=None, m_pole=None, draws=None, Q_out=None,
+                J_out=None):
+        """cps_rpgd_fleet_relabel: one controller step per recorded row, experiment e = file e, from the recorded states
+        (cuda tensor [R, E, 6]) instead of the plant; no synchronisation.  target_position / target_equilibrium / L / m_pole:
+        cuda tensors [R, E] or None (L / m_pole change predictor "ODE"'s model; the network reads neither); draws as in
+        run(); Q_out [R, E] (allocated when None) receives the controls; J_out [R, E, K] or None.  reset() first is the
+        reference's controller.reset().  Returns Q_out."""
+        eng = self.engine
+        eng.use_current_stream()
+        _check_dev(states, "states", self.device)
+        R = int(states.shape[0]) if states.dim() == 3 else -1
+        if tuple(states.shape) != (R, self.E, 6):
+            raise ValueError(f"states has shape {tuple(states.shape)}, expected (rows, {self.E}, 6)")
+        if Q_out is None:
+            Q_out = torch.empty((R, self.E), device=self.device, dtype=torch.float32)
+        for t, name, numel in ((target_position, "target_position", R * self.E),
+                               (target_equilibrium, "target_equilibrium", R * self.E),
+                               (L, "L", R * self.E), (m_pole, "m_pole", R * self.E),
+                               (draws, "draws", R * self.E * (self.K - self.opt_keep_k) * self.n_ind),
+                               (Q_out, "Q_out", R * self.E), (J_out, "J_out", R * self.E * self.K)):
+            if t is not None:
+                _check_dev(t, name, self.device)
+                if t.numel() != numel:
+                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+        eng._chk(eng.lib.cps_rpgd_fleet_relabel(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
+                                                _ptr(L), _ptr(m_pole), _ptr(draws), _ptr(Q_out), _ptr(J_out)))
+        return Q_out

@@ -18,6 +18,12 @@ controller's warm start -- so it cannot be laid out as a fixed table of rows.  H
 the reference) drives every file on a host thread of its own, and the integrand evaluations of all files are collected
 into lockstep rounds: one masked fleet launch (cps_fleet_relabel_masked) evaluates the pending query of every file that
 still has one, files that are done with the row sit the launch out.  method='nd' is not offered.  No CPU fallback.
+
+RPGD, the reference's default optimizer, relabels the same way (Relabeller(optimizer="rpgd"), controller_config["rpgd"]):
+one RpgdFleet controller period per row of all files with the plant replaced by the recording (cps_rpgd_fleet_relabel).
+Plain rows, `_random_uniform_`, Monte-Carlo `_integrate_` and `_differentiate_` are sequences of rows.  `nquad` is not
+offered under RPGD: files sitting rows out would need their own solve counter, Adam iteration count and number of Adam
+steps, and the RPGD fleet advances those in lockstep.
 """
 from __future__ import annotations
 
@@ -31,34 +37,65 @@ import torch
 from . import _lib as L
 from . import config as cfgmod
 from .core import _check_dev, _ptr
-from .fleet import Fleet
+from .fleet import Fleet, RpgdFleet
 
 STATE_COMPONENTS = ("angle", "angleD", "angle_cos", "angle_sin", "position", "positionD")  # CartPole/state_utilities.py
 _CONTROLLER_ATTRIBUTES = ("target_position", "target_equilibrium", "L", "m_pole")
 
 
 class Relabeller:
-    """E files in lockstep on one device: a Fleet used in replay mode (the plant is not integrated)."""
+    """E files in lockstep on one device: a Fleet (MPPI) used in replay mode (the plant is not integrated).
 
-    def __init__(self, n_files: int, num_rollouts: int = 2000, horizon: int = 50, dt: float = 0.02, substeps: int = 10,
-                 integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal", interp_period: int = 10,
-                 device: int | None = None, noise: str = "philox", seed: int = 0, file_offset: int = 0,
-                 cost_config: dict | None = None, mppi: dict | None = None, no_pairs: bool = False):
-        self.fleet = Fleet(n_files, num_rollouts, horizon, dt=dt, substeps=substeps, integrator=integrator, cost=cost,
-                           interp_period=interp_period, device=device, noise=noise, seed=seed,
-                           experiment_offset=file_offset, no_pairs=no_pairs)
+    optimizer="rpgd": an RpgdFleet instead, built from RpgdFleet's keywords (num_rollouts, mpc_horizon, outer_its,
+    resamp_per, period_interpolation_inducing_points, ..., integrator="neural" with network=spec); dt, substeps,
+    integrator, cost, cost_config, device, noise, seed and file_offset keep their meaning.  horizon, interp_period, mppi and
+    no_pairs are MPPI's and raise ValueError there."""
+
+    def __init__(self, n_files: int, num_rollouts: int | None = None, horizon: int | None = None, dt: float = 0.02,
+                 substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
+                 interp_period: int | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
+                 file_offset: int = 0, cost_config: dict | None = None, mppi: dict | None = None, no_pairs: bool = False,
+                 optimizer: str = "mppi", **rpgd):
+        if optimizer not in ("mppi", "rpgd"):
+            raise ValueError(f"optimizer must be 'mppi' or 'rpgd', got {optimizer!r}")
+        self.optimizer = optimizer
+        if optimizer == "rpgd":
+            given = [k for k, v in (("horizon", horizon), ("interp_period", interp_period), ("mppi", mppi)) if v is not None]
+            if no_pairs:
+                given.append("no_pairs")
+            if given:
+                raise ValueError(f"{given} are MPPI keywords; RPGD takes mpc_horizon / period_interpolation_inducing_points")
+            if num_rollouts is not None:
+                rpgd["num_rollouts"] = num_rollouts
+            self.fleet = RpgdFleet(n_files, dt=dt, substeps=substeps, integrator=integrator, cost=cost,
+                                   cost_config=cost_config, device=device, noise=noise, seed=seed,
+                                   experiment_offset=file_offset, **rpgd)
+        else:
+            if rpgd:
+                raise TypeError(f"unexpected keyword arguments {sorted(rpgd)} (RPGD keywords need optimizer='rpgd')")
+            self.fleet = Fleet(n_files, 2000 if num_rollouts is None else num_rollouts, 50 if horizon is None else horizon,
+                               dt=dt, substeps=substeps, integrator=integrator, cost=cost,
+                               interp_period=10 if interp_period is None else interp_period, device=device, noise=noise,
+                               seed=seed, experiment_offset=file_offset, no_pairs=no_pairs)
         self.engine = self.fleet.engine
         self.E, self.K, self.T, self.n_ind, self.device = n_files, self.fleet.K, self.fleet.T, self.fleet.n_ind, self.fleet.device
-        if cost_config is not None:
-            self.engine.set_cost_params(cfgmod.cost_vector(cost, cost_config))
-        if mppi:
-            self.engine.set_mppi_params(**mppi)
+        if optimizer == "mppi":
+            if cost_config is not None:
+                self.engine.set_cost_params(cfgmod.cost_vector(cost, cost_config))
+            if mppi:
+                self.engine.set_mppi_params(**mppi)
 
     def close(self):
         self.fleet.close()
 
-    def reset(self, period: int = 0):
-        """controller.reset() of every file (:109-110)."""
+    def reset(self, period: int = 0, init_draws=None):
+        """controller.reset() of every file (:109-110).  RPGD: init_draws as RpgdFleet.reset takes them ('supplied'
+        fleets: cuda tensor [E, K, n_ind]; a 'philox' fleet draws its own)."""
+        if self.optimizer == "rpgd":
+            self.fleet.reset(np.zeros((self.E, 6), dtype=np.float32), period, init_draws=init_draws)
+            return
+        if init_draws is not None:
+            raise ValueError("init_draws are RPGD's; an MPPI relabeller starts from a zero warm start")
         self.engine.use_current_stream()
         self.engine._chk(self.engine.lib.cps_fleet_reset(self.engine._h, int(period)))
 
@@ -66,7 +103,12 @@ class Relabeller:
                        noise=None, Q_out=None, J_out=None, active=None):
         """cps_fleet_relabel on cuda tensors: states [R, E, 6]; attributes [R, E] or None; noise [R, E, n_ind, K] for a
         'supplied' fleet; active [R, E] int32 or None: files with 0 sit the row out (cps_fleet_relabel_masked).
-        Returns Q_out [R, E] (no synchronisation)."""
+        RPGD: cps_rpgd_fleet_relabel, noise = the resampling draws [R, E, K - opt_keep_k, n_ind] of a 'supplied' fleet;
+        no `active`.  Returns Q_out [R, E] (no synchronisation)."""
+        if self.optimizer == "rpgd":
+            if active is not None:
+                raise NotImplementedError("RPGD relabelling advances every file in lockstep: no per-file mask")
+            return self.fleet.relabel(states, target_position, target_equilibrium, pole_length, m_pole, noise, Q_out, J_out)
         eng = self.engine
         eng.use_current_stream()
         _check_dev(states, "states", self.device)
@@ -302,16 +344,37 @@ def nquad_rows(relabeller: Relabeller, states, attrs, features, ranges, num_eval
     return labels, calls
 
 
+# keys of config_optimizers.yml's rpgd block that do not change the labels (logging, the reference's unused rtol) or
+# that only the uniform sampling distribution reads, which RpgdFleet refuses itself
+_RPGD_IGNORED = ("optimizer_logging", "calculate_optimal_trajectory", "rtol", "sample_whole_control_space",
+                 "uniform_dist_min", "uniform_dist_max")
+
+
+def rpgd_relabeller_keywords(block: dict) -> dict:
+    """Relabeller(optimizer="rpgd") keywords from controller_config["rpgd"]: the rpgd block of config_optimizers.yml plus
+    integrator / cost / cost_config / network / noise / device / file_offset; `seed: null` keeps the default seed."""
+    kw = {k: v for k, v in dict(block).items() if k not in _RPGD_IGNORED}
+    if kw.get("seed", 0) is None:
+        del kw["seed"]
+    return kw
+
+
 def add_control_along_trajectories(dfs, controller_config, controller_output_variable_name="Q_calculated",
                                    integration_method="monte_carlo", integration_num_evals=64, save_output_only=False,
                                    df_modifier=lambda df: df, relabeller: Relabeller | None = None, seed=None,
-                                   noise=None, **kwargs):
-    """The reference's function (:53-140) for one DataFrame or a LIST of them (one per recorded file), MPPI as the
-    controller.  controller_config: 'state_components' (default: the six CartPole state columns),
+                                   noise=None, init_draws=None, **kwargs):
+    """The reference's function (:53-140) for one DataFrame or a LIST of them (one per recorded file), MPPI or RPGD as
+    the controller.  controller_config: 'state_components' (default: the six CartPole state columns),
     'environment_attributes_dict' (controller attribute -> CSV column, with the reference's suffix conventions) and
-    optionally 'mppi' (keyword arguments of Relabeller: num_rollouts, horizon, integrator, cost, ...).
+    optionally 'mppi' (keyword arguments of Relabeller: num_rollouts, horizon, integrator, cost, ...) or 'rpgd' (the rpgd
+    block of config_optimizers.yml plus integrator, cost, network, ...: an RpgdFleet relabels; not with 'mppi').
+    noise: a 'supplied' relabeller's draws per expanded row ([rows, E, n_ind, K] MPPI, [rows, E, K - opt_keep_k, n_ind]
+    RPGD); init_draws: a 'supplied' RPGD relabeller's reset draws [E, K, n_ind].
     Returns DataFrame(s) with the label column appended (or only the labels with save_output_only)."""
     import pandas as pd
+    if "mppi" in controller_config and "rpgd" in controller_config:
+        raise ValueError("controller_config takes one optimizer: 'mppi' or 'rpgd', not both")
+    rpgd = "rpgd" in controller_config or getattr(relabeller, "optimizer", "mppi") == "rpgd"
     single = isinstance(dfs, pd.DataFrame)
     files = [dfs] if single else list(dfs)
     if not files:
@@ -335,6 +398,10 @@ def add_control_along_trajectories(dfs, controller_config, controller_output_var
     if features and integration_method not in ("monte_carlo", "nquad"):
         raise ValueError("Invalid integration method. Choose 'nquad' or 'monte_carlo'.")
     nquad_mode = bool(features) and integration_method == "nquad"
+    if nquad_mode and rpgd:
+        raise NotImplementedError("integration_method='nquad' is not offered under RPGD: its files sit rows out, which "
+                                  "would need a solve counter, Adam iteration count and Adam steps per file; use "
+                                  "'monte_carlo'")
     unknown = [k for k in features + diff_features if k not in _CONTROLLER_ATTRIBUTES]
     if unknown:
         raise ValueError(f"cannot sweep {unknown}: the controller's attributes are {_CONTROLLER_ATTRIBUTES}")
@@ -373,11 +440,17 @@ def add_control_along_trajectories(dfs, controller_config, controller_output_var
             sweep[:, j * DIFF_WINDOW:(j + 1) * DIFF_WINDOW] = (base[:, None] + offsets[None, :]).astype(np.float32)
     own = relabeller is None
     if own:
-        relabeller = Relabeller(E, **dict(controller_config.get("mppi", {})))
+        if "rpgd" in controller_config:
+            relabeller = Relabeller(E, optimizer="rpgd", **rpgd_relabeller_keywords(controller_config["rpgd"]))
+        else:
+            relabeller = Relabeller(E, **dict(controller_config.get("mppi", {})))
     if relabeller.E != E:
         raise ValueError(f"the relabeller was built for {relabeller.E} files, got {E}")
     try:
-        relabeller.reset()
+        if init_draws is None:
+            relabeller.reset()
+        else:
+            relabeller.reset(init_draws=init_draws)
         if nquad_mode:
             labels_nq, _ = nquad_rows(relabeller, states, attrs, features, ranges, integration_num_evals, rows, noise=noise)
             Q = np.zeros((R, E), dtype=np.float32)

@@ -465,6 +465,25 @@ int cps_rpgd_fleet_set_states(cps_handle *h, const float *s_host, const float *i
  * may each be NULL. */
 int cps_rpgd_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *draws_dev,
                         float *record_dev, float *J_out_dev, float *Q_opt_out_dev);
+/* Offline relabelling under RPGD: add_control_along_trajectories
+ * (SI_Toolkit/src/SI_Toolkit/General/preprocess_data_add_control_along_trajectories.py:53-140) with optimizer_rpgd_tf as the
+ * controller, E recorded files in lockstep (experiment e of the fleet = file e).  controller.reset() of every file is
+ * cps_rpgd_fleet_set_states (the states it takes are overwritten by the first row).  Then one row of all files is one
+ * controller period of cps_rpgd_fleet_step with the plant stage replaced: each file's state is its recorded row
+ * states_dev [n_rows][E][6], the control goes to Q_out_dev [n_rows][E] and to the file's u_prev, nothing is integrated and
+ * no record is written.  The arithmetic per file and row is exactly one optimizer_rpgd_b200.step with the row's attributes
+ * tp_dev / te_dev / L_dev / m_pole_dev [n_rows][E] (NULL: 0 / +1 / the handle's L / m_pole).  Between rows a file keeps its
+ * plans, Adam moments, ages and u_prev; the solve counter and Adam's iteration count are shared (lockstep).  L / m_pole
+ * change the controller's model on CPS_EULER_CROMER (folded on the device per row and file with fold_ode's expressions,
+ * so the handle's own values give the handle's constants bit for bit); the neural predictor reads neither, so there they
+ * are accepted and change nothing.  draws_dev [n_rows][E][K - opt_keep_k][n_ind] as in cps_rpgd_fleet_step (NULL on a
+ * Philox fleet, whose counters use the period counter and experiment_offset: the draws are those cps_rpgd_fleet_draws
+ * returns, whatever the split of the files over handles); J_out_dev [n_rows][E][K] or NULL.  Launches per row as per
+ * period: 3 + 4 x (Adam steps) with CPS_EULER_CROMER, 3 + 2 x (Adam steps) with CPS_PREDICTOR_NEURAL, whatever E.  After
+ * the call the fleet's states are the last row's recorded states. */
+int cps_rpgd_fleet_relabel(cps_handle *h, int n_rows, const float *states_dev, const float *tp_dev, const float *te_dev,
+                           const float *L_dev, const float *m_pole_dev, const float *draws_dev, float *Q_out_dev,
+                           float *J_out_dev);
 /* s_host [E][6], u_prev_host [E]; either may be NULL.  Synchronises. */
 int cps_rpgd_fleet_get_states(cps_handle *h, float *s_host, float *u_prev_host);
 /* Optimizer state: Q_host, m_host, v_host [E][K][T], ages_host [E][K], the shared Adam iteration and solve counters; any
