@@ -27,6 +27,15 @@ def _check_dev(t, name, device, dtype=torch.float32):
     return t
 
 
+def _check_sizes(device, *checks):
+    """_check_dev and the element count of every (tensor, name, numel) whose tensor is not None."""
+    for t, name, numel in checks:
+        if t is not None:
+            _check_dev(t, name, device)
+            if t.numel() != numel:
+                raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+
+
 INTEGRATORS = {"ODE_v0": L.EULER_V0, "ODE": L.EULER_CROMER, "neural": L.PREDICTOR_NEURAL}
 COSTS = {None: L.COST_NONE, "none": L.COST_NONE, "default": L.COST_DEFAULT,
          "quadratic_boundary": L.COST_QUADRATIC_BOUNDARY,
@@ -146,12 +155,8 @@ class Engine:
         if tuple(noise.shape[:2]) != self.noise_shape(noise_layout) or noise.numel() != self.n_noise * self.K:
             raise ValueError(f"noise has shape {tuple(noise.shape)}, expected {self.noise_shape(noise_layout)}")
         unom_ptr = self.lib.cps_mppi_u_nom_dev(self._h) if u_nom is None else _check_dev(u_nom, "u_nom", self.device).data_ptr()
-        for t, name, numel in ((J_out, "J_out", self.K), (traj_out, "traj_out", self.K * (self.T + 1) * 6),
-                               (u_run_out, "u_run_out", self.K * self.T)):
-            if t is not None:
-                _check_dev(t, name, self.device)
-                if t.numel() != numel:
-                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+        _check_sizes(self.device, (J_out, "J_out", self.K), (traj_out, "traj_out", self.K * (self.T + 1) * 6),
+                     (u_run_out, "u_run_out", self.K * self.T))
         self._chk(self.lib.cps_mppi_step(self._h, _ptr(s), _ptr(noise), noise_layout, float(u_prev),
                                          C.c_void_p(unom_ptr), _ptr(self._u_dev), _ptr(J_out), _ptr(traj_out),
                                          traj_layout, _ptr(u_run_out)))
@@ -196,12 +201,8 @@ class Engine:
         _check_dev(delta_u, "delta_u", self.device)
         if delta_u.numel() != self.K * self.T:
             raise ValueError(f"delta_u has {delta_u.numel()} elements, expected {self.K * self.T}")
-        for t, name, numel in ((S_out, "S_out", self.K), (traj_out, "traj_out", self.K * (self.T + 1) * 6),
-                               (u_upd_out, "u_upd_out", self.T)):
-            if t is not None:
-                _check_dev(t, name, self.device)
-                if t.numel() != numel:
-                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+        _check_sizes(self.device, (S_out, "S_out", self.K), (traj_out, "traj_out", self.K * (self.T + 1) * 6),
+                     (u_upd_out, "u_upd_out", self.T))
         self._chk(self.lib.cps_legacy_step(self._h, _ptr(s), _ptr(delta_u), layout, _ptr(self._u_dev), _ptr(S_out),
                                            _ptr(traj_out), traj_layout, _ptr(u_upd_out)))
         return self._u_dev

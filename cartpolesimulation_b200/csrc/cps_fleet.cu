@@ -72,10 +72,7 @@ struct FleetArgs {
     const float *L_row, *mp_row;  // [E] controller-model pole length / mass of this row, or null (handle's values)
     float *Q_out;               // [E] controls computed for this row
     const int *active;          // [E] or null: files with 0 sit this row out (controller state untouched, no output)
-    float k, m_cart, g, J_fric, M_fric, u_max;  // physical constants for the device-side fold of (L, m_pole)
-    float m_pole_fixed;         // ODE_v0 takes only L from the variable parameters
-    float L_default, mp_default;  // the handle's L / m_pole "for controller" when only one of the arrays is given
-    double h_step;                // substep dt / n in double, for the device-side fold
+    FoldInputs fold;            // the device-side fold of (L, m_pole)
 };
 
 // cps_fleet_noise: materialise the draws the kernel generates, [E][n_ind][K]
@@ -83,7 +80,7 @@ __global__ void __launch_bounds__(256) fleet_noise_kernel(unsigned long long see
                                                           int K, int n_ind, float *out) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x, e = blockIdx.y;
     if (k >= K || e >= E) return;
-    fleet_draws(seed, period, e_offset + (unsigned)e, (unsigned)k, n_ind, out + ((size_t)e * n_ind) * K + k, K);
+    philox_normals(seed, (unsigned)k, 0u, period, e_offset + (unsigned)e, n_ind, out + ((size_t)e * n_ind) * K + k, K);
 }
 
 // The controller's view after `pushed` ring pushes: delayed + interpolated state (latency_adder.py:67-71), measurement
@@ -151,11 +148,12 @@ __global__ void __launch_bounds__(256, 4) fleet_kernel(const __grid_constant__ F
     if (PHILOX) {
         if (PAIR) {
             const int k = 2 * (blockIdx.x * blockDim.x + tid);
-            fleet_draws(a.seed, a.period, a.e_offset + (unsigned)e, (unsigned)min(k, mp.K - 2), mp.n_ind, s_eps + 2 * tid, per_block);
-            fleet_draws(a.seed, a.period, a.e_offset + (unsigned)e, (unsigned)min(k + 1, mp.K - 1), mp.n_ind, s_eps + 2 * tid + 1, per_block);
+            philox_normals(a.seed, (unsigned)min(k, mp.K - 2), 0u, a.period, a.e_offset + (unsigned)e, mp.n_ind, s_eps + 2 * tid, per_block);
+            philox_normals(a.seed, (unsigned)min(k + 1, mp.K - 1), 0u, a.period, a.e_offset + (unsigned)e, mp.n_ind, s_eps + 2 * tid + 1,
+                           per_block);
         } else {
             const int k = blockIdx.x * blockDim.x + tid;
-            fleet_draws(a.seed, a.period, a.e_offset + (unsigned)e, (unsigned)min(k, mp.K - 1), mp.n_ind, s_eps + tid, per_block);
+            philox_normals(a.seed, (unsigned)min(k, mp.K - 1), 0u, a.period, a.e_offset + (unsigned)e, mp.n_ind, s_eps + tid, per_block);
         }
     }
     __syncthreads();
@@ -181,8 +179,8 @@ __global__ void __launch_bounds__(256, 4) fleet_kernel(const __grid_constant__ F
     io.px.world = 0;
     OdeParams ode = a.ode;
     if (a.L_row || a.mp_row)
-        fold_ode_device<INTEG>(a, a.L_row ? (double)a.L_row[e] : (double)a.L_default,
-                               a.mp_row ? (double)a.mp_row[e] : (double)a.mp_default, ode);
+        fold_ode_device<INTEG>(a.fold, a.L_row ? (double)a.L_row[e] : (double)a.fold.L_default,
+                               a.mp_row ? (double)a.mp_row[e] : (double)a.fold.mp_default, ode);
     const bool last = PAIR ? mppi_solve_block2<INTEG, COST, NSUB, false>(ode, s_cost, mp, io, smem, blockIdx.x, a.bpe)
                            : mppi_solve_block<INTEG, COST, SC_ROTATE, CPS_NOISE_INDUCING, false, false, 0, false>(ode, s_cost, mp, io, smem,
                                                                                                        blockIdx.x, a.bpe);
@@ -216,23 +214,15 @@ __global__ void __launch_bounds__(256, 4) fleet_kernel(const __grid_constant__ F
     const float u = __fmul_rn(P.u_max, Q);
     double aDD, pDD;
     plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
-    if (a.record) {
-        float *r = a.record + (size_t)e * CPS_FLEET_RECORD;
-        r[0] = (float)a.time;
-        r[1] = s[IDX_ANGLE]; r[2] = s[IDX_ANGLED]; r[3] = (float)aDD; r[4] = s[IDX_COS]; r[5] = s[IDX_SIN];
-        r[6] = s[IDX_POS]; r[7] = s[IDX_POSD]; r[8] = (float)pDD;
-        r[9] = Qc; r[10] = Q; r[11] = u; r[12] = tp; r[13] = te; r[14] = 0.0f; r[15] = 0.0f;
-    }
+    if (a.record) plant_record(a.record + (size_t)e * CPS_FLEET_RECORD, a.time, s, aDD, pDD, Qc, Q, u, tp, te);
     float *ring = M.on ? M.ring + (size_t)e * M.ring_len * 6 : nullptr;
-    for (int i = 0; i < P.n_sim; ++i) {
-        plant_tick(P, s, aDD, pDD);
-        plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
+    plant_ticks(P, s, u, aDD, pDD, [&](int i) {
         if (M.on) {   // add_current_state_to_latency_buffer (latency_adder.py:36-47)
             float *slot = ring + (size_t)((M.pushed + i) % M.ring_len) * 6;
 #pragma unroll
             for (int c = 0; c < 6; ++c) slot[c] = s[c];
         }
-    }
+    });
     float *so = a.s + (size_t)e * 8;
 #pragma unroll
     for (int c = 0; c < 6; ++c) so[c] = s[c];
@@ -277,17 +267,10 @@ __global__ void __launch_bounds__(128) fleet_net_plant_kernel(const __grid_const
     const float u = __fmul_rn(P.u_max, Q);
     double aDD, pDD;
     plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
-    if (a.record) {
-        float *r = a.record + (size_t)e * CPS_FLEET_RECORD;
-        r[0] = (float)a.time;
-        r[1] = s[IDX_ANGLE]; r[2] = s[IDX_ANGLED]; r[3] = (float)aDD; r[4] = s[IDX_COS]; r[5] = s[IDX_SIN];
-        r[6] = s[IDX_POS]; r[7] = s[IDX_POSD]; r[8] = (float)pDD;
-        r[9] = Q; r[10] = Q; r[11] = u; r[12] = a.tp ? a.tp[e] : 0.0f; r[13] = a.te ? a.te[e] : 1.0f; r[14] = 0.0f; r[15] = 0.0f;
-    }
-    for (int i = 0; i < P.n_sim; ++i) {
-        plant_tick(P, s, aDD, pDD);
-        plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
-    }
+    if (a.record)
+        plant_record(a.record + (size_t)e * CPS_FLEET_RECORD, a.time, s, aDD, pDD, Q, Q, u, a.tp ? a.tp[e] : 0.0f,
+                     a.te ? a.te[e] : 1.0f);
+    plant_ticks(P, s, u, aDD, pDD, [](int) {});
     float *so = a.s + (size_t)e * 8;
 #pragma unroll
     for (int c = 0; c < 6; ++c) so[c] = s[c];
@@ -355,41 +338,6 @@ static fleet_fn pick_fleet(int integ, int cost, bool philox, bool pair, bool n10
     return integ == CPS_EULER_V0 ? pick_fleet1<0>(cost, philox, pair, n10) : pick_fleet1<1>(cost, philox, pair, n10);
 }
 
-// A fleet whose controller predicts with the loaded network: per experiment a hidden state next to the ODE fleet's state,
-// warm start and last control; partials and tickets for the network kernel's tiling; a draw workspace for Philox.
-static int fleet_create_neural(cps_handle *h, const cps_fleet_config *cfg) {
-    NetFleetPlan p;
-    int rc = cps_net_mppi_fleet_plan(h, cfg->n_experiments, "cps_fleet_create", &p);
-    if (rc != CPS_OK) return rc;
-    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    cps_fleet_free(h);
-    FleetState *F = new (std::nothrow) FleetState();
-    if (!F) return fail(h, CPS_ERR_INVALID, "cps_fleet_create: out of host memory");
-    memset(F, 0, sizeof(*F));
-    F->cfg = *cfg;
-    F->E = cfg->n_experiments;
-    F->neural = 1;
-    F->htot = cps_net_state_size(h);
-    F->bpe = p.tiles;
-    h->fleet = F;
-    const size_t E = F->E, K = h->cfg.num_rollouts, T = h->cfg.horizon, hn = F->htot > 0 ? F->htot : 1;
-    F->part_cap = E * p.tiles * (h->n_red + 2);
-    CUDA_TRY(h, cudaMalloc(&F->d_s, sizeof(float) * E * 8));
-    CUDA_TRY(h, cudaMalloc(&F->d_unom, sizeof(float) * E * T));
-    CUDA_TRY(h, cudaMalloc(&F->d_uprev, sizeof(float) * E));
-    CUDA_TRY(h, cudaMalloc(&F->d_partials, sizeof(float) * F->part_cap));
-    CUDA_TRY(h, cudaMalloc(&F->d_tickets, sizeof(unsigned) * E));
-    CUDA_TRY(h, cudaMalloc(&F->d_h, sizeof(float) * E * hn));
-    if (cfg->noise_source == CPS_FLEET_NOISE_PHILOX) CUDA_TRY(h, cudaMalloc(&F->d_noise, sizeof(float) * E * h->n_ind * K));
-    CUDA_TRY(h, cudaMemset(F->d_s, 0, sizeof(float) * E * 8));
-    CUDA_TRY(h, cudaMemset(F->d_unom, 0, sizeof(float) * E * T));
-    CUDA_TRY(h, cudaMemset(F->d_uprev, 0, sizeof(float) * E));
-    CUDA_TRY(h, cudaMemset(F->d_tickets, 0, sizeof(unsigned) * E));
-    CUDA_TRY(h, cudaMemset(F->d_h, 0, sizeof(float) * E * hn));
-    CUDA_TRY(h, cudaDeviceSynchronize());
-    return CPS_OK;
-}
-
 extern "C" int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg) {
     if (!h) return CPS_ERR_INVALID;
     if (!cfg || cfg->struct_size != (int)sizeof(cps_fleet_config))
@@ -402,7 +350,10 @@ extern "C" int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg) {
     if (h->cfg.noise_mode != CPS_NOISE_INDUCING)
         return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_create: fleets use inducing-point noise (CPS_NOISE_INDUCING)");
     if (cfg->n_experiments > 65535) return fail(h, CPS_ERR_INVALID, "cps_fleet_create: at most 65535 experiments per handle");
-    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) return fleet_create_neural(h, cfg);
+    const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
+    NetFleetPlan p;
+    int rc;
+    if (neural && (rc = cps_net_mppi_fleet_plan(h, cfg->n_experiments, "cps_fleet_create", &p)) != CPS_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     cps_fleet_free(h);
     FleetState *F = new (std::nothrow) FleetState();
@@ -411,30 +362,71 @@ extern "C" int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg) {
     F->cfg = *cfg;
     F->E = cfg->n_experiments;
     const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
-    // large fleets are throughput work: two rollouts per thread in packed FP32 (mppi_solve_block2) from 65536 rollouts
-    // per launch on, as for a single solve (tools/ab_fleet_pairs.py: 14 % faster at E = 256 and 1024, 30 % slower at E <= 16)
-    F->pair = (K % 2 == 0 && K >= 64 && (long long)cfg->n_experiments * K >= CPS_MPPI_PAIR_MIN_ROLLOUTS &&
-               !(h->cfg.flags & CPS_FLAG_NO_PAIRS)) ? 1 : 0;
-    const int threads = F->pair ? K / 2 : K;   // threads per experiment
-    F->block = threads >= 256 ? 256 : ((threads + 31) / 32) * 32;
-    F->bpe = (threads + F->block - 1) / F->block;
-    MppiParams mp_geo = h->mp;
-    const size_t draws = (cfg->noise_source == CPS_FLEET_NOISE_PHILOX) ? (size_t)h->n_ind * F->block * (F->pair ? 2 : 1) : 0;
-    F->smem = sizeof(float) * mppi_smem_floats(mp_geo, h->cfg.cost_id, F->block, F->pair ? 2 : 1, draws);
-    F->rs_off = mp_geo.rs_off;
-    if (F->smem > 200 * 1024) { delete F; return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_create: horizon too large for shared memory"); }
+    if (neural) {
+        // the controller predicts with the loaded network: per experiment a hidden state, partials and tickets for the
+        // network kernel's tiling, a draw workspace for Philox
+        F->neural = 1;
+        F->htot = cps_net_state_size(h);
+        F->bpe = p.tiles;
+    } else {
+        // large fleets are throughput work: two rollouts per thread in packed FP32 (mppi_solve_block2) from 65536 rollouts
+        // per launch on, as for a single solve (tools/ab_fleet_pairs.py: 14 % faster at E = 256 and 1024, 30 % slower at E <= 16)
+        F->pair = (K % 2 == 0 && K >= 64 && (long long)cfg->n_experiments * K >= CPS_MPPI_PAIR_MIN_ROLLOUTS &&
+                   !(h->cfg.flags & CPS_FLAG_NO_PAIRS)) ? 1 : 0;
+        const int threads = F->pair ? K / 2 : K;   // threads per experiment
+        F->block = threads >= 256 ? 256 : ((threads + 31) / 32) * 32;
+        F->bpe = (threads + F->block - 1) / F->block;
+        MppiParams mp_geo = h->mp;
+        const size_t draws = (cfg->noise_source == CPS_FLEET_NOISE_PHILOX) ? (size_t)h->n_ind * F->block * (F->pair ? 2 : 1) : 0;
+        F->smem = sizeof(float) * mppi_smem_floats(mp_geo, h->cfg.cost_id, F->block, F->pair ? 2 : 1, draws);
+        F->rs_off = mp_geo.rs_off;
+        if (F->smem > 200 * 1024) { delete F; return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_create: horizon too large for shared memory"); }
+    }
     h->fleet = F;
-    const size_t E = F->E;
+    const size_t E = F->E, hn = F->htot > 0 ? F->htot : 1;
+    F->part_cap = E * F->bpe * (h->n_red + 2);
     CUDA_TRY(h, cudaMalloc(&F->d_s, sizeof(float) * E * 8));
     CUDA_TRY(h, cudaMalloc(&F->d_unom, sizeof(float) * E * T));
     CUDA_TRY(h, cudaMalloc(&F->d_uprev, sizeof(float) * E));
-    CUDA_TRY(h, cudaMalloc(&F->d_partials, sizeof(float) * E * F->bpe * (h->n_red + 2)));
+    CUDA_TRY(h, cudaMalloc(&F->d_partials, sizeof(float) * F->part_cap));
     CUDA_TRY(h, cudaMalloc(&F->d_tickets, sizeof(unsigned) * E));
     CUDA_TRY(h, cudaMemset(F->d_s, 0, sizeof(float) * E * 8));
     CUDA_TRY(h, cudaMemset(F->d_unom, 0, sizeof(float) * E * T));
     CUDA_TRY(h, cudaMemset(F->d_uprev, 0, sizeof(float) * E));
     CUDA_TRY(h, cudaMemset(F->d_tickets, 0, sizeof(unsigned) * E));
+    if (neural) {
+        CUDA_TRY(h, cudaMalloc(&F->d_h, sizeof(float) * E * hn));
+        CUDA_TRY(h, cudaMemset(F->d_h, 0, sizeof(float) * E * hn));
+        if (cfg->noise_source == CPS_FLEET_NOISE_PHILOX) CUDA_TRY(h, cudaMalloc(&F->d_noise, sizeof(float) * E * h->n_ind * K));
+    }
     CUDA_TRY(h, cudaDeviceSynchronize());
+    return CPS_OK;
+}
+
+int fleet_states_to_device(cps_handle *h, const float *s_host, float *s_dev, int E, const char *who) {
+    float *tmp = new (std::nothrow) float[(size_t)E * 8];
+    if (!tmp) return fail(h, CPS_ERR_INVALID, "%s: out of host memory", who);
+    for (int e = 0; e < E; ++e) {
+        for (int c = 0; c < 6; ++c) tmp[(size_t)e * 8 + c] = s_host[(size_t)e * 6 + c];
+        tmp[(size_t)e * 8 + 6] = tmp[(size_t)e * 8 + 7] = 0.0f;
+    }
+    cudaError_t er = cudaMemcpyAsync(s_dev, tmp, sizeof(float) * (size_t)E * 8, cudaMemcpyHostToDevice, h->stream);
+    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
+    delete[] tmp;
+    CUDA_TRY(h, er);
+    return CPS_OK;
+}
+
+int fleet_states_to_host(cps_handle *h, const float *s_dev, float *s_host, int E, const char *who) {
+    float *tmp = new (std::nothrow) float[(size_t)E * 8];
+    if (!tmp) return fail(h, CPS_ERR_INVALID, "%s: out of host memory", who);
+    cudaError_t er = cudaMemcpyAsync(tmp, s_dev, sizeof(float) * (size_t)E * 8, cudaMemcpyDeviceToHost, h->stream);
+    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
+    if (er == cudaSuccess)
+        for (int e = 0; e < E; ++e)
+            for (int c = 0; c < 6; ++c) s_host[(size_t)e * 6 + c] = tmp[(size_t)e * 8 + c];
+    delete[] tmp;
+    CUDA_TRY(h, er);
     return CPS_OK;
 }
 
@@ -444,26 +436,17 @@ extern "C" int cps_fleet_set_states(cps_handle *h, const float *s_host, long lon
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_set_states: no fleet (cps_fleet_create)");
     if (!s_host || period < 0) return fail(h, CPS_ERR_INVALID, "cps_fleet_set_states: bad argument");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    float *tmp = new (std::nothrow) float[(size_t)F->E * 8];
-    if (!tmp) return fail(h, CPS_ERR_INVALID, "cps_fleet_set_states: out of host memory");
-    for (int e = 0; e < F->E; ++e) {
-        for (int c = 0; c < 6; ++c) tmp[(size_t)e * 8 + c] = s_host[(size_t)e * 6 + c];
-        tmp[(size_t)e * 8 + 6] = tmp[(size_t)e * 8 + 7] = 0.0f;
-    }
-    cudaError_t er = cudaMemcpyAsync(F->d_s, tmp, sizeof(float) * (size_t)F->E * 8, cudaMemcpyHostToDevice, h->stream);
-    if (er == cudaSuccess) er = cudaMemsetAsync(F->d_unom, 0, sizeof(float) * (size_t)F->E * h->cfg.horizon, h->stream);
-    if (er == cudaSuccess) er = cudaMemsetAsync(F->d_uprev, 0, sizeof(float) * (size_t)F->E, h->stream);
-    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
-    delete[] tmp;
-    CUDA_TRY(h, er);
+    CUDA_TRY(h, cudaMemsetAsync(F->d_unom, 0, sizeof(float) * (size_t)F->E * h->cfg.horizon, h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(F->d_uprev, 0, sizeof(float) * (size_t)F->E, h->stream));
+    int rc = fleet_states_to_device(h, s_host, F->d_s, F->E, "cps_fleet_set_states");
+    if (rc != CPS_OK) return rc;
     F->period = period;
     if (F->neural && F->htot > 0) {   // every experiment starts from the handle's stored state (what a fresh predictor holds)
         std::vector<float> h0((size_t)F->htot), all((size_t)F->E * F->htot);
         if (F->htot != cps_net_state_size(h))
             return fail(h, CPS_ERR_INVALID, "cps_fleet_set_states: the loaded network's hidden state differs from the fleet's; "
                         "recreate the fleet (cps_fleet_create)");
-        int rc = cps_net_get_state(h, h0.data());
-        if (rc != CPS_OK) return rc;
+        if ((rc = cps_net_get_state(h, h0.data())) != CPS_OK) return rc;
         for (int e = 0; e < F->E; ++e) memcpy(&all[(size_t)e * F->htot], h0.data(), sizeof(float) * F->htot);
         CUDA_TRY(h, cudaMemcpyAsync(F->d_h, all.data(), sizeof(float) * all.size(), cudaMemcpyHostToDevice, h->stream));
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
@@ -516,16 +499,7 @@ extern "C" int cps_fleet_get_observed(cps_handle *h, float *obs_host) {
     if (!F || !F->pm.on) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_get_observed: no plant-side models (cps_fleet_set_plant_models)");
     if (!obs_host) return fail(h, CPS_ERR_INVALID, "cps_fleet_get_observed: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    float *tmp = new (std::nothrow) float[(size_t)F->E * 8];
-    if (!tmp) return fail(h, CPS_ERR_INVALID, "cps_fleet_get_observed: out of host memory");
-    cudaError_t er = cudaMemcpyAsync(tmp, F->pm.obs, sizeof(float) * (size_t)F->E * 8, cudaMemcpyDeviceToHost, h->stream);
-    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
-    if (er == cudaSuccess)
-        for (int e = 0; e < F->E; ++e)
-            for (int c = 0; c < 6; ++c) obs_host[(size_t)e * 6 + c] = tmp[(size_t)e * 8 + c];
-    delete[] tmp;
-    CUDA_TRY(h, er);
-    return CPS_OK;
+    return fleet_states_to_host(h, F->pm.obs, obs_host, F->E, "cps_fleet_get_observed");
 }
 
 extern "C" int cps_fleet_reset(cps_handle *h, long long period) {
@@ -545,17 +519,8 @@ extern "C" int cps_fleet_get_states(cps_handle *h, float *s_host, float *u_nom_h
     FleetState *F = h->fleet;
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_get_states: no fleet (cps_fleet_create)");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (s_host) {
-        float *tmp = new (std::nothrow) float[(size_t)F->E * 8];
-        if (!tmp) return fail(h, CPS_ERR_INVALID, "cps_fleet_get_states: out of host memory");
-        cudaError_t er = cudaMemcpyAsync(tmp, F->d_s, sizeof(float) * (size_t)F->E * 8, cudaMemcpyDeviceToHost, h->stream);
-        if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
-        if (er == cudaSuccess)
-            for (int e = 0; e < F->E; ++e)
-                for (int c = 0; c < 6; ++c) s_host[(size_t)e * 6 + c] = tmp[(size_t)e * 8 + c];
-        delete[] tmp;
-        CUDA_TRY(h, er);
-    }
+    int rc;
+    if (s_host && (rc = fleet_states_to_host(h, F->d_s, s_host, F->E, "cps_fleet_get_states")) != CPS_OK) return rc;
     if (u_nom_host)
         CUDA_TRY(h, cudaMemcpyAsync(u_nom_host, F->d_unom, sizeof(float) * (size_t)F->E * h->cfg.horizon, cudaMemcpyDeviceToHost, h->stream));
     if (u_prev_host)
@@ -591,6 +556,14 @@ extern "C" long long cps_fleet_period(const cps_handle *h) { return (h && h->fle
 // CostParams for a given target equilibrium: fold_cost() depends on it for quadratic_boundary_grad (weight set, w[9]).
 int cps_fold_cost_for(cps_handle *h, float target_equilibrium, CostParams *out);
 
+// The period's draws: supplied by the caller or generated (Philox), as the fleet was created
+static int fleet_check_noise(cps_handle *h, const FleetState *F, const float *noise_dev, const char *who) {
+    const bool philox = F->cfg.noise_source == CPS_FLEET_NOISE_PHILOX;
+    if (!philox && !noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied noise", who);
+    if (philox && noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its noise (Philox); pass NULL", who);
+    return CPS_OK;
+}
+
 // Shared by cps_fleet_step (closed loop: replay_dev == nullptr) and cps_fleet_relabel (states from a recording).
 static int fleet_launch(cps_handle *h, const char *who, int n_periods, const float *tp_dev, const float *te_dev,
                         const float *noise_dev, float *record_dev, float *J_out_dev, const float *replay_dev,
@@ -599,9 +572,9 @@ static int fleet_launch(cps_handle *h, const char *who, int n_periods, const flo
     FleetState *F = h->fleet;
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no fleet (cps_fleet_create)", who);
     if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "%s: negative number of periods / rows", who);
+    int rc;
+    if ((rc = fleet_check_noise(h, F, noise_dev, who)) != CPS_OK) return rc;
     const bool philox = F->cfg.noise_source == CPS_FLEET_NOISE_PHILOX;
-    if (!philox && !noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied noise", who);
-    if (philox && noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its noise (Philox); pass NULL", who);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     FleetArgs a;
     a.ode = h->ode; a.mp = h->mp;
@@ -610,22 +583,14 @@ static int fleet_launch(cps_handle *h, const char *who, int n_periods, const flo
     if (replay_dev) a.pm.on = 0;   // relabelling feeds recorded states: no plant, no observation chain
     if (a.pm.on && !philox && ((a.pm.ctrl_mode && !ctrl_draws_dev) || (a.pm.meas_on && !meas_draws_dev)))
         return fail(h, CPS_ERR_INVALID, "%s: a fleet with supplied noise needs the plant-side draws as well (cps_fleet_step_noisy)", who);
-    int rc;
     if ((rc = cps_fold_cost_for(h, 1.0f, &a.cost_up)) != CPS_OK) return rc;
     if ((rc = cps_fold_cost_for(h, -1.0f, &a.cost_dn)) != CPS_OK) return rc;
-    PlantParams &P = a.plant;
-    P.k = h->phys[CPS_PH_K]; P.m_cart = h->phys[CPS_PH_M_CART]; P.g = h->phys[CPS_PH_G]; P.J_fric = h->phys[CPS_PH_J_FRIC];
-    P.M_fric = h->phys[CPS_PH_M_FRIC]; P.u_max = h->phys[CPS_PH_U_MAX]; P.thl = h->phys[CPS_PH_TRACK_HALF_LENGTH];
-    P.L = (double)h->phys[CPS_PH_L]; P.m_pole = (double)h->phys[CPS_PH_M_POLE];
-    P.dt = F->cfg.dt_simulation; P.n_sim = F->cfg.sim_substeps;
+    a.plant = plant_params(h, F->cfg.dt_simulation, F->cfg.sim_substeps);
     a.bpe = F->bpe;
     a.s = F->d_s; a.u_nom = F->d_unom; a.u_prev = F->d_uprev;
     a.seed = F->cfg.seed; a.e_offset = (unsigned)F->cfg.experiment_offset;
     a.partials = F->d_partials; a.tickets = F->d_tickets; a.nonfinite = h->d_nonfinite;
-    a.k = P.k; a.m_cart = P.m_cart; a.g = P.g; a.J_fric = P.J_fric; a.M_fric = P.M_fric; a.u_max = P.u_max;
-    a.m_pole_fixed = h->phys[CPS_PH_M_POLE];
-    a.L_default = h->L_var; a.mp_default = h->m_pole_var;
-    a.h_step = (double)h->cfg.dt / (double)h->cfg.substeps;
+    a.fold = fold_inputs(h);
     if (F->pair && noise_dev && ((uintptr_t)noise_dev % 8) != 0)
         return fail(h, CPS_ERR_INVALID, "%s: supplied noise must be 8-byte aligned", who);
     fleet_fn fn = pick_fleet(h->cfg.integrator, h->cfg.cost_id, philox, F->pair != 0, h->ode.n == 10);
@@ -667,12 +632,11 @@ static int fleet_step_neural(cps_handle *h, int n_periods, const float *tp_dev, 
     const char *who = "cps_fleet_step";
     FleetState *F = h->fleet;
     if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "%s: negative number of periods", who);
+    int rc;
+    if ((rc = fleet_check_noise(h, F, noise_dev, who)) != CPS_OK) return rc;
     const bool philox = F->cfg.noise_source == CPS_FLEET_NOISE_PHILOX;
-    if (!philox && !noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied noise", who);
-    if (philox && noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its noise (Philox); pass NULL", who);
     NetFleetPlan p;
-    int rc = cps_net_mppi_fleet_plan(h, F->E, who, &p);
-    if (rc != CPS_OK) return rc;
+    if ((rc = cps_net_mppi_fleet_plan(h, F->E, who, &p)) != CPS_OK) return rc;
     if (cps_net_state_size(h) != F->htot)
         return fail(h, CPS_ERR_INVALID, "%s: the loaded network has %d hidden-state floats, the fleet was created for %d; "
                     "recreate the fleet (cps_fleet_create)", who, cps_net_state_size(h), F->htot);
@@ -690,11 +654,7 @@ static int fleet_step_neural(cps_handle *h, int n_periods, const float *tp_dev, 
     if ((rc = cps_fold_cost_for(h, 1.0f, &cost_up)) != CPS_OK) return rc;
     if ((rc = cps_fold_cost_for(h, -1.0f, &cost_dn)) != CPS_OK) return rc;
     NetPlantArgs pa;
-    PlantParams &P = pa.plant;
-    P.k = h->phys[CPS_PH_K]; P.m_cart = h->phys[CPS_PH_M_CART]; P.g = h->phys[CPS_PH_G]; P.J_fric = h->phys[CPS_PH_J_FRIC];
-    P.M_fric = h->phys[CPS_PH_M_FRIC]; P.u_max = h->phys[CPS_PH_U_MAX]; P.thl = h->phys[CPS_PH_TRACK_HALF_LENGTH];
-    P.L = (double)h->phys[CPS_PH_L]; P.m_pole = (double)h->phys[CPS_PH_M_POLE];
-    P.dt = F->cfg.dt_simulation; P.n_sim = F->cfg.sim_substeps;
+    pa.plant = plant_params(h, F->cfg.dt_simulation, F->cfg.sim_substeps);
     pa.s = F->d_s; pa.u = F->d_uprev; pa.E = F->E;
     const double dt_control = F->cfg.dt_simulation * F->cfg.sim_substeps;
     for (int j = 0; j < n_periods; ++j) {

@@ -1,5 +1,6 @@
-// cps_plant.cuh -- device code shared by the two fleets (cps_fleet.cu: MPPI, cps_rpgd_fleet.cu: RPGD): the plant in the
-// reference's mixed float32 / float64 arithmetic and the counter-based normal draws.
+// cps_plant.cuh -- code shared by the fleets (cps_fleet.cu: MPPI on the ODE or the network, cps_rpgd_fleet.cu: RPGD): the
+// plant in the reference's mixed float32 / float64 arithmetic, the record row, the counter-based normal draws and the
+// device-side fold of the controller's model constants, with the host functions that fill their parameter blocks.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -7,6 +8,7 @@
 #include <cstdint>
 
 #include "cps_device.cuh"
+#include "cps_internal.cuh"
 
 using namespace cps;
 
@@ -16,12 +18,39 @@ struct PlantParams {
     int n_sim;
 };
 
+// The plant of the handle's physical constants, n_sim ticks of dt_simulation per controller period
+static inline PlantParams plant_params(const cps_handle *h, double dt_simulation, int sim_substeps) {
+    PlantParams P;
+    P.k = h->phys[CPS_PH_K]; P.m_cart = h->phys[CPS_PH_M_CART]; P.g = h->phys[CPS_PH_G]; P.J_fric = h->phys[CPS_PH_J_FRIC];
+    P.M_fric = h->phys[CPS_PH_M_FRIC]; P.u_max = h->phys[CPS_PH_U_MAX]; P.thl = h->phys[CPS_PH_TRACK_HALF_LENGTH];
+    P.L = (double)h->phys[CPS_PH_L]; P.m_pole = (double)h->phys[CPS_PH_M_POLE];
+    P.dt = dt_simulation; P.n_sim = sim_substeps;
+    return P;
+}
+
+// What fold_ode_device reads besides L and m_pole: the physical constants, the substep and the handle's L / m_pole "for
+// controller" (used when a fleet is given only one of the per-row arrays).
+struct FoldInputs {
+    float k, m_cart, g, J_fric, M_fric, u_max;
+    float m_pole_fixed;         // ODE_v0 takes only L from the variable parameters
+    float L_default, mp_default;
+    double h_step;              // substep dt / n in double
+};
+
+static inline FoldInputs fold_inputs(const cps_handle *h) {
+    FoldInputs f;
+    f.k = h->phys[CPS_PH_K]; f.m_cart = h->phys[CPS_PH_M_CART]; f.g = h->phys[CPS_PH_G]; f.J_fric = h->phys[CPS_PH_J_FRIC];
+    f.M_fric = h->phys[CPS_PH_M_FRIC]; f.u_max = h->phys[CPS_PH_U_MAX];
+    f.m_pole_fixed = h->phys[CPS_PH_M_POLE];
+    f.L_default = h->L_var; f.mp_default = h->m_pole_var;
+    f.h_step = (double)h->cfg.dt / (double)h->cfg.substeps;
+    return f;
+}
+
 // fold_ode (cps_lib.cu) on the device, same double-precision expressions: the controller's model constants for a
-// per-experiment pole length / mass (add_control_along_trajectories feeds L per recorded row).  `a` is any argument block
-// with the physical constants k, m_cart, g, J_fric, M_fric, u_max, m_pole_fixed and the substep h_step (FleetArgs of
-// cps_fleet.cu, RpgdRowArgs of cps_rpgd_fleet.cu).
-template <int INTEG, class A>
-__device__ __forceinline__ void fold_ode_device(const A &a, double L, double mp_in, OdeParams &o) {
+// per-experiment pole length / mass (add_control_along_trajectories feeds L per recorded row).
+template <int INTEG>
+__device__ __forceinline__ void fold_ode_device(const FoldInputs &a, double L, double mp_in, OdeParams &o) {
     const double k = a.k, mc = a.m_cart, g = a.g, J = a.J_fric, M = a.M_fric, umax = a.u_max;
     const double mp = (INTEG == 0) ? (double)a.m_pole_fixed : mp_in;
     const double kp1 = k + 1.0, Lh = L / 2.0;
@@ -72,12 +101,17 @@ __device__ __forceinline__ void box_muller(unsigned a, unsigned b, float &n0, fl
     n1 = r * sn;
 }
 
-// Draws i = 0..n_ind-1 of rollout k, experiment e_global, controller period `period`; dst[i * stride].
-__device__ __forceinline__ void fleet_draws(unsigned long long seed, unsigned period, unsigned e_global, unsigned k,
-                                            int n_ind, float *dst, long long stride) {
+// Standard normals i = 0..n_ind-1, dst[i * stride], four per counter (w0, w1 + i / 4, period, e_global).  The fleets'
+// streams: the MPPI rollout draws have w0 = rollout, w1 = 0 (second word = draw group < 2^28); the RPGD plan draws have
+// w0 = plan row, w1 = RPGD_DRAWS_RESAMPLE (the resampling solve of `period`) or RPGD_DRAWS_RESET (period 0, the plans of
+// a reset); the plant-side draws of cps_fleet.cu have second word 0xFFFFFFFF.  The second words keep them disjoint.
+#define RPGD_DRAWS_RESAMPLE 0xA0000000u
+#define RPGD_DRAWS_RESET 0xB0000000u
+__device__ __forceinline__ void philox_normals(unsigned long long seed, unsigned w0, unsigned w1, unsigned period,
+                                               unsigned e_global, int n_ind, float *dst, long long stride) {
     const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
     for (int g = 0; 4 * g < n_ind; ++g) {
-        const uint4 r = philox4x32_10(make_uint4(k, (unsigned)g, period, e_global), key);
+        const uint4 r = philox4x32_10(make_uint4(w0, w1 + (unsigned)g, period, e_global), key);
         float n[4];
         box_muller(r.x, r.y, n[0], n[1]);
         box_muller(r.z, r.w, n[2], n[3]);
@@ -137,24 +171,25 @@ __device__ __forceinline__ void plant_tick(const PlantParams &P, float *s, doubl
     s[IDX_ANGLE] = (float)plant_wrap((double)s[IDX_ANGLE]);
 }
 
-// The RPGD fleet's sampling draws (cps_rpgd_fleet.cu): draws i = 0..n_ind-1 of plan row `row`, dst[i * stride].  Counter
-// (row, tag + draw group, period, global experiment): the tag in the second word keeps them apart from the rollout draws
-// above (second word = draw group < 2^28) and from the plant-side draws (second word 0xFFFFFFFF).  tag: RPGD_DRAWS_RESAMPLE
-// for the resampling solve of `period`, RPGD_DRAWS_RESET (period 0) for the plans of a reset.
-// Deliberately a copy of fleet_draws' loop rather than a shared one with a tag argument: fleet_draws is inlined into
-// fleet_kernel, whose code must not change with the RPGD fleet (its SASS is checked byte for byte).
-#define RPGD_DRAWS_RESAMPLE 0xA0000000u
-#define RPGD_DRAWS_RESET 0xB0000000u
-__device__ __forceinline__ void rpgd_draws(unsigned long long seed, unsigned tag, unsigned period, unsigned e_global, unsigned row,
-                                           int n_ind, float *dst, long long stride) {
-    const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
-    for (int g = 0; 4 * g < n_ind; ++g) {
-        const uint4 r = philox4x32_10(make_uint4(row, tag + (unsigned)g, period, e_global), key);
-        float n[4];
-        box_muller(r.x, r.y, n[0], n[1]);
-        box_muller(r.z, r.w, n[2], n[3]);
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-            if (4 * g + q < n_ind) dst[(long long)(4 * g + q) * stride] = n[q];
+// The fleets' record row of one controller period (include/cps.h CPS_FLEET_RECORD): the state the controller was called
+// on with its second derivatives, Qc = the controller's control, Q = the applied one (after control noise), u = u_max Q,
+// and the targets.
+__device__ __forceinline__ void plant_record(float *r, double time, const float *s, double aDD, double pDD, float Qc, float Q,
+                                             float u, float tp, float te) {
+    r[0] = (float)time;
+    r[1] = s[IDX_ANGLE]; r[2] = s[IDX_ANGLED]; r[3] = (float)aDD; r[4] = s[IDX_COS]; r[5] = s[IDX_SIN];
+    r[6] = s[IDX_POS]; r[7] = s[IDX_POSD]; r[8] = (float)pDD;
+    r[9] = Qc; r[10] = Q; r[11] = u; r[12] = tp; r[13] = te; r[14] = 0.0f; r[15] = 0.0f;
+}
+
+// The n_sim ticks of one controller period with u held (CartPole/__init__.py:283-324): (aDD, pDD) enter as the second
+// derivatives of s and leave as those of the new state; on_tick(i) runs after tick i.  The caller computes the first pair
+// (plant_ode) itself: folding that and the record row in here changes how fleet_kernel's solve is scheduled.
+template <class Tick>
+__device__ __forceinline__ void plant_ticks(const PlantParams &P, float *s, float u, double &aDD, double &pDD, Tick on_tick) {
+    for (int i = 0; i < P.n_sim; ++i) {
+        plant_tick(P, s, aDD, pDD);
+        plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
+        on_tick(i);
     }
 }

@@ -62,9 +62,7 @@ struct RpgdRowArgs {
     float *s;                        // [E][8] <- the recorded states
     OdeParams *odes;                 // [E] <- per-experiment model constants, or null (neural, or no per-row L / m_pole)
     OdeParams ode;                   // the handle's fold (the constants that do not depend on L / m_pole)
-    float k, m_cart, g, J_fric, M_fric, u_max, m_pole_fixed;   // fold_ode_device's inputs
-    float L_default, mp_default;     // the handle's L / m_pole "for controller" when only one of the arrays is given
-    double h_step;
+    FoldInputs fold;
     int E;
 };
 
@@ -78,8 +76,8 @@ __global__ void __launch_bounds__(128) rpgd_relabel_row_kernel(const __grid_cons
     for (int c = 0; c < 6; ++c) a.s[(size_t)e * 8 + c] = a.states[(size_t)e * 6 + c];
     if (a.odes) {
         OdeParams o = a.ode;
-        fold_ode_device<CPS_EULER_CROMER>(a, a.L_row ? (double)a.L_row[e] : (double)a.L_default,
-                                          a.mp_row ? (double)a.mp_row[e] : (double)a.mp_default, o);
+        fold_ode_device<CPS_EULER_CROMER>(a.fold, a.L_row ? (double)a.L_row[e] : (double)a.fold.L_default,
+                                          a.mp_row ? (double)a.mp_row[e] : (double)a.fold.mp_default, o);
         a.odes[e] = o;
     }
 }
@@ -126,7 +124,7 @@ __global__ void __launch_bounds__(128) rpgd_fleet_draws_kernel(unsigned long lon
                                                                 unsigned e_offset, int rows, int n_ind, float *out) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x, e = blockIdx.y;
     if (r >= rows) return;
-    rpgd_draws(seed, tag, period, e_offset + (unsigned)e, (unsigned)r, n_ind, out + ((size_t)e * rows + r) * n_ind, 1);
+    philox_normals(seed, (unsigned)r, tag, period, e_offset + (unsigned)e, n_ind, out + ((size_t)e * rows + r) * n_ind, 1);
 }
 
 // optimizer_reset of every experiment (:379-408): plans from the draws [E * K][n_ind], zero moments and ages
@@ -180,7 +178,8 @@ __device__ __forceinline__ void rpgd_finish(const RpgdFinishArgs &a) {
     for (int i = tid; i < K; i += nt) s_J[i] = a.J[(size_t)e * K + i];
     if (a.philox)
         for (int r = tid; r < nf; r += nt)
-            rpgd_draws(a.seed, RPGD_DRAWS_RESAMPLE, a.period, a.e_offset + (unsigned)e, (unsigned)r, a.sp.n_ind, s_d + r * a.sp.n_ind, 1);
+            philox_normals(a.seed, (unsigned)r, RPGD_DRAWS_RESAMPLE, a.period, a.e_offset + (unsigned)e, a.sp.n_ind,
+                           s_d + r * a.sp.n_ind, 1);
     __syncthreads();
     for (int i = tid; i < K; i += nt) {   // plans in front of plan i in torch.sort(J, stable=True)'s order
         const float Ji = s_J[i];
@@ -228,17 +227,10 @@ __device__ __forceinline__ void rpgd_finish(const RpgdFinishArgs &a) {
     const float u = __fmul_rn(P.u_max, Qc);
     double aDD, pDD;
     plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
-    if (a.record) {
-        float *r = a.record + (size_t)e * CPS_FLEET_RECORD;
-        r[0] = (float)a.time;
-        r[1] = s[IDX_ANGLE]; r[2] = s[IDX_ANGLED]; r[3] = (float)aDD; r[4] = s[IDX_COS]; r[5] = s[IDX_SIN];
-        r[6] = s[IDX_POS]; r[7] = s[IDX_POSD]; r[8] = (float)pDD;
-        r[9] = Qc; r[10] = Qc; r[11] = u; r[12] = a.tp ? a.tp[e] : 0.0f; r[13] = a.te ? a.te[e] : 1.0f; r[14] = 0.0f; r[15] = 0.0f;
-    }
-    for (int i = 0; i < P.n_sim; ++i) {
-        plant_tick(P, s, aDD, pDD);
-        plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
-    }
+    if (a.record)
+        plant_record(a.record + (size_t)e * CPS_FLEET_RECORD, a.time, s, aDD, pDD, Qc, Qc, u, a.tp ? a.tp[e] : 0.0f,
+                     a.te ? a.te[e] : 1.0f);
+    plant_ticks(P, s, u, aDD, pDD, [](int) {});
     float *so = a.s + (size_t)e * 8;
 #pragma unroll
     for (int c = 0; c < 6; ++c) so[c] = s[c];
@@ -382,18 +374,9 @@ extern "C" int cps_rpgd_fleet_set_states(cps_handle *h, const float *s_host, con
     if (philox && init_draws_dev)
         return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_set_states: this fleet generates its draws (Philox); pass NULL");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    float *tmp = new (std::nothrow) float[(size_t)F->E * 8];
-    if (!tmp) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_set_states: out of host memory");
-    for (int e = 0; e < F->E; ++e) {
-        for (int c = 0; c < 6; ++c) tmp[(size_t)e * 8 + c] = s_host[(size_t)e * 6 + c];
-        tmp[(size_t)e * 8 + 6] = tmp[(size_t)e * 8 + 7] = 0.0f;
-    }
-    cudaError_t er = cudaMemcpyAsync(F->d_s, tmp, sizeof(float) * (size_t)F->E * 8, cudaMemcpyHostToDevice, h->stream);
-    if (er == cudaSuccess) er = cudaMemsetAsync(F->d_uprev, 0, sizeof(float) * (size_t)F->E, h->stream);
-    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
-    delete[] tmp;
-    CUDA_TRY(h, er);
+    CUDA_TRY(h, cudaMemsetAsync(F->d_uprev, 0, sizeof(float) * (size_t)F->E, h->stream));
     int rc;
+    if ((rc = fleet_states_to_device(h, s_host, F->d_s, F->E, "cps_rpgd_fleet_set_states")) != CPS_OK) return rc;
     if (philox && (rc = draws_launch(h, F, -1, F->d_draws)) != CPS_OK) return rc;
     F->cur = 0;
     const long long n = (long long)F->E * F->K * F->T;
@@ -439,11 +422,7 @@ static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, cons
     a.K = (int)K; a.T = (int)T; a.keep = c.opt_keep_k; a.shift = c.shift_previous;
     a.sp = sample_params(h, F);
     a.u_prev = F->d_uprev; a.s = F->d_s;
-    PlantParams &P = a.plant;
-    P.k = h->phys[CPS_PH_K]; P.m_cart = h->phys[CPS_PH_M_CART]; P.g = h->phys[CPS_PH_G]; P.J_fric = h->phys[CPS_PH_J_FRIC];
-    P.M_fric = h->phys[CPS_PH_M_FRIC]; P.u_max = h->phys[CPS_PH_U_MAX]; P.thl = h->phys[CPS_PH_TRACK_HALF_LENGTH];
-    P.L = (double)h->phys[CPS_PH_L]; P.m_pole = (double)h->phys[CPS_PH_M_POLE];
-    P.dt = c.dt_simulation; P.n_sim = c.sim_substeps;
+    a.plant = plant_params(h, c.dt_simulation, c.sim_substeps);
     const double dt_control = c.dt_simulation * c.sim_substeps;
     // relabelling: the network reads neither L nor m_pole, so only predictor "ODE" folds per-row model constants
     const OdeParams *odes = (replay_dev && !neural && (L_dev || mp_dev)) ? F->d_odes : nullptr;
@@ -452,10 +431,7 @@ static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, cons
     ra.up = up; ra.dn = dn;
     ra.costs = F->d_costs; ra.s = F->d_s; ra.odes = const_cast<OdeParams *>(odes);
     ra.ode = h->ode;
-    ra.k = P.k; ra.m_cart = P.m_cart; ra.g = P.g; ra.J_fric = P.J_fric; ra.M_fric = P.M_fric; ra.u_max = P.u_max;
-    ra.m_pole_fixed = h->phys[CPS_PH_M_POLE];
-    ra.L_default = h->L_var; ra.mp_default = h->m_pole_var;
-    ra.h_step = (double)h->cfg.dt / (double)h->cfg.substeps;
+    ra.fold = fold_inputs(h);
     ra.E = (int)E;
     for (int j = 0; j < n_periods; ++j) {
         const float *tp = tp_dev ? tp_dev + (size_t)j * E : nullptr, *te = te_dev ? te_dev + (size_t)j * E : nullptr;
@@ -533,17 +509,8 @@ extern "C" int cps_rpgd_fleet_get_states(cps_handle *h, float *s_host, float *u_
     if (!F || !F->ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_get_states: no RPGD fleet with states "
                                     "(cps_rpgd_fleet_create, cps_rpgd_fleet_set_states)");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (s_host) {
-        float *tmp = new (std::nothrow) float[(size_t)F->E * 8];
-        if (!tmp) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_get_states: out of host memory");
-        cudaError_t er = cudaMemcpyAsync(tmp, F->d_s, sizeof(float) * (size_t)F->E * 8, cudaMemcpyDeviceToHost, h->stream);
-        if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
-        if (er == cudaSuccess)
-            for (int e = 0; e < F->E; ++e)
-                for (int c = 0; c < 6; ++c) s_host[(size_t)e * 6 + c] = tmp[(size_t)e * 8 + c];
-        delete[] tmp;
-        CUDA_TRY(h, er);
-    }
+    int rc;
+    if (s_host && (rc = fleet_states_to_host(h, F->d_s, s_host, F->E, "cps_rpgd_fleet_get_states")) != CPS_OK) return rc;
     if (u_prev_host)
         CUDA_TRY(h, cudaMemcpyAsync(u_prev_host, F->d_uprev, sizeof(float) * (size_t)F->E, cudaMemcpyDeviceToHost, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));

@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from .core import Engine, _check_dev, _ptr
+from .core import Engine, _check_dev, _check_sizes, _ptr
 
 TRACK_HALF_LENGTH = float(np.float32((44.0e-2 - 4.4e-2) / 2.0))
 
@@ -161,6 +161,32 @@ def make_experiments(n_experiments: int, n_periods: int, cfg: DataGenConfig | No
     return s0, tp, te
 
 
+def _check_fleet_args(kind: str, integrator: str, network, noise: str, dt: float, dt_simulation: float) -> int:
+    """The checks Fleet and RpgdFleet make before they create a handle; returns the plant ticks per controller period."""
+    if integrator == "neural" and network is None:
+        raise NotImplementedError(f"{kind} with integrator='neural' needs the network: pass network=<spec dict as "
+                                  "Engine.net_load takes, e.g. neural.load_model(...)[0]>")
+    if network is not None and integrator != "neural":
+        raise ValueError(f"network= is the neural predictor's model; integrator={integrator!r} takes none")
+    if noise not in ("philox", "supplied"):
+        raise ValueError("noise must be 'philox' or 'supplied'")
+    n_sim = int(round(dt / dt_simulation))
+    if n_sim < 1 or abs(n_sim * dt_simulation - dt) > 1e-9:
+        raise ValueError("dt (control) must be a multiple of dt_simulation")
+    return n_sim
+
+
+def _relabel_rows(fleet, states, Q_out):
+    """The number of rows R of recorded states [R, E, 6] for `fleet`'s relabel, and Q_out (allocated [R, E] when None)."""
+    _check_dev(states, "states", fleet.device)
+    R = int(states.shape[0]) if states.dim() == 3 else -1
+    if tuple(states.shape) != (R, fleet.E, 6):
+        raise ValueError(f"states has shape {tuple(states.shape)}, expected (rows, {fleet.E}, 6)")
+    if Q_out is None:
+        Q_out = torch.empty((R, fleet.E), device=fleet.device, dtype=torch.float32)
+    return R, Q_out
+
+
 class Fleet:
     """E closed-loop experiments on one device = one cps_handle with a fleet attached.
 
@@ -176,13 +202,7 @@ class Fleet:
                  interp_period: int = 10, device: int | None = None, noise: str = "philox", seed: int = 0,
                  experiment_offset: int = 0, dt_simulation: float = 0.002, no_pairs: bool = False,
                  network: dict | None = None, net_kernel: str | None = None):
-        if integrator == "neural" and network is None:
-            raise NotImplementedError("Fleet with integrator='neural' needs the network: pass network=<spec dict as "
-                                      "Engine.net_load takes, e.g. neural.load_model(...)[0]>")
-        if network is not None and integrator != "neural":
-            raise ValueError(f"network= is the neural predictor's model; integrator={integrator!r} takes none")
-        if noise not in ("philox", "supplied"):
-            raise ValueError("noise must be 'philox' or 'supplied'")
+        n_sim = _check_fleet_args("Fleet", integrator, network, noise, dt, dt_simulation)
         self.engine = Engine(num_rollouts, horizon, dt=dt, substeps=substeps, integrator=integrator, cost=cost,
                              interp_period=interp_period, device=device, no_pairs=no_pairs, net_kernel=net_kernel)
         self.neural = network is not None
@@ -190,9 +210,6 @@ class Fleet:
             self.engine.net_load(network)
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(horizon)
         self.n_ind, self.device = self.engine.n_ind, self.engine.device
-        n_sim = int(round(dt / dt_simulation))
-        if abs(n_sim * dt_simulation - dt) > 1e-9:
-            raise ValueError("dt (control) must be a multiple of dt_simulation")
         c = L.cps_fleet_config(C.sizeof(L.cps_fleet_config), self.E, n_sim,
                                L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
                                float(dt_simulation), int(seed), int(experiment_offset))
@@ -284,15 +301,11 @@ class Fleet:
         (cps_fleet_step_noisy); a 'philox' fleet draws them itself when they are None."""
         eng = self.engine
         eng.use_current_stream()
-        for t, name, numel in ((target_position, "target_position", n_periods * self.E),
-                               (target_equilibrium, "target_equilibrium", n_periods * self.E),
-                               (noise, "noise", n_periods * self.E * self.n_ind * self.K),
-                               (record, "record", n_periods * self.E * L.FLEET_RECORD),
-                               (J_out, "J_out", n_periods * self.E * self.K)):
-            if t is not None:
-                _check_dev(t, name, self.device)
-                if t.numel() != numel:
-                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+        _check_sizes(self.device, (target_position, "target_position", n_periods * self.E),
+                     (target_equilibrium, "target_equilibrium", n_periods * self.E),
+                     (noise, "noise", n_periods * self.E * self.n_ind * self.K),
+                     (record, "record", n_periods * self.E * L.FLEET_RECORD),
+                     (J_out, "J_out", n_periods * self.E * self.K))
         if getattr(self, "plant_models", False):
             for t, name in ((ctrl_draws, "ctrl_draws"), (meas_draws, "meas_draws")):
                 if t is not None:
@@ -303,6 +316,34 @@ class Fleet:
         eng._chk(eng.lib.cps_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
                                         _ptr(noise), _ptr(record), _ptr(J_out)))
         return record
+
+    def relabel(self, states, target_position=None, target_equilibrium=None, L=None, m_pole=None, noise=None, Q_out=None,
+                J_out=None, active=None):
+        """cps_fleet_relabel: one controller step per recorded row, experiment e = file e, from the recorded states
+        (cuda tensor [R, E, 6]) instead of the plant; no synchronisation.  target_position / target_equilibrium / L / m_pole:
+        cuda tensors [R, E] or None; noise [R, E, n_ind, K] for a 'supplied' fleet; Q_out [R, E] (allocated when None)
+        receives the controls; J_out [R, E, K] or None; active [R, E] int32 or None: files with 0 sit the row out
+        (cps_fleet_relabel_masked).  Zeroing the warm starts first (Relabeller.reset: cps_fleet_reset) is the reference's
+        controller.reset().  Returns Q_out."""
+        eng = self.engine
+        eng.use_current_stream()
+        R, Q_out = _relabel_rows(self, states, Q_out)
+        _check_sizes(self.device, (target_position, "target_position", R * self.E),
+                     (target_equilibrium, "target_equilibrium", R * self.E),
+                     (L, "L", R * self.E), (m_pole, "m_pole", R * self.E),
+                     (noise, "noise", R * self.E * self.n_ind * self.K),
+                     (Q_out, "Q_out", R * self.E), (J_out, "J_out", R * self.E * self.K))
+        if active is None:
+            eng._chk(eng.lib.cps_fleet_relabel(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
+                                               _ptr(L), _ptr(m_pole), _ptr(noise), _ptr(Q_out), _ptr(J_out)))
+            return Q_out
+        _check_dev(active, "active", self.device, dtype=torch.int32)
+        if active.numel() != R * self.E:
+            raise ValueError("active must be an int32 tensor of shape [rows, files]")
+        eng._chk(eng.lib.cps_fleet_relabel_masked(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
+                                                  _ptr(L), _ptr(m_pole), _ptr(noise), _ptr(Q_out), _ptr(J_out),
+                                                  _ptr(active)))
+        return Q_out
 
 
 class RpgdFleet:
@@ -330,20 +371,11 @@ class RpgdFleet:
                  substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
                  cost_config: dict | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
                  experiment_offset: int = 0, dt_simulation: float = 0.002, network: dict | None = None):
-        if integrator == "neural" and network is None:
-            raise NotImplementedError("RpgdFleet with integrator='neural' needs the network: pass network=<spec dict as "
-                                      "Engine.net_load takes, e.g. neural.load_model(...)[0]>")
-        if network is not None and integrator != "neural":
-            raise ValueError(f"network= is the neural predictor's model; integrator={integrator!r} takes none")
+        n_sim = _check_fleet_args("RpgdFleet", integrator, network, noise, dt, dt_simulation)
         if SAMPLING_DISTRIBUTION == "uniform":
             raise NotImplementedError("RpgdFleet resamples from the normal distribution only (SAMPLING_DISTRIBUTION='normal')")
         if SAMPLING_DISTRIBUTION != "normal":
             raise ValueError(f"RPGD cannot interpret sampling type {SAMPLING_DISTRIBUTION}")
-        if noise not in ("philox", "supplied"):
-            raise ValueError("noise must be 'philox' or 'supplied'")
-        n_sim = int(round(dt / dt_simulation))
-        if n_sim < 1 or abs(n_sim * dt_simulation - dt) > 1e-9:
-            raise ValueError("dt (control) must be a multiple of dt_simulation")
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
         self.outer_its, self.resamp_per, self.shift_previous = int(outer_its), int(resamp_per), int(shift_previous)
         self.first_iter_count = int(warmup_iterations) if warmup else self.outer_its   # as optimizer_rpgd_b200
@@ -378,10 +410,7 @@ class RpgdFleet:
         s = np.ascontiguousarray(states, dtype=np.float32)
         if s.shape != (self.E, 6):
             raise ValueError(f"states must have shape ({self.E}, 6)")
-        if init_draws is not None:
-            _check_dev(init_draws, "init_draws", self.device)
-            if init_draws.numel() != self.E * self.K * self.n_ind:
-                raise ValueError(f"init_draws has {init_draws.numel()} elements, expected {self.E * self.K * self.n_ind}")
+        _check_sizes(self.device, (init_draws, "init_draws", self.E * self.K * self.n_ind))
         self.engine.use_current_stream()
         self.engine._chk(self.engine.lib.cps_rpgd_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP),
                                                                    _ptr(init_draws), int(period)))
@@ -433,44 +462,33 @@ class RpgdFleet:
         Q_opt [n_periods, E, K, T] (plans after the Adam steps) or None."""
         eng = self.engine
         eng.use_current_stream()
-        for t, name, numel in ((target_position, "target_position", n_periods * self.E),
-                               (target_equilibrium, "target_equilibrium", n_periods * self.E),
-                               (draws, "draws", n_periods * self.E * (self.K - self.opt_keep_k) * self.n_ind),
-                               (record, "record", n_periods * self.E * L.FLEET_RECORD),
-                               (J_out, "J_out", n_periods * self.E * self.K),
-                               (Q_opt, "Q_opt", n_periods * self.E * self.K * self.T)):
-            if t is not None:
-                _check_dev(t, name, self.device)
-                if t.numel() != numel:
-                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+        _check_sizes(self.device, (target_position, "target_position", n_periods * self.E),
+                     (target_equilibrium, "target_equilibrium", n_periods * self.E),
+                     (draws, "draws", n_periods * self.E * (self.K - self.opt_keep_k) * self.n_ind),
+                     (record, "record", n_periods * self.E * L.FLEET_RECORD),
+                     (J_out, "J_out", n_periods * self.E * self.K),
+                     (Q_opt, "Q_opt", n_periods * self.E * self.K * self.T))
         eng._chk(eng.lib.cps_rpgd_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
                                              _ptr(draws), _ptr(record), _ptr(J_out), _ptr(Q_opt)))
         return record
 
     def relabel(self, states, target_position=None, target_equilibrium=None, L=None, m_pole=None, draws=None, Q_out=None,
-                J_out=None):
+                J_out=None, active=None):
         """cps_rpgd_fleet_relabel: one controller step per recorded row, experiment e = file e, from the recorded states
         (cuda tensor [R, E, 6]) instead of the plant; no synchronisation.  target_position / target_equilibrium / L / m_pole:
         cuda tensors [R, E] or None (L / m_pole change predictor "ODE"'s model; the network reads neither); draws as in
         run(); Q_out [R, E] (allocated when None) receives the controls; J_out [R, E, K] or None.  reset() first is the
-        reference's controller.reset().  Returns Q_out."""
+        reference's controller.reset().  Returns Q_out.  `active` (Fleet.relabel's per-file mask) is not implemented."""
+        if active is not None:
+            raise NotImplementedError("RPGD relabelling advances every file in lockstep: no per-file mask")
         eng = self.engine
         eng.use_current_stream()
-        _check_dev(states, "states", self.device)
-        R = int(states.shape[0]) if states.dim() == 3 else -1
-        if tuple(states.shape) != (R, self.E, 6):
-            raise ValueError(f"states has shape {tuple(states.shape)}, expected (rows, {self.E}, 6)")
-        if Q_out is None:
-            Q_out = torch.empty((R, self.E), device=self.device, dtype=torch.float32)
-        for t, name, numel in ((target_position, "target_position", R * self.E),
-                               (target_equilibrium, "target_equilibrium", R * self.E),
-                               (L, "L", R * self.E), (m_pole, "m_pole", R * self.E),
-                               (draws, "draws", R * self.E * (self.K - self.opt_keep_k) * self.n_ind),
-                               (Q_out, "Q_out", R * self.E), (J_out, "J_out", R * self.E * self.K)):
-            if t is not None:
-                _check_dev(t, name, self.device)
-                if t.numel() != numel:
-                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
+        R, Q_out = _relabel_rows(self, states, Q_out)
+        _check_sizes(self.device, (target_position, "target_position", R * self.E),
+                     (target_equilibrium, "target_equilibrium", R * self.E),
+                     (L, "L", R * self.E), (m_pole, "m_pole", R * self.E),
+                     (draws, "draws", R * self.E * (self.K - self.opt_keep_k) * self.n_ind),
+                     (Q_out, "Q_out", R * self.E), (J_out, "J_out", R * self.E * self.K))
         eng._chk(eng.lib.cps_rpgd_fleet_relabel(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
                                                 _ptr(L), _ptr(m_pole), _ptr(draws), _ptr(Q_out), _ptr(J_out)))
         return Q_out

@@ -34,9 +34,7 @@ from math import ceil
 import numpy as np
 import torch
 
-from . import _lib as L
 from . import config as cfgmod
-from .core import _check_dev, _ptr
 from .fleet import Fleet, RpgdFleet
 
 STATE_COMPONENTS = ("angle", "angleD", "angle_cos", "angle_sin", "position", "positionD")  # CartPole/state_utilities.py
@@ -101,42 +99,11 @@ class Relabeller:
 
     def relabel_device(self, states, target_position=None, target_equilibrium=None, pole_length=None, m_pole=None,
                        noise=None, Q_out=None, J_out=None, active=None):
-        """cps_fleet_relabel on cuda tensors: states [R, E, 6]; attributes [R, E] or None; noise [R, E, n_ind, K] for a
+        """Fleet.relabel on cuda tensors: states [R, E, 6]; attributes [R, E] or None; noise [R, E, n_ind, K] for a
         'supplied' fleet; active [R, E] int32 or None: files with 0 sit the row out (cps_fleet_relabel_masked).
-        RPGD: cps_rpgd_fleet_relabel, noise = the resampling draws [R, E, K - opt_keep_k, n_ind] of a 'supplied' fleet;
+        RPGD: RpgdFleet.relabel, noise = the resampling draws [R, E, K - opt_keep_k, n_ind] of a 'supplied' fleet;
         no `active`.  Returns Q_out [R, E] (no synchronisation)."""
-        if self.optimizer == "rpgd":
-            if active is not None:
-                raise NotImplementedError("RPGD relabelling advances every file in lockstep: no per-file mask")
-            return self.fleet.relabel(states, target_position, target_equilibrium, pole_length, m_pole, noise, Q_out, J_out)
-        eng = self.engine
-        eng.use_current_stream()
-        _check_dev(states, "states", self.device)
-        R = int(states.shape[0])
-        if tuple(states.shape) != (R, self.E, 6):
-            raise ValueError(f"states has shape {tuple(states.shape)}, expected (rows, {self.E}, 6)")
-        for t, name, numel in ((target_position, "target_position", R * self.E),
-                               (target_equilibrium, "target_equilibrium", R * self.E),
-                               (pole_length, "pole_length", R * self.E), (m_pole, "m_pole", R * self.E),
-                               (noise, "noise", R * self.E * self.n_ind * self.K), (J_out, "J_out", R * self.E * self.K)):
-            if t is not None:
-                _check_dev(t, name, self.device)
-                if t.numel() != numel:
-                    raise ValueError(f"{name} has {t.numel()} elements, expected {numel}")
-        if Q_out is None:
-            Q_out = torch.empty((R, self.E), device=self.device, dtype=torch.float32)
-        _check_dev(Q_out, "Q_out", self.device)
-        if active is not None:
-            _check_dev(active, "active", self.device, dtype=torch.int32)
-            if active.dtype != torch.int32 or active.numel() != R * self.E:
-                raise ValueError("active must be an int32 tensor of shape [rows, files]")
-            eng._chk(eng.lib.cps_fleet_relabel_masked(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
-                                                      _ptr(pole_length), _ptr(m_pole), _ptr(noise), _ptr(Q_out), _ptr(J_out),
-                                                      _ptr(active)))
-            return Q_out
-        eng._chk(eng.lib.cps_fleet_relabel(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
-                                           _ptr(pole_length), _ptr(m_pole), _ptr(noise), _ptr(Q_out), _ptr(J_out)))
-        return Q_out
+        return self.fleet.relabel(states, target_position, target_equilibrium, pole_length, m_pole, noise, Q_out, J_out, active)
 
     def relabel(self, states, target_position=None, target_equilibrium=None, pole_length=None, m_pole=None, noise=None,
                 chunk_rows: int = 4096) -> np.ndarray:
