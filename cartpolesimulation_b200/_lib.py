@@ -71,6 +71,13 @@ class cps_rpgd_fleet_config(C.Structure):
                 ("sample_mean", C.c_float)]
 
 
+class cps_cem_fleet_config(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("n_experiments", C.c_int), ("sim_substeps", C.c_int),
+                ("draw_source", C.c_int), ("dt_simulation", C.c_double), ("seed", C.c_ulonglong),
+                ("experiment_offset", C.c_longlong), ("outer_its", C.c_int), ("first_iter_count", C.c_int),
+                ("best_k", C.c_int), ("initial_stdev", C.c_float), ("stdev_min", C.c_float)]
+
+
 # name -> (restype, argtypes); every symbol include/cps.h declares
 _FP = C.POINTER(C.c_float)
 _VP = C.c_void_p
@@ -140,6 +147,13 @@ SYMBOLS = {
                                            C.POINTER(C.c_longlong)]),
     "cps_rpgd_fleet_period": (C.c_longlong, [_VP]),
     "cps_rpgd_fleet_draws": (C.c_int, [_VP, C.c_longlong, _VP]),
+    "cps_cem_fleet_create": (C.c_int, [_VP, C.POINTER(cps_cem_fleet_config)]),
+    "cps_cem_fleet_set_states": (C.c_int, [_VP, _FP, C.c_longlong]),
+    "cps_cem_fleet_get_states": (C.c_int, [_VP, _FP, _FP]),
+    "cps_cem_fleet_get_distribution": (C.c_int, [_VP, _FP, _FP]),
+    "cps_cem_fleet_step": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "cps_cem_fleet_draws": (C.c_int, [_VP, C.c_longlong, _VP]),
+    "cps_cem_fleet_period": (C.c_longlong, [_VP]),
     "cps_plan_cost": (C.c_int, [_VP, _VP, _VP, C.c_int, C.c_int, C.c_int, C.c_float, _VP, _VP, C.c_int]),
     "cps_plan_random_action": (C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, _VP, _VP, _VP]),
     "cps_plan_random_action_host": (C.c_int, [_VP, _FP, _VP, C.c_int, C.c_float, _FP]),

@@ -246,16 +246,8 @@ __global__ void __launch_bounds__(256, 4) fleet_kernel(const __grid_constant__ F
 
 // Neural fleets (CPS_PREDICTOR_NEURAL): the solve is net_kernel / net_tc_kernel<.., FLEET> (cps_net.cu, cps_net_tc.cu),
 // which leaves each experiment's u in u_prev[e]; this kernel is the plant period that follows, one thread per experiment:
-// fleet_kernel's record row and plant with Q_applied = Q (plant-side models are not offered on neural fleets).
-struct NetPlantArgs {
-    PlantParams plant;
-    float *s;                   // [E][8]
-    const float *u;             // [E] the controls the solve just chose
-    const float *tp, *te;       // [E] targets of this period (null: 0 / +1)
-    float *record;              // [E][CPS_FLEET_RECORD] of this period, or null
-    double time;                // period * dt_control
-    int E;
-};
+// fleet_kernel's record row and plant with Q_applied = Q (plant-side models are not offered on neural fleets).  CEM
+// fleets (cps_cem_fleet.cu) end their periods with it too.
 __global__ void __launch_bounds__(128) fleet_net_plant_kernel(const __grid_constant__ NetPlantArgs a) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= a.E) return;
@@ -274,6 +266,13 @@ __global__ void __launch_bounds__(128) fleet_net_plant_kernel(const __grid_const
     float *so = a.s + (size_t)e * 8;
 #pragma unroll
     for (int c = 0; c < 6; ++c) so[c] = s[c];
+}
+
+int fleet_plant_launch(cps_handle *h, const NetPlantArgs &a) {
+    fleet_net_plant_kernel<<<(a.E + 127) / 128, 128, 0, h->stream>>>(a);
+    h->launches += 1;
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
 }
 
 // (Re)start of the observation chain: ring = the reference's initial buffer (zeros, cos = 1, latency_adder.py:26-28), nothing
@@ -671,8 +670,7 @@ static int fleet_step_neural(cps_handle *h, int n_periods, const float *tp_dev, 
         pa.tp = tp; pa.te = te;
         pa.record = record_dev ? record_dev + (size_t)j * E * CPS_FLEET_RECORD : nullptr;
         pa.time = (double)F->period * dt_control;
-        fleet_net_plant_kernel<<<(F->E + 127) / 128, 128, 0, h->stream>>>(pa);
-        h->launches += 1;
+        if ((rc = fleet_plant_launch(h, pa)) != CPS_OK) return rc;
         F->period += 1;
     }
     CUDA_TRY(h, cudaGetLastError());

@@ -66,6 +66,7 @@ struct FinalizeArgs {
 struct NetState;    // cps_net.cu
 struct FleetState;  // cps_fleet.cu
 struct RpgdFleetState;  // cps_rpgd_fleet.cu
+struct CemFleetState;   // cps_cem_fleet.cu
 struct PlanState;   // cps_plan.cu
 struct GmmState;    // cps_gmm.cu
 struct GradState;   // cps_grad.cu
@@ -117,6 +118,7 @@ struct cps_handle {
     GmmState *gmm;      // CEM with a Gaussian-mixture sampling distribution (cps_cem_gmm_*), owned
     GradState *grad;    // adjoint workspace and Adam moments (cps_plan_cost_grad, cps_rpgd_*), owned
     RpgdFleetState *rfleet;  // closed-loop experiments under RPGD (cps_rpgd_fleet_create), owned
+    CemFleetState *cfleet;   // closed-loop experiments under CEM (cps_cem_fleet_create), owned
 };
 
 extern thread_local std::string g_create_err;
@@ -141,8 +143,32 @@ int fleet_states_to_device(cps_handle *h, const float *s_host, float *s_dev, int
 int fleet_states_to_host(cps_handle *h, const float *s_dev, float *s_host, int E, const char *who);
 // cps_rpgd_fleet.cu
 void cps_rpgd_fleet_free(cps_handle *h);
+// cps_cem_fleet.cu
+void cps_cem_fleet_free(cps_handle *h);
 // cps_plan.cu
 void cps_plan_free(cps_handle *h);
+// CEM fleets: the refusals of cps_cem_fleet_create that concern the planner (those of cps_cem_configure, K above the
+// single-block selection, shared memory of plan_fleet_kernel), and one outer iteration of E experiments: plan_fleet_kernel,
+// then cem_update_fleet_kernel when best_k x T > 2048 (h->launches counts them)
+struct CemFleetIteration {
+    int E, best_k, last_iter;
+    float sd_init, sd_min;
+    const float *s;              // [E][8] states
+    float *u;                    // [E] u_prev of the costs; <- u = elite_Q[0, 0] after the last iteration
+    const float *tp, *te;        // [E] targets of this period (null: 0 / +1)
+    CostParams cost_up, cost_dn; // folded for target_equilibrium = +1 / -1
+    const float *mu, *sd;        // [E][T] the distribution the plans are drawn from
+    float *mu_out, *sd_out;      // [E][T] <- the updated one (clipped and shifted after the last iteration)
+    const float *eps;            // [E][T][K] supplied draws, or null: Philox, counter (plan, w1 + group, period, e_offset + e)
+    unsigned long long seed;
+    unsigned w1, period, e_offset;
+    float *J;                    // [E][K] <- the costs
+    float *Q_out;                // [E][T][K] <- the plans, or null
+    int *elite;                  // [E][K] scratch of the deferred statistics
+    unsigned *tickets;           // [E], zero between launches
+};
+int cps_cem_fleet_check(cps_handle *h, int best_k, float initial_stdev, float stdev_min, int philox, const char *who);
+int cps_cem_fleet_iteration(cps_handle *h, const CemFleetIteration &c);
 // cps_gmm.cu
 void cps_gmm_free(cps_handle *h);
 // cps_grad.cu

@@ -408,6 +408,7 @@ extern "C" void cps_destroy(cps_handle *h) {
     cps_net_free(h);
     cps_fleet_free(h);
     cps_rpgd_fleet_free(h);
+    cps_cem_fleet_free(h);
     cps_plan_free(h);
     cps_gmm_free(h);
     cps_grad_free(h);

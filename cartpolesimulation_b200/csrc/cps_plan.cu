@@ -22,6 +22,7 @@
 #include <new>
 
 #include "cps_internal.cuh"
+#include "cps_plant.cuh"
 
 enum { PLAN_Q = 0, PLAN_CEM = 1 };
 enum { SELECT_NONE = 0, SELECT_ARGMIN = 1, SELECT_CEM = 2 };
@@ -58,6 +59,17 @@ struct PlanArgs {
     float *u_out;                 // [1]
     int *best_out;                // [1] or null: index of the cheapest plan
     int *nonfinite;
+};
+
+// CEM fleets (cps_cem_fleet.cu): the inputs of E experiments, read by plan_fleet_kernel / cem_update_fleet_kernel besides
+// PlanArgs.  There PlanArgs' pointers are the fleet's bases and block (., e) offsets them to experiment e: J and elite
+// [E][K], mu / sd / mu_out / sd_out [E][T], Q (supplied draws) and Q_out [E][T][K] (qs_k = 1, qs_t = K), u_out [E], ticket [E].
+struct PlanFleetExt {
+    const float *s;               // [E][8] states
+    const float *tp, *te;         // [E] targets of this period (null: 0 / +1)
+    CostParams cost_up, cost_dn;  // folded for target_equilibrium = +1 / -1
+    unsigned long long seed;      // Philox draws: counter (plan, w1 + group, period, e_offset + e)
+    unsigned w1, period, e_offset;
 };
 
 struct PlanState {
@@ -517,28 +529,159 @@ __global__ void __launch_bounds__(256) cem_update_kernel(const __grid_constant__
     }
 }
 
+// ---- CEM fleets: the selection and statistics of experiment x = blockIdx.y --------------------------------------------------
+// Draw eps[k][t] of experiment x in the iteration `a` describes: supplied [E][T][K], or Philox (group t / 4 of plan k).
+template <bool PHILOX>
+__device__ __forceinline__ float fleet_draw(const PlanArgs &a, const PlanFleetExt &fx, long long x, int k, int t) {
+    if (!PHILOX) return a.Q[(x * a.T + t) * a.K + k];
+    float n[4];
+    philox_normals(fx.seed, (unsigned)k, fx.w1 + (unsigned)(t >> 2), fx.period, fx.e_offset + (unsigned)x, 4, n, 1);
+    const int c = t & 3;
+    return c == 0 ? n[0] : (c == 1 ? n[1] : (c == 2 ? n[2] : n[3]));
+}
+
+// Run by the last block of experiment x: plan_select on the experiment's K costs (from a copy of the arguments pointed at
+// the experiment, stopping after the elite list), then what plan_select does after it -- u after the last iteration, the
+// statistics (deferred to cem_update_fleet_kernel above 2048 elite entries) -- with the same arithmetic in the same order.
+// PHILOX: the elites' draws are regenerated into s_eps [best_k][T] first.
+template <bool PHILOX>
+__device__ __forceinline__ void cem_fleet_select(const PlanArgs &a, const PlanFleetExt &fx, const float *s_mu,
+                                                 const float *s_sd, float *s_mu2, float *s_sd2, int *s_elite, float *s_eps) {
+    __shared__ PlanArgs s_a;
+    __shared__ int s_best;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nt = blockDim.x, nwarps = nt >> 5;
+    const int K = a.K, T = a.T, bk = min(a.best_k, K);
+    const long long x = blockIdx.y;
+    if (tid == 0) {
+        s_a = a;
+        s_a.J = a.J + x * K;
+        s_a.elite = a.elite + x * K;   // used when the list does not fit in shared memory (deferred statistics)
+        s_a.best_out = &s_best;
+        s_a.defer_stats = 1;   // stop after the elite list ...
+        s_a.last_iter = 0;     // ... without reading the draws
+    }
+    __syncthreads();
+    plan_select<PLAN_CEM>(s_a, s_mu, s_sd, s_mu2, s_sd2, s_elite);   // ends with the elite list visible to the block
+    if (a.last_iter && tid == 0)   // u = elite_Q[0, 0]; thread 0 wrote s_best
+        a.u_out[x] = cem_plan_value(s_mu[0], fleet_draw<PHILOX>(a, fx, x, s_best, 0), s_sd[0], a.lo, a.hi);
+    if (a.defer_stats) return;
+    const int *elite = s_elite;   // statistics here: best_k x T <= 2048, the list is in shared memory
+    if (PHILOX) {
+        const int G4 = (T + 3) / 4;
+        for (int i = tid; i < bk * G4; i += nt) {
+            const int pos = i / G4, g = i - pos * G4;
+            philox_normals(fx.seed, (unsigned)elite[pos], fx.w1 + (unsigned)g, fx.period, fx.e_offset + (unsigned)x,
+                           min(4, T - 4 * g), s_eps + pos * T + 4 * g, 1);
+        }
+        __syncthreads();
+    }
+    const float *Q = a.Q + x * T * K;   // supplied draws of the experiment, [T][K]
+    for (int t = warp; t < T; t += nwarps) {   // as plan_select
+        float sum = 0.0f;
+        for (int e = lane; e < bk; e += 32)
+            sum += cem_plan_value(s_mu[t], PHILOX ? s_eps[e * T + t] : Q[(long long)t * K + elite[e]], s_sd[t], a.lo, a.hi);
+        const float mean = __fdiv_rn(warp_sum(sum), (float)bk);
+        float ss = 0.0f;
+        for (int e = lane; e < bk; e += 32) {
+            const float d =
+                cem_plan_value(s_mu[t], PHILOX ? s_eps[e * T + t] : Q[(long long)t * K + elite[e]], s_sd[t], a.lo, a.hi) - mean;
+            ss = fmaf(d, d, ss);
+        }
+        const float var = __fdiv_rn(warp_sum(ss), (float)bk);
+        if (lane == 0) { s_mu2[t] = mean; s_sd2[t] = sqrtf(var); }
+    }
+    __syncthreads();
+    float *mu_out = a.mu_out + x * T, *sd_out = a.sd_out + x * T;
+    for (int t = tid; t < T; t += nt) {
+        if (!a.last_iter) {
+            mu_out[t] = s_mu2[t];
+            sd_out[t] = s_sd2[t];
+        } else if (t + 1 < T) {
+            mu_out[t] = s_mu2[t + 1];
+            sd_out[t] = clampf(s_sd2[t + 1], a.sd_min, 1.0e8f);
+        } else {
+            mu_out[t] = a.mid;
+            sd_out[t] = a.sd_init;
+        }
+    }
+}
+
+// cem_update_kernel for fleets: block (t, x) updates step t of experiment x, same arithmetic in the same order.
+template <bool PHILOX>
+__global__ void __launch_bounds__(256) cem_update_fleet_kernel(const __grid_constant__ PlanArgs a,
+                                                               const __grid_constant__ PlanFleetExt fx) {
+    __shared__ float s_part[8];
+    __shared__ float s_bc;
+    const int t = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int bk = min(a.best_k, a.K), T = a.T;
+    const long long x = blockIdx.y;
+    const float mu = a.mu[x * T + t], sd = a.sd[x * T + t];
+    const int *elite = a.elite + x * a.K;
+    float sum = 0.0f;
+    for (int e = tid; e < bk; e += 256) sum += cem_plan_value(mu, fleet_draw<PHILOX>(a, fx, x, elite[e], t), sd, a.lo, a.hi);
+    sum = warp_sum(sum);
+    if (lane == 0) s_part[warp] = sum;
+    __syncthreads();
+    if (tid == 0) {
+        float v = 0.0f;
+        for (int w = 0; w < 8; ++w) v += s_part[w];
+        s_bc = __fdiv_rn(v, (float)bk);
+    }
+    __syncthreads();
+    const float mean = s_bc;
+    float ss = 0.0f;
+    for (int e = tid; e < bk; e += 256) {
+        const float d = cem_plan_value(mu, fleet_draw<PHILOX>(a, fx, x, elite[e], t), sd, a.lo, a.hi) - mean;
+        ss = fmaf(d, d, ss);
+    }
+    ss = warp_sum(ss);
+    __syncthreads();
+    if (lane == 0) s_part[warp] = ss;
+    __syncthreads();
+    if (tid != 0) return;
+    float v = 0.0f;
+    for (int w = 0; w < 8; ++w) v += s_part[w];
+    const float stdev = sqrtf(__fdiv_rn(v, (float)bk));
+    float *mu_out = a.mu_out + x * T, *sd_out = a.sd_out + x * T;
+    if (!a.last_iter) {
+        mu_out[t] = mean;
+        sd_out[t] = stdev;
+    } else {   // clip, shift by one step, refill the tail (cem_tf.py:96-99)
+        if (t > 0) { mu_out[t - 1] = mean; sd_out[t - 1] = clampf(stdev, a.sd_min, 1.0e8f); }
+        if (t == T - 1) { mu_out[t] = a.mid; sd_out[t] = a.sd_init; }
+    }
+}
+
 // NSUB = 10: the substeps of the predictors' operating point unrolled (control_step); 0: a.ode.n substeps in a loop.
-template <int INTEG, int COST, int MODE, int NSUB = 0>
-__global__ void __launch_bounds__(256, 4) plan_kernel(const __grid_constant__ PlanArgs a) {
-    extern __shared__ float smem[];   // PLAN_CEM: mu[T], sd[T], mu2[T], sd2[T], elite list [elite_smem]
+// FLEET (PLAN_CEM, plan_fleet_kernel): block (b, e) evaluates plans b * 256.. of experiment e from its state, distribution,
+// u_prev and cost parameters `cost`; the last block of the experiment (its own ticket) selects on its K costs.  PHILOX:
+// the draws come from Philox in the rollout thread, four per call as the horizon advances.  FLEET = false compiles to
+// the code plan_kernel compiled to before the fleet existed.
+template <int INTEG, int COST, int MODE, int NSUB, bool FLEET, bool PHILOX>
+__device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt *fx, const CostParams &cost) {
+    extern __shared__ float smem[];   // PLAN_CEM: mu[T], sd[T], mu2[T], sd2[T], elite list [elite_smem], PHILOX: elites' draws
     __shared__ unsigned s_ticket;
     const int tid = threadIdx.x, T = a.T;
+    const long long x = FLEET ? blockIdx.y : 0;   // the experiment
     float *s_mu = smem, *s_sd = smem + T;
     if (MODE == PLAN_CEM) {
-        for (int t = tid; t < T; t += blockDim.x) { s_mu[t] = a.mu[t]; s_sd[t] = a.sd[t]; }
+        for (int t = tid; t < T; t += blockDim.x) { s_mu[t] = a.mu[x * T + t]; s_sd[t] = a.sd[x * T + t]; }
         __syncthreads();
     }
     const int k = blockIdx.x * blockDim.x + tid;
     const bool active = k < a.K;
     const int kc = min(k, a.K - 1);
 
-    State z = load_state(a.use_inline ? a.s_inline : a.s);
+    State z = load_state(FLEET ? fx->s + x * 8 : (a.use_inline ? a.s_inline : a.s));
     const OdeParams ode = pin_params(a.ode, z.th);
     float c_cost = cosf(z.th);  // the plugins take cos(angle) of the stored angle (default.py:34)
-    const float *q = a.Q + (long long)kc * a.qs_k;
-    float *qo = (MODE == PLAN_CEM && a.Q_out) ? a.Q_out + (long long)kc * a.qs_k : nullptr;
-    float *traj = a.traj_out ? a.traj_out + (long long)kc * a.ts_k : nullptr;
-    float Jacc = 0.0f, up = a.u_prev;
+    // FLEET: plan kc of experiment x in the [E][T][K] draws / plans, one offset for both (qs_k = 1, qs_t = K)
+    const long long qoff = x * T * a.K + kc;
+    const float *q = FLEET ? a.Q + qoff : a.Q + (long long)kc * a.qs_k;
+    float *qo = (MODE == PLAN_CEM && a.Q_out) ? (FLEET ? a.Q_out + qoff : a.Q_out + (long long)kc * a.qs_k) : nullptr;
+    float *traj = (!FLEET && a.traj_out) ? a.traj_out + (long long)kc * a.ts_k : nullptr;   // fleets write no trajectories
+    float Jacc = 0.0f, up = FLEET ? a.u_out[x] : a.u_prev;
+    float nr[4];   // PHILOX: the draws of the current group of four steps, consumed from nr[0]
     // default / quadratic_boundary: the T+1 entries are summed in the reference backend's order (cps_device.cuh RowSumPlan)
     constexpr bool ROWSUM = (COST == COST_DEFAULT || COST == COST_QB);
     const RowSumPlan rsp = row_sum_plan(T + 1);
@@ -546,18 +689,26 @@ __global__ void __launch_bounds__(256, 4) plan_kernel(const __grid_constant__ Pl
     const int ss = blockDim.x;
     float rs_tail = 0.0f;
     if (ROWSUM) row_sum_init(rsp, sl, ss);
-    float qn = q[0];
+    float qn = PHILOX ? 0.0f : q[0];
 #pragma unroll 1
     for (int t = 0; t < T; ++t) {
         float u = qn;
-        if (t + 1 < T) qn = q[(long long)(t + 1) * a.qs_t];  // prefetch under the integration
+        if (PHILOX) {
+            if ((t & 3) == 0)
+                philox_normals(fx->seed, (unsigned)kc, fx->w1 + (unsigned)(t >> 2), fx->period, fx->e_offset + (unsigned)x, 4,
+                               nr, 1);
+            u = nr[0];
+            nr[0] = nr[1]; nr[1] = nr[2]; nr[2] = nr[3];
+        } else if (t + 1 < T) {
+            qn = FLEET ? a.Q[qoff + (long long)(t + 1) * a.K] : q[(long long)(t + 1) * a.qs_t];  // prefetch under the integration
+        }
         if (MODE == PLAN_CEM) {
             u = cem_plan_value(s_mu[t], u, s_sd[t], a.lo, a.hi);
-            if (active && qo) qo[(long long)t * a.qs_t] = u;
+            if (active && qo) (FLEET ? a.Q_out[qoff + (long long)t * a.K] : qo[(long long)t * a.qs_t]) = u;
         }
         if (COST != COST_NONE) {
-            const float st = stage_cost<COST>(a.cost, c_cost, z.w, z.x, u, up);
-            if (ROWSUM) row_sum_push(rsp, sl, ss, rs_tail, t, st - a.cost.max_cost);  // get_stage_cost shift
+            const float st = stage_cost<COST>(cost, c_cost, z.w, z.x, u, up);
+            if (ROWSUM) row_sum_push(rsp, sl, ss, rs_tail, t, st - cost.max_cost);  // get_stage_cost shift
             else Jacc += st;
         }
         if (active && traj) store_state(traj + (long long)t * a.ts_t, a.ts_c, z);
@@ -566,7 +717,7 @@ __global__ void __launch_bounds__(256, 4) plan_kernel(const __grid_constant__ Pl
         up = u;
     }
     if (COST != COST_NONE) {
-        const float term = terminal_cost<COST>(a.cost, z.th, z.x);
+        const float term = terminal_cost<COST>(cost, z.th, z.x);
         if (ROWSUM) {
             row_sum_push(rsp, sl, ss, rs_tail, T, term);
             Jacc = row_sum_finish(rsp, sl, ss, rs_tail);
@@ -577,19 +728,38 @@ __global__ void __launch_bounds__(256, 4) plan_kernel(const __grid_constant__ Pl
     if (active && traj) store_state(traj + (long long)T * a.ts_t, a.ts_c, z);
     const float J = __fdiv_rn(Jacc, (float)(T + 1));  // mean over the T+1 entries (Cost_Functions/__init__.py:90-93)
     if (active) {
-        if (a.J) a.J[k] = J;
+        if (a.J) a.J[(FLEET ? (long long)blockIdx.y : 0LL) * a.K + k] = J;   // blockIdx.y re-read: no register kept over the loop
         if (!isfinite(J)) atomicAdd(a.nonfinite, 1);
     }
     if (a.select == SELECT_NONE) return;
 
     __threadfence();
     __syncthreads();
-    if (tid == 0) s_ticket = atomicAdd(a.ticket, 1u);
+    if (tid == 0) s_ticket = atomicAdd(a.ticket + (FLEET ? blockIdx.y : 0u), 1u);
     __syncthreads();
     if (s_ticket != gridDim.x - 1u) return;
     __threadfence();
-    plan_select<MODE>(a, s_mu, s_sd, smem + 2 * T, smem + 3 * T, reinterpret_cast<int *>(smem + 4 * T));
-    if (tid == 0) *a.ticket = 0u;  // re-arm
+    if (FLEET) {
+        int *s_elite = reinterpret_cast<int *>(smem + 4 * T);
+        cem_fleet_select<PHILOX>(a, *fx, s_mu, s_sd, smem + 2 * T, smem + 3 * T, s_elite,
+                                 reinterpret_cast<float *>(s_elite + a.elite_smem));
+    } else {
+        plan_select<MODE>(a, s_mu, s_sd, smem + 2 * T, smem + 3 * T, reinterpret_cast<int *>(smem + 4 * T));
+    }
+    if (tid == 0) a.ticket[FLEET ? blockIdx.y : 0u] = 0u;  // re-arm
+}
+template <int INTEG, int COST, int MODE, int NSUB = 0>
+__global__ void __launch_bounds__(256, 4) plan_kernel(const __grid_constant__ PlanArgs a) {
+    plan_body<INTEG, COST, MODE, NSUB, false, false>(a, nullptr, a.cost);
+}
+// CEM fleets: grid (ceil(K / 256), E); experiment e's cost parameters are folded for its targets once per block
+template <int INTEG, int COST, int NSUB, bool PHILOX>
+__global__ void __launch_bounds__(256, 4) plan_fleet_kernel(const __grid_constant__ PlanArgs a,
+                                                            const __grid_constant__ PlanFleetExt fx) {
+    __shared__ CostParams s_cost;
+    if (threadIdx.x == 0) s_cost = fold_cost_e(fx.cost_up, fx.cost_dn, fx.tp, fx.te, (int)blockIdx.y);
+    __syncthreads();
+    plan_body<INTEG, COST, PLAN_CEM, NSUB, true, PHILOX>(a, &fx, s_cost);
 }
 
 // Many plans, no selecting block, time-major plans: two plans per thread (k, k + 1) in packed FP32, as mppi_solve_block2
@@ -1016,5 +1186,89 @@ extern "C" int cps_cem_set_distribution(cps_handle *h, const float *mu_host, con
     if (mu_host) CUDA_TRY(h, cudaMemcpyAsync(P->d_mu + P->cur * T, mu_host, sizeof(float) * T, cudaMemcpyHostToDevice, h->stream));
     if (stdev_host) CUDA_TRY(h, cudaMemcpyAsync(P->d_sd + P->cur * T, stdev_host, sizeof(float) * T, cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    return CPS_OK;
+}
+
+// ---- CEM fleets (cps_cem_fleet.cu) ------------------------------------------------------------------------------------
+typedef void (*plan_fleet_fn)(const PlanArgs, const PlanFleetExt);
+template <int INTEG, int NSUB, bool PHILOX>
+static plan_fleet_fn pick_plan_fleet3(int cost) {
+    switch (cost) {
+    case CPS_COST_DEFAULT: return plan_fleet_kernel<INTEG, COST_DEFAULT, NSUB, PHILOX>;
+    case CPS_COST_QUADRATIC_BOUNDARY: return plan_fleet_kernel<INTEG, COST_QB, NSUB, PHILOX>;
+    case CPS_COST_QB_GRAD_MINIMAL: return plan_fleet_kernel<INTEG, COST_GRADMIN, NSUB, PHILOX>;
+    case CPS_COST_QB_GRAD: return plan_fleet_kernel<INTEG, COST_GRAD, NSUB, PHILOX>;
+    default: return nullptr;
+    }
+}
+template <int INTEG, int NSUB>
+static plan_fleet_fn pick_plan_fleet2(int cost, bool philox) {
+    return philox ? pick_plan_fleet3<INTEG, NSUB, true>(cost) : pick_plan_fleet3<INTEG, NSUB, false>(cost);
+}
+template <int INTEG>
+static plan_fleet_fn pick_plan_fleet1(int cost, int n_sub, bool philox) {
+    return n_sub == 10 ? pick_plan_fleet2<INTEG, 10>(cost, philox) : pick_plan_fleet2<INTEG, 0>(cost, philox);
+}
+static plan_fleet_fn pick_plan_fleet(int integ, int cost, int n_sub, bool philox) {
+    return integ == CPS_EULER_V0 ? pick_plan_fleet1<0>(cost, n_sub, philox) : pick_plan_fleet1<1>(cost, n_sub, philox);
+}
+
+// Dynamic shared memory of plan_fleet_kernel (cps_cem_step's layout, plus the elites' regenerated draws with Philox); sets
+// a.defer_stats, a.elite_smem and a.rs_off from a.best_k and a.T.
+static size_t cem_fleet_smem(const cps_handle *h, PlanArgs &a, bool philox) {
+    a.defer_stats = ((long long)a.best_k * a.T > 2048) ? 1 : 0;
+    a.elite_smem = a.defer_stats ? 0 : a.best_k;
+    const size_t base = sizeof(float) * 4 * (size_t)a.T + sizeof(int) * (size_t)a.elite_smem +
+                        ((philox && !a.defer_stats) ? sizeof(float) * (size_t)a.best_k * a.T : 0);
+    return plan_smem(h, a, base, 256, 1);
+}
+
+int cps_cem_fleet_check(cps_handle *h, int best_k, float initial_stdev, float stdev_min, int philox, const char *who) {
+    if (plan_check(h, who) != CPS_OK) return CPS_ERR_UNSUPPORTED;   // the message plan_check left stands
+    const int K = h->cfg.num_rollouts;
+    if (K > CPS_CEM_MULTIBLOCK_MIN)
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: at most %d plans (the multi-block selection is not built for fleets)", who,
+                    CPS_CEM_MULTIBLOCK_MIN);
+    if (best_k < 1 || best_k > K) return fail(h, CPS_ERR_INVALID, "%s: cem_best_k must lie in [1, num_rollouts]", who);
+    if (!(initial_stdev >= 0.0f) || !(stdev_min >= 0.0f)) return fail(h, CPS_ERR_INVALID, "%s: negative stdev", who);
+    PlanArgs a;
+    memset(&a, 0, sizeof(a));
+    a.best_k = best_k; a.T = h->cfg.horizon;
+    if (cem_fleet_smem(h, a, philox != 0) > 200 * 1024)
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: horizon too large for shared memory", who);
+    return CPS_OK;
+}
+
+int cps_cem_fleet_iteration(cps_handle *h, const CemFleetIteration &c) {
+    const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
+    const bool philox = c.eps == nullptr;
+    PlanArgs a;
+    plan_common(h, a, nullptr, 0.0f, K, T);
+    a.Q = c.eps; a.qs_k = 1; a.qs_t = K;
+    a.Q_out = c.Q_out;
+    a.J = c.J;
+    a.select = SELECT_CEM;
+    a.best_k = c.best_k; a.sd_min = c.sd_min; a.sd_init = c.sd_init;
+    a.mid = (a.lo + a.hi) * 0.5f;
+    a.last_iter = c.last_iter;
+    a.ticket = c.tickets; a.elite = c.elite; a.u_out = c.u;
+    a.mu = c.mu; a.sd = c.sd; a.mu_out = c.mu_out; a.sd_out = c.sd_out;
+    const size_t smem = cem_fleet_smem(h, a, philox);
+    PlanFleetExt fx;
+    memset(&fx, 0, sizeof(fx));
+    fx.s = c.s; fx.tp = c.tp; fx.te = c.te;
+    fx.cost_up = c.cost_up; fx.cost_dn = c.cost_dn;
+    fx.seed = c.seed; fx.w1 = c.w1; fx.period = c.period; fx.e_offset = c.e_offset;
+    plan_fleet_fn fn = pick_plan_fleet(h->cfg.integrator, h->cfg.cost_id, h->ode.n, philox);
+    if (!fn) return fail(h, CPS_ERR_UNSUPPORTED, "cps_cem_fleet_step: no kernel for this configuration");
+    if (smem > 48 * 1024) CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fn<<<dim3((unsigned)(K + 255) / 256, (unsigned)c.E), 256, smem, h->stream>>>(a, fx);
+    h->launches += 1;
+    if (a.defer_stats) {
+        if (philox) cem_update_fleet_kernel<true><<<dim3((unsigned)T, (unsigned)c.E), 256, 0, h->stream>>>(a, fx);
+        else cem_update_fleet_kernel<false><<<dim3((unsigned)T, (unsigned)c.E), 256, 0, h->stream>>>(a, fx);
+        h->launches += 1;
+    }
+    CUDA_TRY(h, cudaGetLastError());
     return CPS_OK;
 }

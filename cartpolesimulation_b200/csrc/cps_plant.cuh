@@ -77,6 +77,16 @@ __device__ __forceinline__ void fold_ode_device(const FoldInputs &a, double L, d
     // the rotation constants and w_rot_max depend on the step only: the handle's fold stands
 }
 
+// experiment e's cost parameters for its targets (null: 0 / +1)
+__device__ __forceinline__ CostParams fold_cost_e(const CostParams &up, const CostParams &dn, const float *tp, const float *te,
+                                                  int e) {
+    const float tpe = tp ? tp[e] : 0.0f, tee = te ? te[e] : 1.0f;
+    CostParams c = (tee == 1.0f) ? up : dn;   // quadratic_boundary_grad selects its weight set on the target equilibrium
+    c.target_position = tpe;
+    c.target_equilibrium = tee;
+    return c;
+}
+
 // ---- Philox4x32-10 (Salmon et al., SC'11), the counter-based generator torch / TF / cuRAND also use ---------------------
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
 #pragma unroll
@@ -104,9 +114,12 @@ __device__ __forceinline__ void box_muller(unsigned a, unsigned b, float &n0, fl
 // Standard normals i = 0..n_ind-1, dst[i * stride], four per counter (w0, w1 + i / 4, period, e_global).  The fleets'
 // streams: the MPPI rollout draws have w0 = rollout, w1 = 0 (second word = draw group < 2^28); the RPGD plan draws have
 // w0 = plan row, w1 = RPGD_DRAWS_RESAMPLE (the resampling solve of `period`) or RPGD_DRAWS_RESET (period 0, the plans of
-// a reset); the plant-side draws of cps_fleet.cu have second word 0xFFFFFFFF.  The second words keep them disjoint.
+// a reset); the CEM draws of outer iteration `it` have w0 = plan, w1 = CEM_DRAWS + it * ceil(T / 4) (second word below
+// CEM_DRAWS + 2^28: cps_cem_fleet_create bounds the iterations); the plant-side draws of cps_fleet.cu have second word
+// 0xFFFFFFFF.  The second words keep them disjoint.
 #define RPGD_DRAWS_RESAMPLE 0xA0000000u
 #define RPGD_DRAWS_RESET 0xB0000000u
+#define CEM_DRAWS 0xC0000000u
 __device__ __forceinline__ void philox_normals(unsigned long long seed, unsigned w0, unsigned w1, unsigned period,
                                                unsigned e_global, int n_ind, float *dst, long long stride) {
     const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
@@ -181,6 +194,20 @@ __device__ __forceinline__ void plant_record(float *r, double time, const float 
     r[6] = s[IDX_POS]; r[7] = s[IDX_POSD]; r[8] = (float)pDD;
     r[9] = Qc; r[10] = Q; r[11] = u; r[12] = tp; r[13] = te; r[14] = 0.0f; r[15] = 0.0f;
 }
+
+// The plant period of fleets whose solve leaves each experiment's control in an [E] array (the neural MPPI fleet of
+// cps_fleet.cu, the CEM fleet of cps_cem_fleet.cu): fleet_net_plant_kernel, one thread per experiment, writes the record
+// row with Q_applied = Q and advances the state.  fleet_plant_launch (cps_fleet.cu) launches it on the handle's stream.
+struct NetPlantArgs {
+    PlantParams plant;
+    float *s;                   // [E][8]
+    const float *u;             // [E] the controls the solve just chose
+    const float *tp, *te;       // [E] targets of this period (null: 0 / +1)
+    float *record;              // [E][CPS_FLEET_RECORD] of this period, or null
+    double time;                // period * dt_control
+    int E;
+};
+int fleet_plant_launch(cps_handle *h, const NetPlantArgs &a);
 
 // The n_sim ticks of one controller period with u held (CartPole/__init__.py:283-324): (aDD, pDD) enter as the second
 // derivatives of s and leave as those of the new state; on_tick(i) runs after tick i.  The caller computes the first pair

@@ -36,16 +36,6 @@
 
 namespace {
 
-// experiment e's cost parameters for its targets (null: 0 / +1)
-__device__ __forceinline__ CostParams fold_cost_e(const CostParams &up, const CostParams &dn, const float *tp, const float *te,
-                                                  int e) {
-    const float tpe = tp ? tp[e] : 0.0f, tee = te ? te[e] : 1.0f;
-    CostParams c = (tee == 1.0f) ? up : dn;   // quadratic_boundary_grad selects its weight set on the target equilibrium
-    c.target_position = tpe;
-    c.target_equilibrium = tee;
-    return c;
-}
-
 __global__ void __launch_bounds__(128) rpgd_fleet_cost_kernel(const CostParams up, const CostParams dn, const float *tp,
                                                                const float *te, CostParams *out, int E) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;

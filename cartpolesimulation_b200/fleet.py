@@ -492,3 +492,119 @@ class RpgdFleet:
         eng._chk(eng.lib.cps_rpgd_fleet_relabel(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
                                                 _ptr(L), _ptr(m_pole), _ptr(draws), _ptr(Q_out), _ptr(J_out)))
         return Q_out
+
+
+class CemFleet:
+    """E closed-loop experiments under optimizer_cem_tf (`cem-tf` in Control_Toolkit_ASF/config_controllers.yml) on one
+    device: one cps_handle with a CEM fleet attached (include/cps.h "CEM fleet").
+
+    Every controller period does, for every experiment, what optimizer_cem_b200.step does (cem_outer_it iterations of
+    sampling from the experiment's own distribution, costs, elites and the mean / stdev update; warmup_iterations on the
+    first period after reset() when `warmup`; then the stdev clip, the shift and u = elite_Q[0, 0]), then what Fleet's
+    plant does, with no host round trip.  The keywords are optimizer_cem_b200's (same defaults) and Fleet's.  Predictor
+    "ODE" or "ODE_v0" and the four cost plugins; num_rollouts at most 8192.  The neural predictor and the plant-side models
+    (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+
+    def __init__(self, n_experiments: int, num_rollouts: int = 200, mpc_horizon: int = 35, cem_outer_it: int = 3,
+                 cem_initial_action_stdev: float = 0.5, cem_stdev_min: float = 0.01, cem_best_k: int = 40,
+                 warmup: bool = False, warmup_iterations: int = 250, control_limits=(-1.0, 1.0), dt: float = 0.02,
+                 substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
+                 cost_config: dict | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
+                 experiment_offset: int = 0, dt_simulation: float = 0.002):
+        if integrator == "neural":
+            raise NotImplementedError("CemFleet runs on predictor 'ODE' or 'ODE_v0' (optimizer_cem_b200 has no neural "
+                                      "predictor either)")
+        n_sim = _check_fleet_args("CemFleet", integrator, None, noise, dt, dt_simulation)
+        self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
+        self.outer_its = int(cem_outer_it)
+        self.first_iter_count = int(warmup_iterations) if warmup else self.outer_its   # as optimizer_cem_b200
+        self.noise_source = noise
+        self._reset_period = None
+        lo, hi = (float(np.asarray(x, dtype=np.float32).reshape(-1)[0]) for x in control_limits)
+        self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost, device=device)
+        self.device = self.engine.device
+        if cost_config is not None:
+            self.engine.set_cost_config(cost_config)
+        self.engine.set_mppi_params(lo=lo, hi=hi)
+        c = L.cps_cem_fleet_config(C.sizeof(L.cps_cem_fleet_config), self.E, n_sim,
+                                   L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
+                                   float(dt_simulation), int(seed), int(experiment_offset), self.outer_its,
+                                   self.first_iter_count, int(cem_best_k), float(cem_initial_action_stdev),
+                                   float(cem_stdev_min))
+        self.engine._chk(self.engine.lib.cps_cem_fleet_create(self.engine._h, C.byref(c)))
+
+    def close(self):
+        self.engine.close()
+
+    def set_plant_models(self, *args, **kwargs):
+        raise NotImplementedError("CemFleet has no plant-side models (control disturbance, measurement noise, latency)")
+
+    def reset(self, states, period: int = 0):
+        """optimizer_reset of every experiment (mid-range mean, cem_initial_action_stdev, u_prev = 0, solve counter 0),
+        the initial states [E, 6] and the period counter."""
+        s = np.ascontiguousarray(states, dtype=np.float32)
+        if s.shape != (self.E, 6):
+            raise ValueError(f"states must have shape ({self.E}, 6)")
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_cem_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP), int(period)))
+        self._reset_period = int(period)
+
+    def iterations(self, period: int) -> int:
+        """The outer iterations of controller period `period`: first_iter_count on the period reset() set, else
+        cem_outer_it."""
+        return self.first_iter_count if period == self._reset_period else self.outer_its
+
+    def states(self, with_u_prev: bool = False):
+        s = np.zeros((self.E, 6), dtype=np.float32)
+        u_prev = np.zeros(self.E, dtype=np.float32) if with_u_prev else None
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_cem_fleet_get_states(
+            self.engine._h, s.ctypes.data_as(L._FP), None if u_prev is None else u_prev.ctypes.data_as(L._FP)))
+        return (s, u_prev) if with_u_prev else s
+
+    def distribution(self):
+        """(mean, stdev), each [E, T]: every experiment's sampling distribution.  Synchronises."""
+        mu, sd = np.zeros((self.E, self.T), dtype=np.float32), np.zeros((self.E, self.T), dtype=np.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_cem_fleet_get_distribution(self.engine._h, mu.ctypes.data_as(L._FP),
+                                                                        sd.ctypes.data_as(L._FP)))
+        return mu, sd
+
+    @property
+    def period(self) -> int:
+        return int(self.engine.lib.cps_cem_fleet_period(self.engine._h))
+
+    def nonfinite_costs(self) -> int:
+        """Non-finite plan costs met so far (a NaN state or target makes them so; they sort after every number and stay
+        in their experiment).  Synchronises."""
+        self.engine.use_current_stream()
+        return self.engine.nonfinite_costs()
+
+    def draws(self, period: int) -> torch.Tensor:
+        """The draws a 'philox' fleet uses in `period`: cuda tensor [iterations(period), E, T, K]."""
+        if self._reset_period is None:
+            raise RuntimeError("CemFleet.draws: reset() first (the first period's iteration count depends on it)")
+        out = torch.empty((self.iterations(period), self.E, self.T, self.K), device=self.device, dtype=torch.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_cem_fleet_draws(self.engine._h, int(period), _ptr(out)))
+        return out
+
+    def run(self, n_periods: int, target_position=None, target_equilibrium=None, draws=None, record=None, J_out=None,
+            Q_out=None):
+        """cps_cem_fleet_step: n_periods controller periods, no synchronisation.  target_position / target_equilibrium:
+        cuda tensors [n_periods, E] or None; draws: the periods' standard normals back to back, [sum of iterations(p), E,
+        T, K], for a 'supplied' fleet; record [n_periods, E, 16], J_out [n_periods, E, K] and Q_out [n_periods, E, T, K]
+        (costs and plans of each period's last iteration) or None."""
+        eng = self.engine
+        eng.use_current_stream()
+        p0 = self.period
+        n_it = sum(self.iterations(p0 + j) for j in range(n_periods))
+        _check_sizes(self.device, (target_position, "target_position", n_periods * self.E),
+                     (target_equilibrium, "target_equilibrium", n_periods * self.E),
+                     (draws, "draws", n_it * self.E * self.T * self.K),
+                     (record, "record", n_periods * self.E * L.FLEET_RECORD),
+                     (J_out, "J_out", n_periods * self.E * self.K),
+                     (Q_out, "Q_out", n_periods * self.E * self.T * self.K))
+        eng._chk(eng.lib.cps_cem_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
+                                            _ptr(draws), _ptr(record), _ptr(J_out), _ptr(Q_out)))
+        return record

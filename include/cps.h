@@ -496,6 +496,63 @@ long long cps_rpgd_fleet_period(const cps_handle *h);
  * from the MPPI fleet's rollout and plant-side draws. */
 int cps_rpgd_fleet_draws(cps_handle *h, long long period, float *out_dev);
 
+/* ---- CEM fleet: E closed-loop experiments under optimizer_cem_tf ------------------------------------------------ */
+/* The data generator with controller_mpc and optimizer cem-tf (Control_Toolkit_ASF/config_controllers.yml;
+ * Control_Toolkit/Optimizers/optimizer_cem_tf.py:12-117): per controller period every experiment runs exactly what one
+ * cps_cem_step does from its own state -- first_iter_count outer iterations on the first period after
+ * cps_cem_fleet_set_states (warmup_iterations with warmup, else cem_outer_it), outer_its after that; per iteration
+ * Q = clip(mean + eps * stdev) with separately rounded multiply and add (:66-68), the costs of the K plans from the
+ * experiment's state with its u_prev and targets (:57-61), the best_k cheapest plans (ties to the lowest index, NaN costs
+ * last) and their mean / population stdev per step (:63-83); after the last iteration stdev is clipped to
+ * [stdev_min, 1e8], both vectors are shifted by one step (tail: initial_stdev, mid-range mean) and u = elite_Q[0, 0]
+ * (:96-99) -- then the plant advances one controller period with Q = u and writes the record row of cps_fleet_step.
+ * u becomes the experiment's u_prev for the next period's costs.  Each experiment owns its distribution (mean, stdev
+ * [T]), u_prev, state and targets (target_position / target_equilibrium select the folded cost parameters per experiment
+ * and period, as in cps_fleet_step); all advance in lockstep, so the solve counter is shared.
+ * Draws: standard normals [n_it][E][T][K] per period (K fastest; n_it that period's iteration count), consecutive periods
+ * back to back in one cps_cem_fleet_step call (CPS_FLEET_NOISE_SUPPLIED), or generated in the rollout threads
+ * (CPS_FLEET_NOISE_PHILOX): counter (plan k, CEM tag + it x ceil(T / 4) + group of four steps, period,
+ * experiment_offset + e), key = seed, disjoint from the MPPI and RPGD fleets' streams; cps_cem_fleet_draws materialises
+ * them.  Launches per period: n_it x (1, or 2 when best_k x T > 2048: the elite statistics then run as a second kernel
+ * with one block per (step, experiment)) + 1 for the plant, whatever E (cps_launch_count).
+ * The handle: predictor CPS_EULER_CROMER or CPS_EULER_V0, one of the four cost plugins, K <= 8192 (the single-block
+ * selection of cps_cem_step), control limits from cps_set_mppi_params (lo, hi).  The neural predictor, no cost plugin or
+ * the legacy cost, CPS_FLAG_SUBSTEP_SINCOS / CPS_FLAG_FAST_DIV, K > 8192 or a horizon whose buffers do not fit shared
+ * memory: CPS_ERR_UNSUPPORTED.  best_k outside [1, K], a negative stdev, outer_its or first_iter_count < 1, dt not a
+ * multiple of dt_simulation: CPS_ERR_INVALID.
+ * Non-finite costs (e.g. from a NaN state or target) are not an error: they sort after every number, stay in their
+ * experiment, and every one is added to the handle's counter (cps_nonfinite_costs). */
+typedef struct cps_cem_fleet_config {
+    int struct_size;                 /* = sizeof(cps_cem_fleet_config) */
+    int n_experiments;               /* E on this device, at most 65535 */
+    int sim_substeps;                /* plant ticks per controller period */
+    int draw_source;                 /* CPS_FLEET_NOISE_SUPPLIED | CPS_FLEET_NOISE_PHILOX: the sampling draws */
+    double dt_simulation;            /* plant tick, 0.002 s */
+    unsigned long long seed;
+    long long experiment_offset;     /* global index of local experiment 0 (Philox counters) */
+    int outer_its, first_iter_count; /* cem_outer_it; the first period's count (warmup_iterations or cem_outer_it) */
+    int best_k;                      /* cem_best_k */
+    float initial_stdev, stdev_min;  /* cem_initial_action_stdev, cem_stdev_min */
+} cps_cem_fleet_config;
+int cps_cem_fleet_create(cps_handle *h, const cps_cem_fleet_config *cfg);
+/* optimizer_reset for every experiment (mean mid-range, stdev initial_stdev, as cps_cem_reset), u_prev = 0, solve counter
+ * 0; states s_host [E][6] (angle_cos / angle_sin taken as given); the period counter.  Synchronises. */
+int cps_cem_fleet_set_states(cps_handle *h, const float *s_host, long long period);
+/* s_host [E][6], u_prev_host [E]; either may be NULL.  Synchronises. */
+int cps_cem_fleet_get_states(cps_handle *h, float *s_host, float *u_prev_host);
+/* The sampling distribution of every experiment: mean_host, stdev_host [E][T]; either may be NULL.  Synchronises. */
+int cps_cem_fleet_get_distribution(cps_handle *h, float *mean_host, float *stdev_host);
+/* n_periods controller periods, stream-ordered, no synchronisation.  tp_dev / te_dev [n_periods][E] or NULL (0 / +1);
+ * draws_dev: the periods' draws back to back (see above; NULL on a Philox fleet); record_dev [n_periods][E][CPS_FLEET_RECORD],
+ * J_out_dev [n_periods][E][K] and Q_out_dev [n_periods][E][T][K] (costs and plans of each period's last iteration) may each
+ * be NULL. */
+int cps_cem_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *draws_dev,
+                       float *record_dev, float *J_out_dev, float *Q_out_dev);
+/* The draws a Philox fleet uses in controller period `period`: out_dev [n_it][E][T][K], n_it = first_iter_count for the
+ * period set by cps_cem_fleet_set_states, else outer_its. */
+int cps_cem_fleet_draws(cps_handle *h, long long period, float *out_dev);
+long long cps_cem_fleet_period(const cps_handle *h);
+
 /* ---- forward-only planners: predict_and_cost and the selection step (SURVEY 8f row f3) ----------------------- */
 /* optimizer_random_action_tf / optimizer_cem_tf / optimizer_cem_gmm_tf evaluate K candidate input plans from one state
  * with predictor.predict_core(s, Q) followed by cost_function.get_trajectory_cost(trajectory, Q, u_prev)
@@ -621,8 +678,8 @@ int cps_net_last_kernel(const cps_handle *h);
 /* Which kernel the last cps_rollout / cps_rollout_host chunk of this handle launched: 0 none yet, 1 rollout_kernel (one
  * cartpole per thread), 2 rollout_pair_kernel (two per thread, packed FP32; large time-major batches). */
 int cps_rollout_last_kernel(const cps_handle *h);
-/* Cumulative count of non-finite trajectory costs seen by cps_mppi_step, cps_plan_cost_grad / cps_rpgd_grad_step and
- * cps_rpgd_fleet_step since cps_create (the reference propagates NaN silently; this library does the same arithmetic but
+/* Cumulative count of non-finite trajectory costs seen by cps_mppi_step, cps_plan_cost_grad / cps_rpgd_grad_step,
+ * cps_rpgd_fleet_step and cps_cem_fleet_step since cps_create (the reference propagates NaN silently; this library does the same arithmetic but
  * counts it).  Synchronises. */
 int cps_nonfinite_costs(cps_handle *h, int *count_out);
 
