@@ -75,12 +75,21 @@ struct FleetArgs {
     FoldInputs fold;            // the device-side fold of (L, m_pole)
 };
 
-// cps_fleet_noise: materialise the draws the kernel generates, [E][n_ind][K]
-__global__ void __launch_bounds__(256) fleet_noise_kernel(unsigned long long seed, unsigned period, unsigned e_offset, int E,
-                                                          int K, int n_ind, float *out) {
-    const int k = blockIdx.x * blockDim.x + threadIdx.x, e = blockIdx.y;
-    if (k >= K || e >= E) return;
-    philox_normals(seed, (unsigned)k, 0u, period, e_offset + (unsigned)e, n_ind, out + ((size_t)e * n_ind) * K + k, K);
+// FleetDrawsArgs (cps_plant.cuh): blocks of 256 rows of one experiment along x, the layers along z, so E is not bounded
+// by gridDim.y
+__global__ void __launch_bounds__(256) fleet_draws_kernel(const FleetDrawsArgs a) {
+    const unsigned bpe = (unsigned)(a.rows + 255) / 256;
+    const int e = (int)(blockIdx.x / bpe), r = (int)(blockIdx.x % bpe) * 256 + (int)threadIdx.x, l = (int)blockIdx.z;
+    if (r >= a.rows) return;
+    philox_normals(a.seed, (unsigned)r, a.tag + (unsigned)l * a.tag_step, a.period, a.e_offset + (unsigned)e, a.n,
+                   a.out + l * a.s_layer + e * a.s_exp + r * a.s_row, a.s_elem);
+}
+
+int fleet_draws_launch(cps_handle *h, const FleetDrawsArgs &a, int layers) {
+    fleet_draws_kernel<<<dim3((unsigned)(a.rows + 255) / 256 * (unsigned)a.E, 1, (unsigned)layers), 256, 0, h->stream>>>(a);
+    h->launches += 1;
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
 }
 
 // The controller's view after `pushed` ring pushes: delayed + interpolated state (latency_adder.py:67-71), measurement
@@ -251,21 +260,7 @@ __global__ void __launch_bounds__(256, 4) fleet_kernel(const __grid_constant__ F
 __global__ void __launch_bounds__(128) fleet_net_plant_kernel(const __grid_constant__ NetPlantArgs a) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= a.E) return;
-    const PlantParams &P = a.plant;
-    float s[6];
-#pragma unroll
-    for (int c = 0; c < 6; ++c) s[c] = a.s[(size_t)e * 8 + c];
-    const float Q = a.u[e];
-    const float u = __fmul_rn(P.u_max, Q);
-    double aDD, pDD;
-    plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
-    if (a.record)
-        plant_record(a.record + (size_t)e * CPS_FLEET_RECORD, a.time, s, aDD, pDD, Q, Q, u, a.tp ? a.tp[e] : 0.0f,
-                     a.te ? a.te[e] : 1.0f);
-    plant_ticks(P, s, u, aDD, pDD, [](int) {});
-    float *so = a.s + (size_t)e * 8;
-#pragma unroll
-    for (int c = 0; c < 6; ++c) so[c] = s[c];
+    plant_period_held(a.plant, a.s, e, a.u[e], a.record, a.time, a.tp, a.te);
 }
 
 int fleet_plant_launch(cps_handle *h, const NetPlantArgs &a) {
@@ -288,28 +283,113 @@ __global__ void fleet_observe_reset_kernel(PlantModels M, const float *s, int E)
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------------------
+// the fleets' [E][8] device states (6 used) -> [E][6] host states; synchronises the handle's stream
+static int fleet_states_to_host(cps_handle *h, const float *s_dev, float *s_host, int E, const char *who) {
+    float *tmp = new (std::nothrow) float[(size_t)E * 8];
+    if (!tmp) return fail(h, CPS_ERR_INVALID, "%s: out of host memory", who);
+    cudaError_t er = cudaMemcpyAsync(tmp, s_dev, sizeof(float) * (size_t)E * 8, cudaMemcpyDeviceToHost, h->stream);
+    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
+    if (er == cudaSuccess)
+        for (int e = 0; e < E; ++e)
+            for (int c = 0; c < 6; ++c) s_host[(size_t)e * 6 + c] = tmp[(size_t)e * 8 + c];
+    delete[] tmp;
+    CUDA_TRY(h, er);
+    return CPS_OK;
+}
+
+int fleet_core_init(cps_handle *h, FleetCore &c, int n_experiments, int sim_substeps, int source, double dt_simulation,
+                    unsigned long long seed, long long experiment_offset, const char *who) {
+    if (n_experiments < 1 || sim_substeps < 1 || !(dt_simulation > 0.0))
+        return fail(h, CPS_ERR_INVALID, "%s: need n_experiments >= 1, sim_substeps >= 1, dt_simulation > 0", who);
+    if (source != CPS_FLEET_NOISE_SUPPLIED && source != CPS_FLEET_NOISE_PHILOX)
+        return fail(h, CPS_ERR_INVALID, "%s: unknown draw source %d", who, source);
+    const double dt = (double)h->cfg.dt;
+    if (std::fabs(sim_substeps * dt_simulation - dt) > 1e-6 * dt)
+        return fail(h, CPS_ERR_INVALID, "%s: dt (control) must be sim_substeps x dt_simulation", who);
+    memset(&c, 0, sizeof(c));
+    c.E = n_experiments; c.n_sim = sim_substeps; c.philox = source == CPS_FLEET_NOISE_PHILOX;
+    c.dt_sim = dt_simulation; c.seed = seed; c.e_offset = (unsigned)experiment_offset;
+    return CPS_OK;
+}
+
+int fleet_core_alloc(cps_handle *h, FleetCore &c) {
+    CUDA_TRY(h, cudaMalloc(&c.d_s, sizeof(float) * (size_t)c.E * 8));
+    CUDA_TRY(h, cudaMalloc(&c.d_uprev, sizeof(float) * (size_t)c.E));
+    CUDA_TRY(h, cudaMemsetAsync(c.d_s, 0, sizeof(float) * (size_t)c.E * 8, h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(c.d_uprev, 0, sizeof(float) * (size_t)c.E, h->stream));
+    return CPS_OK;
+}
+
+void fleet_core_free(FleetCore &c) {
+    cudaFree(c.d_s); cudaFree(c.d_uprev);
+}
+
+int fleet_core_set_states(cps_handle *h, FleetCore &c, const float *s_host, long long period, const char *who) {
+    if (!s_host || period < 0) return fail(h, CPS_ERR_INVALID, "%s: bad argument", who);
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    CUDA_TRY(h, cudaMemsetAsync(c.d_uprev, 0, sizeof(float) * (size_t)c.E, h->stream));
+    std::vector<float> s((size_t)c.E * 8, 0.0f);   // [E][8], columns 6, 7 zero
+    for (int e = 0; e < c.E; ++e) memcpy(&s[(size_t)e * 8], s_host + (size_t)e * 6, sizeof(float) * 6);
+    CUDA_TRY(h, cudaMemcpyAsync(c.d_s, s.data(), sizeof(float) * s.size(), cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    c.period = period;
+    return CPS_OK;
+}
+
+int fleet_core_get_states(cps_handle *h, const FleetCore &c, float *s_host, float *u_prev_host, const char *who) {
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    int rc;
+    if (s_host && (rc = fleet_states_to_host(h, c.d_s, s_host, c.E, who)) != CPS_OK) return rc;
+    if (u_prev_host)
+        CUDA_TRY(h, cudaMemcpyAsync(u_prev_host, c.d_uprev, sizeof(float) * (size_t)c.E, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    return CPS_OK;
+}
+
+int fleet_core_check_draws(cps_handle *h, const FleetCore &c, const float *draws_dev, bool reads, const char *who) {
+    if (!c.philox && !draws_dev && reads) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied draws", who);
+    if (c.philox && draws_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its draws (Philox); pass NULL", who);
+    return CPS_OK;
+}
+
+FleetRow fleet_core_row(const FleetCore &c, int j, const float *tp_dev, const float *te_dev, float *record_dev) {
+    const size_t E = c.E;
+    FleetRow r;
+    r.tp = tp_dev ? tp_dev + (size_t)j * E : nullptr;
+    r.te = te_dev ? te_dev + (size_t)j * E : nullptr;
+    r.record = record_dev ? record_dev + (size_t)j * E * CPS_FLEET_RECORD : nullptr;
+    r.period = (unsigned)c.period;
+    r.time = (double)c.period * (c.dt_sim * c.n_sim);
+    return r;
+}
+
+int fleet_fold_costs(cps_handle *h, CostParams *up, CostParams *dn) {
+    int rc;
+    if ((rc = cps_fold_cost_for(h, 1.0f, up)) != CPS_OK) return rc;
+    return cps_fold_cost_for(h, -1.0f, dn);
+}
+
 struct FleetState {
-    cps_fleet_config cfg;
-    int E, bpe, block, pair;   // pair: two rollouts per thread (packed FP32), K even
+    FleetCore core;            // the MPPI fleet may step and read its states before cps_fleet_set_states (zero states)
+    int bpe, block, pair;      // pair: two rollouts per thread (packed FP32), K even
     size_t smem;
     int rs_off;                // MppiParams::rs_off for this geometry
-    float *d_s, *d_unom, *d_uprev, *d_partials;
+    float *d_unom, *d_partials;
     unsigned *d_tickets;
-    long long period;
-    CostParams cost_up, cost_dn;
     PlantModels pm;            // plant-side models (cps_fleet_set_plant_models); pm.pushed counts the ring pushes
     // neural fleets (CPS_PREDICTOR_NEURAL): the controller runs net_kernel / net_tc_kernel<.., FLEET>
     int neural;
     int htot;                  // hidden-state floats per experiment of the network the fleet was created for
     float *d_h;                // [E][htot] each experiment's hidden state
-    float *d_noise;            // Philox: [E][n_ind][K] the period's draws (fleet_noise_kernel), read like supplied ones
+    float *d_noise;            // Philox: [E][n_ind][K] the period's draws (fleet_draws_kernel), read like supplied ones
     size_t part_cap;           // floats allocated at d_partials
 };
 
 void cps_fleet_free(cps_handle *h) {
     FleetState *F = h->fleet;
     if (!F) return;
-    cudaFree(F->d_s); cudaFree(F->d_unom); cudaFree(F->d_uprev); cudaFree(F->d_partials); cudaFree(F->d_tickets);
+    fleet_core_free(F->core);
+    cudaFree(F->d_unom); cudaFree(F->d_partials); cudaFree(F->d_tickets);
     cudaFree(F->pm.obs); cudaFree(F->pm.ring);
     cudaFree(F->d_h); cudaFree(F->d_noise);
     delete F;
@@ -339,27 +419,27 @@ static fleet_fn pick_fleet(int integ, int cost, bool philox, bool pair, bool n10
 
 extern "C" int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg) {
     if (!h) return CPS_ERR_INVALID;
+    const char *who = "cps_fleet_create";
     if (!cfg || cfg->struct_size != (int)sizeof(cps_fleet_config))
-        return fail(h, CPS_ERR_INVALID, "cps_fleet_create: cps_fleet_config size mismatch");
-    if (cfg->n_experiments < 1 || cfg->sim_substeps < 1 || !(cfg->dt_simulation > 0.0))
-        return fail(h, CPS_ERR_INVALID, "cps_fleet_create: need n_experiments >= 1, sim_substeps >= 1, dt_simulation > 0");
-    if (cfg->noise_source != CPS_FLEET_NOISE_SUPPLIED && cfg->noise_source != CPS_FLEET_NOISE_PHILOX)
-        return fail(h, CPS_ERR_INVALID, "cps_fleet_create: unknown noise source %d", cfg->noise_source);
-    if (h->cfg.cost_id == CPS_COST_NONE) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_create: the handle has no cost function");
+        return fail(h, CPS_ERR_INVALID, "%s: cps_fleet_config size mismatch", who);
+    FleetCore core;
+    int rc;
+    if ((rc = fleet_core_init(h, core, cfg->n_experiments, cfg->sim_substeps, cfg->noise_source, cfg->dt_simulation, cfg->seed,
+                              cfg->experiment_offset, who)) != CPS_OK)
+        return rc;
+    if (h->cfg.cost_id == CPS_COST_NONE) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: the handle has no cost function", who);
     if (h->cfg.noise_mode != CPS_NOISE_INDUCING)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_create: fleets use inducing-point noise (CPS_NOISE_INDUCING)");
-    if (cfg->n_experiments > 65535) return fail(h, CPS_ERR_INVALID, "cps_fleet_create: at most 65535 experiments per handle");
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: fleets use inducing-point noise (CPS_NOISE_INDUCING)", who);
+    if (core.E > 65535) return fail(h, CPS_ERR_INVALID, "%s: at most 65535 experiments per handle", who);
     const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
     NetFleetPlan p;
-    int rc;
-    if (neural && (rc = cps_net_mppi_fleet_plan(h, cfg->n_experiments, "cps_fleet_create", &p)) != CPS_OK) return rc;
+    if (neural && (rc = cps_net_mppi_fleet_plan(h, core.E, who, &p)) != CPS_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     cps_fleet_free(h);
     FleetState *F = new (std::nothrow) FleetState();
-    if (!F) return fail(h, CPS_ERR_INVALID, "cps_fleet_create: out of host memory");
+    if (!F) return fail(h, CPS_ERR_INVALID, "%s: out of host memory", who);
     memset(F, 0, sizeof(*F));
-    F->cfg = *cfg;
-    F->E = cfg->n_experiments;
+    F->core = core;
     const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
     if (neural) {
         // the controller predicts with the loaded network: per experiment a hidden state, partials and tickets for the
@@ -370,62 +450,32 @@ extern "C" int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg) {
     } else {
         // large fleets are throughput work: two rollouts per thread in packed FP32 (mppi_solve_block2) from 65536 rollouts
         // per launch on, as for a single solve (tools/ab_fleet_pairs.py: 14 % faster at E = 256 and 1024, 30 % slower at E <= 16)
-        F->pair = (K % 2 == 0 && K >= 64 && (long long)cfg->n_experiments * K >= CPS_MPPI_PAIR_MIN_ROLLOUTS &&
+        F->pair = (K % 2 == 0 && K >= 64 && (long long)core.E * K >= CPS_MPPI_PAIR_MIN_ROLLOUTS &&
                    !(h->cfg.flags & CPS_FLAG_NO_PAIRS)) ? 1 : 0;
         const int threads = F->pair ? K / 2 : K;   // threads per experiment
         F->block = threads >= 256 ? 256 : ((threads + 31) / 32) * 32;
         F->bpe = (threads + F->block - 1) / F->block;
         MppiParams mp_geo = h->mp;
-        const size_t draws = (cfg->noise_source == CPS_FLEET_NOISE_PHILOX) ? (size_t)h->n_ind * F->block * (F->pair ? 2 : 1) : 0;
+        const size_t draws = core.philox ? (size_t)h->n_ind * F->block * (F->pair ? 2 : 1) : 0;
         F->smem = sizeof(float) * mppi_smem_floats(mp_geo, h->cfg.cost_id, F->block, F->pair ? 2 : 1, draws);
         F->rs_off = mp_geo.rs_off;
-        if (F->smem > 200 * 1024) { delete F; return fail(h, CPS_ERR_UNSUPPORTED, "cps_fleet_create: horizon too large for shared memory"); }
+        if (F->smem > 200 * 1024) { delete F; return fail(h, CPS_ERR_UNSUPPORTED, "%s: horizon too large for shared memory", who); }
     }
     h->fleet = F;
-    const size_t E = F->E, hn = F->htot > 0 ? F->htot : 1;
+    const size_t E = core.E, hn = F->htot > 0 ? F->htot : 1;
     F->part_cap = E * F->bpe * (h->n_red + 2);
-    CUDA_TRY(h, cudaMalloc(&F->d_s, sizeof(float) * E * 8));
+    if ((rc = fleet_core_alloc(h, F->core)) != CPS_OK) return rc;
     CUDA_TRY(h, cudaMalloc(&F->d_unom, sizeof(float) * E * T));
-    CUDA_TRY(h, cudaMalloc(&F->d_uprev, sizeof(float) * E));
     CUDA_TRY(h, cudaMalloc(&F->d_partials, sizeof(float) * F->part_cap));
     CUDA_TRY(h, cudaMalloc(&F->d_tickets, sizeof(unsigned) * E));
-    CUDA_TRY(h, cudaMemset(F->d_s, 0, sizeof(float) * E * 8));
     CUDA_TRY(h, cudaMemset(F->d_unom, 0, sizeof(float) * E * T));
-    CUDA_TRY(h, cudaMemset(F->d_uprev, 0, sizeof(float) * E));
     CUDA_TRY(h, cudaMemset(F->d_tickets, 0, sizeof(unsigned) * E));
     if (neural) {
         CUDA_TRY(h, cudaMalloc(&F->d_h, sizeof(float) * E * hn));
         CUDA_TRY(h, cudaMemset(F->d_h, 0, sizeof(float) * E * hn));
-        if (cfg->noise_source == CPS_FLEET_NOISE_PHILOX) CUDA_TRY(h, cudaMalloc(&F->d_noise, sizeof(float) * E * h->n_ind * K));
+        if (core.philox) CUDA_TRY(h, cudaMalloc(&F->d_noise, sizeof(float) * E * h->n_ind * K));
     }
     CUDA_TRY(h, cudaDeviceSynchronize());
-    return CPS_OK;
-}
-
-int fleet_states_to_device(cps_handle *h, const float *s_host, float *s_dev, int E, const char *who) {
-    float *tmp = new (std::nothrow) float[(size_t)E * 8];
-    if (!tmp) return fail(h, CPS_ERR_INVALID, "%s: out of host memory", who);
-    for (int e = 0; e < E; ++e) {
-        for (int c = 0; c < 6; ++c) tmp[(size_t)e * 8 + c] = s_host[(size_t)e * 6 + c];
-        tmp[(size_t)e * 8 + 6] = tmp[(size_t)e * 8 + 7] = 0.0f;
-    }
-    cudaError_t er = cudaMemcpyAsync(s_dev, tmp, sizeof(float) * (size_t)E * 8, cudaMemcpyHostToDevice, h->stream);
-    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
-    delete[] tmp;
-    CUDA_TRY(h, er);
-    return CPS_OK;
-}
-
-int fleet_states_to_host(cps_handle *h, const float *s_dev, float *s_host, int E, const char *who) {
-    float *tmp = new (std::nothrow) float[(size_t)E * 8];
-    if (!tmp) return fail(h, CPS_ERR_INVALID, "%s: out of host memory", who);
-    cudaError_t er = cudaMemcpyAsync(tmp, s_dev, sizeof(float) * (size_t)E * 8, cudaMemcpyDeviceToHost, h->stream);
-    if (er == cudaSuccess) er = cudaStreamSynchronize(h->stream);
-    if (er == cudaSuccess)
-        for (int e = 0; e < E; ++e)
-            for (int c = 0; c < 6; ++c) s_host[(size_t)e * 6 + c] = tmp[(size_t)e * 8 + c];
-    delete[] tmp;
-    CUDA_TRY(h, er);
     return CPS_OK;
 }
 
@@ -433,26 +483,23 @@ extern "C" int cps_fleet_set_states(cps_handle *h, const float *s_host, long lon
     if (!h) return CPS_ERR_INVALID;
     FleetState *F = h->fleet;
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_set_states: no fleet (cps_fleet_create)");
-    if (!s_host || period < 0) return fail(h, CPS_ERR_INVALID, "cps_fleet_set_states: bad argument");
-    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    CUDA_TRY(h, cudaMemsetAsync(F->d_unom, 0, sizeof(float) * (size_t)F->E * h->cfg.horizon, h->stream));
-    CUDA_TRY(h, cudaMemsetAsync(F->d_uprev, 0, sizeof(float) * (size_t)F->E, h->stream));
-    int rc = fleet_states_to_device(h, s_host, F->d_s, F->E, "cps_fleet_set_states");
-    if (rc != CPS_OK) return rc;
-    F->period = period;
+    int rc;
+    if ((rc = fleet_core_set_states(h, F->core, s_host, period, "cps_fleet_set_states")) != CPS_OK) return rc;
+    const int E = F->core.E;
+    CUDA_TRY(h, cudaMemsetAsync(F->d_unom, 0, sizeof(float) * (size_t)E * h->cfg.horizon, h->stream));
     if (F->neural && F->htot > 0) {   // every experiment starts from the handle's stored state (what a fresh predictor holds)
-        std::vector<float> h0((size_t)F->htot), all((size_t)F->E * F->htot);
+        std::vector<float> h0((size_t)F->htot), all((size_t)E * F->htot);
         if (F->htot != cps_net_state_size(h))
             return fail(h, CPS_ERR_INVALID, "cps_fleet_set_states: the loaded network's hidden state differs from the fleet's; "
                         "recreate the fleet (cps_fleet_create)");
         if ((rc = cps_net_get_state(h, h0.data())) != CPS_OK) return rc;
-        for (int e = 0; e < F->E; ++e) memcpy(&all[(size_t)e * F->htot], h0.data(), sizeof(float) * F->htot);
+        for (int e = 0; e < E; ++e) memcpy(&all[(size_t)e * F->htot], h0.data(), sizeof(float) * F->htot);
         CUDA_TRY(h, cudaMemcpyAsync(F->d_h, all.data(), sizeof(float) * all.size(), cudaMemcpyHostToDevice, h->stream));
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     }
     if (F->pm.on) {   // ring = the reference's initial buffer; the first solve sees the true state
         F->pm.pushed = 0;
-        fleet_observe_reset_kernel<<<(F->E + 127) / 128, 128, 0, h->stream>>>(F->pm, F->d_s, F->E);
+        fleet_observe_reset_kernel<<<(E + 127) / 128, 128, 0, h->stream>>>(F->pm, F->core.d_s, E);
         h->launches += 1;
         CUDA_TRY(h, cudaGetLastError());
     }
@@ -469,7 +516,7 @@ extern "C" int cps_fleet_set_plant_models(cps_handle *h, const cps_fleet_plant_m
         return fail(h, CPS_ERR_INVALID, "cps_fleet_set_plant_models: cps_fleet_plant_models size mismatch");
     if (m->control_noise_mode < 0 || m->control_noise_mode > 2) return fail(h, CPS_ERR_INVALID, "cps_fleet_set_plant_models: control_noise_mode must be 0 (OFF), 1 (additive) or 2 (truncnorm)");
     if (m->control_noise_mode == 2 && !(m->control_noise_mult > 0.0f)) return fail(h, CPS_ERR_INVALID, "cps_fleet_set_plant_models: truncnorm needs a positive scale");
-    const double lat_len = m->latency / F->cfg.dt_simulation;
+    const double lat_len = m->latency / F->core.dt_sim;
     if (!(m->latency >= 0.0) || lat_len > 200.0)   // MAX_LATENCY_LEN (latency_adder.py:8,74-75)
         return fail(h, CPS_ERR_INVALID, "cps_fleet_set_plant_models: latency must lie in [0, 200 plant ticks]");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
@@ -483,10 +530,11 @@ extern "C" int cps_fleet_set_plant_models(cps_handle *h, const cps_fleet_plant_m
     M.ring_len = M.lat_int + 2;
     M.on = (M.ctrl_mode || M.meas_on || m->latency > 0.0) ? 1 : 0;
     if (!M.on) return CPS_OK;
-    CUDA_TRY(h, cudaMalloc(&M.obs, sizeof(float) * (size_t)F->E * 8));
-    CUDA_TRY(h, cudaMalloc(&M.ring, sizeof(float) * (size_t)F->E * M.ring_len * 6));
+    const int E = F->core.E;
+    CUDA_TRY(h, cudaMalloc(&M.obs, sizeof(float) * (size_t)E * 8));
+    CUDA_TRY(h, cudaMalloc(&M.ring, sizeof(float) * (size_t)E * M.ring_len * 6));
     M.pushed = 0;
-    fleet_observe_reset_kernel<<<(F->E + 127) / 128, 128, 0, h->stream>>>(M, F->d_s, F->E);
+    fleet_observe_reset_kernel<<<(E + 127) / 128, 128, 0, h->stream>>>(M, F->core.d_s, E);
     h->launches += 1;
     CUDA_TRY(h, cudaGetLastError());
     return CPS_OK;
@@ -498,7 +546,7 @@ extern "C" int cps_fleet_get_observed(cps_handle *h, float *obs_host) {
     if (!F || !F->pm.on) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_get_observed: no plant-side models (cps_fleet_set_plant_models)");
     if (!obs_host) return fail(h, CPS_ERR_INVALID, "cps_fleet_get_observed: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    return fleet_states_to_host(h, F->pm.obs, obs_host, F->E, "cps_fleet_get_observed");
+    return fleet_states_to_host(h, F->pm.obs, obs_host, F->core.E, "cps_fleet_get_observed");
 }
 
 extern "C" int cps_fleet_reset(cps_handle *h, long long period) {
@@ -507,9 +555,9 @@ extern "C" int cps_fleet_reset(cps_handle *h, long long period) {
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_reset: no fleet (cps_fleet_create)");
     if (period < 0) return fail(h, CPS_ERR_INVALID, "cps_fleet_reset: period < 0");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    CUDA_TRY(h, cudaMemsetAsync(F->d_unom, 0, sizeof(float) * (size_t)F->E * h->cfg.horizon, h->stream));
-    CUDA_TRY(h, cudaMemsetAsync(F->d_uprev, 0, sizeof(float) * (size_t)F->E, h->stream));
-    F->period = period;
+    CUDA_TRY(h, cudaMemsetAsync(F->d_unom, 0, sizeof(float) * (size_t)F->core.E * h->cfg.horizon, h->stream));
+    CUDA_TRY(h, cudaMemsetAsync(F->core.d_uprev, 0, sizeof(float) * (size_t)F->core.E, h->stream));
+    F->core.period = period;
     return CPS_OK;
 }
 
@@ -518,14 +566,10 @@ extern "C" int cps_fleet_get_states(cps_handle *h, float *s_host, float *u_nom_h
     FleetState *F = h->fleet;
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_get_states: no fleet (cps_fleet_create)");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    int rc;
-    if (s_host && (rc = fleet_states_to_host(h, F->d_s, s_host, F->E, "cps_fleet_get_states")) != CPS_OK) return rc;
     if (u_nom_host)
-        CUDA_TRY(h, cudaMemcpyAsync(u_nom_host, F->d_unom, sizeof(float) * (size_t)F->E * h->cfg.horizon, cudaMemcpyDeviceToHost, h->stream));
-    if (u_prev_host)
-        CUDA_TRY(h, cudaMemcpyAsync(u_prev_host, F->d_uprev, sizeof(float) * (size_t)F->E, cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    return CPS_OK;
+        CUDA_TRY(h, cudaMemcpyAsync(u_nom_host, F->d_unom, sizeof(float) * (size_t)F->core.E * h->cfg.horizon,
+                                    cudaMemcpyDeviceToHost, h->stream));
+    return fleet_core_get_states(h, F->core, s_host, u_prev_host, "cps_fleet_get_states");
 }
 
 // [E][htot] hidden states of a neural fleet, host <-> device; synchronises
@@ -535,7 +579,7 @@ static int fleet_net_states_io(cps_handle *h, float *host, bool get, const char 
     if (!F || !F->neural) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no fleet with the neural predictor (cps_fleet_create)", who);
     if (!host) return fail(h, CPS_ERR_INVALID, "%s: null pointer", who);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    const size_t bytes = sizeof(float) * (size_t)F->E * F->htot;
+    const size_t bytes = sizeof(float) * (size_t)F->core.E * F->htot;
     if (bytes) {
         CUDA_TRY(h, get ? cudaMemcpyAsync(host, F->d_h, bytes, cudaMemcpyDeviceToHost, h->stream)
                         : cudaMemcpyAsync(F->d_h, host, bytes, cudaMemcpyHostToDevice, h->stream));
@@ -550,17 +594,12 @@ extern "C" int cps_fleet_set_net_states(cps_handle *h, const float *in_host) {
     return fleet_net_states_io(h, const_cast<float *>(in_host), false, "cps_fleet_set_net_states");
 }
 
-extern "C" long long cps_fleet_period(const cps_handle *h) { return (h && h->fleet) ? h->fleet->period : -1; }
+extern "C" long long cps_fleet_period(const cps_handle *h) { return (h && h->fleet) ? h->fleet->core.period : -1; }
 
-// CostParams for a given target equilibrium: fold_cost() depends on it for quadratic_boundary_grad (weight set, w[9]).
-int cps_fold_cost_for(cps_handle *h, float target_equilibrium, CostParams *out);
-
-// The period's draws: supplied by the caller or generated (Philox), as the fleet was created
-static int fleet_check_noise(cps_handle *h, const FleetState *F, const float *noise_dev, const char *who) {
-    const bool philox = F->cfg.noise_source == CPS_FLEET_NOISE_PHILOX;
-    if (!philox && !noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied noise", who);
-    if (philox && noise_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its noise (Philox); pass NULL", who);
-    return CPS_OK;
+// The rollout draws [E][n_ind][K] of `period` (counter: rollout, draw group, period, experiment)
+static FleetDrawsArgs fleet_noise_args(const cps_handle *h, const FleetCore &c, long long period, float *out) {
+    const int K = h->cfg.num_rollouts;
+    return {c.seed, 0u, 0u, (unsigned)period, c.e_offset, c.E, K, h->n_ind, 0, (long long)h->n_ind * K, 1, K, out};
 }
 
 // Shared by cps_fleet_step (closed loop: replay_dev == nullptr) and cps_fleet_relabel (states from a recording).
@@ -571,38 +610,35 @@ static int fleet_launch(cps_handle *h, const char *who, int n_periods, const flo
     FleetState *F = h->fleet;
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no fleet (cps_fleet_create)", who);
     if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "%s: negative number of periods / rows", who);
+    FleetCore &c = F->core;
     int rc;
-    if ((rc = fleet_check_noise(h, F, noise_dev, who)) != CPS_OK) return rc;
-    const bool philox = F->cfg.noise_source == CPS_FLEET_NOISE_PHILOX;
+    if ((rc = fleet_core_check_draws(h, c, noise_dev, true, who)) != CPS_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     FleetArgs a;
     a.ode = h->ode; a.mp = h->mp;
     a.mp.rs_off = F->rs_off;
     a.pm = F->pm;
     if (replay_dev) a.pm.on = 0;   // relabelling feeds recorded states: no plant, no observation chain
-    if (a.pm.on && !philox && ((a.pm.ctrl_mode && !ctrl_draws_dev) || (a.pm.meas_on && !meas_draws_dev)))
+    if (a.pm.on && !c.philox && ((a.pm.ctrl_mode && !ctrl_draws_dev) || (a.pm.meas_on && !meas_draws_dev)))
         return fail(h, CPS_ERR_INVALID, "%s: a fleet with supplied noise needs the plant-side draws as well (cps_fleet_step_noisy)", who);
-    if ((rc = cps_fold_cost_for(h, 1.0f, &a.cost_up)) != CPS_OK) return rc;
-    if ((rc = cps_fold_cost_for(h, -1.0f, &a.cost_dn)) != CPS_OK) return rc;
-    a.plant = plant_params(h, F->cfg.dt_simulation, F->cfg.sim_substeps);
+    if ((rc = fleet_fold_costs(h, &a.cost_up, &a.cost_dn)) != CPS_OK) return rc;
+    a.plant = plant_params(h, c.dt_sim, c.n_sim);
     a.bpe = F->bpe;
-    a.s = F->d_s; a.u_nom = F->d_unom; a.u_prev = F->d_uprev;
-    a.seed = F->cfg.seed; a.e_offset = (unsigned)F->cfg.experiment_offset;
+    a.s = c.d_s; a.u_nom = F->d_unom; a.u_prev = c.d_uprev;
+    a.seed = c.seed; a.e_offset = c.e_offset;
     a.partials = F->d_partials; a.tickets = F->d_tickets; a.nonfinite = h->d_nonfinite;
     a.fold = fold_inputs(h);
     if (F->pair && noise_dev && ((uintptr_t)noise_dev % 8) != 0)
         return fail(h, CPS_ERR_INVALID, "%s: supplied noise must be 8-byte aligned", who);
-    fleet_fn fn = pick_fleet(h->cfg.integrator, h->cfg.cost_id, philox, F->pair != 0, h->ode.n == 10);
+    fleet_fn fn = pick_fleet(h->cfg.integrator, h->cfg.cost_id, c.philox, F->pair != 0, h->ode.n == 10);
     if (!fn) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no kernel for this configuration", who);
     if (F->smem > 48 * 1024) CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)F->smem));
-    const size_t E = F->E, K = h->cfg.num_rollouts;
-    const double dt_control = F->cfg.dt_simulation * F->cfg.sim_substeps;
-    const dim3 grid(F->bpe, F->E);
+    const size_t E = c.E, K = h->cfg.num_rollouts;
+    const dim3 grid(F->bpe, c.E);
     for (int j = 0; j < n_periods; ++j) {
-        a.tp = tp_dev ? tp_dev + (size_t)j * E : nullptr;
-        a.te = te_dev ? te_dev + (size_t)j * E : nullptr;
+        const FleetRow row = fleet_core_row(c, j, tp_dev, te_dev, record_dev);
+        a.tp = row.tp; a.te = row.te; a.record = row.record;
         a.noise = noise_dev ? noise_dev + (size_t)j * E * h->n_ind * K : nullptr;
-        a.record = record_dev ? record_dev + (size_t)j * E * CPS_FLEET_RECORD : nullptr;
         a.J_out = J_out_dev ? J_out_dev + (size_t)j * E * K : nullptr;
         a.replay_s = replay_dev ? replay_dev + (size_t)j * E * 6 : nullptr;
         a.L_row = L_dev ? L_dev + (size_t)j * E : nullptr;
@@ -612,13 +648,13 @@ static int fleet_launch(cps_handle *h, const char *who, int n_periods, const flo
         if (a.pm.on) {
             a.pm.pushed = F->pm.pushed;
             a.pm.ctrl_draws = ctrl_draws_dev ? ctrl_draws_dev + (size_t)j * E : nullptr;
-            a.pm.meas_draws = meas_draws_dev ? meas_draws_dev + (size_t)j * F->cfg.sim_substeps * E * 4 : nullptr;
-            F->pm.pushed += F->cfg.sim_substeps;
+            a.pm.meas_draws = meas_draws_dev ? meas_draws_dev + (size_t)j * c.n_sim * E * 4 : nullptr;
+            F->pm.pushed += c.n_sim;
         }
-        a.period = (unsigned)F->period;
-        a.time = (double)F->period * dt_control;
+        a.period = row.period;
+        a.time = row.time;
         fn<<<grid, F->block, F->smem, h->stream>>>(a);
-        F->period += 1;
+        c.period += 1;
         h->launches += 1;
     }
     CUDA_TRY(h, cudaGetLastError());
@@ -630,17 +666,17 @@ static int fleet_step_neural(cps_handle *h, int n_periods, const float *tp_dev, 
                              float *record_dev, float *J_out_dev) {
     const char *who = "cps_fleet_step";
     FleetState *F = h->fleet;
+    FleetCore &c = F->core;
     if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "%s: negative number of periods", who);
     int rc;
-    if ((rc = fleet_check_noise(h, F, noise_dev, who)) != CPS_OK) return rc;
-    const bool philox = F->cfg.noise_source == CPS_FLEET_NOISE_PHILOX;
+    if ((rc = fleet_core_check_draws(h, c, noise_dev, true, who)) != CPS_OK) return rc;
     NetFleetPlan p;
-    if ((rc = cps_net_mppi_fleet_plan(h, F->E, who, &p)) != CPS_OK) return rc;
+    if ((rc = cps_net_mppi_fleet_plan(h, c.E, who, &p)) != CPS_OK) return rc;
     if (cps_net_state_size(h) != F->htot)
         return fail(h, CPS_ERR_INVALID, "%s: the loaded network has %d hidden-state floats, the fleet was created for %d; "
                     "recreate the fleet (cps_fleet_create)", who, cps_net_state_size(h), F->htot);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    const size_t E = F->E, K = h->cfg.num_rollouts, need = E * p.tiles * (h->n_red + 2);
+    const size_t E = c.E, K = h->cfg.num_rollouts, need = E * p.tiles * (h->n_red + 2);
     if (need > F->part_cap) {   // a different tiling than at create (CPS_TC_ROWS)
         cudaFree(F->d_partials);
         F->d_partials = nullptr;
@@ -650,28 +686,21 @@ static int fleet_step_neural(cps_handle *h, int n_periods, const float *tp_dev, 
     }
     F->bpe = p.tiles;
     CostParams cost_up, cost_dn;
-    if ((rc = cps_fold_cost_for(h, 1.0f, &cost_up)) != CPS_OK) return rc;
-    if ((rc = cps_fold_cost_for(h, -1.0f, &cost_dn)) != CPS_OK) return rc;
+    if ((rc = fleet_fold_costs(h, &cost_up, &cost_dn)) != CPS_OK) return rc;
     NetPlantArgs pa;
-    pa.plant = plant_params(h, F->cfg.dt_simulation, F->cfg.sim_substeps);
-    pa.s = F->d_s; pa.u = F->d_uprev; pa.E = F->E;
-    const double dt_control = F->cfg.dt_simulation * F->cfg.sim_substeps;
+    pa.plant = plant_params(h, c.dt_sim, c.n_sim);
+    pa.s = c.d_s; pa.u = c.d_uprev; pa.E = c.E;
     for (int j = 0; j < n_periods; ++j) {
-        const float *tp = tp_dev ? tp_dev + (size_t)j * E : nullptr, *te = te_dev ? te_dev + (size_t)j * E : nullptr;
+        const FleetRow row = fleet_core_row(c, j, tp_dev, te_dev, record_dev);
         const float *noise = noise_dev ? noise_dev + (size_t)j * E * h->n_ind * K : F->d_noise;
-        if (philox) {   // the draws cps_fleet_noise returns for this period
-            fleet_noise_kernel<<<dim3((unsigned)(K + 255) / 256, F->E), 256, 0, h->stream>>>(
-                F->cfg.seed, (unsigned)F->period, (unsigned)F->cfg.experiment_offset, F->E, (int)K, h->n_ind, F->d_noise);
-            h->launches += 1;
-        }
-        if ((rc = cps_net_mppi_fleet(h, F->E, p, F->d_s, F->d_unom, F->d_uprev, F->d_h, tp, te, cost_up, cost_dn, noise,
+        if (c.philox && (rc = fleet_draws_launch(h, fleet_noise_args(h, c, c.period, F->d_noise), 1)) != CPS_OK)
+            return rc;   // the draws cps_fleet_noise returns for this period
+        if ((rc = cps_net_mppi_fleet(h, c.E, p, c.d_s, F->d_unom, c.d_uprev, F->d_h, row.tp, row.te, cost_up, cost_dn, noise,
                                      F->d_partials, F->d_tickets, J_out_dev ? J_out_dev + (size_t)j * E * K : nullptr)) != CPS_OK)
             return rc;
-        pa.tp = tp; pa.te = te;
-        pa.record = record_dev ? record_dev + (size_t)j * E * CPS_FLEET_RECORD : nullptr;
-        pa.time = (double)F->period * dt_control;
+        pa.tp = row.tp; pa.te = row.te; pa.record = row.record; pa.time = row.time;
         if ((rc = fleet_plant_launch(h, pa)) != CPS_OK) return rc;
-        F->period += 1;
+        c.period += 1;
     }
     CUDA_TRY(h, cudaGetLastError());
     return CPS_OK;
@@ -724,11 +753,5 @@ extern "C" int cps_fleet_noise(cps_handle *h, long long period, float *out_dev) 
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_fleet_noise: no fleet (cps_fleet_create)");
     if (!out_dev || period < 0) return fail(h, CPS_ERR_INVALID, "cps_fleet_noise: bad argument");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    const int K = h->cfg.num_rollouts;
-    const dim3 grid((K + 255) / 256, F->E);
-    fleet_noise_kernel<<<grid, 256, 0, h->stream>>>(F->cfg.seed, (unsigned)period, (unsigned)F->cfg.experiment_offset, F->E, K,
-                                                    h->n_ind, out_dev);
-    h->launches += 1;
-    CUDA_TRY(h, cudaGetLastError());
-    return CPS_OK;
+    return fleet_draws_launch(h, fleet_noise_args(h, F->core, period, out_dev), 1);
 }

@@ -138,9 +138,6 @@ static inline size_t mppi_smem_floats(MppiParams &mp, int cost_id, int block, in
 
 // cps_fleet.cu
 void cps_fleet_free(cps_handle *h);
-// [E][6] host states <-> the fleets' [E][8] device states (columns 6, 7 zero); both synchronise the handle's stream
-int fleet_states_to_device(cps_handle *h, const float *s_host, float *s_dev, int E, const char *who);
-int fleet_states_to_host(cps_handle *h, const float *s_dev, float *s_host, int E, const char *who);
 // cps_rpgd_fleet.cu
 void cps_rpgd_fleet_free(cps_handle *h);
 // cps_cem_fleet.cu

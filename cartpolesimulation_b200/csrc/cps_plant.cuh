@@ -1,6 +1,7 @@
-// cps_plant.cuh -- code shared by the fleets (cps_fleet.cu: MPPI on the ODE or the network, cps_rpgd_fleet.cu: RPGD): the
-// plant in the reference's mixed float32 / float64 arithmetic, the record row, the counter-based normal draws and the
-// device-side fold of the controller's model constants, with the host functions that fill their parameter blocks.
+// cps_plant.cuh -- code shared by the fleets (cps_fleet.cu: MPPI on the ODE or the network, cps_rpgd_fleet.cu: RPGD,
+// cps_cem_fleet.cu: CEM): the plant in the reference's mixed float32 / float64 arithmetic, the record row, the
+// counter-based normal draws and the device-side fold of the controller's model constants, with the host functions that
+// fill their parameter blocks; and FleetCore, the host-side state every fleet carries (cps_fleet.cu defines its functions).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -134,6 +135,19 @@ __device__ __forceinline__ void philox_normals(unsigned long long seed, unsigned
     }
 }
 
+// What a Philox fleet draws in one period, materialised (cps_fleet_noise, cps_rpgd_fleet_draws, cps_cem_fleet_draws, and
+// the draw workspaces of the neural MPPI period and the RPGD reset): per layer l < `layers`, experiment e < E and row
+// r < rows, philox_normals(seed, r, tag + l * tag_step, period, e_offset + e, n) into out + l * s_layer + e * s_exp +
+// r * s_row with element stride s_elem.  fleet_draws_launch (cps_fleet.cu) launches it on the handle's stream.
+struct FleetDrawsArgs {
+    unsigned long long seed;
+    unsigned tag, tag_step, period, e_offset;
+    int E, rows, n;
+    long long s_layer, s_exp, s_row, s_elem;
+    float *out;
+};
+int fleet_draws_launch(cps_handle *h, const FleetDrawsArgs &a, int layers);
+
 // ---- the plant (device restatement of oracle/cps_oracle.c: ode_plant, plant_integrate; no FMA contraction) ------------
 __device__ __forceinline__ void plant_ode(const PlantParams &P, float ca, float sa, float angleD, float positionD, float u,
                                           double &angleDD, double &positionDD) {
@@ -220,3 +234,56 @@ __device__ __forceinline__ void plant_ticks(const PlantParams &P, float *s, floa
         on_tick(i);
     }
 }
+
+// Experiment e's plant period with Q held and no plant-side models (fleet_net_plant_kernel, rpgd_fleet_finish_kernel):
+// the record row with Q_applied = Q when `record` is given, the n_sim ticks, the new state into s [E][8].
+__device__ __forceinline__ void plant_period_held(const PlantParams &P, float *s_all, int e, float Q, float *record, double time,
+                                                  const float *tp, const float *te) {
+    float s[6];
+#pragma unroll
+    for (int c = 0; c < 6; ++c) s[c] = s_all[(size_t)e * 8 + c];
+    const float u = __fmul_rn(P.u_max, Q);
+    double aDD, pDD;
+    plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
+    if (record)
+        plant_record(record + (size_t)e * CPS_FLEET_RECORD, time, s, aDD, pDD, Q, Q, u, tp ? tp[e] : 0.0f, te ? te[e] : 1.0f);
+    plant_ticks(P, s, u, aDD, pDD, [](int) {});
+    float *so = s_all + (size_t)e * 8;
+#pragma unroll
+    for (int c = 0; c < 6; ++c) so[c] = s[c];
+}
+
+// ---- host side: what every fleet keeps besides its optimizer ---------------------------------------------------------
+// The header all fleet config structs begin with (struct_size, n_experiments, sim_substeps, draw source, dt_simulation,
+// seed, experiment_offset) once validated, the plant states and each experiment's last control, and the period counter.
+struct FleetCore {
+    int E, n_sim, philox;
+    double dt_sim;
+    unsigned long long seed;
+    unsigned e_offset;
+    float *d_s, *d_uprev;       // [E][8], [E]
+    long long period;
+    int ready;                  // states have been set (the RPGD and CEM fleets refuse to run before)
+};
+// Validates the header into c (no allocation): n_experiments >= 1, sim_substeps >= 1, dt_simulation > 0, a known draw
+// source and sim_substeps x dt_simulation = the handle's dt.  The bound on E belongs to each fleet's solve grid.
+int fleet_core_init(cps_handle *h, FleetCore &c, int n_experiments, int sim_substeps, int source, double dt_simulation,
+                    unsigned long long seed, long long experiment_offset, const char *who);
+int fleet_core_alloc(cps_handle *h, FleetCore &c);   // d_s, d_uprev, zeroed
+void fleet_core_free(FleetCore &c);
+// States [E][6] from the host (argument check, u_prev = 0, period counter); synchronises.
+int fleet_core_set_states(cps_handle *h, FleetCore &c, const float *s_host, long long period, const char *who);
+// States [E][6] and u_prev [E] to the host, either may be null; synchronises the handle's stream.
+int fleet_core_get_states(cps_handle *h, const FleetCore &c, float *s_host, float *u_prev_host, const char *who);
+// Draws supplied by the caller or generated (Philox), as the fleet was created; `reads` false: this call reads none.
+int fleet_core_check_draws(cps_handle *h, const FleetCore &c, const float *draws_dev, bool reads, const char *who);
+// Row j of the [n_periods][E] target tables and of the [n_periods][E][CPS_FLEET_RECORD] records, for the current period.
+struct FleetRow {
+    const float *tp, *te;
+    float *record;
+    unsigned period;            // Philox counter
+    double time;                // period * dt_control
+};
+FleetRow fleet_core_row(const FleetCore &c, int j, const float *tp_dev, const float *te_dev, float *record_dev);
+// The handle's cost parameters folded for target_equilibrium = +1 and -1 (quadratic_boundary_grad selects its set on it).
+int fleet_fold_costs(cps_handle *h, CostParams *up, CostParams *dn);

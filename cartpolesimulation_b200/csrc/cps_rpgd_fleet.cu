@@ -109,14 +109,6 @@ struct SampleParams {
     float stdev, mean, lo, hi;
 };
 
-// cps_rpgd_fleet_draws: rows [E][rows][n_ind]
-__global__ void __launch_bounds__(128) rpgd_fleet_draws_kernel(unsigned long long seed, unsigned tag, unsigned period,
-                                                                unsigned e_offset, int rows, int n_ind, float *out) {
-    const int r = blockIdx.x * blockDim.x + threadIdx.x, e = blockIdx.y;
-    if (r >= rows) return;
-    philox_normals(seed, (unsigned)r, tag, period, e_offset + (unsigned)e, n_ind, out + ((size_t)e * rows + r) * n_ind, 1);
-}
-
 // optimizer_reset of every experiment (:379-408): plans from the draws [E * K][n_ind], zero moments and ages
 __global__ void __launch_bounds__(256) rpgd_fleet_reset_kernel(const float *draws, float *Q, float *m, float *v, int *ages,
                                                                 long long n, int T, const SampleParams sp) {
@@ -206,24 +198,8 @@ __device__ __forceinline__ void rpgd_finish(const RpgdFinishArgs &a) {
     // ---- the plant: one controller period with Q held (CartPole/__init__.py:283-324), as fleet_kernel without plant-side models
     const float Qc = Q[(size_t)s_src[0] * T];   // u_nom[0] of the cheapest improved plan
     a.u_prev[e] = Qc;                           // the returned control enters the next solve's cost
-    if (REPLAY) {
-        a.Q_out[e] = Qc;
-        return;
-    }
-    const PlantParams &P = a.plant;
-    float s[6];
-#pragma unroll
-    for (int c = 0; c < 6; ++c) s[c] = a.s[(size_t)e * 8 + c];
-    const float u = __fmul_rn(P.u_max, Qc);
-    double aDD, pDD;
-    plant_ode(P, s[IDX_COS], s[IDX_SIN], s[IDX_ANGLED], s[IDX_POSD], u, aDD, pDD);
-    if (a.record)
-        plant_record(a.record + (size_t)e * CPS_FLEET_RECORD, a.time, s, aDD, pDD, Qc, Qc, u, a.tp ? a.tp[e] : 0.0f,
-                     a.te ? a.te[e] : 1.0f);
-    plant_ticks(P, s, u, aDD, pDD, [](int) {});
-    float *so = a.s + (size_t)e * 8;
-#pragma unroll
-    for (int c = 0; c < 6; ++c) so[c] = s[c];
+    if (REPLAY) a.Q_out[e] = Qc;
+    else plant_period_held(a.plant, a.s, e, Qc, a.record, a.time, a.tp, a.te);
 }
 __global__ void __launch_bounds__(128) rpgd_fleet_finish_kernel(const __grid_constant__ RpgdFinishArgs a) {
     rpgd_finish<false>(a);
@@ -236,9 +212,9 @@ __global__ void __launch_bounds__(128) rpgd_relabel_finish_kernel(const __grid_c
 
 // ---- host side ---------------------------------------------------------------------------------------------------------
 struct RpgdFleetState {
+    FleetCore core;
     cps_rpgd_fleet_config cfg;
-    int E, K, T, nf;                  // nf = K - opt_keep_k fresh plans per resampling solve
-    float *d_s, *d_uprev;             // [E][8], [E]
+    int K, T, nf;                     // nf = K - opt_keep_k fresh plans per resampling solve
     float *d_Q[2], *d_m[2], *d_v[2];  // ping-pong plans and Adam moments [E][K][T]
     int *d_ages[2];                   // [E][K]
     int cur;                          // which half holds the current plans
@@ -248,14 +224,13 @@ struct RpgdFleetState {
     OdeParams *d_odes;                // [E] relabelling: each experiment's model constants for its row's L / m_pole (ODE only)
     float *d_draws;                   // Philox reset draws [E][K][n_ind]
     size_t finish_smem;
-    int ready;                        // cps_rpgd_fleet_set_states has run
-    long long period, solves, adam_iterations;
+    long long solves, adam_iterations;
 };
 
 void cps_rpgd_fleet_free(cps_handle *h) {
     RpgdFleetState *F = h->rfleet;
     if (!F) return;
-    cudaFree(F->d_s); cudaFree(F->d_uprev);
+    fleet_core_free(F->core);
     for (int i = 0; i < 2; ++i) { cudaFree(F->d_Q[i]); cudaFree(F->d_m[i]); cudaFree(F->d_v[i]); cudaFree(F->d_ages[i]); }
     cudaFree(F->d_ck); cudaFree(F->d_jac); cudaFree(F->d_J); cudaFree(F->d_G); cudaFree(F->d_costs); cudaFree(F->d_draws);
     cudaFree(F->d_odes);
@@ -273,52 +248,48 @@ static SampleParams sample_params(const cps_handle *h, const RpgdFleetState *F) 
 
 extern "C" int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config *cfg) {
     if (!h) return CPS_ERR_INVALID;
+    const char *who = "cps_rpgd_fleet_create";
     if (!cfg || cfg->struct_size != (int)sizeof(cps_rpgd_fleet_config))
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: cps_rpgd_fleet_config size mismatch");
+        return fail(h, CPS_ERR_INVALID, "%s: cps_rpgd_fleet_config size mismatch", who);
     const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
     if (h->cfg.integrator != CPS_EULER_CROMER && !neural)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: the adjoint of an RPGD fleet is built for predictor \"ODE\" "
-                    "(Euler-Cromer) and the neural predictor");
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: the adjoint of an RPGD fleet is built for predictor \"ODE\" (Euler-Cromer) and "
+                    "the neural predictor", who);
     if (h->cfg.cost_id != CPS_COST_QB_GRAD_MINIMAL && h->cfg.cost_id != CPS_COST_QB_GRAD)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: the adjoint is built for the quadratic_boundary_grad_minimal and "
-                    "quadratic_boundary_grad plugins");
-    if (!neural && h->cfg.substeps > 32)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: at most 32 substeps per control step");
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: the adjoint is built for the quadratic_boundary_grad_minimal and "
+                    "quadratic_boundary_grad plugins", who);
+    if (!neural && h->cfg.substeps > 32) return fail(h, CPS_ERR_UNSUPPORTED, "%s: at most 32 substeps per control step", who);
     const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
-    if (K > 4096) return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: at most 4096 plans (ranks by counting)");
-    if (cfg->n_experiments < 1 || cfg->sim_substeps < 1 || !(cfg->dt_simulation > 0.0))
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: need n_experiments >= 1, sim_substeps >= 1, dt_simulation > 0");
-    if ((long long)cfg->n_experiments * K > (1LL << 30))
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: at most 2^30 plans (n_experiments x K) per handle");
-    if (cfg->draw_source != CPS_FLEET_NOISE_SUPPLIED && cfg->draw_source != CPS_FLEET_NOISE_PHILOX)
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: unknown draw source %d", cfg->draw_source);
-    if (cfg->opt_keep_k < 1 || cfg->opt_keep_k > K)
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: opt_keep_k must lie in [1, K]");
-    if (cfg->shift_previous < 0) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: shift_previous < 0");
+    if (K > 4096) return fail(h, CPS_ERR_UNSUPPORTED, "%s: at most 4096 plans (ranks by counting)", who);
+    FleetCore core;
+    int rc;
+    if ((rc = fleet_core_init(h, core, cfg->n_experiments, cfg->sim_substeps, cfg->draw_source, cfg->dt_simulation, cfg->seed,
+                              cfg->experiment_offset, who)) != CPS_OK)
+        return rc;
+    if ((long long)core.E * K > (1LL << 30))
+        return fail(h, CPS_ERR_INVALID, "%s: at most 2^30 plans (n_experiments x K) per handle", who);
+    if (cfg->opt_keep_k < 1 || cfg->opt_keep_k > K) return fail(h, CPS_ERR_INVALID, "%s: opt_keep_k must lie in [1, K]", who);
+    if (cfg->shift_previous < 0) return fail(h, CPS_ERR_INVALID, "%s: shift_previous < 0", who);
     if (cfg->outer_its < 0 || cfg->first_iter_count < 0 || cfg->resamp_per < 1)
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: need outer_its >= 0, first_iter_count >= 0, resamp_per >= 1");
-    const double dt = (double)h->cfg.dt;
-    if (std::fabs(cfg->sim_substeps * cfg->dt_simulation - dt) > 1e-6 * dt)
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: dt (control) must be sim_substeps x dt_simulation");
+        return fail(h, CPS_ERR_INVALID, "%s: need outer_its >= 0, first_iter_count >= 0, resamp_per >= 1", who);
     const int nf = K - cfg->opt_keep_k;
-    const size_t smem = sizeof(float) * (2 * (size_t)K + (cfg->draw_source == CPS_FLEET_NOISE_PHILOX ? (size_t)nf * h->n_ind : 0));
+    const size_t smem = sizeof(float) * (2 * (size_t)K + (core.philox ? (size_t)nf * h->n_ind : 0));
     if (smem > 227 * 1024)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_rpgd_fleet_create: (K - opt_keep_k) x n_ind too large for the finish kernel's "
-                    "shared memory");
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: (K - opt_keep_k) x n_ind too large for the finish kernel's shared memory", who);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    int rc;   // neural: the network checks of cps_plan_cost_grad, and the workspace sized now rather than mid-run
-    if (neural && (rc = cps_net_grad_fleet_prepare(h, cfg->n_experiments, "cps_rpgd_fleet_create")) != CPS_OK) return rc;
+    // neural: the network checks of cps_plan_cost_grad, and the workspace sized now rather than mid-run
+    if (neural && (rc = cps_net_grad_fleet_prepare(h, core.E, who)) != CPS_OK) return rc;
     cps_rpgd_fleet_free(h);
     RpgdFleetState *F = new (std::nothrow) RpgdFleetState();
-    if (!F) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_create: out of host memory");
+    if (!F) return fail(h, CPS_ERR_INVALID, "%s: out of host memory", who);
     memset(F, 0, sizeof(*F));
+    F->core = core;
     F->cfg = *cfg;
-    F->E = cfg->n_experiments; F->K = K; F->T = T; F->nf = nf;
+    F->K = K; F->T = T; F->nf = nf;
     F->finish_smem = smem;
     h->rfleet = F;
-    const size_t E = F->E, EK = E * K, n = EK * T;
-    CUDA_TRY(h, cudaMalloc(&F->d_s, sizeof(float) * E * 8));
-    CUDA_TRY(h, cudaMalloc(&F->d_uprev, sizeof(float) * E));
+    const size_t E = core.E, EK = E * K, n = EK * T;
+    if ((rc = fleet_core_alloc(h, F->core)) != CPS_OK) return rc;
     for (int i = 0; i < 2; ++i) {
         CUDA_TRY(h, cudaMalloc(&F->d_Q[i], sizeof(float) * n));
         CUDA_TRY(h, cudaMalloc(&F->d_m[i], sizeof(float) * n));
@@ -333,7 +304,7 @@ extern "C" int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config 
     CUDA_TRY(h, cudaMalloc(&F->d_J, sizeof(float) * EK));
     CUDA_TRY(h, cudaMalloc(&F->d_G, sizeof(float) * n));
     CUDA_TRY(h, cudaMalloc(&F->d_costs, sizeof(CostParams) * E));
-    if (cfg->draw_source == CPS_FLEET_NOISE_PHILOX) CUDA_TRY(h, cudaMalloc(&F->d_draws, sizeof(float) * EK * h->n_ind));
+    if (core.philox) CUDA_TRY(h, cudaMalloc(&F->d_draws, sizeof(float) * EK * h->n_ind));
     if (smem > 48 * 1024) {
         CUDA_TRY(h, cudaFuncSetAttribute((const void *)rpgd_fleet_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         CUDA_TRY(h, cudaFuncSetAttribute((const void *)rpgd_relabel_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -341,48 +312,38 @@ extern "C" int cps_rpgd_fleet_create(cps_handle *h, const cps_rpgd_fleet_config 
     return CPS_OK;
 }
 
+// The Philox draws [E][rows][n_ind]: period -1 those of a reset (K rows), else the resampling draws of `period`
 static int draws_launch(cps_handle *h, RpgdFleetState *F, long long period, float *out_dev) {
     const bool reset = period < 0;
     const int rows = reset ? F->K : F->nf;
     if (rows == 0) return CPS_OK;
-    const dim3 grid((rows + 127) / 128, F->E);
-    rpgd_fleet_draws_kernel<<<grid, 128, 0, h->stream>>>(F->cfg.seed, reset ? RPGD_DRAWS_RESET : RPGD_DRAWS_RESAMPLE,
-                                                          reset ? 0u : (unsigned)period, (unsigned)F->cfg.experiment_offset,
-                                                          rows, h->n_ind, out_dev);
-    h->launches += 1;
-    CUDA_TRY(h, cudaGetLastError());
-    return CPS_OK;
+    const FleetDrawsArgs d = {F->core.seed, reset ? RPGD_DRAWS_RESET : RPGD_DRAWS_RESAMPLE, 0u, reset ? 0u : (unsigned)period,
+                              F->core.e_offset, F->core.E, rows, h->n_ind, 0, (long long)rows * h->n_ind, h->n_ind, 1, out_dev};
+    return fleet_draws_launch(h, d, 1);
 }
 
 extern "C" int cps_rpgd_fleet_set_states(cps_handle *h, const float *s_host, const float *init_draws_dev, long long period) {
     if (!h) return CPS_ERR_INVALID;
+    const char *who = "cps_rpgd_fleet_set_states";
     RpgdFleetState *F = h->rfleet;
-    if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_set_states: no RPGD fleet (cps_rpgd_fleet_create)");
-    const bool philox = F->cfg.draw_source == CPS_FLEET_NOISE_PHILOX;
-    if (!s_host || period < 0) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_set_states: bad argument");
-    if (!philox && !init_draws_dev) return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_set_states: this fleet expects supplied draws");
-    if (philox && init_draws_dev)
-        return fail(h, CPS_ERR_INVALID, "cps_rpgd_fleet_set_states: this fleet generates its draws (Philox); pass NULL");
-    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    CUDA_TRY(h, cudaMemsetAsync(F->d_uprev, 0, sizeof(float) * (size_t)F->E, h->stream));
+    if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no RPGD fleet (cps_rpgd_fleet_create)", who);
+    FleetCore &c = F->core;
     int rc;
-    if ((rc = fleet_states_to_device(h, s_host, F->d_s, F->E, "cps_rpgd_fleet_set_states")) != CPS_OK) return rc;
-    if (philox && (rc = draws_launch(h, F, -1, F->d_draws)) != CPS_OK) return rc;
+    if ((rc = fleet_core_check_draws(h, c, init_draws_dev, true, who)) != CPS_OK) return rc;
+    if ((rc = fleet_core_set_states(h, c, s_host, period, who)) != CPS_OK) return rc;
+    if (c.philox && (rc = draws_launch(h, F, -1, F->d_draws)) != CPS_OK) return rc;
     F->cur = 0;
-    const long long n = (long long)F->E * F->K * F->T;
+    const long long n = (long long)c.E * F->K * F->T;
     const int grid = (int)((n + 255) / 256 < 4096 ? (n + 255) / 256 : 4096);
-    rpgd_fleet_reset_kernel<<<grid, 256, 0, h->stream>>>(philox ? F->d_draws : init_draws_dev, F->d_Q[0], F->d_m[0], F->d_v[0],
+    rpgd_fleet_reset_kernel<<<grid, 256, 0, h->stream>>>(c.philox ? F->d_draws : init_draws_dev, F->d_Q[0], F->d_m[0], F->d_v[0],
                                                           F->d_ages[0], n, F->T, sample_params(h, F));
     h->launches += 1;
     CUDA_TRY(h, cudaGetLastError());
-    F->period = period;
     F->solves = 0;
     F->adam_iterations = 0;
-    F->ready = 1;
+    c.ready = 1;
     return CPS_OK;
 }
-
-int cps_fold_cost_for(cps_handle *h, float target_equilibrium, CostParams *out);
 
 // Shared by cps_rpgd_fleet_step (closed loop: replay_dev == nullptr) and cps_rpgd_fleet_relabel (states from a recording).
 static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, const float *tp_dev, const float *te_dev,
@@ -390,56 +351,54 @@ static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, cons
                              const float *replay_dev, const float *L_dev, const float *mp_dev, float *Q_out_dev) {
     RpgdFleetState *F = h->rfleet;
     if (!F) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no RPGD fleet (cps_rpgd_fleet_create)", who);
-    if (!F->ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no states yet (cps_rpgd_fleet_set_states)", who);
+    FleetCore &fc = F->core;
+    if (!fc.ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: no states yet (cps_rpgd_fleet_set_states)", who);
     if (n_periods < 0) return fail(h, CPS_ERR_INVALID, "%s: negative number of periods / rows", who);
-    const bool philox = F->cfg.draw_source == CPS_FLEET_NOISE_PHILOX;
-    if (!philox && !draws_dev && F->nf > 0) return fail(h, CPS_ERR_INVALID, "%s: this fleet expects supplied draws", who);
-    if (philox && draws_dev) return fail(h, CPS_ERR_INVALID, "%s: this fleet generates its draws (Philox); pass NULL", who);
+    int rc;
+    if ((rc = fleet_core_check_draws(h, fc, draws_dev, F->nf > 0, who)) != CPS_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     const bool neural = h->cfg.integrator == CPS_PREDICTOR_NEURAL;
-    int rc;   // neural: the network may have been reloaded since create (another size): check it, grow the workspace
-    if (neural && (rc = cps_net_grad_fleet_prepare(h, F->E, who)) != CPS_OK) return rc;
+    // neural: the network may have been reloaded since create (another size): check it, grow the workspace
+    if (neural && (rc = cps_net_grad_fleet_prepare(h, fc.E, who)) != CPS_OK) return rc;
     CostParams up, dn;
-    if ((rc = cps_fold_cost_for(h, 1.0f, &up)) != CPS_OK) return rc;
-    if ((rc = cps_fold_cost_for(h, -1.0f, &dn)) != CPS_OK) return rc;
+    if ((rc = fleet_fold_costs(h, &up, &dn)) != CPS_OK) return rc;
     const cps_rpgd_fleet_config &c = F->cfg;
-    const size_t E = F->E, K = F->K, T = F->T;
+    const size_t E = fc.E, K = F->K, T = F->T;
     const int EK = (int)(E * K);
     RpgdFinishArgs a;
     memset(&a, 0, sizeof(a));
-    a.philox = philox ? 1 : 0;
-    a.seed = c.seed; a.e_offset = (unsigned)c.experiment_offset;
+    a.philox = fc.philox;
+    a.seed = fc.seed; a.e_offset = fc.e_offset;
     a.K = (int)K; a.T = (int)T; a.keep = c.opt_keep_k; a.shift = c.shift_previous;
     a.sp = sample_params(h, F);
-    a.u_prev = F->d_uprev; a.s = F->d_s;
-    a.plant = plant_params(h, c.dt_simulation, c.sim_substeps);
-    const double dt_control = c.dt_simulation * c.sim_substeps;
+    a.u_prev = fc.d_uprev; a.s = fc.d_s;
+    a.plant = plant_params(h, fc.dt_sim, fc.n_sim);
     // relabelling: the network reads neither L nor m_pole, so only predictor "ODE" folds per-row model constants
     const OdeParams *odes = (replay_dev && !neural && (L_dev || mp_dev)) ? F->d_odes : nullptr;
     RpgdRowArgs ra;
     memset(&ra, 0, sizeof(ra));
     ra.up = up; ra.dn = dn;
-    ra.costs = F->d_costs; ra.s = F->d_s; ra.odes = const_cast<OdeParams *>(odes);
+    ra.costs = F->d_costs; ra.s = fc.d_s; ra.odes = const_cast<OdeParams *>(odes);
     ra.ode = h->ode;
     ra.fold = fold_inputs(h);
     ra.E = (int)E;
     for (int j = 0; j < n_periods; ++j) {
-        const float *tp = tp_dev ? tp_dev + (size_t)j * E : nullptr, *te = te_dev ? te_dev + (size_t)j * E : nullptr;
+        const FleetRow row = fleet_core_row(fc, j, tp_dev, te_dev, record_dev);
         if (replay_dev) {
-            ra.tp = tp; ra.te = te;
+            ra.tp = row.tp; ra.te = row.te;
             ra.states = replay_dev + (size_t)j * E * 6;
             ra.L_row = L_dev ? L_dev + (size_t)j * E : nullptr;
             ra.mp_row = mp_dev ? mp_dev + (size_t)j * E : nullptr;
             rpgd_relabel_row_kernel<<<(unsigned)((E + 127) / 128), 128, 0, h->stream>>>(ra);
         } else {
-            rpgd_fleet_cost_kernel<<<(unsigned)((E + 127) / 128), 128, 0, h->stream>>>(up, dn, tp, te, F->d_costs, (int)E);
+            rpgd_fleet_cost_kernel<<<(unsigned)((E + 127) / 128), 128, 0, h->stream>>>(up, dn, row.tp, row.te, F->d_costs, (int)E);
         }
         h->launches += 1;
         float *Q = F->d_Q[F->cur], *m = F->d_m[F->cur], *v = F->d_v[F->cur];
         const int its = F->solves == 0 ? c.first_iter_count : c.outer_its;
         for (int it = 0; it < its; ++it) {   // grad_step (:166-180)
-            rc = neural ? cps_net_grad_fleet(h, (int)E, F->d_s, Q, F->d_costs, F->d_uprev, F->d_J, F->d_G)
-                        : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, F->d_ck, F->d_jac, F->d_J, F->d_G,
+            rc = neural ? cps_net_grad_fleet(h, (int)E, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_J, F->d_G)
+                        : cps_grad_fleet(h, EK, (int)K, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_ck, F->d_jac, F->d_J, F->d_G,
                                          odes);
             if (rc != CPS_OK) return rc;
             F->adam_iterations += 1;
@@ -451,20 +410,18 @@ static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, cons
                 return rc;
         }
         // get_action (:182-224): the costs of the improved plans
-        rc = neural ? cps_net_grad_fleet(h, (int)E, F->d_s, Q, F->d_costs, F->d_uprev, F->d_J, nullptr)
-                    : cps_grad_fleet(h, EK, (int)K, F->d_s, Q, F->d_costs, F->d_uprev, nullptr, nullptr, F->d_J, nullptr, odes);
+        rc = neural ? cps_net_grad_fleet(h, (int)E, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_J, nullptr)
+                    : cps_grad_fleet(h, EK, (int)K, fc.d_s, Q, F->d_costs, fc.d_uprev, nullptr, nullptr, F->d_J, nullptr, odes);
         if (rc != CPS_OK) return rc;
         const int nxt = F->cur ^ 1;
         a.J = F->d_J; a.Q = Q; a.m = m; a.v = v; a.ages = F->d_ages[F->cur];
         a.Q2 = F->d_Q[nxt]; a.m2 = F->d_m[nxt]; a.v2 = F->d_v[nxt]; a.ages2 = F->d_ages[nxt];
         a.resample = (F->solves % c.resamp_per == 0) ? 1 : 0;
-        a.draws = (!philox && a.resample) ? draws_dev + (size_t)j * E * F->nf * h->n_ind : nullptr;
-        a.period = (unsigned)F->period;
-        a.tp = tp; a.te = te;
-        a.record = record_dev ? record_dev + (size_t)j * E * CPS_FLEET_RECORD : nullptr;
+        a.draws = (!fc.philox && a.resample) ? draws_dev + (size_t)j * E * F->nf * h->n_ind : nullptr;
+        a.period = row.period;
+        a.tp = row.tp; a.te = row.te; a.record = row.record; a.time = row.time;
         a.J_out = J_out_dev ? J_out_dev + (size_t)j * E * K : nullptr;
         a.Q_opt = Q_opt_out_dev ? Q_opt_out_dev + (size_t)j * E * K * T : nullptr;
-        a.time = (double)F->period * dt_control;
         a.Q_out = Q_out_dev ? Q_out_dev + (size_t)j * E : nullptr;
         if (replay_dev) rpgd_relabel_finish_kernel<<<(unsigned)E, 128, F->finish_smem, h->stream>>>(a);
         else rpgd_fleet_finish_kernel<<<(unsigned)E, 128, F->finish_smem, h->stream>>>(a);
@@ -472,7 +429,7 @@ static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, cons
         CUDA_TRY(h, cudaGetLastError());
         F->cur = nxt;
         F->solves += 1;
-        F->period += 1;
+        fc.period += 1;
     }
     return CPS_OK;
 }
@@ -496,37 +453,32 @@ extern "C" int cps_rpgd_fleet_relabel(cps_handle *h, int n_rows, const float *st
 extern "C" int cps_rpgd_fleet_get_states(cps_handle *h, float *s_host, float *u_prev_host) {
     if (!h) return CPS_ERR_INVALID;
     RpgdFleetState *F = h->rfleet;
-    if (!F || !F->ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_get_states: no RPGD fleet with states "
-                                    "(cps_rpgd_fleet_create, cps_rpgd_fleet_set_states)");
-    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    int rc;
-    if (s_host && (rc = fleet_states_to_host(h, F->d_s, s_host, F->E, "cps_rpgd_fleet_get_states")) != CPS_OK) return rc;
-    if (u_prev_host)
-        CUDA_TRY(h, cudaMemcpyAsync(u_prev_host, F->d_uprev, sizeof(float) * (size_t)F->E, cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    return CPS_OK;
+    if (!F || !F->core.ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_get_states: no RPGD fleet with states "
+                                          "(cps_rpgd_fleet_create, cps_rpgd_fleet_set_states)");
+    return fleet_core_get_states(h, F->core, s_host, u_prev_host, "cps_rpgd_fleet_get_states");
 }
 
 extern "C" int cps_rpgd_fleet_get_plans(cps_handle *h, float *Q_host, float *m_host, float *v_host, int *ages_host,
                                         long long *adam_iterations, long long *solves) {
     if (!h) return CPS_ERR_INVALID;
     RpgdFleetState *F = h->rfleet;
-    if (!F || !F->ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_get_plans: no RPGD fleet with states "
-                                    "(cps_rpgd_fleet_create, cps_rpgd_fleet_set_states)");
+    if (!F || !F->core.ready) return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_rpgd_fleet_get_plans: no RPGD fleet with states "
+                                          "(cps_rpgd_fleet_create, cps_rpgd_fleet_set_states)");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    const size_t n = (size_t)F->E * F->K * F->T;
+    const size_t n = (size_t)F->core.E * F->K * F->T;
     if (Q_host) CUDA_TRY(h, cudaMemcpyAsync(Q_host, F->d_Q[F->cur], sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
     if (m_host) CUDA_TRY(h, cudaMemcpyAsync(m_host, F->d_m[F->cur], sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
     if (v_host) CUDA_TRY(h, cudaMemcpyAsync(v_host, F->d_v[F->cur], sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
     if (ages_host)
-        CUDA_TRY(h, cudaMemcpyAsync(ages_host, F->d_ages[F->cur], sizeof(int) * (size_t)F->E * F->K, cudaMemcpyDeviceToHost, h->stream));
+        CUDA_TRY(h, cudaMemcpyAsync(ages_host, F->d_ages[F->cur], sizeof(int) * (size_t)F->core.E * F->K, cudaMemcpyDeviceToHost,
+                                    h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (adam_iterations) *adam_iterations = F->adam_iterations;
     if (solves) *solves = F->solves;
     return CPS_OK;
 }
 
-extern "C" long long cps_rpgd_fleet_period(const cps_handle *h) { return (h && h->rfleet) ? h->rfleet->period : -1; }
+extern "C" long long cps_rpgd_fleet_period(const cps_handle *h) { return (h && h->rfleet) ? h->rfleet->core.period : -1; }
 
 extern "C" int cps_rpgd_fleet_draws(cps_handle *h, long long period, float *out_dev) {
     if (!h) return CPS_ERR_INVALID;

@@ -187,7 +187,71 @@ def _relabel_rows(fleet, states, Q_out):
     return R, Q_out
 
 
-class Fleet:
+class _FleetBase:
+    """What the MPPI, RPGD and CEM fleets do alike: one Engine with one fleet of the kind `_abi` names (the C ABI's
+    function prefix) attached, created from the config header every fleet config struct begins with."""
+    _abi = ""
+
+    def _fn(self, name):
+        return getattr(self.engine.lib, f"{self._abi}_{name}")
+
+    def _setup_engine(self, control_limits, cost_config):
+        """The optimizers' control limits (set_mppi_params lo, hi) and an optional cost configuration."""
+        lo, hi = (float(np.asarray(x, dtype=np.float32).reshape(-1)[0]) for x in control_limits)
+        if cost_config is not None:
+            self.engine.set_cost_config(cost_config)
+        self.engine.set_mppi_params(lo=lo, hi=hi)
+
+    def _create(self, config, n_sim: int, noise: str, dt_simulation: float, seed: int, experiment_offset: int, *rest):
+        """<abi>_create with the header (struct_size, E, sim_substeps, draw source, dt_simulation, seed,
+        experiment_offset) followed by the fleet's own fields `rest`."""
+        c = config(C.sizeof(config), self.E, n_sim, L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
+                   float(dt_simulation), int(seed), int(experiment_offset), *rest)
+        self.noise_source = noise
+        self.engine._chk(self._fn("create")(self.engine._h, C.byref(c)))
+
+    def close(self):
+        self.engine.close()
+
+    def _host_states(self, states) -> np.ndarray:
+        s = np.ascontiguousarray(states, dtype=np.float32)
+        if s.shape != (self.E, 6):
+            raise ValueError(f"states must have shape ({self.E}, 6)")
+        self.engine.use_current_stream()
+        return s
+
+    def states(self, with_u_prev: bool = False):
+        s = np.zeros((self.E, 6), dtype=np.float32)
+        u_prev = np.zeros(self.E, dtype=np.float32) if with_u_prev else None
+        self.engine.use_current_stream()
+        self.engine._chk(self._fn("get_states")(self.engine._h, s.ctypes.data_as(L._FP),
+                                                None if u_prev is None else u_prev.ctypes.data_as(L._FP)))
+        return (s, u_prev) if with_u_prev else s
+
+    @property
+    def period(self) -> int:
+        return int(self._fn("period")(self.engine._h))
+
+    def nonfinite_costs(self) -> int:
+        """Non-finite plan costs met so far (a NaN state or target makes them so; such costs sort after every number, as
+        torch.sort does, stay in their experiment, and the run goes on).  Synchronises."""
+        self.engine.use_current_stream()
+        return self.engine.nonfinite_costs()
+
+    def set_plant_models(self, *args, **kwargs):
+        raise NotImplementedError(f"{type(self).__name__} has no plant-side models (control disturbance, measurement noise, "
+                                  "latency)")
+
+    def _check_rows(self, rows: int, target_position, target_equilibrium, record, J_out, *more):
+        """Device and size of the [rows, E] targets, record [rows, E, 16], J_out [rows, E, K] and `more` ((tensor, name,
+        numel) as _check_sizes takes them) of run / relabel; the engine on the current stream."""
+        self.engine.use_current_stream()
+        _check_sizes(self.device, (target_position, "target_position", rows * self.E),
+                     (target_equilibrium, "target_equilibrium", rows * self.E),
+                     (record, "record", rows * self.E * L.FLEET_RECORD), (J_out, "J_out", rows * self.E * self.K), *more)
+
+
+class Fleet(_FleetBase):
     """E closed-loop experiments on one device = one cps_handle with a fleet attached.
 
     Predictor "ODE" / "ODE_v0", or "neural" with `network`: the spec dict Engine.net_load takes
@@ -196,6 +260,7 @@ class Fleet:
     CartPole ODE.  Each experiment then owns a hidden state (net_states / set_net_states), set to the network's stored
     state by reset() and advanced on (u, s) after every solve, as optimizer_mppi does.  Plant-side models are not offered
     on neural fleets (set_plant_models raises NotImplementedError)."""
+    _abi = "cps_fleet"
 
     def __init__(self, n_experiments: int, num_rollouts: int = 2000, horizon: int = 50, dt: float = 0.02,
                  substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
@@ -210,20 +275,10 @@ class Fleet:
             self.engine.net_load(network)
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(horizon)
         self.n_ind, self.device = self.engine.n_ind, self.engine.device
-        c = L.cps_fleet_config(C.sizeof(L.cps_fleet_config), self.E, n_sim,
-                               L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
-                               float(dt_simulation), int(seed), int(experiment_offset))
-        self.noise_source = noise
-        self.engine._chk(self.engine.lib.cps_fleet_create(self.engine._h, C.byref(c)))
-
-    def close(self):
-        self.engine.close()
+        self._create(L.cps_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset)
 
     def reset(self, states, period: int = 0):
-        s = np.ascontiguousarray(states, dtype=np.float32)
-        if s.shape != (self.E, 6):
-            raise ValueError(f"states must have shape ({self.E}, 6)")
-        self.engine.use_current_stream()
+        s = self._host_states(states)
         self.engine._chk(self.engine.lib.cps_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP), int(period)))
 
     def states(self, with_u_nom: bool = False):
@@ -235,10 +290,6 @@ class Fleet:
             self.engine._h, s.ctypes.data_as(L._FP), None if u_nom is None else u_nom.ctypes.data_as(L._FP),
             None if u_prev is None else u_prev.ctypes.data_as(L._FP)))
         return (s, u_nom, u_prev) if with_u_nom else s
-
-    @property
-    def period(self) -> int:
-        return int(self.engine.lib.cps_fleet_period(self.engine._h))
 
     def noise(self, period: int) -> torch.Tensor:
         """The draws the Philox source uses in `period`: cuda tensor [E, n_ind, K]."""
@@ -300,12 +351,8 @@ class Fleet:
         (set_plant_models): ctrl_draws [n_periods, E] and meas_draws [n_periods, sim_substeps, E, 4] supply their draws
         (cps_fleet_step_noisy); a 'philox' fleet draws them itself when they are None."""
         eng = self.engine
-        eng.use_current_stream()
-        _check_sizes(self.device, (target_position, "target_position", n_periods * self.E),
-                     (target_equilibrium, "target_equilibrium", n_periods * self.E),
-                     (noise, "noise", n_periods * self.E * self.n_ind * self.K),
-                     (record, "record", n_periods * self.E * L.FLEET_RECORD),
-                     (J_out, "J_out", n_periods * self.E * self.K))
+        self._check_rows(n_periods, target_position, target_equilibrium, record, J_out,
+                         (noise, "noise", n_periods * self.E * self.n_ind * self.K))
         if getattr(self, "plant_models", False):
             for t, name in ((ctrl_draws, "ctrl_draws"), (meas_draws, "meas_draws")):
                 if t is not None:
@@ -326,13 +373,10 @@ class Fleet:
         (cps_fleet_relabel_masked).  Zeroing the warm starts first (Relabeller.reset: cps_fleet_reset) is the reference's
         controller.reset().  Returns Q_out."""
         eng = self.engine
-        eng.use_current_stream()
         R, Q_out = _relabel_rows(self, states, Q_out)
-        _check_sizes(self.device, (target_position, "target_position", R * self.E),
-                     (target_equilibrium, "target_equilibrium", R * self.E),
-                     (L, "L", R * self.E), (m_pole, "m_pole", R * self.E),
-                     (noise, "noise", R * self.E * self.n_ind * self.K),
-                     (Q_out, "Q_out", R * self.E), (J_out, "J_out", R * self.E * self.K))
+        self._check_rows(R, target_position, target_equilibrium, None, J_out, (L, "L", R * self.E),
+                         (m_pole, "m_pole", R * self.E), (noise, "noise", R * self.E * self.n_ind * self.K),
+                         (Q_out, "Q_out", R * self.E))
         if active is None:
             eng._chk(eng.lib.cps_fleet_relabel(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
                                                _ptr(L), _ptr(m_pole), _ptr(noise), _ptr(Q_out), _ptr(J_out)))
@@ -346,7 +390,7 @@ class Fleet:
         return Q_out
 
 
-class RpgdFleet:
+class RpgdFleet(_FleetBase):
     """E closed-loop experiments under RPGD, the reference's shipped default optimizer (Control_Toolkit_ASF/
     config_controllers.yml:2), on one device: one cps_handle with an RPGD fleet attached (include/cps.h "RPGD fleet").
 
@@ -361,6 +405,7 @@ class RpgdFleet:
     optimizer_rpgd_b200 and the reference's RPGD.  Cost quadratic_boundary_grad_minimal or quadratic_boundary_grad;
     uniform resampling and the plant-side models (Fleet.set_plant_models) are not implemented and raise
     NotImplementedError."""
+    _abi = "cps_rpgd_fleet"
 
     def __init__(self, n_experiments: int, num_rollouts: int = 16, mpc_horizon: int = 35, outer_its: int = 4,
                  resamp_per: int = 10, opt_keep_k_ratio: float = 0.75, period_interpolation_inducing_points: int = 4,
@@ -380,48 +425,24 @@ class RpgdFleet:
         self.outer_its, self.resamp_per, self.shift_previous = int(outer_its), int(resamp_per), int(shift_previous)
         self.first_iter_count = int(warmup_iterations) if warmup else self.outer_its   # as optimizer_rpgd_b200
         self.opt_keep_k = int(max(int(self.K * opt_keep_k_ratio), 1))
-        self.noise_source = noise
-        lo, hi = (float(np.asarray(x, dtype=np.float32).reshape(-1)[0]) for x in control_limits)
         self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost,
                              interp_period=period_interpolation_inducing_points, device=device)
         self.n_ind, self.device = self.engine.n_ind, self.engine.device
-        if cost_config is not None:
-            self.engine.set_cost_config(cost_config)
-        self.engine.set_mppi_params(lo=lo, hi=hi)
+        self._setup_engine(control_limits, cost_config)
         if network is not None:
             self.engine.net_load(network)
-        c = L.cps_rpgd_fleet_config(C.sizeof(L.cps_rpgd_fleet_config), self.E, n_sim,
-                                    L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
-                                    float(dt_simulation), int(seed), int(experiment_offset), self.outer_its,
-                                    self.first_iter_count, self.resamp_per, self.opt_keep_k, self.shift_previous,
-                                    float(learning_rate), float(adam_beta_1), float(adam_beta_2), float(adam_epsilon),
-                                    float(gradmax_clip), float(sample_stdev), float(sample_mean))
-        self.engine._chk(self.engine.lib.cps_rpgd_fleet_create(self.engine._h, C.byref(c)))
-
-    def close(self):
-        self.engine.close()
-
-    def set_plant_models(self, *args, **kwargs):
-        raise NotImplementedError("RpgdFleet has no plant-side models (control disturbance, measurement noise, latency)")
+        self._create(L.cps_rpgd_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset, self.outer_its,
+                     self.first_iter_count, self.resamp_per, self.opt_keep_k, self.shift_previous, float(learning_rate),
+                     float(adam_beta_1), float(adam_beta_2), float(adam_epsilon), float(gradmax_clip), float(sample_stdev),
+                     float(sample_mean))
 
     def reset(self, states, period: int = 0, init_draws=None):
         """optimizer_reset of every experiment and the initial states [E, 6].  init_draws: cuda tensor [E, K, n_ind] of
         standard normals for the initial plans ('supplied' fleets; a 'philox' fleet draws them, see draws(-1))."""
-        s = np.ascontiguousarray(states, dtype=np.float32)
-        if s.shape != (self.E, 6):
-            raise ValueError(f"states must have shape ({self.E}, 6)")
+        s = self._host_states(states)
         _check_sizes(self.device, (init_draws, "init_draws", self.E * self.K * self.n_ind))
-        self.engine.use_current_stream()
         self.engine._chk(self.engine.lib.cps_rpgd_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP),
                                                                    _ptr(init_draws), int(period)))
-
-    def states(self, with_u_prev: bool = False):
-        s = np.zeros((self.E, 6), dtype=np.float32)
-        u_prev = np.zeros(self.E, dtype=np.float32) if with_u_prev else None
-        self.engine.use_current_stream()
-        self.engine._chk(self.engine.lib.cps_rpgd_fleet_get_states(
-            self.engine._h, s.ctypes.data_as(L._FP), None if u_prev is None else u_prev.ctypes.data_as(L._FP)))
-        return (s, u_prev) if with_u_prev else s
 
     def plans(self) -> dict:
         """The optimizer state of every experiment: Q, m, v [E, K, T], ages [E, K] (int32), and the shared Adam iteration
@@ -434,16 +455,6 @@ class RpgdFleet:
             self.engine._h, Q.ctypes.data_as(L._FP), m.ctypes.data_as(L._FP), v.ctypes.data_as(L._FP),
             ages.ctypes.data_as(C.POINTER(C.c_int)), C.byref(it), C.byref(solves)))
         return dict(Q=Q, m=m, v=v, ages=ages, adam_iterations=int(it.value), solves=int(solves.value))
-
-    @property
-    def period(self) -> int:
-        return int(self.engine.lib.cps_rpgd_fleet_period(self.engine._h))
-
-    def nonfinite_costs(self) -> int:
-        """Non-finite plan costs met so far (a NaN state or target makes them so; such costs sort after every number, as
-        torch.sort does, and the run goes on).  Synchronises."""
-        self.engine.use_current_stream()
-        return self.engine.nonfinite_costs()
 
     def draws(self, period: int) -> torch.Tensor:
         """The draws a 'philox' fleet uses: period >= 0 its resampling draws [E, K - opt_keep_k, n_ind]; period = -1 the
@@ -461,13 +472,9 @@ class RpgdFleet:
         resampling periods only); record [n_periods, E, 16], J_out [n_periods, E, K] (costs of the improved plans) and
         Q_opt [n_periods, E, K, T] (plans after the Adam steps) or None."""
         eng = self.engine
-        eng.use_current_stream()
-        _check_sizes(self.device, (target_position, "target_position", n_periods * self.E),
-                     (target_equilibrium, "target_equilibrium", n_periods * self.E),
-                     (draws, "draws", n_periods * self.E * (self.K - self.opt_keep_k) * self.n_ind),
-                     (record, "record", n_periods * self.E * L.FLEET_RECORD),
-                     (J_out, "J_out", n_periods * self.E * self.K),
-                     (Q_opt, "Q_opt", n_periods * self.E * self.K * self.T))
+        self._check_rows(n_periods, target_position, target_equilibrium, record, J_out,
+                         (draws, "draws", n_periods * self.E * (self.K - self.opt_keep_k) * self.n_ind),
+                         (Q_opt, "Q_opt", n_periods * self.E * self.K * self.T))
         eng._chk(eng.lib.cps_rpgd_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
                                              _ptr(draws), _ptr(record), _ptr(J_out), _ptr(Q_opt)))
         return record
@@ -482,19 +489,16 @@ class RpgdFleet:
         if active is not None:
             raise NotImplementedError("RPGD relabelling advances every file in lockstep: no per-file mask")
         eng = self.engine
-        eng.use_current_stream()
         R, Q_out = _relabel_rows(self, states, Q_out)
-        _check_sizes(self.device, (target_position, "target_position", R * self.E),
-                     (target_equilibrium, "target_equilibrium", R * self.E),
-                     (L, "L", R * self.E), (m_pole, "m_pole", R * self.E),
-                     (draws, "draws", R * self.E * (self.K - self.opt_keep_k) * self.n_ind),
-                     (Q_out, "Q_out", R * self.E), (J_out, "J_out", R * self.E * self.K))
+        self._check_rows(R, target_position, target_equilibrium, None, J_out, (L, "L", R * self.E),
+                         (m_pole, "m_pole", R * self.E),
+                         (draws, "draws", R * self.E * (self.K - self.opt_keep_k) * self.n_ind), (Q_out, "Q_out", R * self.E))
         eng._chk(eng.lib.cps_rpgd_fleet_relabel(eng._h, R, _ptr(states), _ptr(target_position), _ptr(target_equilibrium),
                                                 _ptr(L), _ptr(m_pole), _ptr(draws), _ptr(Q_out), _ptr(J_out)))
         return Q_out
 
 
-class CemFleet:
+class CemFleet(_FleetBase):
     """E closed-loop experiments under optimizer_cem_tf (`cem-tf` in Control_Toolkit_ASF/config_controllers.yml) on one
     device: one cps_handle with a CEM fleet attached (include/cps.h "CEM fleet").
 
@@ -504,6 +508,7 @@ class CemFleet:
     plant does, with no host round trip.  The keywords are optimizer_cem_b200's (same defaults) and Fleet's.  Predictor
     "ODE" or "ODE_v0" and the four cost plugins; num_rollouts at most 8192.  The neural predictor and the plant-side models
     (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+    _abi = "cps_cem_fleet"
 
     def __init__(self, n_experiments: int, num_rollouts: int = 200, mpc_horizon: int = 35, cem_outer_it: int = 3,
                  cem_initial_action_stdev: float = 0.5, cem_stdev_min: float = 0.01, cem_best_k: int = 40,
@@ -518,34 +523,17 @@ class CemFleet:
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
         self.outer_its = int(cem_outer_it)
         self.first_iter_count = int(warmup_iterations) if warmup else self.outer_its   # as optimizer_cem_b200
-        self.noise_source = noise
         self._reset_period = None
-        lo, hi = (float(np.asarray(x, dtype=np.float32).reshape(-1)[0]) for x in control_limits)
         self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost, device=device)
         self.device = self.engine.device
-        if cost_config is not None:
-            self.engine.set_cost_config(cost_config)
-        self.engine.set_mppi_params(lo=lo, hi=hi)
-        c = L.cps_cem_fleet_config(C.sizeof(L.cps_cem_fleet_config), self.E, n_sim,
-                                   L.FLEET_NOISE_PHILOX if noise == "philox" else L.FLEET_NOISE_SUPPLIED,
-                                   float(dt_simulation), int(seed), int(experiment_offset), self.outer_its,
-                                   self.first_iter_count, int(cem_best_k), float(cem_initial_action_stdev),
-                                   float(cem_stdev_min))
-        self.engine._chk(self.engine.lib.cps_cem_fleet_create(self.engine._h, C.byref(c)))
-
-    def close(self):
-        self.engine.close()
-
-    def set_plant_models(self, *args, **kwargs):
-        raise NotImplementedError("CemFleet has no plant-side models (control disturbance, measurement noise, latency)")
+        self._setup_engine(control_limits, cost_config)
+        self._create(L.cps_cem_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset, self.outer_its,
+                     self.first_iter_count, int(cem_best_k), float(cem_initial_action_stdev), float(cem_stdev_min))
 
     def reset(self, states, period: int = 0):
         """optimizer_reset of every experiment (mid-range mean, cem_initial_action_stdev, u_prev = 0, solve counter 0),
         the initial states [E, 6] and the period counter."""
-        s = np.ascontiguousarray(states, dtype=np.float32)
-        if s.shape != (self.E, 6):
-            raise ValueError(f"states must have shape ({self.E}, 6)")
-        self.engine.use_current_stream()
+        s = self._host_states(states)
         self.engine._chk(self.engine.lib.cps_cem_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP), int(period)))
         self._reset_period = int(period)
 
@@ -554,14 +542,6 @@ class CemFleet:
         cem_outer_it."""
         return self.first_iter_count if period == self._reset_period else self.outer_its
 
-    def states(self, with_u_prev: bool = False):
-        s = np.zeros((self.E, 6), dtype=np.float32)
-        u_prev = np.zeros(self.E, dtype=np.float32) if with_u_prev else None
-        self.engine.use_current_stream()
-        self.engine._chk(self.engine.lib.cps_cem_fleet_get_states(
-            self.engine._h, s.ctypes.data_as(L._FP), None if u_prev is None else u_prev.ctypes.data_as(L._FP)))
-        return (s, u_prev) if with_u_prev else s
-
     def distribution(self):
         """(mean, stdev), each [E, T]: every experiment's sampling distribution.  Synchronises."""
         mu, sd = np.zeros((self.E, self.T), dtype=np.float32), np.zeros((self.E, self.T), dtype=np.float32)
@@ -569,16 +549,6 @@ class CemFleet:
         self.engine._chk(self.engine.lib.cps_cem_fleet_get_distribution(self.engine._h, mu.ctypes.data_as(L._FP),
                                                                         sd.ctypes.data_as(L._FP)))
         return mu, sd
-
-    @property
-    def period(self) -> int:
-        return int(self.engine.lib.cps_cem_fleet_period(self.engine._h))
-
-    def nonfinite_costs(self) -> int:
-        """Non-finite plan costs met so far (a NaN state or target makes them so; they sort after every number and stay
-        in their experiment).  Synchronises."""
-        self.engine.use_current_stream()
-        return self.engine.nonfinite_costs()
 
     def draws(self, period: int) -> torch.Tensor:
         """The draws a 'philox' fleet uses in `period`: cuda tensor [iterations(period), E, T, K]."""
@@ -596,15 +566,10 @@ class CemFleet:
         T, K], for a 'supplied' fleet; record [n_periods, E, 16], J_out [n_periods, E, K] and Q_out [n_periods, E, T, K]
         (costs and plans of each period's last iteration) or None."""
         eng = self.engine
-        eng.use_current_stream()
         p0 = self.period
         n_it = sum(self.iterations(p0 + j) for j in range(n_periods))
-        _check_sizes(self.device, (target_position, "target_position", n_periods * self.E),
-                     (target_equilibrium, "target_equilibrium", n_periods * self.E),
-                     (draws, "draws", n_it * self.E * self.T * self.K),
-                     (record, "record", n_periods * self.E * L.FLEET_RECORD),
-                     (J_out, "J_out", n_periods * self.E * self.K),
-                     (Q_out, "Q_out", n_periods * self.E * self.T * self.K))
+        self._check_rows(n_periods, target_position, target_equilibrium, record, J_out,
+                         (draws, "draws", n_it * self.E * self.T * self.K), (Q_out, "Q_out", n_periods * self.E * self.T * self.K))
         eng._chk(eng.lib.cps_cem_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
                                             _ptr(draws), _ptr(record), _ptr(J_out), _ptr(Q_out)))
         return record

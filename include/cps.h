@@ -328,6 +328,8 @@ typedef struct cps_fleet_config {
     unsigned long long seed;
     long long experiment_offset;     /* global index of local experiment 0 (sharding over GPUs) */
 } cps_fleet_config;
+/* CPS_ERR_INVALID: n_experiments outside [1, 65535], sim_substeps < 1, dt_simulation <= 0, an unknown noise source, or dt
+ * (control) not sim_substeps x dt_simulation. */
 int cps_fleet_create(cps_handle *h, const cps_fleet_config *cfg);
 /* s_host [E][6]: initial states (angle_cos / angle_sin are taken as given).  Zeroes u_nom and the last control
  * (optimizer_reset + Q_ccrc = 0, CartPole/__init__.py:871) and sets the period counter. */
