@@ -107,6 +107,12 @@ class Engine:
     def _chk(self, rc):
         L.check(rc, self._h)
 
+    def _s_host_from(self, s_np):
+        """The host-form entry points' state argument: s_np's 6 entries as float32 in a buffer the handle reads."""
+        for i in range(6):
+            self._s_host[i] = s_np[i]
+        return self._s_host
+
     def use_current_stream(self):
         s = torch.cuda.current_stream(self.device).cuda_stream
         if s != self._stream:
@@ -168,9 +174,7 @@ class Engine:
         _check_dev(noise, "noise", self.device)
         if noise.numel() != self.n_noise * self.K:
             raise ValueError(f"noise has {noise.numel()} elements, expected {self.n_noise * self.K}")
-        for i in range(6):
-            self._s_host[i] = s_np[i]
-        self._chk(self.lib.cps_mppi_step_host(self._h, self._s_host, _ptr(noise), noise_layout, float(u_prev),
+        self._chk(self.lib.cps_mppi_step_host(self._h, self._s_host_from(s_np), _ptr(noise), noise_layout, float(u_prev),
                                               self._u_host))
         return self._u_host[0]
 
@@ -212,9 +216,7 @@ class Engine:
         self.use_current_stream()
         if delta_u_np.dtype != np.float32 or not delta_u_np.flags.c_contiguous or delta_u_np.size != self.K * self.T:
             raise ValueError(f"delta_u must be a C-contiguous float32 array of {self.K * self.T} elements")
-        for i in range(6):
-            self._s_host[i] = s_np[i]
-        self._chk(self.lib.cps_legacy_step_host(self._h, self._s_host, C.c_void_p(delta_u_np.ctypes.data), layout,
+        self._chk(self.lib.cps_legacy_step_host(self._h, self._s_host_from(s_np), C.c_void_p(delta_u_np.ctypes.data), layout,
                                                 self._u_host))
         return self._u_host[0]
 
@@ -224,9 +226,7 @@ class Engine:
         self.use_current_stream()
         if knots_np.dtype != np.float32 or not knots_np.flags.c_contiguous or knots_np.ndim != 2 or knots_np.shape[0] != self.K:
             raise ValueError(f"knots must be a C-contiguous float32 array [K = {self.K}, n_knots]")
-        for i in range(6):
-            self._s_host[i] = s_np[i]
-        self._chk(self.lib.cps_legacy_step_host_knots(self._h, self._s_host, C.c_void_p(knots_np.ctypes.data),
+        self._chk(self.lib.cps_legacy_step_host_knots(self._h, self._s_host_from(s_np), C.c_void_p(knots_np.ctypes.data),
                                                       int(knots_np.shape[1]), int(knot_step), self._u_host))
         return self._u_host[0]
 
@@ -305,11 +305,9 @@ class Engine:
         return self._u_dev
 
     # -- rollouts -------------------------------------------------------------------------------------
-    def rollout(self, s0, Q, q_layout=L.ROLLOUT_MAJOR, traj_layout=L.ROLLOUT_MAJOR, want_traj=True,
-                want_final=False, traj_out=None, final_out=None):
-        """cps_rollout on device tensors.  s0: [6] or [B,6]; Q: [B,T] (ROLLOUT_MAJOR) or [T,B] (TIME_MAJOR).
-        Returns (traj, final): traj is [B,T+1,6] (ROLLOUT_MAJOR) or [T+1,6,B] (TIME_MAJOR)."""
-        self.use_current_stream()
+    def _rollout_io(self, s0, Q, q_layout, traj_layout, want_traj, traj_out):
+        """(Q as 2-D, B, T, batched, traj_out) of a device rollout from s0 [6] (shared) or [B, 6]; traj_out allocated
+        when wanted and not given."""
         _check_dev(s0, "s0", self.device)
         _check_dev(Q, "Q", self.device)
         Q2 = Q.reshape(Q.shape[0], Q.shape[1])
@@ -323,6 +321,14 @@ class Engine:
         if want_traj and traj_out is None:
             shape = (B, T + 1, 6) if traj_layout == L.ROLLOUT_MAJOR else (T + 1, 6, B)
             traj_out = torch.empty(shape, device=self.device, dtype=torch.float32)
+        return Q2, B, T, batched, traj_out
+
+    def rollout(self, s0, Q, q_layout=L.ROLLOUT_MAJOR, traj_layout=L.ROLLOUT_MAJOR, want_traj=True,
+                want_final=False, traj_out=None, final_out=None):
+        """cps_rollout on device tensors.  s0: [6] or [B,6]; Q: [B,T] (ROLLOUT_MAJOR) or [T,B] (TIME_MAJOR).
+        Returns (traj, final): traj is [B,T+1,6] (ROLLOUT_MAJOR) or [T+1,6,B] (TIME_MAJOR)."""
+        self.use_current_stream()
+        Q2, B, T, batched, traj_out = self._rollout_io(s0, Q, q_layout, traj_layout, want_traj, traj_out)
         if want_final and final_out is None:
             final_out = torch.empty((B, 6), device=self.device, dtype=torch.float32)
         self._chk(self.lib.cps_rollout(self._h, _ptr(s0), batched, _ptr(Q2), q_layout, B, T, _ptr(traj_out),
@@ -382,16 +388,7 @@ class Engine:
                     want_h=False, traj_out=None):
         """cps_net_rollout on device tensors; h0 None = the stored hidden state, [Htot] shared, or [B, Htot]."""
         self.use_current_stream()
-        _check_dev(s0, "s0", self.device)
-        _check_dev(Q, "Q", self.device)
-        Q2 = Q.reshape(Q.shape[0], Q.shape[1])
-        B, T = (Q2.shape if q_layout == L.ROLLOUT_MAJOR else Q2.shape[::-1])
-        if s0.numel() == 6:
-            batched = 0
-        elif s0.shape[0] == B and s0.numel() == 6 * B:
-            batched = 1
-        else:
-            raise ValueError("Batch size of control input contradict batch size of initial state")
+        Q2, B, T, batched, traj_out = self._rollout_io(s0, Q, q_layout, traj_layout, want_traj, traj_out)
         h_b = 0
         if h0 is not None:
             _check_dev(h0, "h0", self.device)
@@ -401,9 +398,6 @@ class Engine:
                 h_b = 1
             else:
                 raise ValueError(f"h0 has {h0.numel()} elements, expected {self.net_htot} or {self.net_htot * B}")
-        if want_traj and traj_out is None:
-            shape = (B, T + 1, 6) if traj_layout == L.ROLLOUT_MAJOR else (T + 1, 6, B)
-            traj_out = torch.empty(shape, device=self.device, dtype=torch.float32)
         h_final = torch.empty((B, self.net_htot), device=self.device, dtype=torch.float32) if want_h else None
         self._chk(self.lib.cps_net_rollout(self._h, _ptr(s0), batched, _ptr(Q2), q_layout, B, T, _ptr(h0), h_b,
                                            _ptr(traj_out), traj_layout, _ptr(h_final)))
@@ -463,13 +457,17 @@ class Engine:
         return out
 
     # -- forward-only planners (random action, CEM) ----------------------------------------------------
-    def _q_dims(self, Q, layout):
+    def _q_dims(self, Q, layout, name=None):
+        """(K, T) of plans Q in `layout`; given a `name`, they must be the handle's K plans of T steps."""
         if Q.dim() < 2:
             raise ValueError("Q must be [K, T] (ROLLOUT_MAJOR) or [T, K] (TIME_MAJOR)")
         a, b = int(Q.shape[0]), int(Q.shape[1])
         if Q.numel() != a * b:
             raise ValueError("one control input only: trailing dimensions of Q must be 1")
-        return (b, a) if layout == L.TIME_MAJOR else (a, b)
+        dims = (b, a) if layout == L.TIME_MAJOR else (a, b)
+        if name is not None and dims != (self.K, self.T):
+            raise ValueError(f"{name} has shape {tuple(Q.shape)}, expected K = {self.K}, T = {self.T}")
+        return dims
 
     def plan_cost(self, s, Q, q_layout=L.ROLLOUT_MAJOR, u_prev=0.0, want_traj=False, traj_layout=L.ROLLOUT_MAJOR):
         """predict_and_cost of the forward-only optimizers (cps_plan_cost): J [K], and the trajectories if asked."""
@@ -491,8 +489,7 @@ class Engine:
         self.use_current_stream()
         _check_dev(s, "s", self.device)
         _check_dev(Q, "Q", self.device)
-        if self._q_dims(Q, q_layout) != (self.K, self.T):
-            raise ValueError(f"Q has shape {tuple(Q.shape)}, expected K = {self.K}, T = {self.T}")
+        self._q_dims(Q, q_layout, "Q")
         if best_out is not None:
             _check_dev(best_out, "best_out", self.device, torch.int32)
         self._chk(self.lib.cps_plan_random_action(self._h, _ptr(s), _ptr(Q), q_layout, float(u_prev), _ptr(self._u_dev),
@@ -502,11 +499,8 @@ class Engine:
     def plan_random_action_host(self, s_np, Q, q_layout=L.ROLLOUT_MAJOR, u_prev=0.0) -> float:
         self.use_current_stream()
         _check_dev(Q, "Q", self.device)
-        if self._q_dims(Q, q_layout) != (self.K, self.T):
-            raise ValueError(f"Q has shape {tuple(Q.shape)}, expected K = {self.K}, T = {self.T}")
-        for i in range(6):
-            self._s_host[i] = s_np[i]
-        self._chk(self.lib.cps_plan_random_action_host(self._h, self._s_host, _ptr(Q), q_layout, float(u_prev),
+        self._q_dims(Q, q_layout, "Q")
+        self._chk(self.lib.cps_plan_random_action_host(self._h, self._s_host_from(s_np), _ptr(Q), q_layout, float(u_prev),
                                                        self._u_host))
         return self._u_host[0]
 
@@ -522,8 +516,7 @@ class Engine:
         _check_dev(eps, "eps", self.device)
         if eps.dim() < 3 or eps.numel() != eps.shape[0] * self.K * self.T:
             raise ValueError(f"eps has shape {tuple(eps.shape)}, expected [iterations, K, T] or [iterations, T, K]")
-        if self._q_dims(eps[0], layout) != (self.K, self.T):
-            raise ValueError(f"eps has shape {tuple(eps.shape)}, expected K = {self.K}, T = {self.T}")
+        self._q_dims(eps[0], layout, "eps[0]")
         return int(eps.shape[0])
 
     def cem_step(self, s, eps, eps_layout=L.ROLLOUT_MAJOR, u_prev=0.0, Q_out=None, J_out=None):
@@ -538,9 +531,7 @@ class Engine:
     def cem_step_host(self, s_np, eps, eps_layout=L.ROLLOUT_MAJOR, u_prev=0.0) -> float:
         self.use_current_stream()
         n_it = self._cem_eps(eps, eps_layout)
-        for i in range(6):
-            self._s_host[i] = s_np[i]
-        self._chk(self.lib.cps_cem_step_host(self._h, self._s_host, _ptr(eps), eps_layout, n_it, float(u_prev),
+        self._chk(self.lib.cps_cem_step_host(self._h, self._s_host_from(s_np), _ptr(eps), eps_layout, n_it, float(u_prev),
                                              self._u_host))
         return self._u_host[0]
 
@@ -594,9 +585,7 @@ class Engine:
     def cem_gmm_step_host(self, s_np, eps, u01, layout=L.ROLLOUT_MAJOR, u_prev=0.0) -> float:
         self.use_current_stream()
         n_it = self._gmm_draws(eps, u01, layout)
-        for i in range(6):
-            self._s_host[i] = s_np[i]
-        self._chk(self.lib.cps_cem_gmm_step_host(self._h, self._s_host, _ptr(eps), _ptr(u01), layout, n_it, float(u_prev),
+        self._chk(self.lib.cps_cem_gmm_step_host(self._h, self._s_host_from(s_np), _ptr(eps), _ptr(u01), layout, n_it, float(u_prev),
                                                  self._u_host))
         return self._u_host[0]
 
@@ -628,8 +617,7 @@ class Engine:
         self.use_current_stream()
         _check_dev(s, "s", self.device)
         _check_dev(Q, "Q", self.device)
-        if self._q_dims(Q, q_layout) != (self.K, self.T):
-            raise ValueError(f"Q has shape {tuple(Q.shape)}, expected K = {self.K}, T = {self.T}")
+        self._q_dims(Q, q_layout, "Q")
         G = torch.empty_like(Q)
         J = torch.empty(self.K, device=self.device) if want_J else None
         self._chk(self.lib.cps_plan_cost_grad(self._h, _ptr(s), _ptr(Q), q_layout, float(u_prev), _ptr(J), _ptr(G)))

@@ -260,10 +260,8 @@ extern "C" int cps_cem_gmm_reset(cps_handle *h) {
 
 extern "C" int cps_cem_gmm_configure(cps_handle *h, int best_k, float initial_stdev, float stdev_min) {
     if (!h) return CPS_ERR_INVALID;
-    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
-        return fail(h, CPS_ERR_UNSUPPORTED, "cps_cem_gmm_configure: ODE predictors only");
-    if (h->cfg.cost_id == CPS_COST_NONE || h->cfg.cost_id == CPS_COST_LEGACY_MPPI)
-        return fail(h, CPS_ERR_NOT_CONFIGURED, "cps_cem_gmm_configure: the handle has no cost-function plugin");
+    const int rc = cps_plan_check(h, "cps_cem_gmm_configure");   // every solve runs cps_plan_cost
+    if (rc != CPS_OK) return rc;
     if (best_k < 2 || best_k > h->cfg.num_rollouts)   // the two cheapest elites seed the two clusters
         return fail(h, CPS_ERR_INVALID, "cps_cem_gmm_configure: cem_best_k must lie in [2, num_rollouts]");
     if (!(initial_stdev >= 0.0f) || !(stdev_min >= 0.0f)) return fail(h, CPS_ERR_INVALID, "cps_cem_gmm_configure: negative stdev");
@@ -327,15 +325,10 @@ extern "C" int cps_cem_gmm_step_host(cps_handle *h, const float *s_host, const f
     if (!h) return CPS_ERR_INVALID;
     if (!s_host || !u_out_host) return fail(h, CPS_ERR_INVALID, "cps_cem_gmm_step_host: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    float *u_dst = h->h_pin_dev ? h->h_pin_dev + 8 : h->d_u;
-    h->inline_s = s_host;   // the state travels in plan_kernel's parameter block
-    int rc = cps_cem_gmm_step(h, h->d_s, eps_dev, u01_dev, layout, n_iterations, u_prev, u_dst, nullptr, nullptr);
-    h->inline_s = nullptr;
-    if (rc != CPS_OK) return rc;
-    if (!h->h_pin_dev) CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    *u_out_host = h->h_pin[8];
-    return CPS_OK;
+    // the state travels in plan_kernel's parameter block
+    return solve_host(h, s_host, u_out_host, true, [&](const float *s_dev, float *u_dev) {
+        return cps_cem_gmm_step(h, s_dev, eps_dev, u01_dev, layout, n_iterations, u_prev, u_dev, nullptr, nullptr);
+    });
 }
 
 extern "C" int cps_cem_gmm_get_distribution(cps_handle *h, float *loc_host, float *scale_host, float *p1_host) {

@@ -49,8 +49,6 @@ struct GradArgs {
     OdeParams ode;
     CostParams cost;
     const float *s;
-    float s_inline[6];
-    int use_inline;
     const float *Q;
     long long qs_k, qs_t;
     int K, T;
@@ -117,7 +115,7 @@ __device__ __forceinline__ void grad_fwd(const GradArgs &a, const FleetGradExt &
     const CostParams &C = FLEET ? fx.costs[e] : a.cost;
     const int T = a.T, K = a.K;
     const bool want_ck = !FLEET || a.ck != nullptr;
-    State z = load_state(FLEET ? a.s + (long long)e * 8 : (a.use_inline ? a.s_inline : a.s));
+    State z = load_state(FLEET ? a.s + (long long)e * 8 : a.s);
     const OdeParams ode = pin_params(ODE_E ? odes[e] : a.ode, z.th);
     float c_cost = cosf(z.th);
     const float *q = a.Q + (long long)k * a.qs_k;
@@ -485,8 +483,6 @@ extern "C" int cps_plan_cost_grad(cps_handle *h, const float *s_dev, const float
     memset(&a, 0, sizeof(a));
     a.ode = h->ode; a.cost = h->cost;
     a.s = s_dev;
-    a.use_inline = h->inline_s ? 1 : 0;
-    for (int c = 0; c < 6; ++c) a.s_inline[c] = h->inline_s ? h->inline_s[c] : 0.0f;
     a.Q = Q_dev;
     if (q_layout == CPS_TIME_MAJOR) { a.qs_k = 1; a.qs_t = K; a.gs_k = 1; a.gs_t = K; }
     else { a.qs_k = T; a.qs_t = 1; a.gs_k = T; a.gs_t = 1; }

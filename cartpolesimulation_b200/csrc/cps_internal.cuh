@@ -4,6 +4,7 @@
 
 #include <cstdarg>
 #include <cstdio>
+#include <cstring>
 #include <string>
 
 #include "../../include/cps.h"
@@ -94,7 +95,7 @@ struct cps_handle {
     size_t n_lknots;  // bytes allocated at d_lknots
     float *h_pin;  // pinned: [0..6) s, [8] u
     float *h_pin_dev;        // device view of h_pin (mapped): the solve writes u straight into host memory
-    const float *inline_s;   // set by cps_mppi_step_host around its cps_mppi_step call
+    const float *inline_s;   // set by solve_host around the launch of a solve that reads its state inline
     int grid, block;
     size_t smem;
     int shard;
@@ -144,6 +145,8 @@ void cps_rpgd_fleet_free(cps_handle *h);
 void cps_cem_fleet_free(cps_handle *h);
 // cps_plan.cu
 void cps_plan_free(cps_handle *h);
+// the refusals every forward-only planner shares: neural predictor, no cost plugin, substep sin/cos or fast division
+int cps_plan_check(cps_handle *h, const char *who);
 // CEM fleets: the refusals of cps_cem_fleet_create that concern the planner (those of cps_cem_configure, K above the
 // single-block selection, shared memory of plan_fleet_kernel), and one outer iteration of E experiments: plan_fleet_kernel,
 // then cem_update_fleet_kernel when best_k x T > 2048 (h->launches counts them)
@@ -224,4 +227,38 @@ static inline int fail(cps_handle *h, int code, const char *fmt, ...) {
         cudaError_t e_ = (expr);                                                                   \
         if (e_ != cudaSuccess) return fail(h, CPS_ERR_CUDA, "%s: %s", #expr, cudaGetErrorString(e_)); \
     } while (0)
+
+// ---- host form of a solve (the *_host entry points) --------------------------------------------------------------------
+// The argument blocks of MppiArgs / PlanArgs carry the state of a host-form solve when h->inline_s is set.
+template <class Args>
+static inline void fill_inline_state(const cps_handle *h, Args &a) {
+    a.use_inline = h->inline_s ? 1 : 0;
+    for (int c = 0; c < 6; ++c) a.s_inline[c] = h->inline_s ? h->inline_s[c] : 0.0f;
+}
+
+// The u-return half: u_dev is h->d_u (copied back) or the mapped h_pin_dev + 8 (already in host memory); synchronises.
+static inline int return_u_host(cps_handle *h, const float *u_dev, float *u_out_host) {
+    if (u_dev == h->d_u) CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    *u_out_host = h->h_pin[8];
+    return CPS_OK;
+}
+
+// One host-form solve, after cudaSetDevice: the state goes in, launch(s_dev, u_dev) enqueues the solve, u comes back.
+// direct (the kernel reads the state from its parameter block): the state rides inline and, with mapped memory, u is
+// written straight into host memory -- one stream operation.  Otherwise the state is copied through h_pin to d_s and u back
+// from d_u.
+template <class Launch>
+static inline int solve_host(cps_handle *h, const float *s_host, float *u_out_host, bool direct, Launch launch) {
+    float *u_dev = direct && h->h_pin_dev ? h->h_pin_dev + 8 : h->d_u;
+    if (!direct) {
+        memcpy(h->h_pin, s_host, sizeof(float) * 6);
+        CUDA_TRY(h, cudaMemcpyAsync(h->d_s, h->h_pin, sizeof(float) * 6, cudaMemcpyHostToDevice, h->stream));
+    }
+    h->inline_s = direct ? s_host : nullptr;
+    const int rc = launch((const float *)h->d_s, u_dev);
+    h->inline_s = nullptr;
+    if (rc != CPS_OK) return rc;
+    return return_u_host(h, u_dev, u_out_host);
+}
 

@@ -167,15 +167,11 @@ extern "C" int cps_legacy_step_host(cps_handle *h, const float *s_host, const fl
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     const size_t n_du = sizeof(float) * (size_t)h->cfg.num_rollouts * h->cfg.horizon;
     if (!h->d_ldu) CUDA_TRY(h, cudaMalloc(&h->d_ldu, n_du));
-    memcpy(h->h_pin, s_host, sizeof(float) * 6);
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_s, h->h_pin, sizeof(float) * 6, cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_ldu, delta_u_host, n_du, cudaMemcpyHostToDevice, h->stream));
-    rc = cps_legacy_step(h, h->d_s, h->d_ldu, layout, h->d_u, nullptr, nullptr, CPS_ROLLOUT_MAJOR, nullptr);
-    if (rc != CPS_OK) return rc;
-    CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    *u_out_host = h->h_pin[8];
-    return CPS_OK;
+    // stream order: state, delta_u, the solve, u
+    return solve_host(h, s_host, u_out_host, false, [&](const float *s_dev, float *u_dev) {
+        CUDA_TRY(h, cudaMemcpyAsync(h->d_ldu, delta_u_host, n_du, cudaMemcpyHostToDevice, h->stream));
+        return cps_legacy_step(h, s_dev, h->d_ldu, layout, u_dev, nullptr, nullptr, CPS_ROLLOUT_MAJOR, nullptr);
+    });
 }
 
 // SAMPLING_TYPE "interpolated" (controller_mppi_cartpole.py:430-451) on the device: the reference draws the perturbation at
@@ -216,18 +212,14 @@ extern "C" int cps_legacy_step_host_knots(cps_handle *h, const float *s_host, co
         CUDA_TRY(h, cudaMalloc(&h->d_lknots, n_kn));
         h->n_lknots = n_kn;
     }
-    memcpy(h->h_pin, s_host, sizeof(float) * 6);
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_s, h->h_pin, sizeof(float) * 6, cudaMemcpyHostToDevice, h->stream));
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_lknots, knots_host, n_kn, cudaMemcpyHostToDevice, h->stream));
-    const long long n = (long long)K * T;
-    legacy_interp_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->d_lknots, h->d_ldu, K, T, n_knots, knot_step);
-    h->launches += 1;
-    rc = cps_legacy_step(h, h->d_s, h->d_ldu, CPS_ROLLOUT_MAJOR, h->d_u, nullptr, nullptr, CPS_ROLLOUT_MAJOR, nullptr);
-    if (rc != CPS_OK) return rc;
-    CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    *u_out_host = h->h_pin[8];
-    return CPS_OK;
+    // stream order: state, knots, interpolation, the solve, u
+    return solve_host(h, s_host, u_out_host, false, [&](const float *s_dev, float *u_dev) {
+        CUDA_TRY(h, cudaMemcpyAsync(h->d_lknots, knots_host, n_kn, cudaMemcpyHostToDevice, h->stream));
+        const long long n = (long long)K * T;
+        legacy_interp_kernel<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(h->d_lknots, h->d_ldu, K, T, n_knots, knot_step);
+        h->launches += 1;
+        return cps_legacy_step(h, s_dev, h->d_ldu, CPS_ROLLOUT_MAJOR, u_dev, nullptr, nullptr, CPS_ROLLOUT_MAJOR, nullptr);
+    });
 }
 
 extern "C" int cps_legacy_get_perturbations(cps_handle *h, float *delta_u_host) {
@@ -252,12 +244,7 @@ extern "C" int cps_legacy_advance(cps_handle *h, float *u_out_host) {
     legacy_advance_kernel<<<1, 128, sizeof(float) * (size_t)T, h->stream>>>(h->d_unom, h->d_uprev, h->d_u, T);
     h->launches += 1;
     CUDA_TRY(h, cudaGetLastError());
-    if (u_out_host) {
-        CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-        *u_out_host = h->h_pin[8];
-    }
-    return CPS_OK;
+    return u_out_host ? return_u_host(h, h->d_u, u_out_host) : CPS_OK;
 }
 
 extern "C" int cps_legacy_reset(cps_handle *h) {

@@ -546,8 +546,7 @@ extern "C" int cps_mppi_step(cps_handle *h, const float *s_dev, const float *noi
                                  traj_layout, u_run_out_dev);
     MppiArgs a;
     a.ode = h->ode; a.cost = h->cost; a.mp = h->mp;
-    a.use_inline = h->inline_s ? 1 : 0;
-    for (int c = 0; c < 6; ++c) a.s_inline[c] = h->inline_s ? h->inline_s[c] : 0.0f;
+    fill_inline_state(h, a);
     SolveIO &io = a.io;
     io.s = s_dev; io.noise = noise_dev;
     const long long K = h->cfg.num_rollouts;
@@ -594,27 +593,12 @@ extern "C" int cps_mppi_step_host(cps_handle *h, const float *s_host, const floa
     if (h->shard)   // a sharded solve ends with the merged partial record, not with a control: there is no u to return
         return fail(h, CPS_ERR_INVALID, "cps_mppi_step_host: the handle is in shard mode (cps_mppi_set_shard); use cps_mppi_step + cps_mppi_finalize");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (h->cfg.integrator != CPS_PREDICTOR_NEURAL && h->h_pin_dev) {
-        // ODE predictors: ONE operation on the stream.  The state rides in the kernel's parameter block and the block that
-        // finishes the update writes u straight into mapped pinned host memory; no copy in either direction.
-        h->inline_s = s_host;
-        int rc = cps_mppi_step(h, h->d_s, noise_dev, noise_layout, u_prev, h->d_unom, h->h_pin_dev + 8, nullptr, nullptr,
-                               CPS_ROLLOUT_MAJOR, nullptr);
-        h->inline_s = nullptr;
-        if (rc != CPS_OK) return rc;
-        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-        *u_out_host = h->h_pin[8];
-        return CPS_OK;
-    }
-    memcpy(h->h_pin, s_host, sizeof(float) * 6);
-    CUDA_TRY(h, cudaMemcpyAsync(h->d_s, h->h_pin, sizeof(float) * 6, cudaMemcpyHostToDevice, h->stream));
-    int rc = cps_mppi_step(h, h->d_s, noise_dev, noise_layout, u_prev, h->d_unom, h->d_u, nullptr, nullptr,
-                           CPS_ROLLOUT_MAJOR, nullptr);
-    if (rc != CPS_OK) return rc;
-    CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    *u_out_host = h->h_pin[8];
-    return CPS_OK;
+    // ODE predictors: ONE operation on the stream.  The state rides in the kernel's parameter block and the block that
+    // finishes the update writes u straight into mapped pinned host memory; no copy in either direction.
+    return solve_host(h, s_host, u_out_host, h->cfg.integrator != CPS_PREDICTOR_NEURAL, [&](const float *s_dev, float *u_dev) {
+        return cps_mppi_step(h, s_dev, noise_dev, noise_layout, u_prev, h->d_unom, u_dev, nullptr, nullptr, CPS_ROLLOUT_MAJOR,
+                             nullptr);
+    });
 }
 
 __global__ void fill_kernel(float *p, int n, float v) {

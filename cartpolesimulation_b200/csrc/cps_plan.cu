@@ -927,7 +927,7 @@ static int plan_state(cps_handle *h, PlanState **out) {
     return CPS_OK;
 }
 
-static int plan_check(cps_handle *h, const char *who) {
+int cps_plan_check(cps_handle *h, const char *who) {
     if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
         return fail(h, CPS_ERR_UNSUPPORTED, "%s: ODE predictors only (neural predictor: cps_plan_cost, or cps_net_rollout + cps_trajectory_cost)", who);
     if (h->cfg.cost_id == CPS_COST_NONE || h->cfg.cost_id == CPS_COST_LEGACY_MPPI)
@@ -941,8 +941,7 @@ static void plan_common(cps_handle *h, PlanArgs &a, const float *s_dev, float u_
     memset(&a, 0, sizeof(a));
     a.ode = h->ode; a.cost = h->cost;
     a.s = s_dev;
-    a.use_inline = h->inline_s ? 1 : 0;
-    for (int c = 0; c < 6; ++c) a.s_inline[c] = h->inline_s ? h->inline_s[c] : 0.0f;
+    fill_inline_state(h, a);
     a.lo = h->mppi_in[5]; a.hi = h->mppi_in[6];
     a.inv_T1 = 1.0f / (float)(T + 1);
     a.u_prev = u_prev;
@@ -966,7 +965,7 @@ extern "C" int cps_plan_cost(cps_handle *h, const float *s_dev, const float *Q_d
     if (K < 1 || T < 1) return fail(h, CPS_ERR_INVALID, "cps_plan_cost: K and T must be positive");
     if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
         return cps_net_plan_cost(h, s_dev, Q_dev, q_layout, K, T, u_prev, J_out_dev, traj_out_dev, traj_layout);
-    int rc = plan_check(h, "cps_plan_cost");
+    int rc = cps_plan_check(h, "cps_plan_cost");
     if (rc != CPS_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     PlanArgs a;
@@ -997,7 +996,7 @@ extern "C" int cps_plan_random_action(cps_handle *h, const float *s_dev, const f
                                       float *u_out_dev, float *J_out_dev, int *best_out_dev) {
     if (!h) return CPS_ERR_INVALID;
     if (!s_dev || !Q_dev || !u_out_dev) return fail(h, CPS_ERR_INVALID, "cps_plan_random_action: null pointer");
-    int rc = plan_check(h, "cps_plan_random_action");
+    int rc = cps_plan_check(h, "cps_plan_random_action");
     if (rc != CPS_OK) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     PlanState *P;
@@ -1029,15 +1028,9 @@ extern "C" int cps_plan_random_action_host(cps_handle *h, const float *s_host, c
     if (!s_host || !u_out_host) return fail(h, CPS_ERR_INVALID, "cps_plan_random_action_host: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     // one stream operation: state in the parameter block, control written into mapped pinned host memory
-    float *u_dst = h->h_pin_dev ? h->h_pin_dev + 8 : h->d_u;
-    h->inline_s = s_host;
-    int rc = cps_plan_random_action(h, h->d_s, Q_dev, q_layout, u_prev, u_dst, nullptr, nullptr);
-    h->inline_s = nullptr;
-    if (rc != CPS_OK) return rc;
-    if (!h->h_pin_dev) CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    *u_out_host = h->h_pin[8];
-    return CPS_OK;
+    return solve_host(h, s_host, u_out_host, true, [&](const float *s_dev, float *u_dev) {
+        return cps_plan_random_action(h, s_dev, Q_dev, q_layout, u_prev, u_dev, nullptr, nullptr);
+    });
 }
 
 // ---- CEM --------------------------------------------------------------------------------------------------------------
@@ -1061,7 +1054,7 @@ extern "C" int cps_cem_reset(cps_handle *h) {
 
 extern "C" int cps_cem_configure(cps_handle *h, int best_k, float initial_stdev, float stdev_min) {
     if (!h) return CPS_ERR_INVALID;
-    int rc = plan_check(h, "cps_cem_configure");
+    int rc = cps_plan_check(h, "cps_cem_configure");
     if (rc != CPS_OK) return rc;
     if (best_k < 1 || best_k > h->cfg.num_rollouts)
         return fail(h, CPS_ERR_INVALID, "cps_cem_configure: cem_best_k must lie in [1, num_rollouts]");
@@ -1154,15 +1147,9 @@ extern "C" int cps_cem_step_host(cps_handle *h, const float *s_host, const float
     if (!h) return CPS_ERR_INVALID;
     if (!s_host || !u_out_host) return fail(h, CPS_ERR_INVALID, "cps_cem_step_host: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    float *u_dst = h->h_pin_dev ? h->h_pin_dev + 8 : h->d_u;
-    h->inline_s = s_host;
-    int rc = cps_cem_step(h, h->d_s, eps_dev, eps_layout, n_iterations, u_prev, u_dst, nullptr, nullptr);
-    h->inline_s = nullptr;
-    if (rc != CPS_OK) return rc;
-    if (!h->h_pin_dev) CUDA_TRY(h, cudaMemcpyAsync(h->h_pin + 8, h->d_u, sizeof(float), cudaMemcpyDeviceToHost, h->stream));
-    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-    *u_out_host = h->h_pin[8];
-    return CPS_OK;
+    return solve_host(h, s_host, u_out_host, true, [&](const float *s_dev, float *u_dev) {
+        return cps_cem_step(h, s_dev, eps_dev, eps_layout, n_iterations, u_prev, u_dev, nullptr, nullptr);
+    });
 }
 
 extern "C" int cps_cem_get_distribution(cps_handle *h, float *mu_host, float *stdev_host) {
@@ -1224,7 +1211,7 @@ static size_t cem_fleet_smem(const cps_handle *h, PlanArgs &a, bool philox) {
 }
 
 int cps_cem_fleet_check(cps_handle *h, int best_k, float initial_stdev, float stdev_min, int philox, const char *who) {
-    if (plan_check(h, who) != CPS_OK) return CPS_ERR_UNSUPPORTED;   // the message plan_check left stands
+    if (cps_plan_check(h, who) != CPS_OK) return CPS_ERR_UNSUPPORTED;   // the message cps_plan_check left stands
     const int K = h->cfg.num_rollouts;
     if (K > CPS_CEM_MULTIBLOCK_MIN)
         return fail(h, CPS_ERR_UNSUPPORTED, "%s: at most %d plans (the multi-block selection is not built for fleets)", who,

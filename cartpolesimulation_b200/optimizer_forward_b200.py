@@ -22,122 +22,17 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from . import config as cfgmod
-from .core import Engine
-from .optimizer_mppi_b200 import CudaNormalGenerator, _extract_cost, _extract_net_spec, _extract_predictor
-from .predictors import read_variable
+from .optimizer_mppi_b200 import _template_optimizer
 
 
-class CudaGenerator(CudaNormalGenerator):
-    """normal / uniform draws on the device with the call shapes of tf.random.Generator."""
-
-    def uniform(self, shape, minval=0.0, maxval=1.0, dtype=torch.float32):
-        out = torch.empty(tuple(shape), device=self.device, dtype=dtype)
-        return out.uniform_(float(minval), float(maxval), generator=self.rng)
-
-
-class _forward_optimizer:
-    supported_computation_libraries = ("Numpy", "TF", "Pytorch")
-    PREDICTORS = ("ODE", "ODE_v0")   # predictor types configure accepts
-    NOISE_RING = 256   # solves per device RNG call when the optimizer draws its own numbers
-
-    def _ring_draw(self, shape, draw):
-        """One solve's draws (tensor of `shape`) out of a ring filled by a single generator call per NOISE_RING solves:
-        a device RNG launch costs ~8 us of host time, a good part of a solve at these sizes."""
-        ring = getattr(self, "_ring", None)
-        if ring is None or tuple(ring.shape[1:]) != tuple(shape) or self._ring_i >= ring.shape[0]:
-            n = max(1, min(self.NOISE_RING, (64 << 20) // (4 * int(np.prod(shape)))))
-            self._ring = draw((n,) + tuple(shape))
-            self._ring_i = 0
-        out = self._ring[self._ring_i]
-        self._ring_i += 1
-        return out
-
-    def __init__(self, predictor, cost_function, control_limits, computation_library=None, seed=None,
-                 mpc_horizon: int = 35, num_rollouts: int = 200, optimizer_logging: bool = False,
-                 calculate_optimal_trajectory: bool = False, device=None, **kwargs):
-        self.lib = computation_library
-        self.num_rollouts = int(num_rollouts)
-        self.mpc_horizon = int(mpc_horizon)
-        self.cost_function = cost_function
-        self.predictor = predictor
-        self.u = 0.0  # template_optimizer.__init__ (Optimizers/__init__.py:35)
-        self.num_states = None
-        self.num_control_inputs = None
-        lo, hi = control_limits
-        self.action_low = np.asarray(lo, dtype=np.float32).reshape(-1)
-        self.action_high = np.asarray(hi, dtype=np.float32).reshape(-1)
-        self.seed = seed
-        self.logging_values = {}
-        self.optimizer_logging = bool(optimizer_logging)
-        self._device_arg = device
-        self.engine = None
-        self.rng = None
-        self._own_rng = None
-        self._var = None
-
+class _forward_optimizer(_template_optimizer):
     def configure(self, num_states: int, num_control_inputs: int, default_configure: bool = True, dt: float = None,
                   predictor_specification: str = None, **kwargs):
-        if int(num_control_inputs) != 1 or int(num_states) != 6:
-            raise ValueError(f"{type(self).__name__} implements the CartPole path: 6 states, 1 control input")
-        self.num_states, self.num_control_inputs = int(num_states), int(num_control_inputs)
-        ptype, n = _extract_predictor(self.predictor, predictor_specification)
-        if ptype not in self.PREDICTORS:
-            raise NotImplementedError(f"{type(self).__name__} supports the {' / '.join(self.PREDICTORS)} predictors, not "
-                                      f"{ptype!r} (no CPU fallback)")
-        net_spec = _extract_net_spec(self.predictor) if ptype == "neural" else None
         if dt is None:
             dt = getattr(self.predictor, "dt", None) or 0.02
-        cost_name, cost_cfg = _extract_cost(self.cost_function)
-        self.dt = float(dt)
-        self.engine = Engine(num_rollouts=self.num_rollouts, horizon=self.mpc_horizon, dt=self.dt, substeps=n,
-                             integrator=ptype, cost=cost_name, device=self._device_arg)
-        self.device = self.engine.device
-        self.cost_name, self.predictor_type = cost_name, ptype
-        if net_spec is not None:
-            self.engine.net_load(net_spec)
-        self.engine.set_cost_params(cfgmod.cost_vector(cost_name, cost_cfg))
-        # only the control limits of this block are used by the planners
-        self.engine.set_mppi_params(lo=float(self.action_low[0]), hi=float(self.action_high[0]))
-        self._own_rng = CudaGenerator(self.seed, self.device)
-        self.rng = self._own_rng
-        self._var = None
-        self._configure_engine()
+        self._configure(num_states, num_control_inputs, dt, predictor_specification)
         if default_configure:
             self.optimizer_reset()
-
-    def _configure_engine(self):
-        pass
-
-    @property
-    def optimizer_name(self):
-        return self.__class__.__name__.replace("optimizer_", "").replace("_", "-").lower()
-
-    def _refresh_variable_parameters(self):
-        vp = getattr(self.cost_function, "variable_parameters", None)
-        if vp is None:
-            vp = getattr(getattr(self.cost_function, "cost_function", None), "variable_parameters", None)
-        var = (read_variable(vp, "target_position", 0.0), read_variable(vp, "target_equilibrium", 1.0),
-               read_variable(vp, "L", cfgmod.DEFAULT_PHYSICS["L"]),
-               read_variable(vp, "m_pole", cfgmod.DEFAULT_PHYSICS["m_pole"]))
-        if var != self._var:
-            self.engine.set_variable_parameters(*var)
-            self._var = var
-
-    def refresh_cost_parameters(self):
-        _, cfg = _extract_cost(self.cost_function)
-        self.engine.set_cost_params(cfgmod.cost_vector(self.cost_name, cfg))
-
-    def _state(self, s):
-        if self.engine is None:
-            raise RuntimeError(f"{type(self).__name__}.step called before configure")
-        s = np.asarray(s, dtype=np.float32).reshape(-1)
-        if s.shape[0] != 6:
-            raise ValueError(f"state must have 6 entries, got {s.shape[0]}")
-        if self.optimizer_logging:
-            self.logging_values = {"s_logged": s.copy()}
-        self._refresh_variable_parameters()
-        return s
 
     def _log_rollouts(self, s, Q_kt):
         """Q_logged / J_logged / rollout_trajectories_logged of the reference: a second evaluation of the final plans
@@ -158,7 +53,7 @@ class optimizer_random_action_b200(_forward_optimizer):
         K, T = self.num_rollouts, self.mpc_horizon
         lo, hi = float(self.action_low[0]), float(self.action_high[0])
         if self.rng is self._own_rng:
-            return self._ring_draw((T, K), lambda shp: self._own_rng.uniform(shp, lo, hi)), L.TIME_MAJOR
+            return self._ring_draw("uniform", (T, K), lo, hi), L.TIME_MAJOR
         Q = self.rng.uniform(shape=[K, T, 1], minval=lo, maxval=hi, dtype=torch.float32)  # reference call (:58-63)
         return torch.as_tensor(Q).to(device=self.device, dtype=torch.float32).reshape(K, T).contiguous(), L.ROLLOUT_MAJOR
 
@@ -166,7 +61,7 @@ class optimizer_random_action_b200(_forward_optimizer):
         s = self._state(s)
         Q, layout = self._draw()
         self._u_prev_logged = self.u
-        u = self.engine.plan_random_action_host(s, Q, layout, float(np.asarray(self.u).reshape(-1)[0]))
+        u = self.engine.plan_random_action_host(s, Q, layout, self._u_prev())
         self.u = np.array(u, dtype=np.float32)
         if self.optimizer_logging:
             self._log_rollouts(s, Q.t() if layout == L.TIME_MAJOR else Q)
@@ -224,7 +119,7 @@ class optimizer_cem_b200(_forward_optimizer):
         if self.rng is self._own_rng:
             if iterations != self.cem_outer_it:   # the warm-up solve
                 return self._own_rng.normal((iterations, T, K)), L.TIME_MAJOR
-            return self._ring_draw((iterations, T, K), self._own_rng.normal), L.TIME_MAJOR
+            return self._ring_draw("normal", (iterations, T, K)), L.TIME_MAJOR
         eps = [torch.as_tensor(self.rng.normal(shape=(K, T, 1), dtype=torch.float32)).reshape(K, T)
                for _ in range(iterations)]  # one reference-shaped call per outer iteration (:66-67)
         return torch.stack(eps).to(device=self.device, dtype=torch.float32).contiguous(), L.ROLLOUT_MAJOR
@@ -233,12 +128,12 @@ class optimizer_cem_b200(_forward_optimizer):
         s = self._state(s)
         iterations = self.warmup_iterations if self.warmup and self.count == 0 else self.cem_outer_it
         eps, layout = self._draw(iterations)
-        u_prev = float(np.asarray(self.u).reshape(-1)[0])
+        u_prev = self._u_prev()
         self._u_prev_logged = self.u
         if self.optimizer_logging:
             K, T = self.num_rollouts, self.mpc_horizon
             Q = torch.empty((T, K) if layout == L.TIME_MAJOR else (K, T), device=self.device)
-            u_dev = self.engine.cem_step(torch.from_numpy(s).to(self.device), eps, layout, u_prev, Q_out=Q)
+            u_dev = self.engine.cem_step(self._state_dev(s), eps, layout, u_prev, Q_out=Q)
             u = float(u_dev.cpu()[0])
         else:
             u = self.engine.cem_step_host(s, eps, layout, u_prev)
@@ -291,15 +186,8 @@ class optimizer_cem_gmm_b200(_forward_optimizer):
     def _draw(self):
         K, T, it = self.num_rollouts, self.mpc_horizon, self.cem_outer_it
         if self.rng is self._own_rng:
-            eps = self._ring_draw((it, 2, T, K), self._own_rng.normal)
-            ring = getattr(self, "_uring", None)
-            if ring is None or self._uring_i >= ring.shape[0]:
-                n = max(1, min(self.NOISE_RING, (64 << 20) // (4 * it * T * K)))
-                self._uring = self._own_rng.uniform((n, it, T, K))
-                self._uring_i = 0
-            u01 = self._uring[self._uring_i]
-            self._uring_i += 1
-            return eps, u01, L.TIME_MAJOR
+            # two rings, each with its own refill step; the normal one is drawn first
+            return self._ring_draw("normal", (it, 2, T, K)), self._ring_draw("uniform", (it, T, K)), L.TIME_MAJOR
         eps, u01 = [], []
         for _ in range(it):
             eps.append(torch.as_tensor(self.rng.normal(shape=(K, T, 1, 2), dtype=torch.float32)).reshape(K, T, 2))
@@ -310,12 +198,12 @@ class optimizer_cem_gmm_b200(_forward_optimizer):
     def step(self, s: np.ndarray, time=None):
         s = self._state(s)
         eps, u01, layout = self._draw()
-        u_prev = float(np.asarray(self.u).reshape(-1)[0])
+        u_prev = self._u_prev()
         self._u_prev_logged = self.u
         if self.optimizer_logging:
             K, T = self.num_rollouts, self.mpc_horizon
             Q = torch.empty((T, K) if layout == L.TIME_MAJOR else (K, T), device=self.device)
-            u_dev = self.engine.cem_gmm_step(torch.from_numpy(s).to(self.device), eps, u01, layout, u_prev, Q_out=Q)
+            u_dev = self.engine.cem_gmm_step(self._state_dev(s), eps, u01, layout, u_prev, Q_out=Q)
             u = float(u_dev.cpu()[0])
         else:
             u = self.engine.cem_gmm_step_host(s, eps, u01, layout, u_prev)
@@ -413,13 +301,8 @@ class optimizer_rpgd_b200(_forward_optimizer):
     def step(self, s: np.ndarray, time=None):
         s = self._state(s)
         K, T, keep = self.num_rollouts, self.mpc_horizon, self.opt_keep_k
-        if getattr(self, "_s_pin", None) is None:   # pinned staging: the state's copy is stream-ordered, no synchronisation
-            self._s_pin = torch.empty(6, dtype=torch.float32).pin_memory()
-            self._s_dev = torch.empty(6, dtype=torch.float32, device=self.device)
-        self._s_pin.copy_(torch.from_numpy(s))
-        self._s_dev.copy_(self._s_pin, non_blocking=True)
-        s_dev = self._s_dev
-        u_prev = float(np.asarray(self.u).reshape(-1)[0])
+        s_dev = self._state_dev(s)
+        u_prev = self._u_prev()
         for _ in range(self.first_iter_count if self.count == 0 else self.outer_its):   # grad_step (:166-180)
             self.engine.rpgd_grad_step(s_dev, self.Q_tf, u_prev, self.learning_rate, self.adam_beta_1, self.adam_beta_2,
                                        self.adam_epsilon, self.gradmax_clip)

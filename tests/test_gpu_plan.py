@@ -199,6 +199,11 @@ def test_planner_errors():
     no_cost = Engine(64, 10, integrator="ODE", cost=None, device=0)
     with pytest.raises(RuntimeError):
         no_cost.plan_cost(s, torch.zeros((64, 10), device="cuda"))
+    for flag in ("fast_div", "substep_sincos"):   # the planners' rotation substeps only: refused at configure, nothing launched
+        gmm = Engine(64, 10, integrator="ODE", cost="quadratic_boundary_grad_minimal", device=0, **{flag: True})
+        with pytest.raises(NotImplementedError):   # CPS_ERR_UNSUPPORTED
+            gmm.cem_gmm_configure(8, 0.5, 0.01)
+        assert gmm.launch_count() == 0
 
 
 # ---- the optimizer mirrors ---------------------------------------------------------------------------------------------
