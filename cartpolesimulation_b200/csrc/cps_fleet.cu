@@ -92,6 +92,23 @@ int fleet_draws_launch(cps_handle *h, const FleetDrawsArgs &a, int layers) {
     return CPS_OK;
 }
 
+// fleet_draws_kernel's layout and grid with uniforms in [lo, lo + span)
+__global__ void __launch_bounds__(256) fleet_uniforms_kernel(const FleetDrawsArgs a, float lo, float span) {
+    const unsigned bpe = (unsigned)(a.rows + 255) / 256;
+    const int e = (int)(blockIdx.x / bpe), r = (int)(blockIdx.x % bpe) * 256 + (int)threadIdx.x, l = (int)blockIdx.z;
+    if (r >= a.rows) return;
+    philox_uniforms(a.seed, (unsigned)r, a.tag + (unsigned)l * a.tag_step, a.period, a.e_offset + (unsigned)e, a.n,
+                    a.out + l * a.s_layer + e * a.s_exp + r * a.s_row, a.s_elem, lo, span);
+}
+
+int fleet_uniforms_launch(cps_handle *h, const FleetDrawsArgs &a, int layers, float lo, float span) {
+    fleet_uniforms_kernel<<<dim3((unsigned)(a.rows + 255) / 256 * (unsigned)a.E, 1, (unsigned)layers), 256, 0, h->stream>>>(
+        a, lo, span);
+    h->launches += 1;
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
+}
+
 // The controller's view after `pushed` ring pushes: delayed + interpolated state (latency_adder.py:67-71), measurement
 // noise (noise_adder.py:69-84, draws n[0..3] = angle, position, angleD, positionD; null: none) and the cos / sin refresh of
 // update_vertical_angle_offset with a zero offset (CartPole/__init__.py:348-358).  float64 like the reference's buffer.

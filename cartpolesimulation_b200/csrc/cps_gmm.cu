@@ -25,6 +25,7 @@
 #include <new>
 
 #include "cps_internal.cuh"
+#include "cps_plant.cuh"
 
 struct GmmState {
     int best_k;
@@ -65,8 +66,7 @@ __global__ void __launch_bounds__(256) gmm_sample_kernel(const __grid_constant__
         const int t = (int)(i / a.K), k = (int)(i - (long long)t * a.K);
         const int c = (a.u01[(long long)t * a.us_t + (long long)k * a.us_k] < p1) ? 0 : 1;
         const float e = a.eps[(long long)c * a.es_c + (long long)t * a.es_t + (long long)k * a.es_k];
-        // tfpd.Normal.sample: loc + scale * eps, separately rounded; then tf.clip_by_value (:60-61)
-        const float q = fminf(fmaxf(__fadd_rn(a.dist[c * a.T + t], __fmul_rn(a.dist[(2 + c) * a.T + t], e)), a.lo), a.hi);
+        const float q = gmm_plan_value(a.dist[c * a.T + t], a.dist[(2 + c) * a.T + t], e, a.lo, a.hi);
         a.Q[i] = q;
         if (a.Q_out) a.Q_out[(long long)k * a.qo_k + (long long)t * a.qo_t] = q;
     }
@@ -78,15 +78,19 @@ __device__ __forceinline__ float warp_sum_f(float v) {
     return v;
 }
 
-// One block of 256 threads.
-__global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__ GmmArgs a) {
+// One CEM-GMM selection and update by one block of 256 threads (gmm_update_kernel, gmm_update_fleet_kernel): J [K] the
+// costs, elite [2 K] scratch (elite indices ascending, then their cluster flags), dist loc[2][T], scale[2][T], p1 <- the
+// update, *u_out <- u after the last iteration.  The plans are read through q_elite(t, e, k) (step t of elite e, plan k)
+// and q_best(t, j, b) (step t of the j-th cheapest plan, plan b); rows(b0, b1) runs once the two cheapest are known.
+template <class Rows, class QElite, class QBest>
+__device__ __forceinline__ void gmm_update_block(const float *J, int K, int T, int bk, int last_iter, float sd_min, int *elite,
+                                                 float *dist, float *u_out, Rows rows, QElite q_elite, QBest q_best) {
     __shared__ unsigned s_hist[256];
     __shared__ unsigned s_prefix, s_remaining;
     __shared__ int s_scan[8], s_base_eq, s_base_el;
     __shared__ unsigned long long s_best[8];
     __shared__ int s_b0, s_b1, s_n1;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nt = blockDim.x, nwarps = nt >> 5;
-    const int K = a.K, T = a.T, bk = a.best_k;
 
     // ---- the best_k-th smallest key: 8-bit radix select, most significant digit first ---------------------------------
     if (tid == 0) { s_prefix = 0u; s_remaining = (unsigned)bk; }
@@ -96,7 +100,7 @@ __global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__
         __syncthreads();
         const unsigned prefix = s_prefix, mask = (shift == 24) ? 0u : ~((1u << (shift + 8)) - 1u);
         for (int i = tid; i < K; i += nt) {
-            const unsigned key = order_key(__ldcg(a.J + i));
+            const unsigned key = order_key(__ldcg(J + i));
             if ((key & mask) == prefix) atomicAdd(&s_hist[(key >> shift) & 255u], 1u);
         }
         __syncthreads();
@@ -117,7 +121,7 @@ __global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__
     __syncthreads();
     for (int base = 0; base < K; base += nt) {
         const int i = base + tid;
-        const unsigned key = (i < K) ? order_key(__ldcg(a.J + i)) : 0xFFFFFFFFu;
+        const unsigned key = (i < K) ? order_key(__ldcg(J + i)) : 0xFFFFFFFFu;
         const bool is_eq = i < K && key == kth;
         // rank of this plan among the equal keys seen so far
         unsigned bal = __ballot_sync(0xffffffffu, is_eq);
@@ -138,7 +142,7 @@ __global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__
         for (int w = 0; w < warp; ++w) el_base += s_scan[w];
         int el_total = 0;
         for (int w = 0; w < nwarps; ++w) el_total += s_scan[w];
-        if (take) a.elite[el_base + el_before] = i;
+        if (take) elite[el_base + el_before] = i;
         __syncthreads();
         if (tid == 0) { s_base_eq += eq_total; s_base_el += el_total; }
         __syncthreads();
@@ -148,9 +152,9 @@ __global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__
     for (int pass = 0; pass < 2; ++pass) {
         unsigned long long best = ~0ull;
         for (int e = tid; e < bk; e += nt) {
-            const int k = a.elite[e];
+            const int k = elite[e];
             if (pass == 1 && k == s_b0) continue;
-            const unsigned long long c = ((unsigned long long)order_key(__ldcg(a.J + k)) << 32) | (unsigned)k;
+            const unsigned long long c = ((unsigned long long)order_key(__ldcg(J + k)) << 32) | (unsigned)k;
             best = c < best ? c : best;
         }
 #pragma unroll
@@ -167,22 +171,23 @@ __global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__
         __syncthreads();
     }
     const int b0 = s_b0, b1 = s_b1;
+    rows(b0, b1);
 
     // ---- cluster of every elite: nearer of the two in the Euclidean norm over the horizon (:72-77), one warp per elite ----
-    int *flag = a.elite + bk;   // 0: first cluster, 1: second
+    int *flag = elite + bk;   // 0: first cluster, 1: second
     if (tid == 0) s_n1 = 0;
     __syncthreads();
     int n1_local = 0;
     for (int e = warp; e < bk; e += nwarps) {
-        const int k = a.elite[e];
+        const int k = elite[e];
         int f;
         if (k == b0) f = 0;
         else if (k == b1) f = 1;
         else {
             float d0 = 0.0f, d1 = 0.0f;
             for (int t = lane; t < T; t += 32) {
-                const float q = a.Q[(long long)t * K + k];
-                const float x0 = q - a.Q[(long long)t * K + b0], x1 = q - a.Q[(long long)t * K + b1];
+                const float q = q_elite(t, e, k);
+                const float x0 = q - q_best(t, 0, b0), x1 = q - q_best(t, 1, b1);
                 d0 = fmaf(x0, x0, d0);
                 d1 = fmaf(x1, x1, d1);
             }
@@ -200,13 +205,13 @@ __global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__
     for (int t = warp; t < T; t += nwarps) {
         float s0 = 0.0f, s1 = 0.0f;
         for (int e = lane; e < bk; e += 32) {
-            const float q = a.Q[(long long)t * K + a.elite[e]];
+            const float q = q_elite(t, e, elite[e]);
             if (flag[e] == 0) s0 += q; else s1 += q;
         }
         const float m0 = __fdiv_rn(warp_sum_f(s0), (float)n1), m1 = __fdiv_rn(warp_sum_f(s1), (float)n2);
         float v0 = 0.0f, v1 = 0.0f;
         for (int e = lane; e < bk; e += 32) {
-            const float q = a.Q[(long long)t * K + a.elite[e]];
+            const float q = q_elite(t, e, elite[e]);
             if (flag[e] == 0) { const float d = q - m0; v0 = fmaf(d, d, v0); }
             else { const float d = q - m1; v1 = fmaf(d, d, v1); }
         }
@@ -214,23 +219,81 @@ __global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__
         v1 = sqrtf(__fdiv_rn(warp_sum_f(v1), (float)n2));
         if (lane == 0) {
             // written one step earlier after the last iteration: the shift of :111-118
-            const int dst = a.last_iter ? t - 1 : t;
-            const float sd0 = fminf(fmaxf(v0, a.sd_min), 1.0e4f), sd1 = fminf(fmaxf(v1, a.sd_min), 1.0e4f);
+            const int dst = last_iter ? t - 1 : t;
+            const float sd0 = fminf(fmaxf(v0, sd_min), 1.0e4f), sd1 = fminf(fmaxf(v1, sd_min), 1.0e4f);
             if (dst >= 0) {
-                a.dist[dst] = m0; a.dist[T + dst] = m1; a.dist[2 * T + dst] = sd0; a.dist[3 * T + dst] = sd1;
+                dist[dst] = m0; dist[T + dst] = m1; dist[2 * T + dst] = sd0; dist[3 * T + dst] = sd1;
             }
-            if (a.last_iter && t == T - 1) {   // the last entry is repeated
-                a.dist[t] = m0; a.dist[T + t] = m1; a.dist[2 * T + t] = sd0; a.dist[3 * T + t] = sd1;
+            if (last_iter && t == T - 1) {   // the last entry is repeated
+                dist[t] = m0; dist[T + t] = m1; dist[2 * T + t] = sd0; dist[3 * T + t] = sd1;
             }
         }
     }
     if (tid == 0) {
-        a.dist[4 * T] = __fdiv_rn((float)n1, (float)bk);   // prob_Q_1 (:79-80)
-        if (a.last_iter) *a.u_out = a.Q[b0];               // elite_Q[0, 0, :] (:108): step 0 of the cheapest plan
+        dist[4 * T] = __fdiv_rn((float)n1, (float)bk);   // prob_Q_1 (:79-80)
+        if (last_iter) *u_out = q_best(0, 0, b0);        // elite_Q[0, 0, :] (:108): step 0 of the cheapest plan
     }
 }
 
+// One block of 256 threads: the sampled plans are a.Q [T][K].
+__global__ void __launch_bounds__(256) gmm_update_kernel(const __grid_constant__ GmmArgs a) {
+    auto q = [&a](int t, int, int k) { return a.Q[(long long)t * a.K + k]; };
+    gmm_update_block(a.J, a.K, a.T, a.best_k, a.last_iter, a.sd_min, a.elite, a.dist, a.u_out, [](int, int) {}, q, q);
+}
+
+// CEM-GMM fleets: block x runs gmm_update_block on experiment x.  The elites' plans are rebuilt into a.rows [best_k][T]
+// from the mixture they were sampled from and their draws (supplied, or regenerated from Philox as the rollouts drew them).
+template <bool PHILOX>
+__global__ void __launch_bounds__(256) gmm_update_fleet_kernel(const __grid_constant__ GmmFleetUpdate a) {
+    __shared__ int s_pos[2];   // positions of the two cheapest plans in the elite list
+    const long long x = blockIdx.x;
+    const int K = a.K, T = a.T, bk = a.best_k, G4 = (T + 3) / 4;
+    const float *d = a.dist + x * (4 * T + 1);
+    float *W = a.rows + x * bk * T;
+    int *elite = a.elite + x * 2 * K;
+    auto rows = [&](int b0, int b1) {
+        const float p1 = d[4 * T];
+        for (int i = threadIdx.x; i < bk * G4; i += blockDim.x) {
+            const int pos = i / G4, g = i - pos * G4, k = elite[pos], n = min(4, T - 4 * g);
+            float e0[4], e1[4], u[4];
+            if (PHILOX) {
+                const unsigned eg = a.e_offset + (unsigned)x;
+                philox_normals(a.seed, (unsigned)k, a.w1 + (unsigned)g, a.period, eg, n, e0, 1);
+                philox_normals(a.seed, (unsigned)k, a.w1 + (unsigned)(G4 + g), a.period, eg, n, e1, 1);
+                philox_uniforms(a.seed, (unsigned)k, a.w1 + (unsigned)(2 * G4 + g), a.period, eg, n, u, 1, 0.0f, 1.0f);
+            } else {
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    const long long t = min(4 * g + q, T - 1);
+                    e0[q] = a.eps[(x * 2 * T + t) * K + k];
+                    e1[q] = a.eps[(x * 2 * T + T + t) * K + k];
+                    u[q] = a.u01[(x * T + t) * K + k];
+                }
+            }
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                const int t = 4 * g + q, c = (u[q] < p1) ? 0 : 1;
+                if (q < n) W[pos * T + t] = gmm_plan_value(d[c * T + t], d[(2 + c) * T + t], c ? e1[q] : e0[q], a.lo, a.hi);
+            }
+            if (g == 0 && k == b0) s_pos[0] = pos;
+            if (g == 0 && k == b1) s_pos[1] = pos;
+        }
+        __syncthreads();
+    };
+    gmm_update_block(a.J + x * K, K, T, bk, a.last_iter, a.sd_min, elite, a.dist_out + x * (4 * T + 1), a.u + x, rows,
+                     [&](int t, int e, int) { return W[e * T + t]; },
+                     [&](int t, int j, int) { return W[s_pos[j] * T + t]; });
+}
+
 }  // namespace
+
+int cps_gmm_fleet_update(cps_handle *h, const GmmFleetUpdate &a) {
+    if (a.eps) gmm_update_fleet_kernel<false><<<a.E, 256, 0, h->stream>>>(a);
+    else gmm_update_fleet_kernel<true><<<a.E, 256, 0, h->stream>>>(a);
+    h->launches += 1;
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
+}
 
 void cps_gmm_free(cps_handle *h) {
     GmmState *G = h->gmm;

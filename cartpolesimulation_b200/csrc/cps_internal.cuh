@@ -68,7 +68,8 @@ struct NetState;    // cps_net.cu
 struct FleetState;  // cps_fleet.cu
 struct RpgdFleetState;  // cps_rpgd_fleet.cu
 struct CemFleetState;   // cps_cem_fleet.cu
-struct PlanState;   // cps_plan.cu
+struct ForwardFleetState;   // cps_forward_fleets.cu
+struct PlanState;  // cps_plan.cu
 struct GmmState;    // cps_gmm.cu
 struct GradState;   // cps_grad.cu
 
@@ -120,6 +121,8 @@ struct cps_handle {
     GradState *grad;    // adjoint workspace and Adam moments (cps_plan_cost_grad, cps_rpgd_*), owned
     RpgdFleetState *rfleet;  // closed-loop experiments under RPGD (cps_rpgd_fleet_create), owned
     CemFleetState *cfleet;   // closed-loop experiments under CEM (cps_cem_fleet_create), owned
+    ForwardFleetState *gfleet;   // ... under CEM-GMM (cps_cem_gmm_fleet_create), owned
+    ForwardFleetState *rafleet;  // ... under random action (cps_random_action_fleet_create), owned
 };
 
 extern thread_local std::string g_create_err;
@@ -143,6 +146,8 @@ void cps_fleet_free(cps_handle *h);
 void cps_rpgd_fleet_free(cps_handle *h);
 // cps_cem_fleet.cu
 void cps_cem_fleet_free(cps_handle *h);
+// cps_forward_fleets.cu
+void cps_forward_fleets_free(cps_handle *h);
 // cps_plan.cu
 void cps_plan_free(cps_handle *h);
 // the refusals every forward-only planner shares: neural predictor, no cost plugin, substep sin/cos or fast division
@@ -169,8 +174,46 @@ struct CemFleetIteration {
 };
 int cps_cem_fleet_check(cps_handle *h, int best_k, float initial_stdev, float stdev_min, int philox, const char *who);
 int cps_cem_fleet_iteration(cps_handle *h, const CemFleetIteration &c);
+// CEM-GMM and random-action fleets (cps_forward_fleets.cu): the refusals of their creates that concern the planner (gmm:
+// those of cps_cem_gmm_configure; both: K above the single-block selection, shared memory of the rollout kernel), and the
+// rollouts of one iteration of E experiments, one launch of plan_forward_fleet_kernel, grid (ceil(K / 256), E).  gmm: the
+// plans Q = clip(loc[c][t] + scale[c][t] eps_c) from each experiment's mixture, costs into J, no selection; random action:
+// the plans as given (or lo + (hi - lo) u from Philox), costs, and in the last block of each experiment u = Q[argmin J, 0].
+struct ForwardFleetRollouts {
+    int gmm, E;
+    const float *s;              // [E][8] states
+    float *u;                    // [E] u_prev of the costs; random action: <- u
+    const float *tp, *te;        // [E] targets of this period (null: 0 / +1)
+    CostParams cost_up, cost_dn; // folded for target_equilibrium = +1 / -1
+    const float *dist;           // gmm: [E][4T + 1] loc[2][T], scale[2][T], p1 the plans are drawn from
+    const float *Q;              // supplied: random action plans [E][T][K]; gmm normals [E][2][T][K]; null: Philox
+    const float *u01;            // gmm, supplied: uniforms [E][T][K]
+    unsigned long long seed;     // Philox: counter (plan, w1 + draw word, period, e_offset + e), cps_plant.cuh
+    unsigned w1, period, e_offset;
+    float *J;                    // [E][K] <- the costs
+    float *Q_out;                // [E][T][K] <- the plans, or null
+    unsigned *tickets;           // [E], zero between launches (random action)
+};
+int cps_forward_fleet_check(cps_handle *h, int gmm, int best_k, float initial_stdev, float stdev_min, const char *who);
+int cps_forward_fleet_rollouts(cps_handle *h, const ForwardFleetRollouts &c);
 // cps_gmm.cu
 void cps_gmm_free(cps_handle *h);
+// CEM-GMM fleets: the selection and update of one iteration for E experiments, gmm_update_fleet_kernel, grid E, per
+// experiment the arithmetic of gmm_update_kernel in the same order
+struct GmmFleetUpdate {
+    int E, K, T, best_k, last_iter;
+    float lo, hi, sd_min;
+    const float *J;              // [E][K] the costs
+    const float *dist;           // [E][4T + 1] the mixture the plans were drawn from
+    float *dist_out;             // [E][4T + 1] <- the update (shifted after the last iteration)
+    const float *eps, *u01;      // supplied draws of this iteration [E][2][T][K], [E][T][K], or null: Philox
+    unsigned long long seed;
+    unsigned w1, period, e_offset;
+    int *elite;                  // [E][2K] scratch: elite indices, cluster flags
+    float *rows;                 // [E][best_k][T] scratch: the elites' plans
+    float *u;                    // [E] <- u = elite_Q[0, 0] after the last iteration
+};
+int cps_gmm_fleet_update(cps_handle *h, const GmmFleetUpdate &a);
 // cps_grad.cu
 #define CPS_GRAD_REC 20   /* floats per (control step, plan) record: M[3][4], r[4], cost partials (3), control term */
 void cps_grad_free(cps_handle *h);

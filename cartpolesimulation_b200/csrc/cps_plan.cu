@@ -24,7 +24,7 @@
 #include "cps_internal.cuh"
 #include "cps_plant.cuh"
 
-enum { PLAN_Q = 0, PLAN_CEM = 1 };
+enum { PLAN_Q = 0, PLAN_CEM = 1, PLAN_GMM = 2 };
 enum { SELECT_NONE = 0, SELECT_ARGMIN = 1, SELECT_CEM = 2 };
 
 struct PlanArgs {
@@ -70,6 +70,7 @@ struct PlanFleetExt {
     CostParams cost_up, cost_dn;  // folded for target_equilibrium = +1 / -1
     unsigned long long seed;      // Philox draws: counter (plan, w1 + group, period, e_offset + e)
     unsigned w1, period, e_offset;
+    const float *u01;             // CEM-GMM fleets, supplied draws: the component-picking uniforms [E][T][K]
 };
 
 struct PlanState {
@@ -652,11 +653,46 @@ __global__ void __launch_bounds__(256) cem_update_fleet_kernel(const __grid_cons
     }
 }
 
+// ---- random-action fleets: the argmin of experiment x = blockIdx.y -----------------------------------------------------
+// Run by the last block of experiment x: plan_select on the experiment's K costs from a copy of the arguments pointed at
+// the experiment, u = Q[argmin J, 0].  Supplied plans: plan_select reads Q[best, 0] of the experiment's [T][K] plans.
+// PHILOX: there is no plan buffer, so plan_select's read is pointed at s_u and thread 0 regenerates the cheapest plan's
+// first input as the rollout thread drew it.
+template <bool PHILOX>
+__device__ __forceinline__ void ra_fleet_select(const PlanArgs &a, const PlanFleetExt &fx) {
+    __shared__ PlanArgs s_a;
+    __shared__ int s_best;
+    __shared__ float s_u;
+    const long long x = blockIdx.y;
+    if (threadIdx.x == 0) {
+        s_a = a;
+        s_a.J = a.J + x * a.K;
+        s_a.best_out = &s_best;
+        s_a.u_out = &s_u;
+        s_a.Q = PHILOX ? &s_u : a.Q + x * a.T * a.K;
+        s_a.qs_k = PHILOX ? 0 : 1;
+    }
+    __syncthreads();
+    plan_select<PLAN_Q>(s_a, nullptr, nullptr, nullptr, nullptr, nullptr);
+    if (threadIdx.x == 0) {   // thread 0 wrote s_best and s_u
+        float u = s_u;
+        if (PHILOX)
+            philox_uniforms(fx.seed, (unsigned)s_best, fx.w1, fx.period, fx.e_offset + (unsigned)x, 1, &u, 1, a.lo,
+                            __fsub_rn(a.hi, a.lo));
+        a.u_out[x] = u;
+    }
+}
+
 // NSUB = 10: the substeps of the predictors' operating point unrolled (control_step); 0: a.ode.n substeps in a loop.
 // FLEET (PLAN_CEM, plan_fleet_kernel): block (b, e) evaluates plans b * 256.. of experiment e from its state, distribution,
 // u_prev and cost parameters `cost`; the last block of the experiment (its own ticket) selects on its K costs.  PHILOX:
 // the draws come from Philox in the rollout thread, four per call as the horizon advances.  FLEET = false compiles to
 // the code plan_kernel compiled to before the fleet existed.
+// FLEET with PLAN_Q (random-action fleets, plan_forward_fleet_kernel): the plans [E][T][K] as given, or with PHILOX
+// lo + (hi - lo) u from uniforms; the last block of the experiment takes the argmin (ra_fleet_select).  FLEET with
+// PLAN_GMM (CEM-GMM fleets): the experiment's mixture loc[2][T], scale[2][T], p1 goes to shared memory and every plan entry
+// is gmm_plan_value of the component its uniform picks, from normals [E][2][T][K] and uniforms fx->u01 [E][T][K] or from
+// Philox (three calls per four steps: both components' normals and the uniforms); no selection here.
 template <int INTEG, int COST, int MODE, int NSUB, bool FLEET, bool PHILOX>
 __device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt *fx, const CostParams &cost) {
     extern __shared__ float smem[];   // PLAN_CEM: mu[T], sd[T], mu2[T], sd2[T], elite list [elite_smem], PHILOX: elites' draws
@@ -666,6 +702,10 @@ __device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt 
     float *s_mu = smem, *s_sd = smem + T;
     if (MODE == PLAN_CEM) {
         for (int t = tid; t < T; t += blockDim.x) { s_mu[t] = a.mu[x * T + t]; s_sd[t] = a.sd[x * T + t]; }
+        __syncthreads();
+    }
+    if (MODE == PLAN_GMM) {   // a.mu: the mixtures [E][4T + 1]
+        for (int i = tid; i < 4 * T + 1; i += blockDim.x) smem[i] = a.mu[x * (4 * T + 1) + i];
         __syncthreads();
     }
     const int k = blockIdx.x * blockDim.x + tid;
@@ -681,7 +721,7 @@ __device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt 
     float *qo = (MODE == PLAN_CEM && a.Q_out) ? (FLEET ? a.Q_out + qoff : a.Q_out + (long long)kc * a.qs_k) : nullptr;
     float *traj = (!FLEET && a.traj_out) ? a.traj_out + (long long)kc * a.ts_k : nullptr;   // fleets write no trajectories
     float Jacc = 0.0f, up = FLEET ? a.u_out[x] : a.u_prev;
-    float nr[4];   // PHILOX: the draws of the current group of four steps, consumed from nr[0]
+    float nr[4];   // PHILOX: the draws (PLAN_GMM: the plan entries) of the current group of four steps, consumed from nr[0]
     // default / quadratic_boundary: the T+1 entries are summed in the reference backend's order (cps_device.cuh RowSumPlan)
     constexpr bool ROWSUM = (COST == COST_DEFAULT || COST == COST_QB);
     const RowSumPlan rsp = row_sum_plan(T + 1);
@@ -689,14 +729,40 @@ __device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt 
     const int ss = blockDim.x;
     float rs_tail = 0.0f;
     if (ROWSUM) row_sum_init(rsp, sl, ss);
-    float qn = PHILOX ? 0.0f : q[0];
+    float qn = (PHILOX || MODE == PLAN_GMM) ? 0.0f : q[0];
 #pragma unroll 1
     for (int t = 0; t < T; ++t) {
         float u = qn;
-        if (PHILOX) {
-            if ((t & 3) == 0)
-                philox_normals(fx->seed, (unsigned)kc, fx->w1 + (unsigned)(t >> 2), fx->period, fx->e_offset + (unsigned)x, 4,
-                               nr, 1);
+        if (MODE == PLAN_GMM) {
+            if (PHILOX) {   // the group's four plan entries are formed at once, so only they stay in registers
+                if ((t & 3) == 0) {
+                    float n1[4], nu[4];
+                    const unsigned g = (unsigned)(t >> 2), G4 = (unsigned)((T + 3) >> 2), eg = fx->e_offset + (unsigned)x;
+                    philox_normals(fx->seed, (unsigned)kc, fx->w1 + g, fx->period, eg, 4, nr, 1);
+                    philox_normals(fx->seed, (unsigned)kc, fx->w1 + G4 + g, fx->period, eg, 4, n1, 1);
+                    philox_uniforms(fx->seed, (unsigned)kc, fx->w1 + 2 * G4 + g, fx->period, eg, 4, nu, 1, 0.0f, 1.0f);
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        const int tq = min(t + q, T - 1), c = (nu[q] < smem[4 * T]) ? 0 : 1;
+                        nr[q] = gmm_plan_value(smem[c * T + tq], smem[(2 + c) * T + tq], c ? n1[q] : nr[q], a.lo, a.hi);
+                    }
+                }
+                u = nr[0];
+                nr[0] = nr[1]; nr[1] = nr[2]; nr[2] = nr[3];
+            } else {
+                const long long o = (x * 2 * T + t) * a.K + kc;
+                const int c = (fx->u01[qoff + (long long)t * a.K] < smem[4 * T]) ? 0 : 1;
+                u = gmm_plan_value(smem[c * T + t], smem[(2 + c) * T + t], a.Q[o + c * (long long)T * a.K], a.lo, a.hi);
+            }
+        } else if (PHILOX) {
+            if ((t & 3) == 0) {
+                if (MODE == PLAN_Q)
+                    philox_uniforms(fx->seed, (unsigned)kc, fx->w1 + (unsigned)(t >> 2), fx->period,
+                                    fx->e_offset + (unsigned)x, 4, nr, 1, a.lo, __fsub_rn(a.hi, a.lo));
+                else
+                    philox_normals(fx->seed, (unsigned)kc, fx->w1 + (unsigned)(t >> 2), fx->period,
+                                   fx->e_offset + (unsigned)x, 4, nr, 1);
+            }
             u = nr[0];
             nr[0] = nr[1]; nr[1] = nr[2]; nr[2] = nr[3];
         } else if (t + 1 < T) {
@@ -706,6 +772,7 @@ __device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt 
             u = cem_plan_value(s_mu[t], u, s_sd[t], a.lo, a.hi);
             if (active && qo) (FLEET ? a.Q_out[qoff + (long long)t * a.K] : qo[(long long)t * a.qs_t]) = u;
         }
+        if (FLEET && MODE != PLAN_CEM && active && a.Q_out) a.Q_out[qoff + (long long)t * a.K] = u;
         if (COST != COST_NONE) {
             const float st = stage_cost<COST>(cost, c_cost, z.w, z.x, u, up);
             if (ROWSUM) row_sum_push(rsp, sl, ss, rs_tail, t, st - cost.max_cost);  // get_stage_cost shift
@@ -739,7 +806,9 @@ __device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt 
     __syncthreads();
     if (s_ticket != gridDim.x - 1u) return;
     __threadfence();
-    if (FLEET) {
+    if (FLEET && MODE == PLAN_Q) {
+        ra_fleet_select<PHILOX>(a, *fx);
+    } else if (FLEET) {
         int *s_elite = reinterpret_cast<int *>(smem + 4 * T);
         cem_fleet_select<PHILOX>(a, *fx, s_mu, s_sd, smem + 2 * T, smem + 3 * T, s_elite,
                                  reinterpret_cast<float *>(s_elite + a.elite_smem));
@@ -760,6 +829,15 @@ __global__ void __launch_bounds__(256, 4) plan_fleet_kernel(const __grid_constan
     if (threadIdx.x == 0) s_cost = fold_cost_e(fx.cost_up, fx.cost_dn, fx.tp, fx.te, (int)blockIdx.y);
     __syncthreads();
     plan_body<INTEG, COST, PLAN_CEM, NSUB, true, PHILOX>(a, &fx, s_cost);
+}
+// CEM-GMM (PLAN_GMM) and random-action (PLAN_Q) fleets: plan_fleet_kernel's grid and cost fold
+template <int INTEG, int COST, int MODE, int NSUB, bool PHILOX>
+__global__ void __launch_bounds__(256, 4) plan_forward_fleet_kernel(const __grid_constant__ PlanArgs a,
+                                                                    const __grid_constant__ PlanFleetExt fx) {
+    __shared__ CostParams s_cost;
+    if (threadIdx.x == 0) s_cost = fold_cost_e(fx.cost_up, fx.cost_dn, fx.tp, fx.te, (int)blockIdx.y);
+    __syncthreads();
+    plan_body<INTEG, COST, MODE, NSUB, true, PHILOX>(a, &fx, s_cost);
 }
 
 // Many plans, no selecting block, time-major plans: two plans per thread (k, k + 1) in packed FP32, as mppi_solve_block2
@@ -1256,6 +1334,78 @@ int cps_cem_fleet_iteration(cps_handle *h, const CemFleetIteration &c) {
         else cem_update_fleet_kernel<false><<<dim3((unsigned)T, (unsigned)c.E), 256, 0, h->stream>>>(a, fx);
         h->launches += 1;
     }
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
+}
+
+// ---- CEM-GMM and random-action fleets (cps_forward_fleets.cu) ----------------------------------------------------------
+template <int INTEG, int MODE, int NSUB, bool PHILOX>
+static plan_fleet_fn pick_forward_fleet3(int cost) {
+    switch (cost) {
+    case CPS_COST_DEFAULT: return plan_forward_fleet_kernel<INTEG, COST_DEFAULT, MODE, NSUB, PHILOX>;
+    case CPS_COST_QUADRATIC_BOUNDARY: return plan_forward_fleet_kernel<INTEG, COST_QB, MODE, NSUB, PHILOX>;
+    case CPS_COST_QB_GRAD_MINIMAL: return plan_forward_fleet_kernel<INTEG, COST_GRADMIN, MODE, NSUB, PHILOX>;
+    case CPS_COST_QB_GRAD: return plan_forward_fleet_kernel<INTEG, COST_GRAD, MODE, NSUB, PHILOX>;
+    default: return nullptr;
+    }
+}
+template <int INTEG, int MODE, int NSUB>
+static plan_fleet_fn pick_forward_fleet2(int cost, bool philox) {
+    return philox ? pick_forward_fleet3<INTEG, MODE, NSUB, true>(cost) : pick_forward_fleet3<INTEG, MODE, NSUB, false>(cost);
+}
+template <int INTEG, int MODE>
+static plan_fleet_fn pick_forward_fleet1(int cost, int n_sub, bool philox) {
+    return n_sub == 10 ? pick_forward_fleet2<INTEG, MODE, 10>(cost, philox) : pick_forward_fleet2<INTEG, MODE, 0>(cost, philox);
+}
+static plan_fleet_fn pick_forward_fleet(int integ, int cost, int mode, int n_sub, bool philox) {
+    if (integ == CPS_EULER_V0)
+        return mode == PLAN_GMM ? pick_forward_fleet1<0, PLAN_GMM>(cost, n_sub, philox) : pick_forward_fleet1<0, PLAN_Q>(cost, n_sub, philox);
+    return mode == PLAN_GMM ? pick_forward_fleet1<1, PLAN_GMM>(cost, n_sub, philox) : pick_forward_fleet1<1, PLAN_Q>(cost, n_sub, philox);
+}
+
+// Dynamic shared memory of plan_forward_fleet_kernel: the mixture (gmm), then the row-sum slots; sets a.rs_off.
+static size_t forward_fleet_smem(const cps_handle *h, PlanArgs &a, bool gmm) {
+    return plan_smem(h, a, gmm ? sizeof(float) * (4 * (size_t)a.T + 1) : 0, 256, 1);
+}
+
+int cps_forward_fleet_check(cps_handle *h, int gmm, int best_k, float initial_stdev, float stdev_min, const char *who) {
+    if (cps_plan_check(h, who) != CPS_OK) return CPS_ERR_UNSUPPORTED;   // the message cps_plan_check left stands
+    const int K = h->cfg.num_rollouts;
+    if (K > CPS_CEM_MULTIBLOCK_MIN)
+        return fail(h, CPS_ERR_UNSUPPORTED, "%s: at most %d plans (the multi-block selection is not built for fleets)", who,
+                    CPS_CEM_MULTIBLOCK_MIN);
+    if (gmm && (best_k < 2 || best_k > K)) return fail(h, CPS_ERR_INVALID, "%s: cem_best_k must lie in [2, num_rollouts]", who);
+    if (gmm && (!(initial_stdev >= 0.0f) || !(stdev_min >= 0.0f))) return fail(h, CPS_ERR_INVALID, "%s: negative stdev", who);
+    PlanArgs a;
+    memset(&a, 0, sizeof(a));
+    a.T = h->cfg.horizon;
+    if (forward_fleet_smem(h, a, gmm != 0) > 200 * 1024) return fail(h, CPS_ERR_UNSUPPORTED, "%s: horizon too large for shared memory", who);
+    return CPS_OK;
+}
+
+int cps_forward_fleet_rollouts(cps_handle *h, const ForwardFleetRollouts &c) {
+    const int K = h->cfg.num_rollouts, T = h->cfg.horizon;
+    const bool philox = c.Q == nullptr;
+    PlanArgs a;
+    plan_common(h, a, nullptr, 0.0f, K, T);
+    a.Q = c.Q; a.qs_k = 1; a.qs_t = K;
+    a.Q_out = c.Q_out;
+    a.J = c.J;
+    a.select = c.gmm ? SELECT_NONE : SELECT_ARGMIN;
+    a.ticket = c.tickets; a.u_out = c.u;
+    a.mu = c.dist;
+    const size_t smem = forward_fleet_smem(h, a, c.gmm != 0);
+    PlanFleetExt fx;
+    memset(&fx, 0, sizeof(fx));
+    fx.s = c.s; fx.tp = c.tp; fx.te = c.te;
+    fx.cost_up = c.cost_up; fx.cost_dn = c.cost_dn;
+    fx.seed = c.seed; fx.w1 = c.w1; fx.period = c.period; fx.e_offset = c.e_offset;
+    fx.u01 = c.u01;
+    plan_fleet_fn fn = pick_forward_fleet(h->cfg.integrator, h->cfg.cost_id, c.gmm ? PLAN_GMM : PLAN_Q, h->ode.n, philox);
+    if (!fn) return fail(h, CPS_ERR_UNSUPPORTED, "no kernel for this configuration");
+    if (smem > 48 * 1024) CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fn<<<dim3((unsigned)(K + 255) / 256, (unsigned)c.E), 256, smem, h->stream>>>(a, fx);
+    h->launches += 1;
     CUDA_TRY(h, cudaGetLastError());
     return CPS_OK;
 }

@@ -116,11 +116,17 @@ __device__ __forceinline__ void box_muller(unsigned a, unsigned b, float &n0, fl
 // streams: the MPPI rollout draws have w0 = rollout, w1 = 0 (second word = draw group < 2^28); the RPGD plan draws have
 // w0 = plan row, w1 = RPGD_DRAWS_RESAMPLE (the resampling solve of `period`) or RPGD_DRAWS_RESET (period 0, the plans of
 // a reset); the CEM draws of outer iteration `it` have w0 = plan, w1 = CEM_DRAWS + it * ceil(T / 4) (second word below
-// CEM_DRAWS + 2^28: cps_cem_fleet_create bounds the iterations); the plant-side draws of cps_fleet.cu have second word
-// 0xFFFFFFFF.  The second words keep them disjoint.
+// CEM_DRAWS + 2^28: cps_cem_fleet_create bounds the iterations); the CEM-GMM draws of outer iteration `it` have w0 = plan
+// and, with G4 = ceil(T / 4), second words GMM_DRAWS + 3 G4 it + {0, G4} + group for the two components' normals and
+// GMM_DRAWS + 3 G4 it + 2 G4 + group for the component-picking uniforms (below GMM_DRAWS + 2^28: cps_cem_gmm_fleet_create
+// bounds the iterations); the random-action plans have w0 = plan, w1 = RA_DRAWS + group (uniforms, philox_uniforms; below
+// RA_DRAWS + 2^28 since T is bounded by shared memory); the plant-side draws of cps_fleet.cu have second word 0xFFFFFFFF.
+// The second words keep them disjoint.
 #define RPGD_DRAWS_RESAMPLE 0xA0000000u
 #define RPGD_DRAWS_RESET 0xB0000000u
 #define CEM_DRAWS 0xC0000000u
+#define GMM_DRAWS 0xD0000000u
+#define RA_DRAWS 0xE0000000u
 __device__ __forceinline__ void philox_normals(unsigned long long seed, unsigned w0, unsigned w1, unsigned period,
                                                unsigned e_global, int n_ind, float *dst, long long stride) {
     const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
@@ -135,6 +141,29 @@ __device__ __forceinline__ void philox_normals(unsigned long long seed, unsigned
     }
 }
 
+// Uniforms i = 0..n_ind-1 in [lo, lo + span), dst[i * stride], four per counter (w0, w1 + i / 4, period, e_global): one
+// 24-bit uniform u = (word >> 8) 2^-24 in [0, 1) per Philox word, then lo + span * u with the multiply and the add rounded
+// separately (lo = 0, span = 1 gives u itself).
+__device__ __forceinline__ void philox_uniforms(unsigned long long seed, unsigned w0, unsigned w1, unsigned period,
+                                                unsigned e_global, int n_ind, float *dst, long long stride, float lo,
+                                                float span) {
+    const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
+    for (int g = 0; 4 * g < n_ind; ++g) {
+        const uint4 r = philox4x32_10(make_uint4(w0, w1 + (unsigned)g, period, e_global), key);
+        const unsigned w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+            if (4 * g + q < n_ind)
+                dst[(long long)(4 * g + q) * stride] = __fadd_rn(lo, __fmul_rn(span, (float)(w[q] >> 8) * 5.9604644775390625e-8f));
+    }
+}
+
+// A CEM-GMM plan entry: loc + scale * eps of the picked component, separately rounded, then clipped (tfpd.Normal.sample
+// and tf.clip_by_value, optimizer_cem_gmm_tf.py:60-61); gmm_sample_kernel and the GMM fleet's rollouts share it.
+__device__ __forceinline__ float gmm_plan_value(float loc, float scale, float eps, float lo, float hi) {
+    return fminf(fmaxf(__fadd_rn(loc, __fmul_rn(scale, eps)), lo), hi);
+}
+
 // What a Philox fleet draws in one period, materialised (cps_fleet_noise, cps_rpgd_fleet_draws, cps_cem_fleet_draws, and
 // the draw workspaces of the neural MPPI period and the RPGD reset): per layer l < `layers`, experiment e < E and row
 // r < rows, philox_normals(seed, r, tag + l * tag_step, period, e_offset + e, n) into out + l * s_layer + e * s_exp +
@@ -147,6 +176,8 @@ struct FleetDrawsArgs {
     float *out;
 };
 int fleet_draws_launch(cps_handle *h, const FleetDrawsArgs &a, int layers);
+// The same layout with philox_uniforms(..., lo, span) in place of the normals (the CEM-GMM and random-action fleets).
+int fleet_uniforms_launch(cps_handle *h, const FleetDrawsArgs &a, int layers, float lo, float span);
 
 // ---- the plant (device restatement of oracle/cps_oracle.c: ode_plant, plant_integrate; no FMA contraction) ------------
 __device__ __forceinline__ void plant_ode(const PlantParams &P, float ca, float sa, float angleD, float positionD, float u,

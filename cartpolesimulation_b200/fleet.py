@@ -573,3 +573,126 @@ class CemFleet(_FleetBase):
         eng._chk(eng.lib.cps_cem_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
                                             _ptr(draws), _ptr(record), _ptr(J_out), _ptr(Q_out)))
         return record
+
+
+class CemGmmFleet(_FleetBase):
+    """E closed-loop experiments under optimizer_cem_gmm_tf (`cem-gmm-tf` in Control_Toolkit_ASF/config_controllers.yml) on
+    one device: one cps_handle with a CEM-GMM fleet attached (include/cps.h "CEM-GMM and random-action fleets").
+
+    Every controller period does, for every experiment, what optimizer_cem_gmm_b200.step does (cem_outer_it iterations of
+    sampling from the experiment's own two-component mixture, costs, elites, the two clusters around the two cheapest
+    elites and their mean / stdev / weight; then u = elite_Q[0, 0] and the shift), then what Fleet's plant does, with no
+    host round trip.  The keywords are optimizer_cem_gmm_b200's (same defaults) and Fleet's.  Predictor "ODE" or "ODE_v0"
+    and the four cost plugins; num_rollouts at most 8192, cem_best_k at least 2.  The neural predictor and the plant-side
+    models (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+    _abi = "cps_cem_gmm_fleet"
+
+    def __init__(self, n_experiments: int, num_rollouts: int = 200, mpc_horizon: int = 35, cem_outer_it: int = 3,
+                 cem_initial_action_stdev: float = 0.5, cem_stdev_min: float = 0.01, cem_best_k: int = 40,
+                 control_limits=(-1.0, 1.0), dt: float = 0.02, substeps: int = 10, integrator: str = "ODE",
+                 cost: str = "quadratic_boundary_grad_minimal", cost_config: dict | None = None, device: int | None = None,
+                 noise: str = "philox", seed: int = 0, experiment_offset: int = 0, dt_simulation: float = 0.002):
+        if integrator == "neural":
+            raise NotImplementedError("CemGmmFleet runs on predictor 'ODE' or 'ODE_v0' (optimizer_cem_gmm_b200 has no "
+                                      "neural predictor either)")
+        n_sim = _check_fleet_args("CemGmmFleet", integrator, None, noise, dt, dt_simulation)
+        self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
+        self.outer_its = int(cem_outer_it)
+        self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost, device=device)
+        self.device = self.engine.device
+        self._setup_engine(control_limits, cost_config)
+        self._create(L.cps_cem_gmm_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset, self.outer_its,
+                     int(cem_best_k), float(cem_initial_action_stdev), float(cem_stdev_min))
+
+    def reset(self, states, period: int = 0):
+        """optimizer_reset of every experiment (both components at mid-range with cem_initial_action_stdev, p1 = 0.5,
+        u_prev = 0), the initial states [E, 6] and the period counter."""
+        s = self._host_states(states)
+        self.engine._chk(self.engine.lib.cps_cem_gmm_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP), int(period)))
+
+    def distribution(self):
+        """(loc [E, 2, T], scale [E, 2, T], p1 [E]): every experiment's mixture.  Synchronises."""
+        loc, scale = (np.zeros((self.E, 2, self.T), dtype=np.float32) for _ in range(2))
+        p1 = np.zeros(self.E, dtype=np.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_cem_gmm_fleet_get_distribution(
+            self.engine._h, loc.ctypes.data_as(L._FP), scale.ctypes.data_as(L._FP), p1.ctypes.data_as(L._FP)))
+        return loc, scale, p1
+
+    def draws(self, period: int):
+        """The draws a 'philox' fleet uses in `period`: cuda tensors eps [cem_outer_it, E, 2, T, K] (standard normals of
+        both components) and u01 [cem_outer_it, E, T, K] (the component-picking uniforms)."""
+        eps = torch.empty((self.outer_its, self.E, 2, self.T, self.K), device=self.device, dtype=torch.float32)
+        u01 = torch.empty((self.outer_its, self.E, self.T, self.K), device=self.device, dtype=torch.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_cem_gmm_fleet_draws(self.engine._h, int(period), _ptr(eps), _ptr(u01)))
+        return eps, u01
+
+    def run(self, n_periods: int, target_position=None, target_equilibrium=None, eps=None, u01=None, record=None,
+            J_out=None, Q_out=None):
+        """cps_cem_gmm_fleet_step: n_periods controller periods, no synchronisation.  target_position /
+        target_equilibrium: cuda tensors [n_periods, E] or None; eps [n_periods * cem_outer_it, E, 2, T, K] and u01
+        [n_periods * cem_outer_it, E, T, K] for a 'supplied' fleet; record [n_periods, E, 16], J_out [n_periods, E, K] and
+        Q_out [n_periods, E, T, K] (costs and plans of each period's last iteration) or None."""
+        eng = self.engine
+        n_it = n_periods * self.outer_its
+        self._check_rows(n_periods, target_position, target_equilibrium, record, J_out,
+                         (eps, "eps", n_it * self.E * 2 * self.T * self.K), (u01, "u01", n_it * self.E * self.T * self.K),
+                         (Q_out, "Q_out", n_periods * self.E * self.T * self.K))
+        eng._chk(eng.lib.cps_cem_gmm_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
+                                                _ptr(eps), _ptr(u01), _ptr(record), _ptr(J_out), _ptr(Q_out)))
+        return record
+
+
+class RandomActionFleet(_FleetBase):
+    """E closed-loop experiments under optimizer_random_action_tf (`random-action-tf` in Control_Toolkit_ASF/
+    config_controllers.yml) on one device: one cps_handle with a random-action fleet attached (include/cps.h "CEM-GMM and
+    random-action fleets").
+
+    Every controller period does, for every experiment, what optimizer_random_action_b200.step does (K plans uniform in the
+    control limits, their costs from the experiment's state, u_prev and targets, u = the cheapest plan's first input),
+    then what Fleet's plant does, with no host round trip.  The keywords are optimizer_random_action_b200's (same
+    defaults) and Fleet's.  Predictor "ODE" or "ODE_v0" and the four cost plugins; num_rollouts at most 8192.  The neural
+    predictor and the plant-side models (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+    _abi = "cps_random_action_fleet"
+
+    def __init__(self, n_experiments: int, num_rollouts: int = 200, mpc_horizon: int = 35, control_limits=(-1.0, 1.0),
+                 dt: float = 0.02, substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
+                 cost_config: dict | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
+                 experiment_offset: int = 0, dt_simulation: float = 0.002):
+        if integrator == "neural":
+            raise NotImplementedError("RandomActionFleet runs on predictor 'ODE' or 'ODE_v0' (optimizer_random_action_b200 "
+                                      "has no neural predictor either)")
+        n_sim = _check_fleet_args("RandomActionFleet", integrator, None, noise, dt, dt_simulation)
+        self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
+        self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost, device=device)
+        self.device = self.engine.device
+        self._setup_engine(control_limits, cost_config)
+        self._create(L.cps_random_action_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset)
+
+    def reset(self, states, period: int = 0):
+        """u_prev = 0, the initial states [E, 6] and the period counter."""
+        s = self._host_states(states)
+        self.engine._chk(self.engine.lib.cps_random_action_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP),
+                                                                            int(period)))
+
+    def draws(self, period: int) -> torch.Tensor:
+        """The plans a 'philox' fleet evaluates in `period`: cuda tensor [E, T, K]."""
+        out = torch.empty((self.E, self.T, self.K), device=self.device, dtype=torch.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_random_action_fleet_draws(self.engine._h, int(period), _ptr(out)))
+        return out
+
+    def run(self, n_periods: int, target_position=None, target_equilibrium=None, plans=None, record=None, J_out=None,
+            Q_out=None):
+        """cps_random_action_fleet_step: n_periods controller periods, no synchronisation.  target_position /
+        target_equilibrium: cuda tensors [n_periods, E] or None; plans [n_periods, E, T, K] for a 'supplied' fleet;
+        record [n_periods, E, 16], J_out [n_periods, E, K] and Q_out [n_periods, E, T, K] (the plans evaluated) or None."""
+        eng = self.engine
+        self._check_rows(n_periods, target_position, target_equilibrium, record, J_out,
+                         (plans, "plans", n_periods * self.E * self.T * self.K),
+                         (Q_out, "Q_out", n_periods * self.E * self.T * self.K))
+        eng._chk(eng.lib.cps_random_action_fleet_step(eng._h, int(n_periods), _ptr(target_position),
+                                                      _ptr(target_equilibrium), _ptr(plans), _ptr(record), _ptr(J_out),
+                                                      _ptr(Q_out)))
+        return record

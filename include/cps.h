@@ -555,6 +555,84 @@ int cps_cem_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const 
 int cps_cem_fleet_draws(cps_handle *h, long long period, float *out_dev);
 long long cps_cem_fleet_period(const cps_handle *h);
 
+/* ---- CEM-GMM and random-action fleets: E closed-loop experiments under optimizer_cem_gmm_tf / optimizer_random_action_tf */
+/* The data generator with controller_mpc and optimizer cem-gmm-tf or random-action-tf (Control_Toolkit_ASF/
+ * config_controllers.yml; Control_Toolkit/Optimizers/optimizer_cem_gmm_tf.py:14-140, optimizer_random_action_tf.py:12-86).
+ * CEM-GMM: per controller period every experiment runs exactly what one cps_cem_gmm_step with outer_its iterations does
+ * from its own state, mixture (loc[2][T], scale[2][T], p1), u_prev, targets and draws -- per iteration component
+ * c = 0 iff u01 < p1 and Q = clip(loc[c][t] + scale[c][t] eps_c) with separately rounded multiply and add, the costs, the
+ * best_k cheapest plans (ties to the lowest index, NaN costs last), the two clusters around the two cheapest elites
+ * (nearer in the Euclidean norm, ties to the cheapest), their per-step mean and population stdev clipped to
+ * [stdev_min, 1e4] and p1 = n1 / best_k; after the last iteration u = elite_Q[0, 0] and loc / scale shifted by one step
+ * with the last entry repeated.  Random action: every experiment evaluates K plans uniform in [lo, hi) from its state,
+ * u_prev and targets and takes u = Q[argmin J, 0] (ties to the lowest index).  Then, for both, the plant advances one
+ * controller period with Q = u and writes the record row of cps_fleet_step; u becomes the experiment's u_prev.
+ * Targets select the folded cost parameters per experiment and period, as in cps_fleet_step.
+ * Draws, supplied (CPS_FLEET_NOISE_SUPPLIED; consecutive periods back to back in one _step call) or generated from
+ * Philox4x32-10 (CPS_FLEET_NOISE_PHILOX, key = seed, counters disjoint from the other fleets' streams; _draws materialises
+ * them): CEM-GMM standard normals eps [outer_its][E][2][T][K] and uniforms u01 [outer_its][E][T][K] per period, counter
+ * (plan k, GMM tag + 3 it ceil(T / 4) + {0, ceil(T / 4)} + group of four steps, period, experiment_offset + e) for the two
+ * components' normals and + 2 ceil(T / 4) + group for the uniforms; random action plans [E][T][K] per period, counter
+ * (plan k, RA tag + group of four steps, period, experiment_offset + e).  A Philox uniform is (word >> 8) 2^-24 in [0, 1)
+ * from one 32-bit word; a random-action plan entry is lo + (hi - lo) u with the multiply and the add rounded separately.
+ * Launches per period: 2 outer_its + 1 (CEM-GMM), 2 (random action), whatever E (cps_launch_count).
+ * The handle: predictor CPS_EULER_CROMER or CPS_EULER_V0, one of the four cost plugins, K <= 8192, control limits from
+ * cps_set_mppi_params (lo, hi).  The neural predictor, no cost plugin or the legacy cost, CPS_FLAG_SUBSTEP_SINCOS /
+ * CPS_FLAG_FAST_DIV, K > 8192 or a horizon whose buffers do not fit shared memory: CPS_ERR_UNSUPPORTED.  CEM-GMM best_k
+ * outside [2, K], a negative stdev, outer_its < 1, more than 65535 experiments or dt not a multiple of dt_simulation:
+ * CPS_ERR_INVALID.  Non-finite costs sort after every number, stay in their experiment and are counted
+ * (cps_nonfinite_costs). */
+typedef struct cps_cem_gmm_fleet_config {
+    int struct_size;                 /* = sizeof(cps_cem_gmm_fleet_config) */
+    int n_experiments;               /* E on this device, at most 65535 */
+    int sim_substeps;                /* plant ticks per controller period */
+    int draw_source;                 /* CPS_FLEET_NOISE_SUPPLIED | CPS_FLEET_NOISE_PHILOX */
+    double dt_simulation;            /* plant tick, 0.002 s */
+    unsigned long long seed;
+    long long experiment_offset;     /* global index of local experiment 0 (Philox counters) */
+    int outer_its;                   /* cem_outer_it */
+    int best_k;                      /* cem_best_k */
+    float initial_stdev, stdev_min;  /* cem_initial_action_stdev, cem_stdev_min */
+} cps_cem_gmm_fleet_config;
+int cps_cem_gmm_fleet_create(cps_handle *h, const cps_cem_gmm_fleet_config *cfg);
+/* optimizer_reset for every experiment (both components at mid-range with initial_stdev, p1 = 0.5, as cps_cem_gmm_reset),
+ * u_prev = 0; states s_host [E][6]; the period counter.  Synchronises. */
+int cps_cem_gmm_fleet_set_states(cps_handle *h, const float *s_host, long long period);
+/* s_host [E][6], u_prev_host [E]; either may be NULL.  Synchronises. */
+int cps_cem_gmm_fleet_get_states(cps_handle *h, float *s_host, float *u_prev_host);
+/* Every experiment's mixture: loc_host, scale_host [E][2][T], p1_host [E]; any may be NULL.  Synchronises. */
+int cps_cem_gmm_fleet_get_distribution(cps_handle *h, float *loc_host, float *scale_host, float *p1_host);
+/* n_periods controller periods, stream-ordered, no synchronisation.  tp_dev / te_dev [n_periods][E] or NULL (0 / +1);
+ * eps_dev / u01_dev the periods' draws back to back (NULL on a Philox fleet); record_dev [n_periods][E][CPS_FLEET_RECORD],
+ * J_out_dev [n_periods][E][K] and Q_out_dev [n_periods][E][T][K] (costs and plans of each period's last iteration) may
+ * each be NULL. */
+int cps_cem_gmm_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *eps_dev,
+                           const float *u01_dev, float *record_dev, float *J_out_dev, float *Q_out_dev);
+/* The draws a Philox fleet uses in controller period `period`: eps_out_dev [outer_its][E][2][T][K], u01_out_dev
+ * [outer_its][E][T][K]; either may be NULL. */
+int cps_cem_gmm_fleet_draws(cps_handle *h, long long period, float *eps_out_dev, float *u01_out_dev);
+long long cps_cem_gmm_fleet_period(const cps_handle *h);
+
+typedef struct cps_random_action_fleet_config {
+    int struct_size;                 /* = sizeof(cps_random_action_fleet_config) */
+    int n_experiments;               /* E on this device, at most 65535 */
+    int sim_substeps;                /* plant ticks per controller period */
+    int draw_source;                 /* CPS_FLEET_NOISE_SUPPLIED | CPS_FLEET_NOISE_PHILOX */
+    double dt_simulation;            /* plant tick, 0.002 s */
+    unsigned long long seed;
+    long long experiment_offset;     /* global index of local experiment 0 (Philox counters) */
+} cps_random_action_fleet_config;
+int cps_random_action_fleet_create(cps_handle *h, const cps_random_action_fleet_config *cfg);
+/* u_prev = 0; states s_host [E][6]; the period counter.  Synchronises. */
+int cps_random_action_fleet_set_states(cps_handle *h, const float *s_host, long long period);
+int cps_random_action_fleet_get_states(cps_handle *h, float *s_host, float *u_prev_host);
+/* As cps_cem_gmm_fleet_step; plans_dev [n_periods][E][T][K] (NULL on a Philox fleet); Q_out_dev receives the plans. */
+int cps_random_action_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *plans_dev,
+                                 float *record_dev, float *J_out_dev, float *Q_out_dev);
+/* The plans a Philox fleet evaluates in controller period `period`: out_dev [E][T][K]. */
+int cps_random_action_fleet_draws(cps_handle *h, long long period, float *out_dev);
+long long cps_random_action_fleet_period(const cps_handle *h);
+
 /* ---- forward-only planners: predict_and_cost and the selection step (SURVEY 8f row f3) ----------------------- */
 /* optimizer_random_action_tf / optimizer_cem_tf / optimizer_cem_gmm_tf evaluate K candidate input plans from one state
  * with predictor.predict_core(s, Q) followed by cost_function.get_trajectory_cost(trajectory, Q, u_prev)
