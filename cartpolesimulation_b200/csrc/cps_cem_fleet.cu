@@ -10,6 +10,10 @@
 //                              grid (T, E); after the last iteration the stdev clip, the shift of both vectors and
 //                              u = elite_Q[0, 0] (:96-99), which becomes the experiment's u_prev;
 //   fleet_net_plant_kernel     (cps_fleet.cu) the plant period with Q = u and the record row, one thread per experiment.
+// With the neural predictor an outer iteration is plan_sample_kernel (the plans into [E][K][T], the period's cost
+// parameters into [E]), net_grad_kernel<.., FLEET> (cps_net_grad.cu) for the costs, plan_select_kernel with one block per
+// experiment, and cem_update_fleet_kernel as above: n_it x (3, or 4 with deferred statistics) + 1 launches per period.
+// Every rollout starts from the network's stored hidden state; the fleet keeps none per experiment.
 // Per experiment every iteration is the arithmetic of one cps_cem_step iteration; the solve counter is shared (lockstep):
 // first_iter_count iterations on the first period after cps_cem_fleet_set_states, outer_its after that.  The
 // distribution lives in [2][E][T] ping-pong buffers (an iteration reads one half and writes the other).
@@ -34,6 +38,8 @@ struct CemFleetState {
     float *d_J;                       // [E][K] costs when the caller does not ask for them
     int *d_elite;                     // [E][K] elite lists of the deferred statistics (best_k x T > 2048), else null
     unsigned *d_tickets;              // [E]
+    float *d_P;                       // neural predictor: [E][K][T] the sampled plans
+    CostParams *d_costs;              // neural predictor: [E] the period's folded cost parameters
     long long first_period, solves;
 };
 
@@ -42,6 +48,7 @@ void cps_cem_fleet_free(cps_handle *h) {
     if (!F) return;
     fleet_core_free(F->core);
     cudaFree(F->d_mu); cudaFree(F->d_sd); cudaFree(F->d_J); cudaFree(F->d_elite); cudaFree(F->d_tickets);
+    cudaFree(F->d_P); cudaFree(F->d_costs);
     delete F;
     h->cfleet = nullptr;
 }
@@ -87,6 +94,10 @@ extern "C" int cps_cem_fleet_create(cps_handle *h, const cps_cem_fleet_config *c
     if ((long long)cfg->best_k * T > 2048) CUDA_TRY(h, cudaMalloc(&F->d_elite, sizeof(int) * E * K));
     CUDA_TRY(h, cudaMalloc(&F->d_tickets, sizeof(unsigned) * E));
     CUDA_TRY(h, cudaMemset(F->d_tickets, 0, sizeof(unsigned) * E));
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) {
+        CUDA_TRY(h, cudaMalloc(&F->d_P, sizeof(float) * E * K * T));
+        CUDA_TRY(h, cudaMalloc(&F->d_costs, sizeof(CostParams) * E));
+    }
     return CPS_OK;
 }
 
@@ -132,6 +143,7 @@ extern "C" int cps_cem_fleet_step(cps_handle *h, int n_periods, const float *tp_
     it.s = fc.d_s; it.u = fc.d_uprev;
     it.seed = fc.seed; it.e_offset = fc.e_offset;
     it.elite = F->d_elite; it.tickets = F->d_tickets;
+    it.P = F->d_P; it.costs = F->d_costs;
     NetPlantArgs pa;
     memset(&pa, 0, sizeof(pa));
     pa.plant = plant_params(h, fc.dt_sim, fc.n_sim);

@@ -14,7 +14,11 @@
 //     plan_forward_fleet_kernel   each experiment's K uniform plans in [lo, hi), their costs, and in the last block of the
 //                                 experiment (its own ticket) u = Q[argmin J, 0];
 //   fleet_net_plant_kernel        (cps_fleet.cu) the plant period with Q = u and the record row, one thread per experiment.
-// Launches per period: 2 x cem_outer_it + 1 (CEM-GMM), 2 (random action).  The mixtures live in [2][E][4T + 1] ping-pong
+// Launches per period: 2 x cem_outer_it + 1 (CEM-GMM), 2 (random action).
+// With the neural predictor the rollouts are plan_sample_kernel (the plans into [E][K][T], the period's cost parameters
+// into [E]) and net_grad_kernel<.., FLEET> (cps_net_grad.cu), and random action takes its argmin in plan_select_kernel,
+// one block per experiment: 3 x cem_outer_it + 1 (CEM-GMM), 4 (random action) launches per period.  Every rollout starts
+// from the network's stored hidden state; the fleets keep none per experiment.  The mixtures live in [2][E][4T + 1] ping-pong
 // buffers (an iteration reads one half and writes the other).  No [E][T][K] plan or draw buffer is materialised on a
 // Philox fleet: the update rebuilds the elites' plans, best_k x T per experiment, from the mixture and the regenerated draws.
 #include <cuda_runtime.h>
@@ -40,12 +44,15 @@ struct ForwardFleetState {
     int *d_elite;                     // CEM-GMM: [E][2K] elite indices and cluster flags
     float *d_rows;                    // CEM-GMM: [E][best_k][T] the elites' plans
     unsigned *d_tickets;              // random action: [E]
+    float *d_P;                       // neural predictor: [E][K][T] the sampled plans
+    CostParams *d_costs;              // neural predictor: [E] the period's folded cost parameters
 };
 
 static void forward_fleet_free(ForwardFleetState *&F) {
     if (!F) return;
     fleet_core_free(F->core);
     cudaFree(F->d_dist); cudaFree(F->d_J); cudaFree(F->d_elite); cudaFree(F->d_rows); cudaFree(F->d_tickets);
+    cudaFree(F->d_P); cudaFree(F->d_costs);
     delete F;
     F = nullptr;
 }
@@ -93,6 +100,10 @@ static int forward_fleet_create(cps_handle *h, ForwardFleetState *&slot, int gmm
         CUDA_TRY(h, cudaMalloc(&F->d_tickets, sizeof(unsigned) * E));
         CUDA_TRY(h, cudaMemset(F->d_tickets, 0, sizeof(unsigned) * E));
     }
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) {
+        CUDA_TRY(h, cudaMalloc(&F->d_P, sizeof(float) * E * K * T));
+        CUDA_TRY(h, cudaMalloc(&F->d_costs, sizeof(CostParams) * E));
+    }
     return CPS_OK;
 }
 
@@ -137,6 +148,7 @@ static int forward_fleet_step(cps_handle *h, ForwardFleetState *F, int n_periods
     r.s = fc.d_s; r.u = fc.d_uprev;
     r.seed = fc.seed; r.e_offset = fc.e_offset;
     r.tickets = F->d_tickets;
+    r.P = F->d_P; r.costs = F->d_costs;
     GmmFleetUpdate g;
     memset(&g, 0, sizeof(g));
     g.E = fc.E; g.K = F->K; g.T = F->T; g.best_k = F->best_k;

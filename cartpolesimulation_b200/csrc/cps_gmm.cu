@@ -14,7 +14,7 @@
 //
 // Three launches per outer iteration, nothing returns to the host in between:
 //   gmm_sample_kernel   Q[T][K] from the supplied draws (standard normals for both components, one uniform per element)
-//   plan_kernel         rollouts + cost (cps_plan_cost)
+//   plan_kernel         rollouts + cost (cps_plan_cost; with the neural predictor its net_grad_kernel pass)
 //   gmm_update_kernel   ONE block: radix select of the best_k cheapest plans (ties in index order), the two cheapest of
 //                       them, the distances, the cluster statistics, and after the last iteration u and the shift.
 // The distribution lives on the device: loc[2][T], scale[2][T], p1.
@@ -323,7 +323,7 @@ extern "C" int cps_cem_gmm_reset(cps_handle *h) {
 
 extern "C" int cps_cem_gmm_configure(cps_handle *h, int best_k, float initial_stdev, float stdev_min) {
     if (!h) return CPS_ERR_INVALID;
-    const int rc = cps_plan_check(h, "cps_cem_gmm_configure");   // every solve runs cps_plan_cost
+    const int rc = cps_plan_check(h, "cps_cem_gmm_configure");   // every solve runs cps_plan_cost (ODE or network)
     if (rc != CPS_OK) return rc;
     if (best_k < 2 || best_k > h->cfg.num_rollouts)   // the two cheapest elites seed the two clusters
         return fail(h, CPS_ERR_INVALID, "cps_cem_gmm_configure: cem_best_k must lie in [2, num_rollouts]");
@@ -388,8 +388,8 @@ extern "C" int cps_cem_gmm_step_host(cps_handle *h, const float *s_host, const f
     if (!h) return CPS_ERR_INVALID;
     if (!s_host || !u_out_host) return fail(h, CPS_ERR_INVALID, "cps_cem_gmm_step_host: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    // the state travels in plan_kernel's parameter block
-    return solve_host(h, s_host, u_out_host, true, [&](const float *s_dev, float *u_dev) {
+    // ODE: the state travels in plan_kernel's parameter block; the network kernel reads it from device memory
+    return solve_host(h, s_host, u_out_host, h->cfg.integrator != CPS_PREDICTOR_NEURAL, [&](const float *s_dev, float *u_dev) {
         return cps_cem_gmm_step(h, s_dev, eps_dev, u01_dev, layout, n_iterations, u_prev, u_dev, nullptr, nullptr);
     });
 }

@@ -150,7 +150,8 @@ void cps_cem_fleet_free(cps_handle *h);
 void cps_forward_fleets_free(cps_handle *h);
 // cps_plan.cu
 void cps_plan_free(cps_handle *h);
-// the refusals every forward-only planner shares: neural predictor, no cost plugin, substep sin/cos or fast division
+// the refusals every forward-only planner shares: no cost plugin, substep sin/cos or fast division; with the neural
+// predictor those of cps_plan_cost on a network (cps_net_plan_check) and K above the single-block selection
 int cps_plan_check(cps_handle *h, const char *who);
 // CEM fleets: the refusals of cps_cem_fleet_create that concern the planner (those of cps_cem_configure, K above the
 // single-block selection, shared memory of plan_fleet_kernel), and one outer iteration of E experiments: plan_fleet_kernel,
@@ -171,6 +172,8 @@ struct CemFleetIteration {
     float *Q_out;                // [E][T][K] <- the plans, or null
     int *elite;                  // [E][K] scratch of the deferred statistics
     unsigned *tickets;           // [E], zero between launches
+    float *P;                    // neural predictor: [E][K][T] scratch, the sampled plans net_grad_kernel reads
+    CostParams *costs;           // neural predictor: [E] scratch, the folded cost parameters of this period
 };
 int cps_cem_fleet_check(cps_handle *h, int best_k, float initial_stdev, float stdev_min, int philox, const char *who);
 int cps_cem_fleet_iteration(cps_handle *h, const CemFleetIteration &c);
@@ -193,6 +196,8 @@ struct ForwardFleetRollouts {
     float *J;                    // [E][K] <- the costs
     float *Q_out;                // [E][T][K] <- the plans, or null
     unsigned *tickets;           // [E], zero between launches (random action)
+    float *P;                    // neural predictor: [E][K][T] scratch, the sampled plans net_grad_kernel reads
+    CostParams *costs;           // neural predictor: [E] scratch, the folded cost parameters of this period
 };
 int cps_forward_fleet_check(cps_handle *h, int gmm, int best_k, float initial_stdev, float stdev_min, const char *who);
 int cps_forward_fleet_rollouts(cps_handle *h, const ForwardFleetRollouts &c);
@@ -233,13 +238,15 @@ int cps_net_plan_cost(cps_handle *h, const float *s_dev, const float *Q_dev, int
                       float *J_out_dev, float *traj_out_dev, int traj_layout);
 int cps_net_plan_cost_grad(cps_handle *h, const float *s_dev, const float *Q_dev, int q_layout, float u_prev, float *J_out_dev,
                            float *G_out_dev);
+// the refusals of cps_plan_cost with CPS_PREDICTOR_NEURAL (no network, D_* network, plugin, tensor-core flag, shared memory)
+int cps_net_plan_check(cps_handle *h, const char *who);
 // the RPGD fleet with CPS_PREDICTOR_NEURAL: cps_net_grad_fleet_prepare runs the network checks of cps_plan_cost_grad and
 // sizes the workspace for E experiments; cps_net_grad_fleet is net_grad_kernel over E experiments x K plans [E][K][T] from
 // the fleet's states [E][8], per-experiment cost parameters and u_prev [E]: the gradient (G != nullptr, J and G [E][K][T])
 // or the costs only (G == nullptr), per plan bit-identical to cps_plan_cost_grad / cps_plan_cost
 int cps_net_grad_fleet_prepare(cps_handle *h, int E, const char *who);
 int cps_net_grad_fleet(cps_handle *h, int E, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
-                       const float *u_prev_dev, float *J_dev, float *G_dev);
+                       const float *u_prev_dev, float *J_dev, float *G_dev, const char *who);   // who: for the messages
 int cps_net_mppi_step(cps_handle *h, const float *s_dev, const float *noise_dev, int noise_layout, float u_prev,
                       float *u_nom_dev, float *u_out_dev, float *J_out_dev, float *traj_out_dev, int traj_layout,
                       float *u_run_out_dev);

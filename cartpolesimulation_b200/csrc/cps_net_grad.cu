@@ -516,6 +516,9 @@ int cps_net_plan_cost_grad(cps_handle *h, const float *s_dev, const float *Q_dev
     return launch(h, a, true);
 }
 
+// ---- cps_plan.cu / cps_gmm.cu: the network checks of cps_plan_cost for the forward-only planners -------------------------
+int cps_net_plan_check(cps_handle *h, const char *who) { return check(h, who, false); }
+
 // ---- cps_rpgd_fleet.cu: the plans of E experiments in one launch -----------------------------------------------------------
 int cps_net_grad_fleet_prepare(cps_handle *h, int E, const char *who) {
     int rc = check(h, who, true);
@@ -526,9 +529,9 @@ int cps_net_grad_fleet_prepare(cps_handle *h, int E, const char *who) {
 }
 
 int cps_net_grad_fleet(cps_handle *h, int E, const float *s_dev, const float *Q_dev, const CostParams *costs_dev,
-                       const float *u_prev_dev, float *J_dev, float *G_dev) {
+                       const float *u_prev_dev, float *J_dev, float *G_dev, const char *who) {
     const bool grad = G_dev != nullptr;
-    int rc = check(h, "cps_rpgd_fleet_step", grad);
+    int rc = check(h, who, grad);
     if (rc != CPS_OK) return rc;
     NetState *S = h->net;
     const int K = h->cfg.num_rollouts, T = h->cfg.horizon;

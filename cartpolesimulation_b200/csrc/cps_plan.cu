@@ -84,6 +84,7 @@ struct PlanState {
     unsigned *d_gkmax, *d_ghist;
     int *d_gcnt;
     int configured_cem;
+    float *d_P;                   // neural predictor, CEM: [K][T] the sampled plans net_grad_kernel reads
 };
 
 // cost -> unsigned key with the same order; NaN sorts last
@@ -693,6 +694,8 @@ __device__ __forceinline__ void ra_fleet_select(const PlanArgs &a, const PlanFle
 // PLAN_GMM (CEM-GMM fleets): the experiment's mixture loc[2][T], scale[2][T], p1 goes to shared memory and every plan entry
 // is gmm_plan_value of the component its uniform picks, from normals [E][2][T][K] and uniforms fx->u01 [E][T][K] or from
 // Philox (three calls per four steps: both components' normals and the uniforms); no selection here.
+// The draws and plan entries formed in the horizon loop below are restated by plan_sample_kernel (the neural predictor's
+// plans): a change to either copy -- Philox counters, the GMM groups of four, supplied-draw indexing -- goes into both.
 template <int INTEG, int COST, int MODE, int NSUB, bool FLEET, bool PHILOX>
 __device__ __forceinline__ void plan_body(const PlanArgs &a, const PlanFleetExt *fx, const CostParams &cost) {
     extern __shared__ float smem[];   // PLAN_CEM: mu[T], sd[T], mu2[T], sd2[T], elite list [elite_smem], PHILOX: elites' draws
@@ -840,6 +843,97 @@ __global__ void __launch_bounds__(256, 4) plan_forward_fleet_kernel(const __grid
     plan_body<INTEG, COST, MODE, NSUB, true, PHILOX>(a, &fx, s_cost);
 }
 
+// ---- neural predictor: the plans for net_grad_kernel, then the selection on their costs ------------------------------------
+// plan_sample_kernel, block (b, x), one thread per plan k of experiment x: the plan entries plan_body would form in its
+// horizon loop -- PLAN_CEM clip(mu + eps sd) (cem_plan_value), PLAN_GMM gmm_plan_value of the component the uniform picks,
+// PLAN_Q the uniforms lo + (hi - lo) u (Philox only: supplied random-action plans are evaluated as given) -- from the same
+// draws with the same Philox counters.  Single solve (CEM): draws a.Q and plans P / a.Q_out in the strides qs_k / qs_t.
+// FLEET: draws in the fleets' layouts ([E][T][K], GMM [E][2][T][K] + fx.u01), P [E][K][T] (net_grad_kernel's FLEET
+// layout), a.Q_out [E][T][K]; block (0, x) also folds the experiment's cost parameters of the period into costs[x].
+// The draw generation restates plan_body's horizon loop (kept apart so that plan_body's code is untouched): a change to
+// either copy goes into both; test_gpu_plan_neural.py checks a neural fleet's draws against the ODE fleet's.
+template <int MODE, bool FLEET, bool PHILOX>
+__global__ void __launch_bounds__(256) plan_sample_kernel(const __grid_constant__ PlanArgs a,
+                                                          const __grid_constant__ PlanFleetExt fx, float *P, CostParams *costs) {
+    extern __shared__ float smem[];   // PLAN_CEM: mu[T], sd[T]; PLAN_GMM: loc[2][T], scale[2][T], p1
+    const int tid = threadIdx.x, T = a.T, K = a.K;
+    const long long x = FLEET ? blockIdx.y : 0;
+    if (FLEET && blockIdx.x == 0 && tid == 0) costs[x] = fold_cost_e(fx.cost_up, fx.cost_dn, fx.tp, fx.te, (int)x);
+    if (MODE == PLAN_CEM)
+        for (int t = tid; t < T; t += blockDim.x) { smem[t] = a.mu[x * T + t]; smem[T + t] = a.sd[x * T + t]; }
+    if (MODE == PLAN_GMM)
+        for (int i = tid; i < 4 * T + 1; i += blockDim.x) smem[i] = a.mu[x * (4 * T + 1) + i];
+    __syncthreads();
+    const int k = blockIdx.x * blockDim.x + tid;
+    if (k >= K) return;
+    const long long qoff = x * T * K + k;   // FLEET: plan k of experiment x in the [E][T][K] draws and Q_out
+    float nr[4];
+    for (int t = 0; t < T; ++t) {
+        float u;
+        if (MODE == PLAN_GMM && PHILOX) {   // plan_body's groups of four entries
+            if ((t & 3) == 0) {
+                float n1[4], nu[4];
+                const unsigned g = (unsigned)(t >> 2), G4 = (unsigned)((T + 3) >> 2), eg = fx.e_offset + (unsigned)x;
+                philox_normals(fx.seed, (unsigned)k, fx.w1 + g, fx.period, eg, 4, nr, 1);
+                philox_normals(fx.seed, (unsigned)k, fx.w1 + G4 + g, fx.period, eg, 4, n1, 1);
+                philox_uniforms(fx.seed, (unsigned)k, fx.w1 + 2 * G4 + g, fx.period, eg, 4, nu, 1, 0.0f, 1.0f);
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    const int tq = min(t + q, T - 1), c = (nu[q] < smem[4 * T]) ? 0 : 1;
+                    nr[q] = gmm_plan_value(smem[c * T + tq], smem[(2 + c) * T + tq], c ? n1[q] : nr[q], a.lo, a.hi);
+                }
+            }
+            u = nr[t & 3];
+        } else if (MODE == PLAN_GMM) {
+            const int c = (fx.u01[qoff + (long long)t * K] < smem[4 * T]) ? 0 : 1;
+            u = gmm_plan_value(smem[c * T + t], smem[(2 + c) * T + t], a.Q[(x * 2 * T + c * T + t) * K + k], a.lo, a.hi);
+        } else if (PHILOX) {
+            if ((t & 3) == 0) {
+                if (MODE == PLAN_Q)
+                    philox_uniforms(fx.seed, (unsigned)k, fx.w1 + (unsigned)(t >> 2), fx.period, fx.e_offset + (unsigned)x, 4,
+                                    nr, 1, a.lo, __fsub_rn(a.hi, a.lo));
+                else
+                    philox_normals(fx.seed, (unsigned)k, fx.w1 + (unsigned)(t >> 2), fx.period, fx.e_offset + (unsigned)x, 4,
+                                   nr, 1);
+            }
+            u = nr[t & 3];
+        } else {
+            u = FLEET ? a.Q[qoff + (long long)t * K] : a.Q[(long long)k * a.qs_k + (long long)t * a.qs_t];
+        }
+        if (MODE == PLAN_CEM) u = cem_plan_value(smem[t], u, smem[T + t], a.lo, a.hi);
+        if (FLEET) {
+            P[(x * K + k) * T + t] = u;
+            if (a.Q_out) a.Q_out[qoff + (long long)t * K] = u;
+        } else {
+            const long long o = (long long)k * a.qs_k + (long long)t * a.qs_t;
+            P[o] = u;
+            if (a.Q_out) a.Q_out[o] = u;
+        }
+    }
+}
+
+// The selection plan_body runs in the block that finishes last, as a kernel of its own after net_grad_kernel wrote the
+// costs: one block of 256 threads (plan_select assumes at most 8 warps), FLEET one per experiment x = blockIdx.y.  It reads
+// the same inputs as there: the draws and the distribution the plans were sampled from (CEM: cem_plan_value of them is the
+// sampled plan, bit for bit), the supplied plans, or the Philox draws regenerated; dynamic shared memory as plan_body's.
+template <int MODE, bool FLEET, bool PHILOX>
+__global__ void __launch_bounds__(256) plan_select_kernel(const __grid_constant__ PlanArgs a,
+                                                          const __grid_constant__ PlanFleetExt fx) {
+    extern __shared__ float smem[];   // PLAN_CEM: mu[T], sd[T], mu2[T], sd2[T], elite list [elite_smem], PHILOX: elites' draws
+    const int T = a.T;
+    const long long x = FLEET ? blockIdx.y : 0;
+    float *s_mu = smem, *s_sd = smem + T;
+    if (MODE == PLAN_CEM) {
+        for (int t = threadIdx.x; t < T; t += blockDim.x) { s_mu[t] = a.mu[x * T + t]; s_sd[t] = a.sd[x * T + t]; }
+        __syncthreads();
+    }
+    int *s_elite = reinterpret_cast<int *>(smem + 4 * T);
+    if (FLEET && MODE == PLAN_Q) ra_fleet_select<PHILOX>(a, fx);
+    else if (FLEET) cem_fleet_select<PHILOX>(a, fx, s_mu, s_sd, smem + 2 * T, smem + 3 * T, s_elite,
+                                             reinterpret_cast<float *>(s_elite + a.elite_smem));
+    else plan_select<MODE>(a, s_mu, s_sd, smem + 2 * T, smem + 3 * T, s_elite);
+}
+
 // Many plans, no selecting block, time-major plans: two plans per thread (k, k + 1) in packed FP32, as mppi_solve_block2
 // does for the MPPI solve.  Per plan the arithmetic is that of plan_kernel, so the costs are bit-identical (tested).
 #define CPS_PLAN_PAIR_MIN 65536   /* measured: at 16384 and 32768 plans one per thread is 10-25 % faster (latency regime) */
@@ -967,7 +1061,7 @@ void cps_plan_free(cps_handle *h) {
     PlanState *P = h->plan;
     if (!P) return;
     cudaFree(P->d_J); cudaFree(P->d_mu); cudaFree(P->d_sd); cudaFree(P->d_elite); cudaFree(P->d_best); cudaFree(P->d_ticket);
-    cudaFree(P->d_gbest); cudaFree(P->d_gkmax); cudaFree(P->d_ghist); cudaFree(P->d_gcnt);
+    cudaFree(P->d_gbest); cudaFree(P->d_gkmax); cudaFree(P->d_ghist); cudaFree(P->d_gcnt); cudaFree(P->d_P);
     delete P;
     h->plan = nullptr;
 }
@@ -988,6 +1082,7 @@ static int plan_state(cps_handle *h, PlanState **out) {
     if (e == cudaSuccess) e = cudaMalloc(&P->d_gkmax, sizeof(unsigned));
     if (e == cudaSuccess) e = cudaMalloc(&P->d_ghist, sizeof(unsigned) * 4 * 256);
     if (e == cudaSuccess) e = cudaMalloc(&P->d_gcnt, sizeof(int) * 2 * 1024);
+    if (e == cudaSuccess && h->cfg.integrator == CPS_PREDICTOR_NEURAL) e = cudaMalloc(&P->d_P, sizeof(float) * K * T);
     if (e == cudaSuccess) e = cudaMemset(P->d_gbest, 0xFF, sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaMemset(P->d_gkmax, 0, sizeof(unsigned));
     if (e == cudaSuccess) e = cudaMemset(P->d_ghist, 0, sizeof(unsigned) * 4 * 256);
@@ -996,7 +1091,7 @@ static int plan_state(cps_handle *h, PlanState **out) {
     if (e == cudaSuccess) e = cudaMemset(P->d_sd, 0, sizeof(float) * 2 * T);
     if (e != cudaSuccess) {   // nothing half-built stays attached to the handle
         cudaFree(P->d_J); cudaFree(P->d_mu); cudaFree(P->d_sd); cudaFree(P->d_elite); cudaFree(P->d_best); cudaFree(P->d_ticket);
-        cudaFree(P->d_gbest); cudaFree(P->d_gkmax); cudaFree(P->d_ghist); cudaFree(P->d_gcnt);
+        cudaFree(P->d_gbest); cudaFree(P->d_gkmax); cudaFree(P->d_ghist); cudaFree(P->d_gcnt); cudaFree(P->d_P);
         delete P;
         return fail(h, CPS_ERR_CUDA, "cps_plan: allocating the planner scratch: %s", cudaGetErrorString(e));
     }
@@ -1006,8 +1101,14 @@ static int plan_state(cps_handle *h, PlanState **out) {
 }
 
 int cps_plan_check(cps_handle *h, const char *who) {
-    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
-        return fail(h, CPS_ERR_UNSUPPORTED, "%s: ODE predictors only (neural predictor: cps_plan_cost, or cps_net_rollout + cps_trajectory_cost)", who);
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) {   // every evaluation is cps_plan_cost's, the selection one block
+        const int rc = cps_net_plan_check(h, who);
+        if (rc != CPS_OK) return rc;
+        if (h->cfg.num_rollouts > CPS_CEM_MULTIBLOCK_MIN)
+            return fail(h, CPS_ERR_UNSUPPORTED, "%s: with the neural predictor at most %d plans (the multi-block selection is "
+                        "built for the ODE predictors only)", who, CPS_CEM_MULTIBLOCK_MIN);
+        return CPS_OK;
+    }
     if (h->cfg.cost_id == CPS_COST_NONE || h->cfg.cost_id == CPS_COST_LEGACY_MPPI)
         return fail(h, CPS_ERR_NOT_CONFIGURED, "%s: the handle has no cost-function plugin", who);
     if (h->cfg.flags & (CPS_FLAG_SUBSTEP_SINCOS | CPS_FLAG_FAST_DIV))
@@ -1089,6 +1190,13 @@ extern "C" int cps_plan_random_action(cps_handle *h, const float *s_dev, const f
     a.ticket = P->d_ticket; a.elite = P->d_elite;
     a.u_out = u_out_dev;
     a.best_out = best_out_dev ? best_out_dev : P->d_best;
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) {   // cps_plan_cost's network pass, then the argmin
+        if ((rc = cps_net_plan_cost(h, s_dev, Q_dev, q_layout, K, T, u_prev, a.J, nullptr, 0)) != CPS_OK) return rc;
+        plan_select_kernel<PLAN_Q, false, false><<<1, 256, 0, h->stream>>>(a, PlanFleetExt());
+        h->launches += 1;
+        CUDA_TRY(h, cudaGetLastError());
+        return CPS_OK;
+    }
     int grid, block;
     plan_geometry(K, true, grid, block);
     plan_fn fn = pick_plan(h->cfg.integrator, h->cfg.cost_id, PLAN_Q, h->ode.n);
@@ -1105,8 +1213,9 @@ extern "C" int cps_plan_random_action_host(cps_handle *h, const float *s_host, c
     if (!h) return CPS_ERR_INVALID;
     if (!s_host || !u_out_host) return fail(h, CPS_ERR_INVALID, "cps_plan_random_action_host: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    // one stream operation: state in the parameter block, control written into mapped pinned host memory
-    return solve_host(h, s_host, u_out_host, true, [&](const float *s_dev, float *u_dev) {
+    // ODE: one stream operation, state in the parameter block, control written into mapped pinned host memory; the
+    // network kernel reads the state from device memory
+    return solve_host(h, s_host, u_out_host, h->cfg.integrator != CPS_PREDICTOR_NEURAL, [&](const float *s_dev, float *u_dev) {
         return cps_plan_random_action(h, s_dev, Q_dev, q_layout, u_prev, u_dev, nullptr, nullptr);
     });
 }
@@ -1174,6 +1283,35 @@ extern "C" int cps_cem_step(cps_handle *h, const float *s_dev, const float *eps_
     // one block per horizon step
     a.defer_stats = ((long long)P->best_k * T > 2048) ? 1 : 0;
     a.elite_smem = a.defer_stats ? 0 : P->best_k;   // the update kernel reads the list from global memory
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) {   // per iteration: the plans, cps_plan_cost's network pass, the selection
+        if (smem > 48 * 1024)
+            CUDA_TRY(h, cudaFuncSetAttribute((const void *)plan_select_kernel<PLAN_CEM, false, false>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (sizeof(float) * 2 * (size_t)T > 48 * 1024)
+            CUDA_TRY(h, cudaFuncSetAttribute((const void *)plan_sample_kernel<PLAN_CEM, false, false>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(float) * 2 * (size_t)T)));
+        for (int it = 0; it < n_iterations; ++it) {
+            a.Q = eps_dev + (size_t)it * K * T;
+            a.last_iter = (it == n_iterations - 1) ? 1 : 0;
+            a.Q_out = a.last_iter ? Q_out_dev : nullptr;
+            a.mu = P->d_mu + (size_t)P->cur * T; a.sd = P->d_sd + (size_t)P->cur * T;
+            a.mu_out = P->d_mu + (size_t)(1 - P->cur) * T; a.sd_out = P->d_sd + (size_t)(1 - P->cur) * T;
+            plan_sample_kernel<PLAN_CEM, false, false><<<(K + 255) / 256, 256, sizeof(float) * 2 * T, h->stream>>>(
+                a, PlanFleetExt(), P->d_P, nullptr);
+            h->launches += 1;
+            int rc = cps_net_plan_cost(h, s_dev, P->d_P, eps_layout, K, T, u_prev, a.J, nullptr, 0);
+            if (rc != CPS_OK) return rc;
+            plan_select_kernel<PLAN_CEM, false, false><<<1, 256, smem, h->stream>>>(a, PlanFleetExt());
+            h->launches += 1;
+            if (a.defer_stats) {
+                cem_update_kernel<<<T, 256, 0, h->stream>>>(a);
+                h->launches += 1;
+            }
+            P->cur = 1 - P->cur;
+        }
+        CUDA_TRY(h, cudaGetLastError());
+        return CPS_OK;
+    }
     // many plans: rollouts + costs without a selecting block (the latency geometry of cps_plan_cost), then the selection by
     // the whole grid (cem_select_kernel, cooperative launch, one block per SM) and the statistics kernel
     const bool multi = K > CPS_CEM_MULTIBLOCK_MIN;
@@ -1225,7 +1363,7 @@ extern "C" int cps_cem_step_host(cps_handle *h, const float *s_host, const float
     if (!h) return CPS_ERR_INVALID;
     if (!s_host || !u_out_host) return fail(h, CPS_ERR_INVALID, "cps_cem_step_host: null pointer");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    return solve_host(h, s_host, u_out_host, true, [&](const float *s_dev, float *u_dev) {
+    return solve_host(h, s_host, u_out_host, h->cfg.integrator != CPS_PREDICTOR_NEURAL, [&](const float *s_dev, float *u_dev) {
         return cps_cem_step(h, s_dev, eps_dev, eps_layout, n_iterations, u_prev, u_dev, nullptr, nullptr);
     });
 }
@@ -1278,6 +1416,41 @@ static plan_fleet_fn pick_plan_fleet(int integ, int cost, int n_sub, bool philox
     return integ == CPS_EULER_V0 ? pick_plan_fleet1<0>(cost, n_sub, philox) : pick_plan_fleet1<1>(cost, n_sub, philox);
 }
 
+// Neural fleets, one iteration of E experiments: plan_sample_kernel over (E, K), net_grad_kernel<.., FLEET> over the E x K
+// plans with the single solve's tile, then (CEM, random action) plan_select_kernel with one block per experiment and, for
+// CEM with deferred statistics, cem_update_fleet_kernel; CEM-GMM's selection and update follow in gmm_update_fleet_kernel.
+// `a` and `fx` are what plan_fleet_kernel / plan_forward_fleet_kernel would take; smem: plan_select_kernel's (CEM).
+typedef void (*plan_select_fn)(const PlanArgs, const PlanFleetExt);
+typedef void (*plan_sample_fn)(const PlanArgs, const PlanFleetExt, float *, CostParams *);
+static int neural_fleet_iteration(cps_handle *h, const PlanArgs &a, const PlanFleetExt &fx, int mode, int E, size_t smem,
+                                  float *P, CostParams *costs, const char *who) {
+    const int K = a.K, T = a.T;
+    const bool philox = a.Q == nullptr;
+    const dim3 grid((unsigned)(K + 255) / 256, (unsigned)E);
+    const size_t ssmem = sizeof(float) * (mode == PLAN_GMM ? 4 * (size_t)T + 1 : mode == PLAN_CEM ? 2 * (size_t)T : 0);
+    plan_sample_fn sf = mode == PLAN_CEM ? (philox ? plan_sample_kernel<PLAN_CEM, true, true> : plan_sample_kernel<PLAN_CEM, true, false>)
+                      : mode == PLAN_GMM ? (philox ? plan_sample_kernel<PLAN_GMM, true, true> : plan_sample_kernel<PLAN_GMM, true, false>)
+                                         : (philox ? plan_sample_kernel<PLAN_Q, true, true> : plan_sample_kernel<PLAN_Q, true, false>);
+    if (ssmem > 48 * 1024) CUDA_TRY(h, cudaFuncSetAttribute((const void *)sf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ssmem));
+    sf<<<grid, 256, ssmem, h->stream>>>(a, fx, P, costs);
+    h->launches += 1;
+    CUDA_TRY(h, cudaGetLastError());
+    int rc = cps_net_grad_fleet(h, E, fx.s, P, costs, a.u_out, a.J, nullptr, who);
+    if (rc != CPS_OK || mode == PLAN_GMM) return rc;
+    plan_select_fn fn = mode == PLAN_CEM ? (philox ? plan_select_kernel<PLAN_CEM, true, true> : plan_select_kernel<PLAN_CEM, true, false>)
+                                         : (philox ? plan_select_kernel<PLAN_Q, true, true> : plan_select_kernel<PLAN_Q, true, false>);
+    if (smem > 48 * 1024) CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    fn<<<dim3(1, (unsigned)E), 256, smem, h->stream>>>(a, fx);
+    h->launches += 1;
+    if (mode == PLAN_CEM && a.defer_stats) {
+        if (philox) cem_update_fleet_kernel<true><<<dim3((unsigned)T, (unsigned)E), 256, 0, h->stream>>>(a, fx);
+        else cem_update_fleet_kernel<false><<<dim3((unsigned)T, (unsigned)E), 256, 0, h->stream>>>(a, fx);
+        h->launches += 1;
+    }
+    CUDA_TRY(h, cudaGetLastError());
+    return CPS_OK;
+}
+
 // Dynamic shared memory of plan_fleet_kernel (cps_cem_step's layout, plus the elites' regenerated draws with Philox); sets
 // a.defer_stats, a.elite_smem and a.rs_off from a.best_k and a.T.
 static size_t cem_fleet_smem(const cps_handle *h, PlanArgs &a, bool philox) {
@@ -1324,6 +1497,7 @@ int cps_cem_fleet_iteration(cps_handle *h, const CemFleetIteration &c) {
     fx.s = c.s; fx.tp = c.tp; fx.te = c.te;
     fx.cost_up = c.cost_up; fx.cost_dn = c.cost_dn;
     fx.seed = c.seed; fx.w1 = c.w1; fx.period = c.period; fx.e_offset = c.e_offset;
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL) return neural_fleet_iteration(h, a, fx, PLAN_CEM, c.E, smem, c.P, c.costs, "cps_cem_fleet_step");
     plan_fleet_fn fn = pick_plan_fleet(h->cfg.integrator, h->cfg.cost_id, h->ode.n, philox);
     if (!fn) return fail(h, CPS_ERR_UNSUPPORTED, "cps_cem_fleet_step: no kernel for this configuration");
     if (smem > 48 * 1024) CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1401,6 +1575,9 @@ int cps_forward_fleet_rollouts(cps_handle *h, const ForwardFleetRollouts &c) {
     fx.cost_up = c.cost_up; fx.cost_dn = c.cost_dn;
     fx.seed = c.seed; fx.w1 = c.w1; fx.period = c.period; fx.e_offset = c.e_offset;
     fx.u01 = c.u01;
+    if (h->cfg.integrator == CPS_PREDICTOR_NEURAL)
+        return neural_fleet_iteration(h, a, fx, c.gmm ? PLAN_GMM : PLAN_Q, c.E, 0, c.P, c.costs,
+                                      c.gmm ? "cps_cem_gmm_fleet_step" : "cps_random_action_fleet_step");
     plan_fleet_fn fn = pick_forward_fleet(h->cfg.integrator, h->cfg.cost_id, c.gmm ? PLAN_GMM : PLAN_Q, h->ode.n, philox);
     if (!fn) return fail(h, CPS_ERR_UNSUPPORTED, "no kernel for this configuration");
     if (smem > 48 * 1024) CUDA_TRY(h, cudaFuncSetAttribute((const void *)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

@@ -397,7 +397,7 @@ static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, cons
         float *Q = F->d_Q[F->cur], *m = F->d_m[F->cur], *v = F->d_v[F->cur];
         const int its = F->solves == 0 ? c.first_iter_count : c.outer_its;
         for (int it = 0; it < its; ++it) {   // grad_step (:166-180)
-            rc = neural ? cps_net_grad_fleet(h, (int)E, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_J, F->d_G)
+            rc = neural ? cps_net_grad_fleet(h, (int)E, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_J, F->d_G, who)
                         : cps_grad_fleet(h, EK, (int)K, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_ck, F->d_jac, F->d_J, F->d_G,
                                          odes);
             if (rc != CPS_OK) return rc;
@@ -410,7 +410,7 @@ static int rpgd_fleet_launch(cps_handle *h, const char *who, int n_periods, cons
                 return rc;
         }
         // get_action (:182-224): the costs of the improved plans
-        rc = neural ? cps_net_grad_fleet(h, (int)E, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_J, nullptr)
+        rc = neural ? cps_net_grad_fleet(h, (int)E, fc.d_s, Q, F->d_costs, fc.d_uprev, F->d_J, nullptr, who)
                     : cps_grad_fleet(h, EK, (int)K, fc.d_s, Q, F->d_costs, fc.d_uprev, nullptr, nullptr, F->d_J, nullptr, odes);
         if (rc != CPS_OK) return rc;
         const int nxt = F->cur ^ 1;

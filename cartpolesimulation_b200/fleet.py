@@ -506,8 +506,12 @@ class CemFleet(_FleetBase):
     sampling from the experiment's own distribution, costs, elites and the mean / stdev update; warmup_iterations on the
     first period after reset() when `warmup`; then the stdev clip, the shift and u = elite_Q[0, 0]), then what Fleet's
     plant does, with no host round trip.  The keywords are optimizer_cem_b200's (same defaults) and Fleet's.  Predictor
-    "ODE" or "ODE_v0" and the four cost plugins; num_rollouts at most 8192.  The neural predictor and the plant-side models
-    (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+    "ODE" or "ODE_v0" and the four cost plugins; num_rollouts at most 8192.  Predictor "neural" takes `network`: the spec
+    dict Engine.net_load takes (neural.load_model(...)[0], neural.build_net_spec, neural.synthetic_net_spec), loaded before
+    the fleet is created; plain GRU / Dense networks, cost quadratic_boundary_grad_minimal or quadratic_boundary_grad.
+    The network lives in the controller only; the plant stays the CartPole ODE.  Every rollout starts from the network's
+    stored hidden state and none is kept per experiment (as RpgdFleet).  The plant-side models (Fleet.set_plant_models)
+    are not implemented and raise NotImplementedError."""
     _abi = "cps_cem_fleet"
 
     def __init__(self, n_experiments: int, num_rollouts: int = 200, mpc_horizon: int = 35, cem_outer_it: int = 3,
@@ -515,11 +519,8 @@ class CemFleet(_FleetBase):
                  warmup: bool = False, warmup_iterations: int = 250, control_limits=(-1.0, 1.0), dt: float = 0.02,
                  substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
                  cost_config: dict | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
-                 experiment_offset: int = 0, dt_simulation: float = 0.002):
-        if integrator == "neural":
-            raise NotImplementedError("CemFleet runs on predictor 'ODE' or 'ODE_v0' (optimizer_cem_b200 has no neural "
-                                      "predictor either)")
-        n_sim = _check_fleet_args("CemFleet", integrator, None, noise, dt, dt_simulation)
+                 experiment_offset: int = 0, dt_simulation: float = 0.002, network: dict | None = None):
+        n_sim = _check_fleet_args("CemFleet", integrator, network, noise, dt, dt_simulation)
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
         self.outer_its = int(cem_outer_it)
         self.first_iter_count = int(warmup_iterations) if warmup else self.outer_its   # as optimizer_cem_b200
@@ -527,6 +528,8 @@ class CemFleet(_FleetBase):
         self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost, device=device)
         self.device = self.engine.device
         self._setup_engine(control_limits, cost_config)
+        if network is not None:
+            self.engine.net_load(network)
         self._create(L.cps_cem_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset, self.outer_its,
                      self.first_iter_count, int(cem_best_k), float(cem_initial_action_stdev), float(cem_stdev_min))
 
@@ -583,24 +586,28 @@ class CemGmmFleet(_FleetBase):
     sampling from the experiment's own two-component mixture, costs, elites, the two clusters around the two cheapest
     elites and their mean / stdev / weight; then u = elite_Q[0, 0] and the shift), then what Fleet's plant does, with no
     host round trip.  The keywords are optimizer_cem_gmm_b200's (same defaults) and Fleet's.  Predictor "ODE" or "ODE_v0"
-    and the four cost plugins; num_rollouts at most 8192, cem_best_k at least 2.  The neural predictor and the plant-side
-    models (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+    and the four cost plugins; num_rollouts at most 8192, cem_best_k at least 2.  Predictor "neural" takes `network`: the spec
+    dict Engine.net_load takes (neural.load_model(...)[0], neural.build_net_spec, neural.synthetic_net_spec), loaded before
+    the fleet is created; plain GRU / Dense networks, cost quadratic_boundary_grad_minimal or quadratic_boundary_grad.
+    The network lives in the controller only; the plant stays the CartPole ODE.  Every rollout starts from the network's
+    stored hidden state and none is kept per experiment (as RpgdFleet).  The plant-side models (Fleet.set_plant_models)
+    are not implemented and raise NotImplementedError."""
     _abi = "cps_cem_gmm_fleet"
 
     def __init__(self, n_experiments: int, num_rollouts: int = 200, mpc_horizon: int = 35, cem_outer_it: int = 3,
                  cem_initial_action_stdev: float = 0.5, cem_stdev_min: float = 0.01, cem_best_k: int = 40,
                  control_limits=(-1.0, 1.0), dt: float = 0.02, substeps: int = 10, integrator: str = "ODE",
                  cost: str = "quadratic_boundary_grad_minimal", cost_config: dict | None = None, device: int | None = None,
-                 noise: str = "philox", seed: int = 0, experiment_offset: int = 0, dt_simulation: float = 0.002):
-        if integrator == "neural":
-            raise NotImplementedError("CemGmmFleet runs on predictor 'ODE' or 'ODE_v0' (optimizer_cem_gmm_b200 has no "
-                                      "neural predictor either)")
-        n_sim = _check_fleet_args("CemGmmFleet", integrator, None, noise, dt, dt_simulation)
+                 noise: str = "philox", seed: int = 0, experiment_offset: int = 0, dt_simulation: float = 0.002,
+                 network: dict | None = None):
+        n_sim = _check_fleet_args("CemGmmFleet", integrator, network, noise, dt, dt_simulation)
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
         self.outer_its = int(cem_outer_it)
         self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost, device=device)
         self.device = self.engine.device
         self._setup_engine(control_limits, cost_config)
+        if network is not None:
+            self.engine.net_load(network)
         self._create(L.cps_cem_gmm_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset, self.outer_its,
                      int(cem_best_k), float(cem_initial_action_stdev), float(cem_stdev_min))
 
@@ -652,22 +659,25 @@ class RandomActionFleet(_FleetBase):
     Every controller period does, for every experiment, what optimizer_random_action_b200.step does (K plans uniform in the
     control limits, their costs from the experiment's state, u_prev and targets, u = the cheapest plan's first input),
     then what Fleet's plant does, with no host round trip.  The keywords are optimizer_random_action_b200's (same
-    defaults) and Fleet's.  Predictor "ODE" or "ODE_v0" and the four cost plugins; num_rollouts at most 8192.  The neural
-    predictor and the plant-side models (Fleet.set_plant_models) are not implemented and raise NotImplementedError."""
+    defaults) and Fleet's.  Predictor "ODE" or "ODE_v0" and the four cost plugins; num_rollouts at most 8192.  Predictor "neural" takes `network`: the spec
+    dict Engine.net_load takes (neural.load_model(...)[0], neural.build_net_spec, neural.synthetic_net_spec), loaded before
+    the fleet is created; plain GRU / Dense networks, cost quadratic_boundary_grad_minimal or quadratic_boundary_grad.
+    The network lives in the controller only; the plant stays the CartPole ODE.  Every rollout starts from the network's
+    stored hidden state and none is kept per experiment (as RpgdFleet).  The plant-side models (Fleet.set_plant_models)
+    are not implemented and raise NotImplementedError."""
     _abi = "cps_random_action_fleet"
 
     def __init__(self, n_experiments: int, num_rollouts: int = 200, mpc_horizon: int = 35, control_limits=(-1.0, 1.0),
                  dt: float = 0.02, substeps: int = 10, integrator: str = "ODE", cost: str = "quadratic_boundary_grad_minimal",
                  cost_config: dict | None = None, device: int | None = None, noise: str = "philox", seed: int = 0,
-                 experiment_offset: int = 0, dt_simulation: float = 0.002):
-        if integrator == "neural":
-            raise NotImplementedError("RandomActionFleet runs on predictor 'ODE' or 'ODE_v0' (optimizer_random_action_b200 "
-                                      "has no neural predictor either)")
-        n_sim = _check_fleet_args("RandomActionFleet", integrator, None, noise, dt, dt_simulation)
+                 experiment_offset: int = 0, dt_simulation: float = 0.002, network: dict | None = None):
+        n_sim = _check_fleet_args("RandomActionFleet", integrator, network, noise, dt, dt_simulation)
         self.E, self.K, self.T = int(n_experiments), int(num_rollouts), int(mpc_horizon)
         self.engine = Engine(self.K, self.T, dt=dt, substeps=substeps, integrator=integrator, cost=cost, device=device)
         self.device = self.engine.device
         self._setup_engine(control_limits, cost_config)
+        if network is not None:
+            self.engine.net_load(network)
         self._create(L.cps_random_action_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset)
 
     def reset(self, states, period: int = 0):

@@ -7,8 +7,15 @@ reads (`u`, `logging_values`, `num_rollouts`, `mpc_horizon`, `optimizer_name`; C
 `predict_and_cost` (predictor.predict_core + cost_function.get_trajectory_cost) and the selection on the sorted costs
 run as one CUDA kernel launch per evaluation (cps_plan_random_action / cps_cem_step); a CEM solve is `cem_outer_it`
 launches with no host round trip in between.  The predictor and cost-function objects handed in are only inspected
-for their configuration, so this package's wrappers and the reference's own work alike.  ODE / ODE_v0 predictors (RPGD
-also the neural predictor); no CPU fallback.
+for their configuration, so this package's wrappers and the reference's own work alike.  Predictors ODE, ODE_v0 and
+neural; no CPU fallback.
+
+Neural predictor (a configured PredictorWrapper whose network the engine takes over): plain GRU / Dense networks, cost
+quadratic_boundary_grad_minimal (the shipped configuration) or quadratic_boundary_grad, at most 8192 rollouts; anything
+else raises NotImplementedError.  predict_and_cost of these optimizers is predict_core + get_trajectory_cost
+(optimizer_random_action_tf.py:42-49, optimizer_cem_tf.py:57-61), so, as for RPGD, every rollout starts from the stored
+hidden state of this optimizer's engine and no step writes it.  The plans are sampled into memory, their costs are those
+of `engine.plan_cost` on them bit for bit, and the selection runs in a separate one-block launch.
 
 Semantics kept from the reference: `self.u` (the `u_prev` of the cost's control-change term) is the last RETURNED
 control, 0.0 initially (Optimizers/__init__.py:35); CEM samples Q = clip(mean + normal * stdev) (:66-68), takes the
@@ -22,14 +29,26 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from .optimizer_mppi_b200 import _template_optimizer
+from .optimizer_mppi_b200 import _extract_predictor, _template_optimizer
+
+
+def _has_network(predictor) -> bool:
+    inner = getattr(predictor, "predictor", predictor)
+    return getattr(inner, "net_spec", None) is not None or hasattr(inner, "net_info")
 
 
 class _forward_optimizer(_template_optimizer):
+    PREDICTORS = ("ODE", "ODE_v0", "neural")
+    NO_NETWORK_REFUSAL = NotImplementedError   # a neural predictor without a network to take over
+
     def configure(self, num_states: int, num_control_inputs: int, default_configure: bool = True, dt: float = None,
                   predictor_specification: str = None, **kwargs):
         if dt is None:
             dt = getattr(self.predictor, "dt", None) or 0.02
+        if (self.NO_NETWORK_REFUSAL and _extract_predictor(self.predictor, predictor_specification)[0] == "neural"
+                and not _has_network(self.predictor)):
+            raise self.NO_NETWORK_REFUSAL(f"{type(self).__name__}: the neural predictor needs a configured PredictorWrapper "
+                                      "whose network the engine can load")
         self._configure(num_states, num_control_inputs, dt, predictor_specification)
         if default_configure:
             self.optimizer_reset()
@@ -235,7 +254,7 @@ class optimizer_rpgd_b200(_forward_optimizer):
     (optimizer_mppi.py:191); every rollout and gradient here starts from the stored hidden state of this optimizer's engine
     and leaves it as it was.  A caller that wants the memory to follow the plant calls `engine.net_update(s, u)` after each step."""
 
-    PREDICTORS = ("ODE", "ODE_v0", "neural")
+    NO_NETWORK_REFUSAL = None   # _extract_net_spec's ValueError
 
     def __init__(self, predictor, cost_function, control_limits, computation_library=None, seed=None,
                  mpc_horizon: int = 35, num_rollouts: int = 16, outer_its: int = 4, sample_stdev: float = 0.5,

@@ -518,8 +518,8 @@ int cps_rpgd_fleet_draws(cps_handle *h, long long period, float *out_dev);
  * them.  Launches per period: n_it x (1, or 2 when best_k x T > 2048: the elite statistics then run as a second kernel
  * with one block per (step, experiment)) + 1 for the plant, whatever E (cps_launch_count).
  * The handle: predictor CPS_EULER_CROMER or CPS_EULER_V0, one of the four cost plugins, K <= 8192 (the single-block
- * selection of cps_cem_step), control limits from cps_set_mppi_params (lo, hi).  The neural predictor, no cost plugin or
- * the legacy cost, CPS_FLAG_SUBSTEP_SINCOS / CPS_FLAG_FAST_DIV, K > 8192 or a horizon whose buffers do not fit shared
+ * selection of cps_cem_step), control limits from cps_set_mppi_params (lo, hi); or CPS_PREDICTOR_NEURAL as under
+ * cps_plan_cost.  No cost plugin or the legacy cost, CPS_FLAG_SUBSTEP_SINCOS / CPS_FLAG_FAST_DIV, K > 8192 or a horizon whose buffers do not fit shared
  * memory: CPS_ERR_UNSUPPORTED.  best_k outside [1, K], a negative stdev, outer_its or first_iter_count < 1, dt not a
  * multiple of dt_simulation: CPS_ERR_INVALID.
  * Non-finite costs (e.g. from a NaN state or target) are not an error: they sort after every number, stay in their
@@ -577,7 +577,7 @@ long long cps_cem_fleet_period(const cps_handle *h);
  * from one 32-bit word; a random-action plan entry is lo + (hi - lo) u with the multiply and the add rounded separately.
  * Launches per period: 2 outer_its + 1 (CEM-GMM), 2 (random action), whatever E (cps_launch_count).
  * The handle: predictor CPS_EULER_CROMER or CPS_EULER_V0, one of the four cost plugins, K <= 8192, control limits from
- * cps_set_mppi_params (lo, hi).  The neural predictor, no cost plugin or the legacy cost, CPS_FLAG_SUBSTEP_SINCOS /
+ * cps_set_mppi_params (lo, hi); or CPS_PREDICTOR_NEURAL as under cps_plan_cost.  No cost plugin or the legacy cost, CPS_FLAG_SUBSTEP_SINCOS /
  * CPS_FLAG_FAST_DIV, K > 8192 or a horizon whose buffers do not fit shared memory: CPS_ERR_UNSUPPORTED.  CEM-GMM best_k
  * outside [2, K], a negative stdev, outer_its < 1, more than 65535 experiments or dt not a multiple of dt_simulation:
  * CPS_ERR_INVALID.  Non-finite costs sort after every number, stay in their experiment and are counted
@@ -647,8 +647,20 @@ long long cps_random_action_fleet_period(const cps_handle *h);
  * handle's stored hidden state (read, never written), with quadratic_boundary_grad_minimal or quadratic_boundary_grad, the
  * forward pass of cps_plan_cost_grad (the same J bit for bit; trajectories those of cps_net_rollout on the FP32 kernel).
  * No network loaded: CPS_ERR_NOT_CONFIGURED; differential networks, other cost plugins, CPS_FLAG_NET_TENSOR_CORES or a
- * network whose shared-memory image exceeds 227 KB: CPS_ERR_UNSUPPORTED.  The fused planners below
- * (cps_plan_random_action*, cps_cem_*, cps_cem_gmm_*) stay ODE-only. */
+ * network whose shared-memory image exceeds 227 KB: CPS_ERR_UNSUPPORTED.
+ *
+ * The planners below (cps_plan_random_action*, cps_cem_*, cps_cem_gmm_*) and their fleets take CPS_PREDICTOR_NEURAL
+ * too, with the network loaded before configure / create.  In the reference their predict_and_cost is predict_core +
+ * get_trajectory_cost (optimizer_random_action_tf.py:42-49, optimizer_cem_tf.py:57-61), so, as RPGD: every rollout starts
+ * from the stored hidden state (cps_net_set_state; zero after loading), no solve writes it, and fleets keep no hidden
+ * state per experiment.  Scope: that of cps_plan_cost on a network (refusals as above, at configure / create and at
+ * every solve) and K <= 8192 (the single-block selection; above: CPS_ERR_UNSUPPORTED).  The plans are sampled into
+ * memory (CEM clip(mean + eps stdev), CEM-GMM as cps_cem_gmm_step, random action the caller's plans or the fleets'
+ * Philox uniforms, from the draws and Philox counters of the ODE path), their costs are those of cps_plan_cost on them bit
+ * for bit, and the selection / update runs as a separate one-block kernel (one block per experiment on a fleet), with
+ * the ODE path's arithmetic and NaN handling.  Launches: random action 2 per solve; CEM 3 per iteration (4 when
+ * best_k x T > 2048); CEM-GMM 3 per iteration, as before.  Fleets per period, whatever E: CEM n_it x (3, or 4) + 1,
+ * CEM-GMM 3 outer_its + 1, random action 4.  The host forms copy the state to the device (one extra copy). */
 int cps_plan_cost(cps_handle *h, const float *s_dev, const float *Q_dev, int q_layout, int K, int T, float u_prev,
                   float *J_out_dev, float *traj_out_dev, int traj_layout);
 /* optimizer_random_action_tf.step (:52-79) for the handle's (K, T): u_out_dev[0] = Q[argmin J, 0], ties to the lowest
