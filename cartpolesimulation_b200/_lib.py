@@ -91,6 +91,13 @@ class cps_random_action_fleet_config(C.Structure):
                 ("experiment_offset", C.c_longlong)]
 
 
+class cps_legacy_fleet_config(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("n_experiments", C.c_int), ("sim_substeps", C.c_int),
+                ("draw_source", C.c_int), ("dt_simulation", C.c_double), ("seed", C.c_ulonglong),
+                ("experiment_offset", C.c_longlong), ("sampling_type", C.c_int), ("update_every", C.c_int),
+                ("stdev", C.c_double), ("p_Q", C.c_double)]
+
+
 # name -> (restype, argtypes); every symbol include/cps.h declares
 _FP = C.POINTER(C.c_float)
 _VP = C.c_void_p
@@ -180,6 +187,15 @@ SYMBOLS = {
     "cps_random_action_fleet_step": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),
     "cps_random_action_fleet_draws": (C.c_int, [_VP, C.c_longlong, _VP]),
     "cps_random_action_fleet_period": (C.c_longlong, [_VP]),
+    "cps_legacy_fleet_create": (C.c_int, [_VP, C.POINTER(cps_legacy_fleet_config)]),
+    "cps_legacy_fleet_set_states": (C.c_int, [_VP, _FP, C.c_longlong]),
+    "cps_legacy_fleet_get_states": (C.c_int, [_VP, _FP, _FP]),
+    "cps_legacy_fleet_get_inputs": (C.c_int, [_VP, _FP, _FP]),
+    "cps_legacy_fleet_step": (C.c_int, [_VP, C.c_int, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "cps_legacy_fleet_draws": (C.c_int, [_VP, C.c_longlong, _VP]),
+    "cps_legacy_fleet_act_draws": (C.c_int, [_VP, C.c_longlong, _VP]),
+    "cps_legacy_fleet_perturbations": (C.c_int, [_VP, C.c_longlong, _VP]),
+    "cps_legacy_fleet_period": (C.c_longlong, [_VP]),
     "cps_plan_cost": (C.c_int, [_VP, _VP, _VP, C.c_int, C.c_int, C.c_int, C.c_float, _VP, _VP, C.c_int]),
     "cps_plan_random_action": (C.c_int, [_VP, _VP, _VP, C.c_int, C.c_float, _VP, _VP, _VP]),
     "cps_plan_random_action_host": (C.c_int, [_VP, _FP, _VP, C.c_int, C.c_float, _FP]),

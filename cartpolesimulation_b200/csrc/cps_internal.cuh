@@ -69,6 +69,7 @@ struct FleetState;  // cps_fleet.cu
 struct RpgdFleetState;  // cps_rpgd_fleet.cu
 struct CemFleetState;   // cps_cem_fleet.cu
 struct ForwardFleetState;   // cps_forward_fleets.cu
+struct LegacyFleetState;    // cps_legacy.cu
 struct PlanState;  // cps_plan.cu
 struct GmmState;    // cps_gmm.cu
 struct GradState;   // cps_grad.cu
@@ -123,6 +124,7 @@ struct cps_handle {
     CemFleetState *cfleet;   // closed-loop experiments under CEM (cps_cem_fleet_create), owned
     ForwardFleetState *gfleet;   // ... under CEM-GMM (cps_cem_gmm_fleet_create), owned
     ForwardFleetState *rafleet;  // ... under random action (cps_random_action_fleet_create), owned
+    LegacyFleetState *lfleet;    // ... under the legacy controller_mppi_cartpole (cps_legacy_fleet_create), owned
 };
 
 extern thread_local std::string g_create_err;
@@ -148,6 +150,8 @@ void cps_rpgd_fleet_free(cps_handle *h);
 void cps_cem_fleet_free(cps_handle *h);
 // cps_forward_fleets.cu
 void cps_forward_fleets_free(cps_handle *h);
+// cps_legacy.cu
+void cps_legacy_fleet_free(cps_handle *h);
 // cps_plan.cu
 void cps_plan_free(cps_handle *h);
 // the refusals every forward-only planner shares: no cost plugin, substep sin/cos or fast division; with the neural

@@ -410,6 +410,7 @@ extern "C" void cps_destroy(cps_handle *h) {
     cps_rpgd_fleet_free(h);
     cps_cem_fleet_free(h);
     cps_forward_fleets_free(h);
+    cps_legacy_fleet_free(h);
     cps_plan_free(h);
     cps_gmm_free(h);
     cps_grad_free(h);

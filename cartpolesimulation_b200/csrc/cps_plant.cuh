@@ -1,7 +1,8 @@
 // cps_plant.cuh -- code shared by the fleets (cps_fleet.cu: MPPI on the ODE or the network, cps_rpgd_fleet.cu: RPGD,
-// cps_cem_fleet.cu: CEM): the plant in the reference's mixed float32 / float64 arithmetic, the record row, the
-// counter-based normal draws and the device-side fold of the controller's model constants, with the host functions that
-// fill their parameter blocks; and FleetCore, the host-side state every fleet carries (cps_fleet.cu defines its functions).
+// cps_cem_fleet.cu: CEM, cps_forward_fleets.cu: CEM-GMM and random action, cps_legacy_fleet.cu: the legacy controller):
+// the plant in the reference's mixed float32 / float64 arithmetic, the record row, the counter-based normal draws and
+// the device-side fold of the controller's model constants, with the host functions that fill their parameter blocks;
+// and FleetCore, the host-side state every fleet carries (cps_fleet.cu defines its functions).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -120,13 +121,17 @@ __device__ __forceinline__ void box_muller(unsigned a, unsigned b, float &n0, fl
 // and, with G4 = ceil(T / 4), second words GMM_DRAWS + 3 G4 it + {0, G4} + group for the two components' normals and
 // GMM_DRAWS + 3 G4 it + 2 G4 + group for the component-picking uniforms (below GMM_DRAWS + 2^28: cps_cem_gmm_fleet_create
 // bounds the iterations); the random-action plans have w0 = plan, w1 = RA_DRAWS + group (uniforms, philox_uniforms; below
-// RA_DRAWS + 2^28 since T is bounded by shared memory); the plant-side draws of cps_fleet.cu have second word 0xFFFFFFFF.
+// RA_DRAWS + 2^28 since T is bounded by shared memory); the legacy controller fleet's rollout draws (cps_legacy_fleet.cu) have
+// w0 = rollout, w1 = LEGACY_DRAWS + group (below LEGACY_DRAWS + 2^26: T is bounded by shared memory) and its actuator
+// uniform w0 = 0, w1 = LEGACY_ACT; the plant-side draws of cps_fleet.cu have second word 0xFFFFFFFF.
 // The second words keep them disjoint.
 #define RPGD_DRAWS_RESAMPLE 0xA0000000u
 #define RPGD_DRAWS_RESET 0xB0000000u
 #define CEM_DRAWS 0xC0000000u
 #define GMM_DRAWS 0xD0000000u
 #define RA_DRAWS 0xE0000000u
+#define LEGACY_DRAWS 0xF0000000u
+#define LEGACY_ACT 0xFFFFFF00u
 __device__ __forceinline__ void philox_normals(unsigned long long seed, unsigned w0, unsigned w1, unsigned period,
                                                unsigned e_global, int n_ind, float *dst, long long stride) {
     const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));

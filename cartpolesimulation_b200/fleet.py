@@ -706,3 +706,114 @@ class RandomActionFleet(_FleetBase):
                                                       _ptr(target_equilibrium), _ptr(plans), _ptr(record), _ptr(J_out),
                                                       _ptr(Q_out)))
         return record
+
+
+class LegacyFleet(_FleetBase):
+    """E closed-loop experiments under the legacy controller_mppi_cartpole (`mppi-cartpole` in
+    Control_Toolkit_ASF/config_controllers.yml:9-30) on one device: one cps_handle with a legacy fleet attached
+    (include/cps.h "Legacy controller fleet").
+
+    Every controller period does, for every experiment, what controller_mppi_cartpole_b200.step does (on solve periods the
+    K x T perturbations of SAMPLING_TYPE, the unclipped rollouts, q() + phi(), the exp-weighted unclipped update and the
+    zero-fill shift; on the others the shift alone; then the actuator noise and the clip), then what Fleet's plant does,
+    with no host round trip.  The keywords are controller_mppi_cartpole_b200's (config: the "mppi-cartpole" block, missing
+    keys take DEFAULT_CONFIG; **kwargs override it) and Fleet's.  The block's `seed` keys the reference's host generator and
+    has no meaning here: it is accepted and ignored, and `seed=` keys the Philox streams.  Predictor "ODE" or "ODE_v0"
+    (optionally "ODE:n").  The legacy cost has no target equilibrium: target_equilibrium is only recorded.  cost_noise
+    != 0, the "neural" predictor and the plant-side models (Fleet.set_plant_models) raise NotImplementedError."""
+    _abi = "cps_legacy_fleet"
+    SAMPLING = {"iid": 0, "random_walk": 1, "uniform": 2, "repeated": 3, "interpolated": 4}
+
+    def __init__(self, n_experiments: int, config: dict | None = None, dt: float = 0.02, intermediate_steps: int = 10,
+                 actuator_noise: float = 0.0, device: int | None = None, noise: str = "philox", seed: int = 0,
+                 experiment_offset: int = 0, dt_simulation: float = 0.002, **kwargs):
+        from .controller_mppi_cartpole_b200 import DEFAULT_CONFIG
+        cfg = dict(DEFAULT_CONFIG)
+        cfg.update(config or {})
+        cfg.update(kwargs)
+        self.config = cfg
+        spec = str(cfg["predictor_specification"]).split(":")
+        if spec[0] not in ("ODE", "ODE_v0"):
+            raise NotImplementedError(f"LegacyFleet: predictor {spec[0]!r} (ODE and ODE_v0 are built)")
+        if float(cfg["cost_noise"]) != 0.0:
+            raise NotImplementedError("LegacyFleet: cost_noise != 0 would need cost weights per experiment")
+        sampling = "iid" if cfg["SAMPLING_TYPE"] is None else cfg["SAMPLING_TYPE"]
+        if sampling not in self.SAMPLING:
+            raise ValueError(f"LegacyFleet: unknown SAMPLING_TYPE {sampling!r} (one of {sorted(self.SAMPLING)})")
+        n_sim = _check_fleet_args("LegacyFleet", spec[0], None, noise, dt, dt_simulation)
+        self.E, self.K, self.T = int(n_experiments), int(cfg["num_rollouts"]), int(cfg["mpc_horizon"])
+        self.sampling_type, self.update_every = sampling, int(cfg["update_every"])
+        self.intermediate_steps = int(spec[1]) if len(spec) > 1 else int(intermediate_steps)
+        self.dt, self.p_Q = float(dt), float(actuator_noise)
+        self.stdev = float(cfg["SQRTRHOINV"] * (1 / np.sqrt(self.dt)))   # float64, as the mirror's SQRTRHODTINV
+        self.n_draws = {"repeated": 1, "interpolated": int(np.ceil(self.T / 10)) + 1}.get(sampling, self.T)
+        self._reset_period = None
+        self.engine = Engine(self.K, self.T, dt=self.dt, substeps=self.intermediate_steps, integrator=spec[0],
+                             cost="legacy_mppi", noise_mode="direct", device=device)
+        self.device = self.engine.device
+        self.engine.set_cost_params([cfg["dd_weight"], cfg["ep_weight"], cfg["ekp_weight"], cfg["ekc_weight"],
+                                     cfg["ccrc_weight"]])
+        self.engine.set_mppi_params(cc_weight=cfg["cc_weight"], R=cfg["R"], LBD=cfg["LBD"], NU=cfg["NU"],
+                                    SQRTRHOINV=cfg["SQRTRHOINV"])
+        self._create(L.cps_legacy_fleet_config, n_sim, noise, dt_simulation, seed, experiment_offset,
+                     self.SAMPLING[sampling], self.update_every, self.stdev, self.p_Q)
+
+    def reset(self, states, period: int = 0):
+        """Every experiment as a freshly configured controller (u = u_prev = 0, iteration counter restarted so that
+        `period` solves), the initial states [E, 6] and the period counter."""
+        s = self._host_states(states)
+        self.engine._chk(self.engine.lib.cps_legacy_fleet_set_states(self.engine._h, s.ctypes.data_as(L._FP), int(period)))
+        self._reset_period = int(period)
+
+    def solves(self, period: int) -> bool:
+        """Whether controller period `period` runs a solve (iteration % update_every == 0)."""
+        if self._reset_period is None:
+            raise RuntimeError("LegacyFleet: reset() first")
+        return (period - self._reset_period) % self.update_every == 0
+
+    def inputs(self):
+        """(u, u_prev), each [E, T]: every experiment's nominal inputs (already shifted) and previous ones.  Synchronises."""
+        u, up = np.zeros((self.E, self.T), np.float32), np.zeros((self.E, self.T), np.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self.engine.lib.cps_legacy_fleet_get_inputs(self.engine._h, u.ctypes.data_as(L._FP),
+                                                                     up.ctypes.data_as(L._FP)))
+        return u, up
+
+    def _draw(self, name: str, period: int, shape) -> torch.Tensor:
+        out = torch.empty(shape, device=self.device, dtype=torch.float32)
+        self.engine.use_current_stream()
+        self.engine._chk(self._fn(name)(self.engine._h, int(period), _ptr(out)))
+        return out
+
+    def draws(self, period: int) -> torch.Tensor:
+        """The raw draws a 'philox' fleet uses in `period`: cuda tensor [E, K, n_draws] (standard normals, or uniforms in
+        [-1, 1) for "uniform"; n_draws = T, 1 for "repeated", ceil(T / 10) + 1 for "interpolated")."""
+        return self._draw("draws", period, (self.E, self.K, self.n_draws))
+
+    def act_draws(self, period: int) -> torch.Tensor:
+        """The actuator-noise uniforms in [-1, 1) of `period`: cuda tensor [E]."""
+        return self._draw("act_draws", period, (self.E,))
+
+    def perturbations(self, period: int) -> torch.Tensor:
+        """The perturbations delta_u a 'philox' fleet's solve of `period` uses: cuda tensor [E, K, T]."""
+        return self._draw("perturbations", period, (self.E, self.K, self.T))
+
+    def run(self, n_periods: int, target_position=None, target_equilibrium=None, draws=None, act_draws=None, record=None,
+            S_out=None):
+        """cps_legacy_fleet_step: n_periods controller periods, no synchronisation.  target_position / target_equilibrium:
+        cuda tensors [n_periods, E] or None; draws [n_periods, E, K, n_draws] and act_draws [n_periods, E] for a
+        'supplied' fleet (draws are read in solve periods only); record [n_periods, E, 16] and S_out [n_periods, E, K]
+        (rollout costs, written in solve periods) or None."""
+        eng = self.engine
+        p0 = self.period
+        reads = any(self.solves(p0 + j) for j in range(n_periods)) if self._reset_period is not None else False
+        if self.noise_source == "philox" and (draws is not None or act_draws is not None):
+            raise ValueError("LegacyFleet: this fleet generates its draws (Philox); pass draws=None, act_draws=None")
+        if self.noise_source == "supplied" and n_periods > 0 and (act_draws is None or (reads and draws is None)):
+            raise ValueError("LegacyFleet: a 'supplied' fleet needs draws (in solve periods) and act_draws")
+        self._check_rows(n_periods, target_position, target_equilibrium, record, S_out,
+                         (draws, "draws", n_periods * self.E * self.K * self.n_draws),
+                         (act_draws, "act_draws", n_periods * self.E))
+        eng._chk(eng.lib.cps_legacy_fleet_step(eng._h, int(n_periods), _ptr(target_position), _ptr(target_equilibrium),
+                                               _ptr(draws), _ptr(act_draws), _ptr(record), _ptr(S_out)))
+        return record

@@ -229,6 +229,76 @@ int cps_legacy_reset(cps_handle *h);
 int cps_legacy_get_inputs(cps_handle *h, float *u_host, float *u_prev_host);
 int cps_legacy_set_inputs(cps_handle *h, const float *u_host, const float *u_prev_host);
 
+/* ---- Legacy controller fleet: E closed-loop experiments under controller_mppi_cartpole ------------------------- */
+/* The data generator with the legacy controller (`mppi-cartpole`, Control_Toolkit_ASF/config_controllers.yml:9-30): per
+ * controller period every experiment does what one controller_mppi_cartpole_b200.step does from its own state, u [T],
+ * u_prev [T] and target position, then the plant advances one period.
+ *   - Solve periods ((period - reset period) % update_every == 0): the K x T perturbations of the configured sampling type
+ *     from the experiment's raw draws, then the iteration of cps_legacy_step (unclipped rollouts, q() + phi(), the
+ *     exp-weighted unclipped update, Q = u[0], u_prev <- u, zero-fill shift).  Other periods: cps_legacy_advance's shift.
+ *   - Actuator noise: Q <- fl32(Q (1 + p_Q v)) in float64 with v uniform in [-1, 1), then Q clipped to [-1, 1] (NaN kept).
+ *   - The plant period with Q held and the record row of cps_fleet_step with Q_calculated = Q_applied = that Q.
+ * Perturbations from the raw draws (stdev = SQRTRHOINV / sqrt(dt), float64; products and sums in float64, rounded to
+ * float32 where the reference assigns into its float32 array): IID T normals z, du_t = fl32(stdev z_t); RANDOM_WALK
+ * T normals, du_0 = fl32(stdev z_0), du_t = fl32(du_{t-1} + stdev z_t); UNIFORM T uniforms v in [-1, 1), du_t = v_t;
+ * REPEATED one normal, du_t = fl32(stdev z); INTERPOLATED ceil(T / 10) + 1 normals, knots fl32(stdev z_j) at t = 0, 10,
+ * 20, ... and the linear formula of cps_legacy_step_host_knots between them.
+ * Draws: supplied (CPS_FLEET_NOISE_SUPPLIED) raw draws [n_periods][E][K][n_draws] (read in solve periods only) and
+ * actuator uniforms [n_periods][E]; or generated from Philox4x32-10 (CPS_FLEET_NOISE_PHILOX, key = seed) in the rollout
+ * threads, counter (rollout k, LEGACY tag + group of four draws, period, experiment_offset + e), and for the actuator
+ * uniform (0, LEGACY actuator tag, period, experiment_offset + e), disjoint from the other fleets' streams.  A Philox
+ * uniform is -1 + 2 ((word >> 8) 2^-24), the multiply and the add rounded separately.
+ * One launch per period, whatever E (cps_launch_count): solve periods grid (blocks of cps_legacy_step for K, E), each
+ * experiment's partials and merge those of cps_legacy_step; other periods one thread per experiment.
+ * The handle: cost CPS_COST_LEGACY_MPPI (any other: CPS_ERR_NOT_CONFIGURED), predictor CPS_EULER_CROMER or CPS_EULER_V0,
+ * weights from cps_set_cost_params / cps_set_mppi_params, folded at each cps_legacy_fleet_step; L / m_pole of the
+ * controller's model are the handle's.  The legacy cost has no target equilibrium: te_dev is only recorded.
+ * n_experiments above 65535, an unknown sampling type, update_every < 1 or dt not a multiple of dt_simulation:
+ * CPS_ERR_INVALID; a horizon whose perturbations do not fit shared memory: CPS_ERR_UNSUPPORTED.  Non-finite costs (e.g.
+ * from a NaN target) stay in their experiment and are counted (cps_nonfinite_costs). */
+enum {
+    CPS_LEGACY_SAMPLING_IID = 0,            /* the reference's default branch */
+    CPS_LEGACY_SAMPLING_RANDOM_WALK = 1,
+    CPS_LEGACY_SAMPLING_UNIFORM = 2,
+    CPS_LEGACY_SAMPLING_REPEATED = 3,
+    CPS_LEGACY_SAMPLING_INTERPOLATED = 4    /* the shipped SAMPLING_TYPE */
+};
+typedef struct cps_legacy_fleet_config {
+    int struct_size;                 /* = sizeof(cps_legacy_fleet_config) */
+    int n_experiments;               /* E on this device, at most 65535 */
+    int sim_substeps;                /* plant ticks per controller period */
+    int draw_source;                 /* CPS_FLEET_NOISE_SUPPLIED | CPS_FLEET_NOISE_PHILOX */
+    double dt_simulation;            /* plant tick, 0.002 s */
+    unsigned long long seed;
+    long long experiment_offset;     /* global index of local experiment 0 (Philox counters) */
+    int sampling_type;               /* CPS_LEGACY_SAMPLING_* */
+    int update_every;                /* solve every update_every-th period after a reset */
+    double stdev;                    /* SQRTRHOINV * (1 / sqrt(dt)) as the mirror computes it */
+    double p_Q;                      /* actuator_noise */
+} cps_legacy_fleet_config;
+int cps_legacy_fleet_create(cps_handle *h, const cps_legacy_fleet_config *cfg);
+/* Every experiment as a freshly configured controller (u = u_prev = 0, the iteration counter restarted so that `period`
+ * solves); states s_host [E][6]; the period counter.  Synchronises. */
+int cps_legacy_fleet_set_states(cps_handle *h, const float *s_host, long long period);
+/* s_host [E][6] and Q_host [E] (each experiment's last control, after the actuator noise); either may be NULL.
+ * Synchronises. */
+int cps_legacy_fleet_get_states(cps_handle *h, float *s_host, float *Q_host);
+/* u_host and u_prev_host [E][T] (u already shifted for the next period); either may be NULL.  Synchronises. */
+int cps_legacy_fleet_get_inputs(cps_handle *h, float *u_host, float *u_prev_host);
+/* n_periods controller periods, stream-ordered, no synchronisation.  tp_dev / te_dev [n_periods][E] or NULL (0 / +1);
+ * draws_dev [n_periods][E][K][n_draws] and act_draws_dev [n_periods][E] as above (NULL on a Philox fleet);
+ * record_dev [n_periods][E][CPS_FLEET_RECORD] and S_out_dev [n_periods][E][K] (rollout costs, written in solve periods)
+ * may be NULL. */
+int cps_legacy_fleet_step(cps_handle *h, int n_periods, const float *tp_dev, const float *te_dev, const float *draws_dev,
+                          const float *act_draws_dev, float *record_dev, float *S_out_dev);
+/* What a Philox fleet draws in controller period `period`: the raw draws out_dev [E][K][n_draws] (n_draws = T, or 1 for
+ * REPEATED, ceil(T / 10) + 1 for INTERPOLATED), the actuator uniforms out_dev [E], and the perturbations out_dev
+ * [E][K][T] made from the raw draws by the rollouts' own transform (Philox fleets only). */
+int cps_legacy_fleet_draws(cps_handle *h, long long period, float *out_dev);
+int cps_legacy_fleet_act_draws(cps_handle *h, long long period, float *out_dev);
+int cps_legacy_fleet_perturbations(cps_handle *h, long long period, float *out_dev);
+long long cps_legacy_fleet_period(const cps_handle *h);
+
 /* ---- open-loop batched rollouts (the predictor interface) ------------------------------------------------ */
 /* predictor.predict_core(s, Q) (SI_Toolkit/src/SI_Toolkit/Predictors/predictor_ODE.py:86-97,
  * predictor_ODE_v0.py:42-74): B rollouts of T control steps x n substeps.  s0_dev: [B][6] if s0_batched else [6]
